@@ -10,8 +10,11 @@ ranks (resident in HBM), then answer the whole query batch (resident in HBM, res
 N > 1 (torchrun): the text is sharded by position range with a halo, every rank searches all queries on
 its shard, presence masks are OR-ed and the per-shard hit lists gathered over NCCL (kmer_index_b200/sharded.py).
 
-`--impl reference` times the reference's own CPU implementation (oracle/_ref, compiled from
-/root/reference; else the oracle port) on a bounded sample of the same workload on the host cores.
+`--impl reference` times the reference's own CPU implementation (oracle/_ref, compiled from the reference's source
+where oracle/Makefile's REF points; else the oracle port) on a bounded sample of the same workload on the host cores.
+
+`--dump-outputs DIR` (one GPU) writes what the last timed step's search returned for a fixed, seeded sample of the
+queries to DIR/*.npy, so that two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -64,7 +67,15 @@ def parse_args():
                          "answers 1/N of the batch locally; 'peer' = only the directory is replicated, the position parts stay "
                          "where they were sorted and are read over NVLink (CUDA IPC mappings); 'position-range' = text shards with halo, every GPU searches the "
                          "whole batch, hit lists merged on rank 0")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's search result for a fixed sample of the queries to "
+                         "DIR/{query_ids,offsets,positions,status}.npy, 64 MB at most")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.gpus != 1 or args.impl != "ours"):
+        ap.error("--dump-outputs writes the search result of one GPU: it needs --gpus 1 and --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -206,6 +217,46 @@ class ClockSampler:
 
 
 # ------------------------------------------------------------------------------------------------------------
+# --dump-outputs
+# ------------------------------------------------------------------------------------------------------------
+DUMP_QUERIES, DUMP_SEED = 1 << 20, 20251
+DUMP_BYTES = 64 << 20
+
+
+def dump_result(out_dir, res, Q: int, dev, count_only: bool):
+    """Write a DeviceResult of Q queries as DIR/<name>.npy, DUMP_BYTES at most:
+        query_ids  float64 [S]      the sampled queries, ascending: all of them up to DUMP_QUERIES, else a sample
+                                    drawn with DUMP_SEED, so it depends on Q alone
+        offsets    float64 [S + 1]  CSR offsets of the sampled queries' hit lists in `positions`
+        positions  float64 [P]      their positions (empty without hits; not written for a count-only search)
+        status     float32 [S]      their status codes
+    The hit lists are exact in float64 (positions < 2^32). Should the sampled hit lists not fit, the sample is cut to
+    its longest prefix that does."""
+    import torch
+    S = min(Q, DUMP_QUERIES)
+    ids = np.arange(Q) if S == Q else np.sort(np.random.default_rng(DUMP_SEED).choice(Q, S, replace=False))
+    d_ids = torch.from_numpy(ids).to(dev)
+    off = torch.as_tensor(res.offsets(), device=dev)
+    counts = off[d_ids + 1] - off[d_ids]
+    if not count_only:
+        room = (DUMP_BYTES - 4096 - S * (8 + 8 + 4)) // 8    # 4 KiB for the last offset and the .npy headers
+        S = int(torch.searchsorted(torch.cumsum(counts, 0), room, right=True).item())
+        d_ids, counts = d_ids[:S], counts[:S]
+    s_off = torch.zeros(S + 1, dtype=torch.int64, device=dev)
+    torch.cumsum(counts, 0, out=s_off[1:])
+    out = {"query_ids": d_ids.double(), "offsets": s_off.double(),
+           "status": torch.as_tensor(res.status(), device=dev)[d_ids].float()}
+    if not count_only:
+        total = int(s_off[-1].item())
+        src = torch.repeat_interleave(off[d_ids] - s_off[:-1], counts) + torch.arange(total, device=dev)
+        pos = torch.as_tensor(res.positions(), device=dev)[src] if total else torch.empty(0, dtype=torch.int32, device=dev)
+        out["positions"] = (pos.to(torch.int64) & 0xFFFFFFFF).double()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
+# ------------------------------------------------------------------------------------------------------------
 # ours
 # ------------------------------------------------------------------------------------------------------------
 def run_ours(args, wl):
@@ -306,20 +357,30 @@ def run_ours(args, wl):
             return sharded.search_device(ix, q.data_ptr(), q_off.data_ptr(), Ql, m_hi, 1, dev, count_only=count_only)
         return sharded.search_device(ix, q.data_ptr(), q_off.data_ptr(), Q, m_hi, world, dev, count_only=count_only)
 
-    def device_step(profile):
-        """build + search with inputs resident in HBM; returns (build_ms, gather_ms, search_ms, hits, stats)."""
+    def device_step(profile, keep=False):
+        """build + search with inputs resident in HBM; returns (build_ms, gather_ms, search_ms, hits, stats, kept).
+        keep (--dump-outputs, one GPU): the search call sharded.search_device makes, but the index and the result stay
+        open and come back as kept = (index, result); otherwise kept is None. That step's search_ms then leaves out the
+        result's free, which sharded.search_device enqueues before e[3]: four stream-ordered cudaFreeAsync calls."""
         e = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
         e[0].record(stream)
         ix = make_index(profile, text_ptr=text.data_ptr())
         e[1].record(stream)
         finish_build(ix)   # NCCL: part of the build
         e[2].record(stream)
-        hits = search_resident(ix, args.count_only)
+        if keep:
+            res = (ix.count_batch_device if args.count_only else ix.search_batch_device)(q.data_ptr(), q_off.data_ptr(), Q, m_hi)
+            hits = res.n_positions
+        else:
+            hits = search_resident(ix, args.count_only)
         e[3].record(stream)
         torch.cuda.synchronize()
         stats = ix.stats() if profile else None
+        times = e[0].elapsed_time(e[2]), e[1].elapsed_time(e[2]), e[2].elapsed_time(e[3])
+        if keep:
+            return (*times, hits, stats, (ix, res))
         ix.close()
-        return e[0].elapsed_time(e[2]), e[1].elapsed_time(e[2]), e[2].elapsed_time(e[3]), hits, stats
+        return (*times, hits, stats, None)
 
     # ---- warm-up, then exactly K timed steps between barriers
     sampler = ClockSampler(local_rank) if rank == 0 else None   # started early: nvidia-smi needs ~1 s to come up
@@ -328,8 +389,8 @@ def run_ours(args, wl):
     barrier()
     b_ms, g_ms, s_ms, stats_acc, hits = [], [], [], {}, 0
     t_region = time.perf_counter()
-    for _ in range(args.steps):
-        tb, tg, ts, hits, st = device_step(True)
+    for i in range(args.steps):
+        tb, tg, ts, hits, st, kept = device_step(True, keep=bool(args.dump_outputs) and i == args.steps - 1)
         b_ms.append(tb)
         g_ms.append(tg)
         s_ms.append(ts)
@@ -340,6 +401,11 @@ def run_ours(args, wl):
     barrier()
     t_region = time.perf_counter() - t_region
     clocks = sampler.stop() if sampler else None
+    if kept:
+        ix, res = kept
+        dump_result(args.dump_outputs, res, Q, dev, args.count_only)
+        res.free()
+        ix.close()
     # where the cross-GPU part of the last timed build went (rank 0's stream)
     assemble_ms = {}
     for (_, a), (label, b) in zip(assemble_marks, assemble_marks[1:]):

@@ -33,6 +33,26 @@ def have_reference() -> bool:
     return os.path.exists(REF_SO)
 
 
+def hit_digests(offsets, positions) -> np.ndarray:
+    """One 64-bit digest per query of its CSR hit list (positions and their order): what the stored reference answers
+    of tests/golden/live/ keep instead of the lists, which would not fit there."""
+    offsets = np.asarray(offsets, dtype=np.uint64)
+    counts = np.diff(offsets).astype(np.int64)
+    out = np.zeros(counts.size, dtype=np.uint64)
+    if positions.size == 0:
+        return out
+    rank = np.arange(positions.size, dtype=np.uint64) - np.repeat(offsets[:-1], counts)
+    with np.errstate(over="ignore"):
+        w = (np.asarray(positions, dtype=np.uint64) + np.uint64(1)) * np.uint64(0x9E3779B97F4A7C15) + \
+            (rank + np.uint64(1)) * np.uint64(0xC2B2AE3D27D4EB4F)
+        w ^= w >> np.uint64(29)
+        w *= np.uint64(0xBF58476D1CE4E5B9)
+        w ^= w >> np.uint64(32)
+        nz = counts > 0
+        out[nz] = np.add.reduceat(w, offsets[:-1][nz].astype(np.int64))
+    return out
+
+
 def _ptr(a: np.ndarray, t):
     return a.ctypes.data_as(t)
 
@@ -210,14 +230,14 @@ class Oracle(_Base):
 
 
 class Reference(_Base):
-    """The reference itself (kmer::kmer_index from /root/reference), compiled into oracle/_ref/."""
+    """The reference itself (kmer::kmer_index of Clemapfel/kmer_index), compiled into oracle/_ref/."""
     _prefix = "kref"
 
     @classmethod
     def lib(cls):
         if cls._lib is None:
             if not os.path.exists(REF_SO):
-                raise FileNotFoundError(f"{REF_SO} not built (needs /root/reference; run make -C oracle)")
+                raise FileNotFoundError(f"{REF_SO} not built (make -C oracle REF=<kmer_index checkout>)")
             L = C.CDLL(REF_SO)
             L.kref_supported.restype = C.c_int
             L.kref_supported.argtypes = [C.c_uint32, _u32p, C.c_uint32]

@@ -1,8 +1,11 @@
 // Exercises include/kmer_index.hpp the way a user of the reference would (test_main.cpp:21-69 protocol):
 // build single and multi indices with make_kmer_index, search(), compare to_vector() with a plain scan.
 // Exit code 0 = all good. Needs a GPU at run time; compile-only is part of the CPU test suite.
+// argv[1]: directory for the save / load round trip (default: the system's temporary directory).
 #include <cstdio>
 #include <cstdlib>
+#include <filesystem>
+#include <string>
 #include <vector>
 
 #include <kmer_index.hpp>
@@ -44,7 +47,7 @@ static std::vector<uint32_t> scan(std::vector<alphabet_t> const& text, std::vect
         }                                                                    \
     } while (0)
 
-int main()
+int main(int argc, char** argv)
 {
     static_assert(kmer::detail::fast_pow(4, 12) == 16777216);
     static_assert(kmer::detail::fast_pow(2, 63) == 0 && kmer::detail::fast_pow(1, 200) == 1);
@@ -163,7 +166,8 @@ int main()
     }
     // save / load round trip
     {
-        const char* path = "/tmp/kmer_index_hpp_test.kmerb200";
+        const std::string path =
+            ((argc > 1 ? std::filesystem::path(argv[1]) : std::filesystem::temp_directory_path()) / "kmer_index_hpp_test.kmerb200").string();
         multi.save(path);
         auto loaded = kmer::kmer_index<alphabet_t, uint32_t, 10, 11, 12>::load(path);
         std::vector<alphabet_t> q(text.begin() + 4242, text.begin() + 4242 + 17);
@@ -171,7 +175,7 @@ int main()
         bool threw = false;
         try { (void)kmer::kmer_index<alphabet_t, uint32_t, 10>::load(path); } catch (std::invalid_argument const&) { threw = true; }
         REQUIRE(threw);
-        std::remove(path);
+        std::remove(path.c_str());
     }
     std::printf("kmer_index.hpp: all checks passed\n");
     return 0;

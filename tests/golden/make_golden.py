@@ -1,8 +1,8 @@
 """Generate tests/golden/*.npz from the COMPILED REFERENCE (oracle/_ref/libkmer_ref.so).
 
-Run in the build container only (needs /root/reference to have built oracle/_ref):
+Needs a checkout of the reference (Clemapfel/kmer_index) to build oracle/_ref first:
 
-    python tests/golden/make_golden.py
+    make -C oracle REF=/path/to/kmer_index && python tests/golden/make_golden.py
 
 Each fixture stores the inputs explicitly (text ranks, query ranks + offsets) next to the
 reference's outputs (per-query sorted positions in CSR form + status), so the fixtures do not
@@ -18,8 +18,10 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+import test_oracle_golden as live  # noqa: E402
 from kmer_index_b200 import synth  # noqa: E402
-from oracle.bindings import Oracle, Reference  # noqa: E402
+from oracle.bindings import Oracle, Reference, hit_digests  # noqa: E402
 
 OUT = os.path.dirname(os.path.abspath(__file__))
 
@@ -43,7 +45,26 @@ def case(name, text, sigma, ks, q, off):
           f"other={(r_status > 1).sum()} ub={ub.sum()}")
 
 
+def live_case(name, sigma, ks, batches):
+    """live/<name>.npz: the reference's answers to the batches of tests/test_oracle_golden.py's live tests, per query the
+    hit count, the status, the digest of the hit list (hit_digests: the lists themselves would not fit) and the UB flag."""
+    arrays = {}
+    for j, (text, q, off) in enumerate(batches):
+        r_off, r_pos, r_status = Reference(text, sigma, ks).search(q, off)
+        ora = Oracle(text, sigma, ks)
+        ora.search(q, off)
+        arrays.update({f"counts{j}": np.diff(r_off).astype(np.uint32), f"digests{j}": hit_digests(r_off, r_pos),
+                       f"status{j}": r_status, f"ub{j}": ora.last_ub.astype(np.uint8)})
+    os.makedirs(live.LIVE_DIR, exist_ok=True)
+    np.savez_compressed(os.path.join(live.LIVE_DIR, name + ".npz"), **arrays)
+    print(f"live/{name}: {len(batches)} batch(es)")
+
+
 def main():
+    for sigma, ks, mmax in live.LIVE_CASES:
+        live_case(live.live_name("live", sigma, ks), sigma, ks, [live.live_batch(sigma, ks, mmax)])
+    for sigma, ks in live.REFERENCE_SHAPES:
+        live_case(live.live_name("sweep", sigma, ks), sigma, ks, [b[1:] for b in live.sweep_batches(sigma, ks)])
     low = synth.low_entropy_text(7)
     for ks, mmax, Q in [([3], 20, 600), ([5], 32, 800), ([6], 40, 800), ([14], 45, 800), ([16], 70, 800),
                         ([12], 100, 800), ([5, 7, 9, 11, 13], 60, 1200), ([9, 10], 60, 800),

@@ -39,6 +39,6 @@ def test_header_runs(tmp_path):
     exe = _compile(tmp_path)
     import torch
     env = dict(os.environ, KMER_B200_TEST_DEVICES=str(min(torch.cuda.device_count(), 4)))
-    out = subprocess.run([exe], capture_output=True, text=True, timeout=300, env=env)
+    out = subprocess.run([exe, str(tmp_path)], capture_output=True, text=True, timeout=300, env=env)
     assert out.returncode == 0, out.stderr + out.stdout
     assert "all checks passed" in out.stdout

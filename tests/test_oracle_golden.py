@@ -1,9 +1,54 @@
 """CPU: pin the C restatement (oracle/kmer_oracle.c) against the fixtures generated from the compiled
 reference (tests/golden/make_golden.py) and, when oracle/_ref is present, against the reference live."""
+import os
+
 import numpy as np
 import pytest
 
-from conftest import assert_results_equal, golden_cases, load_golden
+from conftest import GOLDEN_DIR, ROOT, assert_results_equal, golden_cases, load_golden
+
+# the reference's answers to the batches of the two live tests below, stored by make_golden.py
+LIVE_DIR = os.path.join(GOLDEN_DIR, "live")
+
+
+def live_name(test, sigma, ks):
+    return f"{test}_s{sigma}_k" + "_".join(map(str, ks))
+
+
+def reference_answers(oracle_mod, name, sigma, ks, batches):
+    """The reference's answer to every (text, q, off) of `batches` as (offsets, positions, status, digests, ub): live
+    when oracle/_ref is built (ub None), else from LIVE_DIR/<name>.npz, which holds per query the hit count, the status,
+    the digest of the hit list (oracle.bindings.hit_digests; positions None) and the oracle's UB flag; else a skip."""
+    if oracle_mod.have_reference():
+        out = []
+        for text, q, off in batches:
+            with oracle_mod.Reference(text, sigma, ks) as r:
+                o, p, s = r.search(q, off)
+            out.append((o, p, s, oracle_mod.hit_digests(o, p), None))
+        return out
+    path = os.path.join(LIVE_DIR, name + ".npz")
+    if not os.path.exists(path):
+        pytest.skip(f"neither oracle/_ref nor {os.path.relpath(path, ROOT)} (tests/golden/make_golden.py stores it)")
+    g = np.load(path)
+    out = []
+    for j in range(len(batches)):
+        o = np.zeros(g[f"counts{j}"].size + 1, dtype=np.uint64)
+        np.cumsum(g[f"counts{j}"], out=o[1:])
+        out.append((o, None, g[f"status{j}"], g[f"digests{j}"], g[f"ub{j}"].astype(bool)))
+    return out
+
+
+def compare_with_reference(oracle_mod, got, ub, want, label):
+    """Exact on the queries the oracle does not flag UB; returns per query whether the two answers are the same."""
+    w_off, w_pos, w_st, w_dig, w_ub = want
+    if w_ub is not None:
+        assert np.array_equal(ub, w_ub), f"{label}: UB flags differ from the stored ones"
+    if w_pos is not None:
+        assert_results_equal(got, (w_off, w_pos, w_st), skip=ub, label=label)
+    same = (np.diff(got[0]) == np.diff(w_off)) & (got[2] == w_st) & (oracle_mod.hit_digests(got[0], got[1]) == w_dig)
+    bad = np.nonzero(~same & ~ub)[0]
+    assert bad.size == 0, f"{label}: queries {bad[:8].tolist()} differ from the reference"
+    return same
 
 
 @pytest.mark.parametrize("name", golden_cases())
@@ -52,18 +97,23 @@ def test_truth_scan_small(oracle_mod):
     assert o.tolist() == [0, 3, 5, 5] and p.tolist() == [0, 2, 6, 0, 2]
 
 
-@pytest.mark.parametrize("sigma,ks,mmax", [(4, [6], 40), (4, [5, 7, 9, 11, 13], 60), (15, [5, 6, 7], 12),
-                                            (27, [3], 9), (5, [4], 14)])
-def test_oracle_matches_live_reference(oracle_mod, sigma, ks, mmax):
-    if not oracle_mod.have_reference():
-        pytest.skip("oracle/_ref not built on this box (needs /root/reference)")
+LIVE_CASES = [(4, [6], 40), (4, [5, 7, 9, 11, 13], 60), (15, [5, 6, 7], 12), (27, [3], 9), (5, [4], 14)]
+
+
+def live_batch(sigma, ks, mmax):
     from kmer_index_b200 import synth
     text = synth.low_entropy_text(11, sigma=sigma)
     q, off = synth.stress_queries(text, 1500, 1, mmax, sigma, 4242 + ks[0], low_sigma=2)
-    with oracle_mod.Oracle(text, sigma, ks) as o, oracle_mod.Reference(text, sigma, ks) as r:
+    return text, q, off
+
+
+@pytest.mark.parametrize("sigma,ks,mmax", LIVE_CASES)
+def test_oracle_matches_live_reference(oracle_mod, sigma, ks, mmax):
+    text, q, off = live_batch(sigma, ks, mmax)
+    want, = reference_answers(oracle_mod, live_name("live", sigma, ks), sigma, ks, [(text, q, off)])
+    with oracle_mod.Oracle(text, sigma, ks) as o:
         got = o.search(q, off)
-        want = r.search(q, off)
-        assert_results_equal(got, want, skip=o.last_ub, label=f"sigma={sigma} ks={ks}")
+        compare_with_reference(oracle_mod, got, np.asarray(o.last_ub).astype(bool), want, f"sigma={sigma} ks={ks}")
 
 
 @pytest.mark.parametrize("name", golden_cases())
@@ -115,6 +165,13 @@ def _sweep_texts(sigma, seed):
     yield f"period {p} with 20 point changes", t
 
 
+def sweep_batches(sigma, ks):
+    from kmer_index_b200 import synth
+    for kind, text in _sweep_texts(sigma, 100 + ks[0]):
+        q, off = synth.stress_queries(text, 300, 1, min(6 * max(ks) + 7, 130), sigma, 7000 + ks[0], low_sigma=2)
+        yield kind, text, q, off
+
+
 @pytest.mark.parametrize("sigma,ks", REFERENCE_SHAPES)
 def test_oracle_matches_live_reference_sweep(oracle_mod, sigma, ks):
     """Every shape the compiled reference was instantiated for (oracle/ref_driver.cpp), four kinds of text (long buckets,
@@ -122,18 +179,14 @@ def test_oracle_matches_live_reference_sweep(oracle_mod, sigma, ks):
     which the reference dereferences an end iterator (kmer_index.hpp:317, :546; the oracle flags them) are skipped in the
     exact comparison -- there the reference's answer depends on stale heap bytes -- but must still agree with the
     oracle's defined value almost always."""
-    if not oracle_mod.have_reference():
-        pytest.skip("oracle/_ref not built on this box (needs /root/reference)")
-    from kmer_index_b200 import synth
+    batches = list(sweep_batches(sigma, ks))
+    wants = reference_answers(oracle_mod, live_name("sweep", sigma, ks), sigma, ks, [b[1:] for b in batches])
     flagged = agree = 0
-    for kind, text in _sweep_texts(sigma, 100 + ks[0]):
-        q, off = synth.stress_queries(text, 300, 1, min(6 * max(ks) + 7, 130), sigma, 7000 + ks[0], low_sigma=2)
-        with oracle_mod.Oracle(text, sigma, ks) as o, oracle_mod.Reference(text, sigma, ks) as r:
-            got, want = o.search(q, off), r.search(q, off)
+    for (kind, text, q, off), want in zip(batches, wants):
+        with oracle_mod.Oracle(text, sigma, ks) as o:
+            got = o.search(q, off)
             ub = np.asarray(o.last_ub).astype(bool)
-            assert_results_equal(got, want, skip=o.last_ub, label=f"sigma={sigma} ks={ks} {kind}")
-            for i in np.nonzero(ub)[0]:
-                flagged += 1
-                agree += bool(got[2][i] == want[2][i] and np.array_equal(got[1][int(got[0][i]):int(got[0][i + 1])],
-                                                                         want[1][int(want[0][i]):int(want[0][i + 1])]))
+        same = compare_with_reference(oracle_mod, got, ub, want, f"sigma={sigma} ks={ks} {kind}")
+        flagged += int(ub.sum())
+        agree += int(same[ub].sum())
     assert agree >= 0.95 * flagged, (agree, flagged)
