@@ -184,6 +184,30 @@ int kmer_b200_search_batch_device(kmer_b200_index *index, const uint8_t *d_q_ran
 int kmer_b200_count_batch_device(kmer_b200_index *index, const uint8_t *d_q_ranks, const uint64_t *d_q_offsets,
                                  uint64_t n_queries, uint64_t max_query_len, uint32_t mode, kmer_b200_result **out);
 
+/* ---- approximate search (no reference analogue): for each query q of length m, every position p, ascending, with
+   p + m <= n and at most max_mismatches substituted symbols between T[p, p+m) and q (Hamming distance; no insertions or
+   deletions, no window past the end of the text). max_mismatches <= 8, else KMER_B200_ERR_INVALID_ARGUMENT. The search
+   seeds from max_mismatches + 1 disjoint exact pieces of the query through the index and verifies every candidate
+   window on the packed text (DESIGN.md section 5, "Approximate search"). Per-query status: KMER_B200_QUERY_UNDEFINED for
+   an empty query, else OK; a query of m <= max_mismatches symbols matches every window. max_mismatches = 0 gives the
+   result of KMER_B200_MODE_CORRECT search. Not available (KMER_B200_ERR_UNSUPPORTED) on a multi-device handle, a
+   position-range shard, a shared-positions index or a key-range part that has not been adopted. Query length is
+   bounded by the shared-memory staging as for exact search. Same host buffers and result layout as
+   kmer_b200_search_batch; the whole batch is staged on the device in one copy. */
+int kmer_b200_search_approx_batch(kmer_b200_index *index, const uint8_t *q_ranks, const uint64_t *q_offsets,
+                                  uint64_t n_queries, uint32_t max_mismatches, kmer_b200_result **out);
+
+/* Same with queries resident in device memory and the result left in device memory (max_query_len >= the longest
+   query in the batch). */
+int kmer_b200_search_approx_batch_device(kmer_b200_index *index, const uint8_t *d_q_ranks, const uint64_t *d_q_offsets,
+                                         uint64_t n_queries, uint64_t max_query_len, uint32_t max_mismatches,
+                                         kmer_b200_result **out);
+
+/* Count-only variant of the device approximate search (offsets and status; no position list is materialised). */
+int kmer_b200_count_approx_batch_device(kmer_b200_index *index, const uint8_t *d_q_ranks, const uint64_t *d_q_offsets,
+                                        uint64_t n_queries, uint64_t max_query_len, uint32_t max_mismatches,
+                                        kmer_b200_result **out);
+
 uint64_t kmer_b200_result_n_queries(const kmer_b200_result *r);
 uint64_t kmer_b200_result_n_positions(const kmer_b200_result *r);
 int kmer_b200_result_on_device(const kmer_b200_result *r);

@@ -444,6 +444,46 @@ namespace kmer
             return kmer_batch_result<position_t>(r);
         }
 
+        // Approximate search (no reference analogue; kmer_b200_search_approx_batch): per query, every position whose window
+        // differs from the query in at most max_mismatches (<= 8) symbols, ascending. Substitutions only; max_mismatches = 0
+        // is exact search in CORRECT mode. The batch is gathered into one rank buffer (a copy of the bytes when the queries
+        // hold their ranks in place) and staged on the device in one copy.
+        template<std::ranges::range queries_t>
+        kmer_batch_result<position_t> search_approx_batch(queries_t const& queries, std::uint32_t max_mismatches) const
+        {
+            using query_t = std::remove_cvref_t<std::ranges::range_reference_t<queries_t const>>;
+            std::vector<std::uint8_t> ranks;
+            std::vector<std::uint64_t> offsets{0};
+            for (auto const& q : queries)
+            {
+                if constexpr (detail::ranks_in_place<query_t>)
+                {
+                    auto const* p = reinterpret_cast<std::uint8_t const*>(std::ranges::data(q));
+                    ranks.insert(ranks.end(), p, p + std::ranges::size(q));
+                }
+                else
+                {
+                    for (auto const& c : q)
+                        ranks.push_back(static_cast<std::uint8_t>(c.to_rank()));
+                }
+                offsets.push_back(ranks.size());
+            }
+            kmer_b200_result* r = nullptr;
+            detail::check(kmer_b200_search_approx_batch(_handle, ranks.data(), offsets.data(), offsets.size() - 1, max_mismatches, &r));
+            return kmer_batch_result<position_t>(r);
+        }
+
+        // one query: its positions within max_mismatches substitutions, ascending; throws for an empty query
+        std::vector<position_t> search_approx(std::vector<alphabet_t> const& query, std::uint32_t max_mismatches) const
+        {
+            std::array<std::vector<alphabet_t> const*, 1> one{&query};
+            auto deref = one | std::views::transform([](auto const* p) -> std::vector<alphabet_t> const& { return *p; });
+            auto batch = search_approx_batch(deref, max_mismatches);
+            if (batch.status[0] != KMER_B200_QUERY_OK)
+                throw std::invalid_argument("approximate search of an empty query is undefined");
+            return std::vector<position_t>(batch.positions.begin(), batch.positions.end());
+        }
+
         // kmer_index_element::search_k (kmer_index.hpp:182-190): the bucket of the k symbols starting at `it`, for one
         // of the index's ks; empty when the k-mer does not occur (the reference returns a null pointer)
         template<std::size_t k, typename iterator_t>

@@ -366,6 +366,32 @@ class KmerIndex:
         L.kmer_b200_result_free(r)
         return BatchResult(offsets, positions, status)
 
+    def search_approx(self, q_ranks, q_offsets, max_mismatches: int, copy: bool = True) -> BatchResult:
+        """Approximate search of a host batch (kmer_b200_search_approx_batch): per query, every position p, ascending,
+        where the text window T[p, p+m) differs from the query in at most max_mismatches (<= 8) symbols. Substitutions
+        only; max_mismatches=0 is exact search in MODE_CORRECT. copy=False: views of the library's pinned buffers (valid
+        until BatchResult.free())."""
+        q = np.ascontiguousarray(np.asarray(q_ranks, dtype=np.uint8))
+        off = np.ascontiguousarray(np.asarray(q_offsets, dtype=np.uint64))
+        r = C.c_void_p()
+        _capi.check(self._L.kmer_b200_search_approx_batch(self._h, q.ctypes.data, off.ctypes.data, off.size - 1,
+                                                          int(max_mismatches), C.byref(r)))
+        return self._host_result(r, off.size - 1, copy)
+
+    def _host_result(self, r, Q: int, copy: bool) -> BatchResult:
+        L = self._L
+        total = L.kmer_b200_result_n_positions(r)
+        offsets = np.ctypeslib.as_array(C.cast(L.kmer_b200_result_offsets(r), _capi.u64p), shape=(Q + 1,))
+        status = (np.ctypeslib.as_array(C.cast(L.kmer_b200_result_status(r), _capi.u8p), shape=(Q,))
+                  if Q else np.zeros(0, dtype=np.uint8))
+        positions = (np.ctypeslib.as_array(C.cast(L.kmer_b200_result_positions(r), _capi.u32p), shape=(total,))
+                     if total else np.zeros(0, dtype=np.uint32))
+        if not copy:
+            return BatchResult(offsets, positions, status, _owner=(L, r))
+        out = BatchResult(offsets.copy(), positions.copy(), status.copy())
+        L.kmer_b200_result_free(r)
+        return out
+
     def search(self, query, mode: int = MODE_DEFAULT) -> np.ndarray:
         """kmer_index::search(query).to_vector() for one query; raises ValueError where the reference throws
         std::invalid_argument (kmer_index.hpp:121,508). A batch of one: correct but latency-bound."""
@@ -390,6 +416,14 @@ class KmerIndex:
 
     def count_batch_device(self, q_ptr: int, off_ptr: int, Q: int, max_len: int, mode: int = MODE_DEFAULT):
         return self._device_call(self._L.kmer_b200_count_batch_device, q_ptr, off_ptr, Q, max_len, mode)
+
+    def search_approx_batch_device(self, q_ptr: int, off_ptr: int, Q: int, max_len: int, max_mismatches: int):
+        """Approximate search (see search_approx) of a device-resident batch; the result stays on the device."""
+        return self._device_call(self._L.kmer_b200_search_approx_batch_device, q_ptr, off_ptr, Q, max_len, max_mismatches)
+
+    def count_approx_batch_device(self, q_ptr: int, off_ptr: int, Q: int, max_len: int, max_mismatches: int):
+        """Count-only approximate search of a device-resident batch: offsets and status, no positions."""
+        return self._device_call(self._L.kmer_b200_count_approx_batch_device, q_ptr, off_ptr, Q, max_len, max_mismatches)
 
     def presence_batch_device(self, q_ptr: int, off_ptr: int, Q: int, max_len: int, present_ptr: int,
                               mode: int = MODE_DEFAULT, fmt: int = 0) -> None:

@@ -88,6 +88,12 @@ SYMBOLS = {
                                                 C.c_uint32, C.POINTER(C.c_void_p)]),
     "kmer_b200_count_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64,
                                                C.c_uint32, C.POINTER(C.c_void_p)]),
+    "kmer_b200_search_approx_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32,
+                                                C.POINTER(C.c_void_p)]),
+    "kmer_b200_search_approx_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64,
+                                                       C.c_uint32, C.POINTER(C.c_void_p)]),
+    "kmer_b200_count_approx_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64,
+                                                      C.c_uint32, C.POINTER(C.c_void_p)]),
     "kmer_b200_result_n_queries": (C.c_uint64, [C.c_void_p]),
     "kmer_b200_result_n_positions": (C.c_uint64, [C.c_void_p]),
     "kmer_b200_result_on_device": (C.c_int, [C.c_void_p]),

@@ -1326,8 +1326,10 @@ struct PackedQueries {
 
 int search_begin(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len,
                  uint32_t mode, const void *d_present_global, uint32_t present_format, uint32_t *d_present4,
-                 PendingSearch *p, const PackedQueries *packed = nullptr) {
+                 PendingSearch *p, const PackedQueries *packed = nullptr, int32_t max_mismatches = -1) {
     using namespace kb;
+    const bool approx = max_mismatches >= 0;  // approximate search: the semantics of CORRECT mode, any query length
+    if (approx) mode = KMER_B200_MODE_CORRECT;
     if (mode == UINT32_MAX) mode = ix->cfg.mode;
     if (mode > KMER_B200_MODE_CORRECT) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "unknown mode");
     // query ids travel as 32-bit values (heavy list, hit list, block indices of the launch)
@@ -1393,7 +1395,9 @@ int search_begin(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off,
         for (int r = 0; r <= kb::kMaxPosParts; ++r) a.parts0.first[r] = E0.part_first[r];
         for (int r = 0; r < kb::kMaxPosParts; ++r) a.parts0.ptr[r] = E0.pos_part[r];
     }
-    a.lean_ok = a.single_k && ix->sigma == 4 && ix->elems[0].dev.shift == 0 && ix->elems[0].key_bytes == 4 && !d_present4 &&
+    a.approx = approx ? 1 : 0;
+    a.max_mismatches = approx ? (uint32_t)max_mismatches : 0;
+    a.lean_ok = !approx && a.single_k && ix->sigma == 4 && ix->elems[0].dev.shift == 0 && ix->elems[0].key_bytes == 4 && !d_present4 &&
                 !d_present_global && ix->cfg.profile < 2 && !std::getenv("KMER_B200_NO_LEAN");
     a.error_flag = p->d_flags;  // per search: a second search on the handle cannot clobber a pending one's flags
     a.gather_count = ix->cfg.profile >= 2 ? ix->d_gathers : nullptr;  // profile = 2: also count gathered sectors
@@ -1401,8 +1405,11 @@ int search_begin(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off,
 
     cudaMemsetAsync(p->d_flags, 0, 4 * sizeof(uint32_t), st);
     ix->prof.begin(K_SEARCH_COUNT, 0);
-    launch_search(a, d_present4 ? (a.gather_count ? kPassCountDeferredAccount : kPassCountDeferred)
-                                : (a.gather_count ? kPassCountAccount : kPassCount), st);
+    if (approx)
+        launch_search_approx(a, a.gather_count ? kPassCountAccount : kPassCount, st);
+    else
+        launch_search(a, d_present4 ? (a.gather_count ? kPassCountDeferredAccount : kPassCountDeferred)
+                                    : (a.gather_count ? kPassCountAccount : kPassCount), st);
     ix->prof.end();
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return bail(fail(KMER_B200_ERR_CUDA, std::string("search (count pass): ") + cudaGetErrorString(e)));
@@ -1482,10 +1489,14 @@ int search_finish(PendingSearch *p, const uint32_t *d_present4_global, SearchFla
         if (dev_alloc(ix, &res->positions, total, false)) return bail(KMER_B200_ERR_OUT_OF_MEMORY);
         a.positions = res->positions;
         ix->prof.begin(K_SEARCH_WRITE, 0);
-        launch_search(a, kPassWrite, st);
+        if (a.approx)
+            launch_search_approx(a, kPassWrite, st);
+        else
+            launch_search(a, kPassWrite, st);
         ix->prof.end();
-        // results written in slab order: sub-k lengths without an auxiliary element, anything seeded from a view
-        if (flags[1] != 0 && (aux_missing != 0 || a.views)) {
+        // results written in slab order: sub-k lengths without an auxiliary element, anything seeded from a view, approximate
+        // hits of several seeds or of a slab
+        if (flags[1] != 0 && (aux_missing != 0 || a.views || a.approx)) {
             uint32_t *d_tmp = nullptr;
             if (dev_alloc(ix, &d_tmp, total, false)) return bail(KMER_B200_ERR_OUT_OF_MEMORY);
             const uint32_t key_bits = bit_length(ix->cfg.shard_begin + ix->n);
@@ -1512,9 +1523,9 @@ int search_finish(PendingSearch *p, const uint32_t *d_present4_global, SearchFla
 // queries already on the device; result stays on the device
 int search_device_impl(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len,
                        uint32_t mode, const void *d_present_global, uint32_t present_format, SearchFlavor flavor,
-                       kmer_b200_result **out, const PackedQueries *packed = nullptr) {
+                       kmer_b200_result **out, const PackedQueries *packed = nullptr, int32_t max_mismatches = -1) {
     PendingSearch p;
-    KB_TRY(search_begin(ix, d_q, d_off, Q, max_len, mode, d_present_global, present_format, nullptr, &p, packed));
+    KB_TRY(search_begin(ix, d_q, d_off, Q, max_len, mode, d_present_global, present_format, nullptr, &p, packed, max_mismatches));
     return search_finish(&p, nullptr, flavor, out);
 }
 
@@ -1542,6 +1553,21 @@ __global__ void max_len_kernel(const uint64_t *__restrict__ off, uint64_t Q, uns
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(0xFFFFFFFFu, m, o));
     if ((threadIdx.x & 31) == 0 && m) atomicMax(out, m);
+}
+
+// Approximate search needs the whole text and every position of every element on this device: refused (with the reason)
+// for the handles where one of them lives elsewhere.
+int approx_check(const kmer_b200_index *ix, uint32_t max_mismatches) {
+    if (max_mismatches > kb::kMaxMismatches) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "approximate search: max_mismatches above 8");
+    if (!ix->replicas.empty()) return fail(KMER_B200_ERR_UNSUPPORTED, "approximate search is not available on a multi-device handle");
+    if (ix->sharded || !ix->reaches_end || ix->cfg.halo != 0)
+        return fail(KMER_B200_ERR_UNSUPPORTED, "approximate search is not available on a position-range shard");
+    if (ix->cfg.reserved & KMER_B200_FLAG_SHARED_POSITIONS)
+        return fail(KMER_B200_ERR_UNSUPPORTED, "approximate search is not available on a shared-positions index");
+    for (size_t e = 0; e < ix->ks.size(); ++e)
+        if (ix->elems[e].dev.key_lo != 0 || ix->elems[e].dev.key_hi != UINT64_MAX)
+            return fail(KMER_B200_ERR_UNSUPPORTED, "approximate search needs the whole key space: adopt the assembled element first");
+    return KMER_B200_OK;
 }
 
 }  // namespace
@@ -1778,6 +1804,28 @@ int kmer_b200_count_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const 
     DeviceGuard guard(ix->device);
     std::lock_guard<std::mutex> lock(ix->mu);
     return search_device_impl(ix, d_q, d_off, Q, max_len, mode, nullptr, 0, kFlavorCountOnly, out);
+}
+
+int kmer_b200_search_approx_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
+                                         uint64_t max_len, uint32_t max_mismatches, kmer_b200_result **out) {
+    if (!ix || !out || !d_off) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    *out = nullptr;
+    KB_TRY(approx_check(ix, max_mismatches));
+    DeviceGuard guard(ix->device);
+    std::lock_guard<std::mutex> lock(ix->mu);
+    return search_device_impl(ix, d_q, d_off, Q, max_len, KMER_B200_MODE_CORRECT, nullptr, 0, kFlavorFull, out, nullptr,
+                              (int32_t)max_mismatches);
+}
+
+int kmer_b200_count_approx_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
+                                        uint64_t max_len, uint32_t max_mismatches, kmer_b200_result **out) {
+    if (!ix || !out || !d_off) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    *out = nullptr;
+    KB_TRY(approx_check(ix, max_mismatches));
+    DeviceGuard guard(ix->device);
+    std::lock_guard<std::mutex> lock(ix->mu);
+    return search_device_impl(ix, d_q, d_off, Q, max_len, KMER_B200_MODE_CORRECT, nullptr, 0, kFlavorCountOnly, out, nullptr,
+                              (int32_t)max_mismatches);
 }
 
 int kmer_b200_search_batch_device_global(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
@@ -2574,6 +2622,87 @@ static int search_batch_host_stream(kmer_b200_index *ix, const uint8_t *q_ranks,
     return code;
 }
 
+// One copy each way: the batch is staged on the device whole, searched, and the result copied back into pinned host buffers.
+// Small exact batches, and every approximate batch (max_mismatches >= 0), take this path. The caller holds the
+// handle's lock and device.
+static int search_batch_host_single_copy(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q,
+                                         uint32_t mode, const uint8_t *lut256, int32_t max_mismatches, kmer_b200_result **out) {
+    cudaStream_t st = ix->stream;
+    const uint64_t n_sym = q_offsets[Q] - q_offsets[0];
+    uint8_t *d_q = nullptr;
+    uint64_t *d_off = nullptr;
+    unsigned long long *d_max = nullptr;
+    struct Staging {  // the device copies of the batch are released on every exit path
+        kmer_b200_index *ix;
+        uint8_t *&q;
+        uint64_t *&off;
+        unsigned long long *&mx;
+        ~Staging() {
+            dev_free(ix, q);
+            dev_free(ix, off);
+            dev_free(ix, mx);
+        }
+    } staging{ix, d_q, d_off, d_max};
+    KB_TRY(dev_alloc(ix, &d_q, n_sym, false));
+    KB_TRY(dev_alloc(ix, &d_off, Q + 1, false));
+    KB_TRY(dev_alloc(ix, &d_max, 1, false));
+    // offsets are rebased on the device side by passing q_ranks - q_offsets[0]
+    KB_CUDA(cudaMemcpyAsync(d_off, q_offsets, (Q + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+    if (n_sym) KB_CUDA(cudaMemcpyAsync(d_q, q_ranks + q_offsets[0], n_sym, cudaMemcpyHostToDevice, st));
+    if (lut256) KB_TRY(translate_on_device(ix, d_q, n_sym, lut256));
+    KB_CUDA(cudaMemsetAsync(d_max, 0, sizeof(unsigned long long), st));
+    if (Q) max_len_kernel<<<(unsigned)std::min<uint64_t>((Q + 255) / 256, (uint64_t)kb::device_sm_count() * 8), 256, 0, st>>>(d_off, Q, d_max);
+    KB_CUDA(cudaMemcpyAsync(&ix->h_pinned[2], d_max, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    KB_CUDA(cudaStreamSynchronize(st));
+    const uint64_t max_len = ix->h_pinned[2];
+    kmer_b200_result *dres = nullptr;
+    int s = search_device_impl(ix, d_q - q_offsets[0], d_off, Q, max_len, mode, nullptr, 0, kFlavorFull, &dres, nullptr,
+                               max_mismatches);
+    if (s != 0) return s;
+    // device result -> pinned host buffers
+    kmer_b200_result *res = new (std::nothrow) kmer_b200_result();
+    if (!res) {
+        kmer_b200_result_free(dres);
+        return fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation failed");
+    }
+    res->index = ix;
+    res->on_device = false;
+    res->n_queries = Q;
+    res->n_positions = dres->n_positions;
+    res->offsets = (uint64_t *)pinned_get((Q + 1) * sizeof(uint64_t), &res->cap_offsets);
+    res->status = (uint8_t *)pinned_get(Q, &res->cap_status);
+    // pinning tens of gigabytes is slow and can starve the host: beyond 8 GiB the positions go to pageable memory
+    const size_t pos_bytes = res->n_positions * sizeof(uint32_t);
+    if (pos_bytes > (8ull << 30)) {
+        res->positions = (uint32_t *)std::malloc(pos_bytes);
+        res->positions_pageable = true;
+        res->cap_positions = pos_bytes;
+    } else {
+        res->positions = (uint32_t *)pinned_get(pos_bytes, &res->cap_positions);
+    }
+    if (!res->offsets || !res->status || !res->positions) {
+        kmer_b200_result_free(dres);
+        kmer_b200_result_free(res);
+        return fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed");
+    }
+    cudaMemcpyAsync(res->offsets, dres->offsets, (Q + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+    if (Q) cudaMemcpyAsync(res->status, dres->status, Q, cudaMemcpyDeviceToHost, st);
+    if (res->n_positions)
+        cudaMemcpyAsync(res->positions, dres->positions, res->n_positions * sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
+    cudaError_t e = cudaStreamSynchronize(st);
+    kmer_b200_result_free(dres);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        kmer_b200_result_free(res);
+        return fail(KMER_B200_ERR_CUDA, std::string("search (D2H): ") + cudaGetErrorString(e));
+    }
+    ix->last_h2d = n_sym + (Q + 1) * sizeof(uint64_t);
+    ix->last_d2h = (Q + 1) * sizeof(uint64_t) + Q + res->n_positions * sizeof(uint32_t);
+    ix->last_host_path = 0, ix->last_raw_pct = 100, ix->last_pack_gbs = 0;
+    *out = res;
+    return KMER_B200_OK;
+}
+
 static int search_batch_host(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q,
                              uint32_t mode, const uint8_t *lut256, kmer_b200_result **out) {
     if (!ix || !out || !q_offsets) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
@@ -2581,7 +2710,6 @@ static int search_batch_host(kmer_b200_index *ix, const uint8_t *q_ranks, const 
     if (!ix->replicas.empty()) return search_batch_multi(ix, q_ranks, q_offsets, Q, mode, lut256, out);
     DeviceGuard guard(ix->device);
     std::lock_guard<std::mutex> lock(ix->mu);
-    cudaStream_t st = ix->stream;
     const uint64_t n_sym = q_offsets[Q] - q_offsets[0];
     if (n_sym && !q_ranks) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "q_ranks is null");
     // batches whose transfer dominates (>= 256 MiB over PCIe) are pipelined in chunks
@@ -2654,82 +2782,23 @@ static int search_batch_host(kmer_b200_index *ix, const uint8_t *q_ranks, const 
         ix->last_host_path = 1, ix->last_raw_pct = 100, ix->last_pack_gbs = 0;
         return search_batch_host_pipelined(ix, q_ranks, q_offsets, Q, mode, out);
     }
-    uint8_t *d_q = nullptr;
-    uint64_t *d_off = nullptr;
-    unsigned long long *d_max = nullptr;
-    struct Staging {  // the device copies of the batch are released on every exit path
-        kmer_b200_index *ix;
-        uint8_t *&q;
-        uint64_t *&off;
-        unsigned long long *&mx;
-        ~Staging() {
-            dev_free(ix, q);
-            dev_free(ix, off);
-            dev_free(ix, mx);
-        }
-    } staging{ix, d_q, d_off, d_max};
-    KB_TRY(dev_alloc(ix, &d_q, n_sym, false));
-    KB_TRY(dev_alloc(ix, &d_off, Q + 1, false));
-    KB_TRY(dev_alloc(ix, &d_max, 1, false));
-    // offsets are rebased on the device side by passing q_ranks - q_offsets[0]
-    KB_CUDA(cudaMemcpyAsync(d_off, q_offsets, (Q + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    if (n_sym) KB_CUDA(cudaMemcpyAsync(d_q, q_ranks + q_offsets[0], n_sym, cudaMemcpyHostToDevice, st));
-    if (lut256) KB_TRY(translate_on_device(ix, d_q, n_sym, lut256));
-    KB_CUDA(cudaMemsetAsync(d_max, 0, sizeof(unsigned long long), st));
-    if (Q) max_len_kernel<<<(unsigned)std::min<uint64_t>((Q + 255) / 256, (uint64_t)kb::device_sm_count() * 8), 256, 0, st>>>(d_off, Q, d_max);
-    KB_CUDA(cudaMemcpyAsync(&ix->h_pinned[2], d_max, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    KB_CUDA(cudaStreamSynchronize(st));
-    const uint64_t max_len = ix->h_pinned[2];
-    kmer_b200_result *dres = nullptr;
-    int s = search_device_impl(ix, d_q - q_offsets[0], d_off, Q, max_len, mode, nullptr, 0, kFlavorFull, &dres);
-    if (s != 0) return s;
-    // device result -> pinned host buffers
-    kmer_b200_result *res = new (std::nothrow) kmer_b200_result();
-    if (!res) {
-        kmer_b200_result_free(dres);
-        return fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation failed");
-    }
-    res->index = ix;
-    res->on_device = false;
-    res->n_queries = Q;
-    res->n_positions = dres->n_positions;
-    res->offsets = (uint64_t *)pinned_get((Q + 1) * sizeof(uint64_t), &res->cap_offsets);
-    res->status = (uint8_t *)pinned_get(Q, &res->cap_status);
-    // pinning tens of gigabytes is slow and can starve the host: beyond 8 GiB the positions go to pageable memory
-    const size_t pos_bytes = res->n_positions * sizeof(uint32_t);
-    if (pos_bytes > (8ull << 30)) {
-        res->positions = (uint32_t *)std::malloc(pos_bytes);
-        res->positions_pageable = true;
-        res->cap_positions = pos_bytes;
-    } else {
-        res->positions = (uint32_t *)pinned_get(pos_bytes, &res->cap_positions);
-    }
-    if (!res->offsets || !res->status || !res->positions) {
-        kmer_b200_result_free(dres);
-        kmer_b200_result_free(res);
-        return fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed");
-    }
-    cudaMemcpyAsync(res->offsets, dres->offsets, (Q + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
-    if (Q) cudaMemcpyAsync(res->status, dres->status, Q, cudaMemcpyDeviceToHost, st);
-    if (res->n_positions)
-        cudaMemcpyAsync(res->positions, dres->positions, res->n_positions * sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
-    cudaError_t e = cudaStreamSynchronize(st);
-    kmer_b200_result_free(dres);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        kmer_b200_result_free(res);
-        return fail(KMER_B200_ERR_CUDA, std::string("search (D2H): ") + cudaGetErrorString(e));
-    }
-    ix->last_h2d = n_sym + (Q + 1) * sizeof(uint64_t);
-    ix->last_d2h = (Q + 1) * sizeof(uint64_t) + Q + res->n_positions * sizeof(uint32_t);
-    ix->last_host_path = 0, ix->last_raw_pct = 100, ix->last_pack_gbs = 0;
-    *out = res;
-    return KMER_B200_OK;
+    return search_batch_host_single_copy(ix, q_ranks, q_offsets, Q, mode, lut256, -1, out);
 }
 
 int kmer_b200_search_batch(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q,
                            uint32_t mode, kmer_b200_result **out) {
     return search_batch_host(ix, q_ranks, q_offsets, Q, mode, nullptr, out);
+}
+
+int kmer_b200_search_approx_batch(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q,
+                                  uint32_t max_mismatches, kmer_b200_result **out) {
+    if (!ix || !out || !q_offsets) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    *out = nullptr;
+    KB_TRY(approx_check(ix, max_mismatches));
+    if (q_offsets[Q] != q_offsets[0] && !q_ranks) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "q_ranks is null");
+    DeviceGuard guard(ix->device);
+    std::lock_guard<std::mutex> lock(ix->mu);
+    return search_batch_host_single_copy(ix, q_ranks, q_offsets, Q, KMER_B200_MODE_CORRECT, nullptr, (int32_t)max_mismatches, out);
 }
 
 int kmer_b200_search_batch_ptrs(kmer_b200_index *ix, const uint8_t *const *q_ptrs, const uint64_t *q_lens, uint64_t Q,

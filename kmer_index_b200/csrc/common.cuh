@@ -60,6 +60,48 @@ __device__ __forceinline__ uint64_t text_window64(const uint64_t *words, uint64_
     return sh ? ((hi << sh) | (lo >> (64 - sh))) : hi;
 }
 
+// T[tpos, tpos+len) == q[qpos, qpos+len), false if the text span leaves the text (qw: the packed query)
+__device__ __forceinline__ bool match_span(const PackedText &T, const uint64_t *qw, uint64_t tpos, uint32_t qpos,
+                                           uint32_t len) {
+    if (tpos + len > T.n) return false;
+    const uint32_t spw = 64 / T.bits;
+    while (len) {
+        const uint32_t c = len < spw ? len : spw;
+        const uint64_t a = text_window64(T.words, tpos, T.bits);
+        const uint64_t b = window64(qw, (uint64_t)qpos, T.bits);
+        if ((a ^ b) >> (64 - c * T.bits)) return false;
+        tpos += c;
+        qpos += c;
+        len -= c;
+    }
+    return true;
+}
+
+// Hamming distance of T[tpos, tpos+len) and q[qpos, qpos+len) (the caller keeps the span inside the text), counted one
+// 64-bit window at a time: XOR the windows, OR-fold every b-bit field onto its lowest bit, keep those bits, popcount.
+// Returns early with a count above `limit` as soon as the count exceeds it.
+__device__ __forceinline__ uint32_t mismatches_span(const PackedText &T, const uint64_t *qw, uint64_t tpos, uint32_t qpos,
+                                                    uint32_t len, uint32_t limit) {
+    const uint32_t spw = 64 / T.bits;
+    const uint64_t low = T.bits == 2 ? 0x5555555555555555ull : (T.bits == 4 ? 0x1111111111111111ull : 0x0101010101010101ull);
+    uint32_t d = 0;
+    while (len) {
+        const uint32_t c = len < spw ? len : spw;
+        uint64_t x = text_window64(T.words, tpos, T.bits) ^ window64(qw, (uint64_t)qpos, T.bits);
+        x |= x >> 1;
+        if (T.bits >= 4) x |= x >> 2;
+        if (T.bits == 8) x |= x >> 4;
+        x &= low;
+        if (c < spw) x &= ~0ull << (64 - c * T.bits);  // the fields of the c symbols at the top
+        d += (uint32_t)__popcll(x);
+        if (d > limit) return d;
+        tpos += c;
+        qpos += c;
+        len -= c;
+    }
+    return d;
+}
+
 // The k-mer hash of the k symbols at the top of window `w` (kmer_index.hpp:56-73).
 // sigma == 4: the 2k-bit field itself. Otherwise Horner over the k symbols (k * bits <= 64).
 __device__ __forceinline__ uint64_t key_from_window(uint64_t w, uint32_t k, uint32_t bits, uint32_t sigma) {

@@ -97,9 +97,18 @@ struct SearchArgs {
     unsigned long long *gather_count;  // device or null: accumulates the 32-byte sectors the batch must gather
     uint32_t *error_flag;            // device u32[4]: [0] bit 0 = query rank >= sigma; [1] = #segments to sort;
                                      // [2..3] = u64 mask of sub-k query lengths that found no auxiliary element
+    uint32_t approx;                 // 1: approximate search (search_approx.cu): every window within max_mismatches substitutions
+    uint32_t max_mismatches;         // e <= kMaxMismatches
 };
 
+// a query with more candidates than this is handed from its group of lanes to the warp-per-query launch
+constexpr uint32_t kHeavyCandidates = 2048;
+
 void launch_search(const SearchArgs &args, SearchPass pass, cudaStream_t stream);
+// approximate search (search_approx.cu): passes kPassCount, kPassCountAccount and kPassWrite of an unsharded index whose
+// elements hold their positions (whole or in peer parts); queries as 1-byte ranks (q_packed unused)
+constexpr uint32_t kMaxMismatches = 8;
+void launch_search_approx(const SearchArgs &args, SearchPass pass, cudaStream_t stream);
 uint32_t search_q_words(uint32_t group, uint32_t bits, uint64_t max_len);
 // deferred count pass epilogue: zero the counts / set THROW according to the combined presence flags
 void launch_finalize_deferred(uint64_t *d_counts, uint8_t *d_status, const uint8_t *d_defer, const uint32_t *d_present4_global,

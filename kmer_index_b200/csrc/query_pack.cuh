@@ -112,4 +112,53 @@ __device__ __forceinline__ bool pack_query_lane(const uint8_t *__restrict__ q_ra
     return (inval & 0x8080808080808080ull) != 0;
 }
 
+// One group of G lanes (lane gl of the group, warp mask gmask) packs the m ranks at q_ranks[off0..] into qw[] (b bits per
+// symbol, MSB-first, + two zero words) and sets bit 0 of *error_flag when a rank is >= sigma. q_total = symbols in
+// q_ranks (bounds the 16-byte reads). A chunk is 8 symbols (one 8-byte load); `lpw` chunks make one 64-bit word. Each
+// lane takes `cpl` consecutive chunks per round so that a round always covers whole words; lanes sharing a word combine
+// their parts with xor-shuffles. The group is converged on return.
+template <int G>
+__device__ __forceinline__ void pack_query_group(const uint8_t *q_ranks, uint64_t off0, uint32_t m, uint64_t q_total,
+                                                 const PackedText &T, uint32_t gl, uint32_t gmask, uint32_t *error_flag,
+                                                 uint64_t *qw) {
+    const uint8_t *qr = q_ranks + off0;
+    const uint32_t lpw = 8 / T.bits;                          // chunks per word: 4, 2, 1
+    const uint32_t cpl = lpw > (uint32_t)G ? lpw / G : 1;     // chunks per lane and round
+    const uint32_t share = lpw / cpl;                         // lanes sharing one word
+    const uint32_t wpr = (uint32_t)G * cpl / lpw;             // words per round
+    const uint64_t guard = (0x80u - (T.sigma > 128 ? 128u : T.sigma)) * 0x0101010101010101ull;
+    bool bad = false;
+    uint32_t round = 0;
+    if (G == 1) {
+        if (T.bits == 2) bad = pack_query_lane<2>(q_ranks, off0, m, q_total, T.sigma, qw);
+        else if (T.bits == 4) bad = pack_query_lane<4>(q_ranks, off0, m, q_total, T.sigma, qw);
+        else bad = pack_query_lane<8>(q_ranks, off0, m, q_total, T.sigma, qw);
+    } else
+    for (uint32_t base = 0; base < m; base += 8 * G * cpl, ++round) {
+        uint64_t w = 0;
+        for (uint32_t c = 0; c < cpl; ++c) {
+            const uint32_t chunk = gl * cpl + c;              // chunk index inside the round
+            const uint32_t s0 = base + 8 * chunk;
+            uint64_t v = 0;
+            if (s0 < m) {
+                v = load8(qr + s0, m - s0, off0 + s0 + 16 <= q_total);
+                if (T.sigma <= 128) {
+                    bad |= (((v + guard) | v) & 0x8080808080808080ull) != 0;
+                } else {
+                    for (uint32_t j = 0; j < 8; ++j) bad |= ((v >> (8 * j)) & 0xFF) >= T.sigma;
+                }
+            }
+            w |= pack8(v, T.bits) << (64 - 8 * T.bits * ((chunk % lpw) + 1));
+        }
+        for (uint32_t o = 1; o < share; o <<= 1) w |= __shfl_xor_sync(gmask, w, o, G);
+        if (gl % share == 0) qw[round * wpr + gl / share] = w;
+    }
+    if (G > 1 && gl == 0) {
+        qw[round * wpr] = 0;
+        qw[round * wpr + 1] = 0;
+    }
+    if ((G == 1 ? bad : __any_sync(gmask, bad)) && gl == 0) atomicOr(error_flag, 1u);
+    if (G > 1) __syncwarp(gmask);
+}
+
 }  // namespace kb

@@ -1,0 +1,266 @@
+// Approximate batched search (sm_100a): for a query q of length m and a budget e <= kMaxMismatches, every window start p
+// with p + m <= n and Hamming(T[p, p+m), q) <= e, ascending. Substitutions only.
+//
+// Pigeonhole seeds: L = floor(m / (e+1)); seed j is the query segment [jL, (j+1)L), j = 0..e. A window within e
+// substitutions matches at least one of these e+1 disjoint segments exactly. Seed j is looked up as
+//   * the k-mer at query offset jL of the element with the largest k <= L (an auxiliary k' = L element included): its
+//     bucket lists every x with T[x, x+k) == q[jL, jL+k), or, when every k is larger than L,
+//   * the whole segment through the prefix slab of the element with the smallest k > L (the buckets of all k-mers that
+//     start with it, bounded by lower_bound_key as the sub-k plan of search_kernels.cu does) plus the k - L starts at the
+//     end of the text where no k-mer starts, compared directly.
+// Candidate x of seed j gives p = x - jL. Seed i lists p exactly when T[p+iL, ...) equals its seed, so p is dropped when
+// an earlier seed i < j matches there: every window is verified once, by its first error-free seed, and no sort or
+// dedup pass is needed. Survivors are verified with mismatches_span on the packed text (early exit above e).
+// One group of G lanes per query, as the general search kernel; two passes (count -> scan -> write); candidate lists
+// longer than kHeavyCandidates go to a warp-per-query launch. Hits of several seeds, or of a slab, are not ascending:
+// such a query is flagged for launch_segment_sort.
+#include <algorithm>
+
+#include "launch.h"
+#include "query_pack.cuh"
+
+namespace kb {
+
+constexpr int kApproxThreads = 256;
+
+// PASS: kPassCount, kPassCountAccount (count + gathered sectors) or kPassWrite. HEAVY: the warp-per-query launch over
+// the heavy list.
+template <int PASS_, int G, bool HEAVY>
+__device__ __forceinline__ void approx_query(const SearchArgs &a, const uint64_t q, uint64_t *smem_q) {
+    constexpr bool kAccount = PASS_ == kPassCountAccount;
+    constexpr int PASS = kAccount ? (int)kPassCount : PASS_;
+    const int lane = threadIdx.x & 31;
+    const int gl = threadIdx.x & (G - 1);
+    const int group = threadIdx.x / G;
+    const uint32_t gshift = (uint32_t)(lane - gl);
+    const uint32_t gfull = G == 32 ? 0xFFFFFFFFu : ((1u << G) - 1);
+    const uint32_t gmask = gfull << gshift;
+    const uint32_t lt_mask = (1u << gl) - 1;
+#define GBALLOT(pred) (G == 1 ? ((pred) ? 1u : 0u) : ((__ballot_sync(gmask, (pred)) >> gshift) & gfull))
+#define GSHFL(v, src) (G == 1 ? (v) : __shfl_sync(gmask, (v), (src), G))
+// the count pass enlists a query with a long candidate list for the warp launch (marked in unsorted[q] bit 1); the
+// write pass follows that mark. Both passes see the same lookups, hence the same decision.
+#define HAND_OFF_IF_HEAVY(len)                                                                          \
+    if (PASS == kPassCount && !HEAVY && G < 32 && a.heavy != nullptr && (len) > (uint64_t)kHeavyCandidates) { \
+        if (gl == 0) {                                                                                  \
+            a.heavy[1 + atomicAdd(a.heavy, 1u)] = (uint32_t)q;                                          \
+            a.counts[q] = 0;                                                                            \
+            a.status[q] = KMER_B200_QUERY_OK;                                                           \
+            a.unsorted[q] = 2;                                                                          \
+        }                                                                                               \
+        return;                                                                                         \
+    }
+
+    uint64_t out_base = 0;
+    if (PASS == kPassWrite) {
+        out_base = a.counts[q];
+        if (a.counts[q + 1] == out_base) return;
+        if (!HEAVY && G < 32 && (a.unsorted[q] & 2)) return;
+    }
+    const DeviceIndex &ix = *a.index;
+    const PackedText T = ix.text;
+    const uint64_t off0 = a.q_offsets[q];
+    const uint64_t m64 = a.q_offsets[q + 1] - off0;
+    const uint32_t e = a.max_mismatches;
+    uint32_t status = KMER_B200_QUERY_OK;
+    if (m64 == 0) status = KMER_B200_QUERY_UNDEFINED;
+    else if (m64 > a.max_len) status = KMER_B200_QUERY_TOO_LONG_FOR_SHARD;  // longer than the caller's max_query_len
+    if (status != KMER_B200_QUERY_OK) {
+        if (PASS == kPassCount && gl == 0) {
+            a.counts[q] = 0;
+            a.status[q] = (uint8_t)status;
+            a.unsorted[q] = 0;
+        }
+        return;
+    }
+    const uint32_t m = (uint32_t)m64;
+    uint64_t *qw = smem_q + (size_t)group * a.q_words;
+    pack_query_group<G>(a.q_ranks, off0, m, a.q_offsets[a.n_queries], T, (uint32_t)gl, gmask, a.error_flag, qw);
+
+    uint32_t n_gather = 0;
+    uint64_t n_hits = 0;
+    bool unsorted = false;
+    if (m <= e || (uint64_t)m > T.n) {
+        // every window is within e substitutions of a query of at most e symbols (or no window fits)
+        const uint64_t n_win = (uint64_t)m > T.n ? 0 : T.n - m + 1;
+        HAND_OFF_IF_HEAVY(n_win)
+        n_hits = n_win;
+        if (PASS == kPassWrite)
+            for (uint64_t p = gl; p < n_win; p += G) a.positions[out_base + p] = (uint32_t)p;
+    } else {
+        const uint32_t L = m / (e + 1);
+        // the seed element: the largest k <= L, else the smallest k (> L), enumerated as prefix slabs
+        uint32_t es = ix.elem_by_k_desc[ix.n_elems - 1];
+        bool slab = true;
+        for (uint32_t i = 0; i < ix.n_elems; ++i) {
+            const uint32_t c = ix.elem_by_k_desc[i];
+            if (ix.elem[c].k <= L) {
+                es = c;
+                slab = false;
+                break;
+            }
+        }
+        if (L < 64 && ix.aux_for_len[L] != 0xFF && (slab || ix.elem[es].k < L)) {
+            es = ix.aux_for_len[L];
+            slab = false;
+        }
+        const Element &E = ix.elem[es];
+        const uint32_t s_len = slab ? L : E.k;      // symbols of a seed that its candidates match exactly
+        const uint32_t n_tail = slab ? E.k - L : 0;  // per slab seed: starts behind the last k-mer, compared directly
+
+        // ---- the e+1 lookups: independent, issued together (lane j % G takes seed j)
+        Range sr[kMaxMismatches + 1];
+        uint64_t total = 0;
+#pragma unroll
+        for (uint32_t j = 0; j <= kMaxMismatches; ++j) {
+            sr[j] = Range{0, 0};
+            if (j <= e && (G == 1 || j % G == (uint32_t)gl)) {
+                if (slab) {
+                    const uint64_t width = ix.pow_sigma[E.k - L];
+                    const uint64_t key = key_at(qw, (uint64_t)j * L, L, T.bits, T.sigma) * width;
+                    const uint64_t lo = lower_bound_key(E, key);
+                    sr[j] = Range{lo, lower_bound_key(E, key + width) - lo};
+                    if (kAccount) n_gather += 2;
+                } else {
+                    sr[j] = bucket_of(E, key_at(qw, (uint64_t)j * L, E.k, T.bits, T.sigma));
+                    if (kAccount) n_gather += 1 + (E.shift ? 1 : 0);
+                }
+                total += sr[j].cnt + n_tail;
+            }
+        }
+        for (int o = G >> 1; o > 0; o >>= 1) total += __shfl_xor_sync(gmask, total, o, G);
+        HAND_OFF_IF_HEAVY(total)
+
+        // ---- candidates, seed by seed
+        uint32_t seeds_with_hits = 0;
+        for (uint32_t j = 0; j <= e; ++j) {
+            const uint64_t lo = GSHFL(sr[j].lo, (int)(j % G));
+            const uint64_t cnt = GSHFL(sr[j].cnt, (int)(j % G));
+            const uint64_t n_cand = cnt + n_tail;
+            const uint32_t so = j * L;  // the seed's query offset
+            uint64_t hits_j = 0;
+            for (uint64_t c0 = 0; c0 < n_cand; c0 += G) {
+                const uint64_t c = c0 + gl;
+                uint64_t p = 0;
+                bool ok = false;
+                if (c < n_cand) {
+                    uint64_t x;
+                    if (c < cnt) {
+                        x = gather32(pos_ptr(E, lo + c));  // a slab spans buckets, so it may span parts
+                        ok = true;
+                        if (kAccount && (((lo + c) & 7) == 0 || c == 0)) ++n_gather;
+                    } else {
+                        x = T.n - E.k + 1 + (c - cnt);
+                        ok = match_span(T, qw, x, so, L);
+                        if (kAccount) ++n_gather;
+                    }
+                    ok = ok && x >= so && x - so + m <= T.n;
+                    p = x - so;
+                    // an earlier seed that matches exactly here has listed p already
+                    for (uint32_t i = 0; ok && i < j; ++i) {
+                        ok = !match_span(T, qw, p + (uint64_t)i * L, i * L, s_len);
+                        if (kAccount) ++n_gather;
+                    }
+                    if (ok) {
+                        ok = mismatches_span(T, qw, p, 0, m, e) <= e;
+                        if (kAccount) n_gather += 1 + (m * T.bits >> 8);
+                    }
+                }
+                const uint32_t b = GBALLOT(ok);
+                if (PASS == kPassWrite && ok) a.positions[out_base + n_hits + __popc(b & lt_mask)] = (uint32_t)p;
+                n_hits += __popc(b);
+                hits_j += __popc(b);
+            }
+            seeds_with_hits += hits_j != 0 ? 1u : 0u;
+        }
+        unsorted = seeds_with_hits > 1 || slab;  // a bucket of one seed is ascending; a slab is ordered by hash
+    }
+    if (kAccount) {
+        for (int o = G >> 1; o > 0; o >>= 1) n_gather += __shfl_xor_sync(gmask, n_gather, o, G);
+        if (gl == 0) atomicAdd(a.gather_count, (unsigned long long)n_gather);
+    }
+    if (PASS == kPassCount && gl == 0) {
+        a.counts[q] = n_hits;
+        a.status[q] = KMER_B200_QUERY_OK;
+        const bool flag = unsorted && n_hits > 1;
+        a.unsorted[q] = (flag ? 1 : 0) | (HEAVY ? 2 : 0);
+        if (flag) atomicAdd(a.error_flag + 1, 1u);  // number of segments the sort pass has to visit
+        if (a.hits != nullptr && n_hits > 0) {
+            // the write pass only visits the queries listed here
+            const uint32_t act = __activemask();
+            const int leader = __ffs(act) - 1;
+            uint32_t slot = 0;
+            if (lane == leader) slot = atomicAdd(a.hits, (uint32_t)__popc(act));
+            slot = __shfl_sync(act, slot, leader) + __popc(act & ((1u << lane) - 1));
+            a.hits[1 + slot] = (uint32_t)q;
+        }
+    }
+#undef HAND_OFF_IF_HEAVY
+#undef GBALLOT
+#undef GSHFL
+}
+
+// count pass: one group per query; write pass: the queries the count pass listed as having hits
+template <int PASS, int G>
+__global__ void __launch_bounds__(kApproxThreads) search_approx_kernel(const SearchArgs a) {
+    constexpr int kGroups = kApproxThreads / G;
+    extern __shared__ uint64_t smem_q[];
+    if (PASS == kPassWrite && a.hits != nullptr) {
+        const uint32_t n_listed = a.hits[0];
+        for (uint64_t i = (uint64_t)blockIdx.x * kGroups + threadIdx.x / G; i < n_listed; i += (uint64_t)gridDim.x * kGroups) {
+            approx_query<PASS, G, false>(a, (uint64_t)a.hits[1 + i], smem_q);
+            __syncwarp();
+        }
+    } else {
+        const uint64_t q = (uint64_t)blockIdx.x * kGroups + threadIdx.x / G;
+        if (q < a.n_queries) approx_query<PASS, G, false>(a, q, smem_q);
+    }
+}
+
+// second launch of a pass: one warp per query of the heavy list (a.heavy[0] = length, a.heavy[1..] = query ids)
+template <int PASS>
+__global__ void __launch_bounds__(kApproxThreads) search_approx_heavy_kernel(const SearchArgs a) {
+    constexpr int kGroups = kApproxThreads / 32;
+    extern __shared__ uint64_t smem_q[];
+    const uint32_t n_heavy = a.heavy[0];
+    for (uint32_t i = blockIdx.x * kGroups + threadIdx.x / 32; i < n_heavy; i += gridDim.x * kGroups) {
+        approx_query<PASS, 32, true>(a, (uint64_t)a.heavy[1 + i], smem_q);
+        __syncwarp();
+    }
+}
+
+template <int PASS, int G>
+static void launch_approx_pg(const SearchArgs &args, cudaStream_t stream) {
+    constexpr int kGroups = kApproxThreads / G;
+    const size_t smem = (size_t)kGroups * args.q_words * sizeof(uint64_t);
+    uint64_t blocks = (args.n_queries + kGroups - 1) / kGroups;
+    if (PASS == kPassWrite && args.hits != nullptr) blocks = std::min<uint64_t>(blocks, (uint64_t)device_sm_count() * 16);
+    cudaFuncSetAttribute(search_approx_kernel<PASS, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    search_approx_kernel<PASS, G><<<(unsigned)blocks, kApproxThreads, smem, stream>>>(args);
+    if (G < 32 && args.heavy != nullptr) {
+        // queries with long candidate lists, if any (the list length lives on the device: fixed grid, no host sync)
+        SearchArgs h = args;
+        h.q_words = search_q_words(32, args.bits, args.max_len);
+        const size_t hsmem = (size_t)(kApproxThreads / 32) * h.q_words * sizeof(uint64_t);
+        cudaFuncSetAttribute(search_approx_heavy_kernel<PASS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hsmem);
+        search_approx_heavy_kernel<PASS><<<device_sm_count() * 2, kApproxThreads, hsmem, stream>>>(h);
+    }
+}
+
+template <int G>
+static void launch_approx_g(const SearchArgs &args, SearchPass pass, cudaStream_t stream) {
+    if (pass == kPassCount) launch_approx_pg<kPassCount, G>(args, stream);
+    if (pass == kPassCountAccount) launch_approx_pg<kPassCountAccount, G>(args, stream);
+    if (pass == kPassWrite) launch_approx_pg<kPassWrite, G>(args, stream);
+}
+
+void launch_search_approx(const SearchArgs &args, SearchPass pass, cudaStream_t stream) {
+    if (args.n_queries == 0) return;
+    if (args.group == 1) launch_approx_g<1>(args, pass, stream);
+    else if (args.group == 2) launch_approx_g<2>(args, pass, stream);
+    else if (args.group == 4) launch_approx_g<4>(args, pass, stream);
+    else if (args.group == 8) launch_approx_g<8>(args, pass, stream);
+    else launch_approx_g<32>(args, pass, stream);
+}
+
+}  // namespace kb

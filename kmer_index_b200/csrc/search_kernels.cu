@@ -30,29 +30,11 @@ constexpr int kSearchThreads = kSearchWarps * 32;
 
 enum PlanKind : int { kExact = 0, kSubK = 1, kContig = 2, kBuggySingle = 3, kMultiSum = 4 };
 
-// T[tpos, tpos+len) == q[qpos, qpos+len), false if the text span leaves the text
-__device__ __forceinline__ bool match_span(const PackedText &T, const uint64_t *qw, uint64_t tpos, uint32_t qpos,
-                                           uint32_t len) {
-    if (tpos + len > T.n) return false;
-    const uint32_t spw = 64 / T.bits;
-    while (len) {
-        const uint32_t c = len < spw ? len : spw;
-        const uint64_t a = text_window64(T.words, tpos, T.bits);
-        const uint64_t b = window64(qw, (uint64_t)qpos, T.bits);
-        if ((a ^ b) >> (64 - c * T.bits)) return false;
-        tpos += c;
-        qpos += c;
-        len -= c;
-    }
-    return true;
-}
-
 // One group of G lanes per query (one lane up to 64 symbols ... a full warp for long queries or long buckets): the scalar part
 // of a query (plan, status) costs a warp instruction per group, not per warp, and G/32 more queries are in
 // flight per SM to cover the chain of dependent gathers (offsets -> ranks -> directory -> bucket -> text).
 // Candidate lists longer than this are not walked by a small group: the query is appended to the batch's
-// "heavy" list and a second launch gives it a full warp (long buckets of repetitive / low-entropy text).
-constexpr uint32_t kHeavyCandidates = 2048;
+// "heavy" list and a second launch gives it a full warp (long buckets of repetitive / low-entropy text): kHeavyCandidates.
 
 // HEAVY = true: the second launch (G = 32) over the heavy list; never hands a query off again.
 // VIEWS = true: elements may be prefix views of the largest k's arrays (shared-positions index, Element::width); compiled
@@ -132,9 +114,6 @@ __device__ __forceinline__ void search_query(const SearchArgs &a, const uint64_t
     const uint32_t m = (uint32_t)m64;
 
     // ---- 1. pack the query (b bits per symbol, MSB-first) -----------------------------------------------
-    // A chunk is 8 symbols (one 8-byte load); `lpw` chunks make one 64-bit word. Each lane takes `cpl`
-    // consecutive chunks per round so that a round always covers whole words; lanes sharing a word combine
-    // their parts with xor-shuffles.
     if (packed_in) {
         // the caller packed the query already: copy its words (and the two zero words the window reads rely on)
         const uint32_t n_words = (m * T.bits + 63) / 64;
@@ -146,44 +125,7 @@ __device__ __forceinline__ void search_query(const SearchArgs &a, const uint64_t
         }
         if (G > 1) __syncwarp(gmask);
     } else {
-        const uint8_t *qr = a.q_ranks + off0;
-        const uint32_t lpw = 8 / T.bits;                          // chunks per word: 4, 2, 1
-        const uint32_t cpl = lpw > (uint32_t)G ? lpw / G : 1;     // chunks per lane and round
-        const uint32_t share = lpw / cpl;                         // lanes sharing one word
-        const uint32_t wpr = (uint32_t)G * cpl / lpw;             // words per round
-        const uint64_t guard = (0x80u - (T.sigma > 128 ? 128u : T.sigma)) * 0x0101010101010101ull;
-        bool bad = false;
-        uint32_t round = 0;
-        if (G == 1) {
-            if (T.bits == 2) bad = pack_query_lane<2>(a.q_ranks, off0, m, q_total, T.sigma, qw);
-            else if (T.bits == 4) bad = pack_query_lane<4>(a.q_ranks, off0, m, q_total, T.sigma, qw);
-            else bad = pack_query_lane<8>(a.q_ranks, off0, m, q_total, T.sigma, qw);
-        } else
-        for (uint32_t base = 0; base < m; base += 8 * G * cpl, ++round) {
-            uint64_t w = 0;
-            for (uint32_t c = 0; c < cpl; ++c) {
-                const uint32_t chunk = gl * cpl + c;              // chunk index inside the round
-                const uint32_t s0 = base + 8 * chunk;
-                uint64_t v = 0;
-                if (s0 < m) {
-                    v = load8(qr + s0, m - s0, off0 + s0 + 16 <= q_total);
-                    if (T.sigma <= 128) {
-                        bad |= (((v + guard) | v) & 0x8080808080808080ull) != 0;
-                    } else {
-                        for (uint32_t j = 0; j < 8; ++j) bad |= ((v >> (8 * j)) & 0xFF) >= T.sigma;
-                    }
-                }
-                w |= pack8(v, T.bits) << (64 - 8 * T.bits * ((chunk % lpw) + 1));
-            }
-            for (uint32_t o = 1; o < share; o <<= 1) w |= __shfl_xor_sync(gmask, w, o, G);
-            if (gl % share == 0) qw[round * wpr + gl / share] = w;
-        }
-        if (G > 1 && gl == 0) {
-            qw[round * wpr] = 0;
-            qw[round * wpr + 1] = 0;
-        }
-        if ((G == 1 ? bad : __any_sync(gmask, bad)) && gl == 0) atomicOr(a.error_flag, 1u);
-        if (G > 1) __syncwarp(gmask);
+        pack_query_group<G>(a.q_ranks, off0, m, q_total, T, (uint32_t)gl, gmask, a.error_flag, qw);
     }
 
     // ---- 2. plan -----------------------------------------------------------------------------------------
