@@ -416,9 +416,9 @@ void kmer_b200_last_search_transfer(const kmer_b200_index *index, uint64_t *h2d_
 /* Bytes the text took over PCIe when the index was built from a host buffer (large 2- / 4-bit texts are partly packed on
    the host threads first); 0 for an index built from device memory or loaded from a file. */
 uint64_t kmer_b200_build_transfer(const kmer_b200_index *index);
-/* Which host pipeline that call took: 0 = one copy each way (small batches), 1 = chunks of 1-byte ranks, 2 = chunks packed
-   query by query on the host threads, 3 = chunks packed as a stream on the host threads (+ raw_pct percent of the chunks
-   sent as 1-byte ranks at the same time; pack_gbs = the host's measured streaming pack rate, 0 when not needed). */
+/* Which host pipeline that call took: 0 = one copy each way (small batches), 3 = chunks, packed as a stream on the host
+   threads, raw_pct percent of them sent as 1-byte ranks at the same time (100: every chunk raw; pack_gbs = the host's
+   measured streaming pack rate, 0 when not needed). The codes 1 and 2 are no longer reported. */
 void kmer_b200_last_search_host_path(const kmer_b200_index *index, uint32_t *pipeline, uint32_t *raw_pct, double *pack_gbs);
 /* Calibration of the random-gather ceiling: n_gathers independent 8-byte reads at random addresses of a
    table_bytes table (>> L2); *ms_out = device time. sectors/s = n_gathers / time. */

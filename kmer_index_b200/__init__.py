@@ -603,7 +603,7 @@ class KmerIndex:
         """Which host pipeline the last host-buffer search took (kmer_b200_last_search_host_path)."""
         a, b, r = C.c_uint32(0), C.c_uint32(0), C.c_double(0)
         self._L.kmer_b200_last_search_host_path(self._h, C.byref(a), C.byref(b), C.byref(r))
-        names = {0: "single copy", 1: "raw chunks", 2: "per-query host pack", 3: "streaming host pack + raw chunks"}
+        names = {0: "single copy", 3: "streaming host pack + raw chunks"}
         return {"pipeline": names.get(int(a.value), str(a.value)), "raw_chunk_pct": int(b.value), "host_pack_gbs": float(r.value)}
 
     @property

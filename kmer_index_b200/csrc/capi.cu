@@ -194,7 +194,7 @@ struct kmer_b200_index {
     cudaStream_t stream = nullptr;
     bool own_stream = false;
     cudaStream_t copy_in = nullptr, copy_out = nullptr;  // host-batch pipeline: H2D / D2H engines next to `stream`
-    cudaStream_t copy_in2 = nullptr;                     // second H2D queue (raw chunks of search_batch_host_stream)
+    cudaStream_t copy_in2 = nullptr;                     // second H2D queue (raw chunks of search_batch_host_chunked)
     kmer_b200_config cfg{};
     uint64_t n = 0;
     uint32_t sigma = 0, bits = 0;
@@ -951,7 +951,7 @@ static int ensure_copy_streams(kmer_b200_index *ix) {
 }
 
 // Streaming pack rate of this host (input bytes per second, all pool threads), measured once per process on the first
-// large batch: decides how many chunks of a pinned batch travel raw (search_batch_host_stream).
+// large batch: decides how many chunks of a pinned batch travel raw (search_batch_host_chunked).
 static double stream_pack_rate(const uint8_t *ranks, uint64_t n, uint32_t bits, uint32_t sigma) {
     static std::mutex mu;
     static double rate = 0;
@@ -984,6 +984,18 @@ static uint32_t raw_chunk_percent(double pack_rate, uint32_t bits, uint64_t n_sy
     return (uint32_t)std::max(0.0, std::min(100.0, raw + 0.5));
 }
 
+// Which of n_chunks chunks travel raw for a share of raw_pct percent: spread evenly (error diffusion), the first one among
+// them -- the copy engine starts on it at once while the host threads pack the next one.
+static std::vector<uint8_t> raw_chunk_choice(uint32_t raw_pct, uint64_t n_chunks) {
+    std::vector<uint8_t> raw(n_chunks, 0);
+    uint32_t acc = raw_pct ? 99 : 0;
+    for (uint64_t c = 0; c < n_chunks; ++c) {
+        acc += std::min(raw_pct, 100u);
+        if (acc >= 100) raw[c] = 1, acc -= 100;
+    }
+    return raw;
+}
+
 // A large host text (2- or 4-bit alphabets) on its way to ix->d_text: cut into chunks of whole words; the host threads
 // pack chunk after chunk as a stream (kb::pack_stream_host) into a pinned ring whose slots are copied straight into
 // their place in the packed text, and -- pinned input only -- the copy engine moves the other chunks as 1-byte ranks at
@@ -1012,15 +1024,8 @@ static int upload_text_stream(kmer_b200_index *ix, const uint8_t *ranks, uint64_
     }
     const uint64_t chunk = 32ull << 20;  // symbols per chunk: a multiple of every spw
     const uint64_t n_chunks = (n + chunk - 1) / chunk;
-    std::vector<uint8_t> raw(n_chunks, 0);
-    uint64_t n_raw = 0;
-    {
-        uint32_t acc = raw_pct ? 99 : 0;
-        for (uint64_t c = 0; c < n_chunks; ++c) {
-            acc += raw_pct;
-            if (acc >= 100) raw[c] = 1, acc -= 100, ++n_raw;
-        }
-    }
+    const std::vector<uint8_t> raw = raw_chunk_choice(raw_pct, n_chunks);
+    const uint64_t n_raw = (uint64_t)std::count(raw.begin(), raw.end(), 1);
     kb::HostPool &pool = kb::HostPool::instance();
     const unsigned T = pool.threads();
     cudaStream_t st = ix->stream;
@@ -1970,6 +1975,38 @@ __global__ void __launch_bounds__(256) widen_lens_kernel(const uint16_t *__restr
     if (i < n) out[i] = lens[i];
 }
 
+// The host copy of a search result of Q queries: offsets and status pinned; null when an allocation failed. The positions
+// are placed by host_result_positions once their number is known.
+static kmer_b200_result *host_result_new(kmer_b200_index *ix, uint64_t Q) {
+    kmer_b200_result *res = new (std::nothrow) kmer_b200_result();
+    if (!res) return nullptr;
+    res->index = ix;
+    res->on_device = false;
+    res->n_queries = Q;
+    res->offsets = (uint64_t *)pinned_get((Q + 1) * sizeof(uint64_t), &res->cap_offsets);
+    res->status = (uint8_t *)pinned_get(Q, &res->cap_status);
+    if (!res->offsets || !res->status) {
+        kmer_b200_result_free(res);
+        return nullptr;
+    }
+    return res;
+}
+
+// Room for n_positions positions: pinned up to 8 GiB, pageable beyond (pinning tens of gigabytes is slow and can starve
+// the host). False when the allocation failed.
+static bool host_result_positions(kmer_b200_result *res, uint64_t n_positions) {
+    res->n_positions = n_positions;
+    const size_t pos_bytes = n_positions * sizeof(uint32_t);
+    if (pos_bytes > (8ull << 30)) {
+        res->positions = (uint32_t *)std::malloc(pos_bytes);
+        res->positions_pageable = true;
+        res->cap_positions = pos_bytes;
+    } else {
+        res->positions = (uint32_t *)pinned_get(pos_bytes, &res->cap_positions);
+    }
+    return res->positions != nullptr;
+}
+
 // A stream of packed symbols (query boundaries ignored: kb::pack_stream_host) -> the fixed-stride per-query words the
 // search kernels take (SearchArgs::q_packed). One thread per output word: a funnel shift of two stream words, the
 // symbols behind the query's end zeroed. `off` = symbol offsets of the queries inside the stream.
@@ -1995,361 +2032,26 @@ __global__ void __launch_bounds__(256) align_stream_kernel(const uint64_t *__res
     out[idx] = v;
 }
 
-// Large host batches are pipelined in chunks of queries: the H2D copy of chunk c+1 (copy engine), the search of
-// chunk c (SMs) and the D2H copy of chunk c-1's offsets and status (the other copy engine) run concurrently, so
-// the call costs about as much as moving its bytes over PCIe once. Position lists stay on the device until the
-// last chunk is done (their total size is only known then) and are copied out in one sweep.
-static int search_batch_host_pipelined(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q,
-                                       uint32_t mode, kmer_b200_result **out) {
-    constexpr int kChunks = 8;
-    cudaStream_t st = ix->stream;
-    KB_TRY(ensure_copy_streams(ix));
-    const uint64_t n_sym = q_offsets[Q] - q_offsets[0];
-    uint8_t *d_q = nullptr;
-    uint64_t *d_off = nullptr;
-    unsigned long long *d_max = nullptr;
-    // The offsets cross the link as 16-bit lengths (2 bytes per query instead of 8; config 5: 0.6 of 4.8 GB less) and are
-    // rebuilt on the device by a prefix sum. The host threads compute chunk c + 1's lengths while chunk c is in flight;
-    // a chunk with a query of 65 536 symbols or more sends its offsets as they are.
-    const bool lens16 = std::getenv("KMER_B200_NO_LENS16") == nullptr;
-    uint16_t *h_lens = nullptr, *d_lens = nullptr;
-    size_t h_lens_cap = 0;
-    uint64_t *d_scan = nullptr;
-    uint64_t chunk_max[kChunks] = {};
-    bool chunk_lens[kChunks] = {};
-    kmer_b200_result *chunk_res[kChunks] = {};
-    cudaEvent_t ev_in[kChunks] = {}, ev_done[kChunks] = {};
-    kmer_b200_result *res = nullptr;
-    auto cleanup = [&](int code) {
-        cudaStreamSynchronize(ix->copy_in);
-        cudaStreamSynchronize(ix->copy_out);
-        cudaStreamSynchronize(st);
-        for (int c = 0; c < kChunks; ++c) {
-            if (chunk_res[c]) kmer_b200_result_free(chunk_res[c]);
-            if (ev_in[c]) cudaEventDestroy(ev_in[c]);
-            if (ev_done[c]) cudaEventDestroy(ev_done[c]);
-        }
-        dev_free(ix, d_q);
-        dev_free(ix, d_off);
-        dev_free(ix, d_max);
-        dev_free(ix, d_lens);
-        dev_free(ix, d_scan);
-        if (h_lens) pinned_put(h_lens, h_lens_cap);
-        if (code != 0 && res) kmer_b200_result_free(res);
-        return code;
-    };
-    const uint64_t per = (Q + kChunks - 1) / kChunks;
-    // every chunk owns per + 1 offsets (its last entry is not shared with the next chunk's first)
-    if (dev_alloc(ix, &d_q, n_sym, false) || dev_alloc(ix, &d_off, Q + 1 + kChunks, false) || dev_alloc(ix, &d_max, kChunks, false))
-        return cleanup(KMER_B200_ERR_OUT_OF_MEMORY);
-    if (lens16) {
-        h_lens = (uint16_t *)pinned_get(Q * sizeof(uint16_t), &h_lens_cap);
-        if (!h_lens || dev_alloc(ix, &d_lens, Q, false) || dev_alloc(ix, &d_scan, kb::offsets_scan_blocks(per) + 1, false))
-            return cleanup(fail(KMER_B200_ERR_OUT_OF_MEMORY, "allocation for the query lengths failed"));
-    }
-    // the allocations above are ordered on `st`; the copy streams must not touch them earlier
-    cudaEvent_t ev_alloc;
-    cudaEventCreateWithFlags(&ev_alloc, cudaEventDisableTiming);
-    cudaMemsetAsync(d_max, 0, kChunks * sizeof(unsigned long long), st);
-    cudaEventRecord(ev_alloc, st);
-    cudaStreamWaitEvent(ix->copy_in, ev_alloc, 0);
-    cudaStreamWaitEvent(ix->copy_out, ev_alloc, 0);
-    cudaEventDestroy(ev_alloc);
-
-    res = new (std::nothrow) kmer_b200_result();
-    if (!res) return cleanup(fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation failed"));
-    res->index = ix;
-    res->on_device = false;
-    res->n_queries = Q;
-    res->offsets = (uint64_t *)pinned_get((Q + 1) * sizeof(uint64_t), &res->cap_offsets);
-    res->status = (uint8_t *)pinned_get(Q, &res->cap_status);
-    if (!res->offsets || !res->status) return cleanup(fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed"));
-
-    // enqueue every chunk's H2D now; the copy engine works through them while the chunks are searched
-    uint64_t c0[kChunks + 1];
-    uint64_t h2d = n_sym;
-    for (int c = 0; c <= kChunks; ++c) c0[c] = std::min<uint64_t>((uint64_t)c * per, Q);
-    for (int c = 0; c < kChunks; ++c) {
-        const uint64_t qa = c0[c], qb = c0[c + 1];
-        cudaEventCreateWithFlags(&ev_in[c], cudaEventDisableTiming);
-        cudaEventCreateWithFlags(&ev_done[c], cudaEventDisableTiming);
-        if (qb > qa) {
-            // the ranks first: the copy engine moves them while the host threads compute this chunk's lengths
-            const uint64_t s0 = q_offsets[qa] - q_offsets[0], s1 = q_offsets[qb] - q_offsets[0];
-            if (s1 > s0) cudaMemcpyAsync(d_q + s0, q_ranks + q_offsets[qa], s1 - s0, cudaMemcpyHostToDevice, ix->copy_in);
-            if (lens16) {
-                kb::HostPool &pool = kb::HostPool::instance();
-                const unsigned T = std::max(1u, std::min(pool.threads(), 64u));
-                uint64_t part_max[64] = {};
-                pool.run(T, [&](unsigned t) { part_max[t] = kb::query_lengths_host(q_offsets, qa, qb, h_lens + qa, t, T); });
-                for (unsigned t = 0; t < T; ++t) chunk_max[c] = std::max(chunk_max[c], part_max[t]);
-                chunk_lens[c] = chunk_max[c] < 65536;
-            }
-            if (chunk_lens[c])
-                cudaMemcpyAsync(d_lens + qa, h_lens + qa, (qb - qa) * sizeof(uint16_t), cudaMemcpyHostToDevice, ix->copy_in);
-            else
-                cudaMemcpyAsync(d_off + qa + c, q_offsets + qa, (qb - qa + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, ix->copy_in);
-            h2d += chunk_lens[c] ? (qb - qa) * sizeof(uint16_t) : (qb - qa + 1) * sizeof(uint64_t);
-        }
-        cudaEventRecord(ev_in[c], ix->copy_in);
-    }
-    uint64_t base = 0;
-    for (int c = 0; c < kChunks; ++c) {
-        const uint64_t qa = c0[c], qb = c0[c + 1], Qc = qb - qa;
-        if (Qc == 0) continue;
-        cudaStreamWaitEvent(st, ev_in[c], 0);
-        uint64_t *d_off_c = d_off + qa + c;
-        uint64_t max_len = chunk_max[c];
-        if (chunk_lens[c]) {
-            // lengths -> offsets: widen, exclusive scan (the total lands in entry Qc), shift to the batch's numbering
-            widen_lens_kernel<<<(unsigned)((Qc + 255) / 256), 256, 0, st>>>(d_lens + qa, Qc, d_off_c);
-            kb::launch_offsets_scan(d_off_c, Qc, d_scan, st);
-            add_base_kernel<<<(unsigned)((Qc + 1 + 255) / 256), 256, 0, st>>>(d_off_c, Qc + 1, q_offsets[qa]);
-        } else {
-            max_len_kernel<<<(unsigned)std::min<uint64_t>((Qc + 255) / 256, (uint64_t)kb::device_sm_count() * 8), 256, 0, st>>>(d_off_c, Qc, d_max + c);
-            cudaMemcpyAsync(&ix->h_pinned[2], d_max + c, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
-            cudaError_t e = cudaStreamSynchronize(st);
-            if (e != cudaSuccess) return cleanup(fail(KMER_B200_ERR_CUDA, std::string("search (H2D): ") + cudaGetErrorString(e)));
-            max_len = ix->h_pinned[2];
-        }
-        int s = search_device_impl(ix, d_q - q_offsets[0], d_off_c, Qc, max_len, mode, nullptr, 0, kFlavorFull, &chunk_res[c]);
-        if (s != 0) return cleanup(s);
-        kmer_b200_result *cr = chunk_res[c];
-        if (base) add_base_kernel<<<(unsigned)((Qc + 1 + 255) / 256), 256, 0, st>>>(cr->offsets, Qc + 1, base);
-        cudaEventRecord(ev_done[c], st);
-        cudaStreamWaitEvent(ix->copy_out, ev_done[c], 0);
-        // the last entry of a chunk's offsets equals the first of the next one: copy Qc entries, the final total below
-        cudaMemcpyAsync(res->offsets + qa, cr->offsets, Qc * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->copy_out);
-        cudaMemcpyAsync(res->status + qa, cr->status, Qc, cudaMemcpyDeviceToHost, ix->copy_out);
-        base += cr->n_positions;
-    }
-    res->n_positions = base;
-    const size_t pos_bytes = base * sizeof(uint32_t);
-    if (pos_bytes > (8ull << 30)) {
-        res->positions = (uint32_t *)std::malloc(pos_bytes);
-        res->positions_pageable = true;
-        res->cap_positions = pos_bytes;
-    } else {
-        res->positions = (uint32_t *)pinned_get(pos_bytes, &res->cap_positions);
-    }
-    if (!res->positions) return cleanup(fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation for the positions failed"));
-    uint64_t at = 0;
-    for (int c = 0; c < kChunks; ++c) {
-        if (!chunk_res[c] || !chunk_res[c]->n_positions) continue;
-        cudaMemcpyAsync(res->positions + at, chunk_res[c]->positions, chunk_res[c]->n_positions * sizeof(uint32_t),
-                        cudaMemcpyDeviceToHost, ix->copy_out);
-        at += chunk_res[c]->n_positions;
-    }
-    cudaError_t e = cudaStreamSynchronize(ix->copy_out);
-    res->offsets[Q] = base;
-    if (e != cudaSuccess) return cleanup(fail(KMER_B200_ERR_CUDA, std::string("search (D2H): ") + cudaGetErrorString(e)));
-    ix->last_h2d = h2d;
-    ix->last_d2h = Q * 9 + pos_bytes;
-    *out = res;
-    return cleanup(0);
-}
-
-// Large host batches, packed on the host: the batch is cut into chunks of queries; the host threads pack chunk c + 2
-// (1 byte per rank -> b-bit words, fixed stride, plus 16-bit lengths: a third of the bytes for dna4) while chunk c + 1
-// crosses PCIe and chunk c is searched; offsets and status of finished chunks leave on the other copy engine. The input
-// may be pageable memory: the packers read it directly, only the packed staging ring is pinned. The call costs about
-// as much as the slower of "pack the batch once with all host cores" and "move the packed bytes once".
-static int search_batch_host_packed(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q,
-                                    uint32_t mode, kmer_b200_result **out) {
-    constexpr int kChunks = 16, kRing = 3;
-    uint64_t h2d = 0;
-    cudaStream_t st = ix->stream;
-    KB_TRY(ensure_copy_streams(ix));
-    kb::HostPool &pool = kb::HostPool::instance();
-    const unsigned T = pool.threads();
-    const uint32_t spw = 64 / ix->bits;
-    const uint64_t per = (Q + kChunks - 1) / kChunks;
-    uint64_t c0[kChunks + 1];
-    for (int c = 0; c <= kChunks; ++c) c0[c] = std::min<uint64_t>((uint64_t)c * per, Q);
-
-    // pinned staging ring: lengths first (their maximum fixes the chunk's stride), then the packed words
-    const uint64_t max_stride = 16;
-    uint16_t *h_lens[kRing] = {};
-    uint64_t *h_words[kRing] = {};
-    size_t cap_lens[kRing] = {}, cap_words[kRing] = {};
-    uint64_t *d_words[kChunks] = {};
-    uint16_t *d_lens[kChunks] = {};
-    uint32_t stride[kChunks] = {};
-    uint64_t max_len[kChunks] = {};
-    kmer_b200_result *chunk_res[kChunks] = {};
-    cudaEvent_t ev_in[kChunks] = {}, ev_done[kChunks] = {}, ev_slot[kRing] = {};
-    kmer_b200_result *res = nullptr;
-    std::vector<uint64_t> part_max(T * 4);
-    std::vector<uint8_t> part_ok(T * 4);
-    bool unsupported = false, bad_rank = false;
-    auto cleanup = [&](int code) {
-        pool.wait();
-        cudaStreamSynchronize(ix->copy_in);
-        cudaStreamSynchronize(ix->copy_out);
-        cudaStreamSynchronize(st);
-        for (int c = 0; c < kChunks; ++c) {
-            if (chunk_res[c]) kmer_b200_result_free(chunk_res[c]);
-            if (ev_in[c]) cudaEventDestroy(ev_in[c]);
-            if (ev_done[c]) cudaEventDestroy(ev_done[c]);
-            dev_free(ix, d_words[c]);
-            dev_free(ix, d_lens[c]);
-        }
-        for (int r = 0; r < kRing; ++r) {
-            if (ev_slot[r]) cudaEventDestroy(ev_slot[r]);
-            pinned_put(h_lens[r], cap_lens[r]);
-            pinned_put(h_words[r], cap_words[r]);
-        }
-        if (code != 0 && res) kmer_b200_result_free(res);
-        return code;
-    };
-    for (int r = 0; r < kRing; ++r) {
-        h_lens[r] = (uint16_t *)pinned_get(per * sizeof(uint16_t), &cap_lens[r]);
-        h_words[r] = (uint64_t *)pinned_get(per * 4 * sizeof(uint64_t), &cap_words[r]);  // grown when a chunk needs more
-        if (!h_lens[r] || !h_words[r]) return cleanup(fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed"));
-        cudaEventCreateWithFlags(&ev_slot[r], cudaEventDisableTiming);
-    }
-    for (int c = 0; c < kChunks; ++c) {
-        cudaEventCreateWithFlags(&ev_in[c], cudaEventDisableTiming);
-        cudaEventCreateWithFlags(&ev_done[c], cudaEventDisableTiming);
-    }
-    res = new (std::nothrow) kmer_b200_result();
-    if (!res) return cleanup(fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation failed"));
-    res->index = ix;
-    res->on_device = false;
-    res->n_queries = Q;
-    res->offsets = (uint64_t *)pinned_get((Q + 1) * sizeof(uint64_t), &res->cap_offsets);
-    res->status = (uint8_t *)pinned_get(Q, &res->cap_status);
-    if (!res->offsets || !res->status) return cleanup(fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed"));
-
-    // stage 1 of chunk c (blocking, short): lengths + longest query -> stride; stage 2 (asynchronous): pack
-    auto start_pack = [&](int c) -> int {
-        const uint64_t qa = c0[c], qb = c0[c + 1];
-        if (qb == qa) return 0;
-        const int slot = c % kRing;
-        if (c >= kRing) cudaEventSynchronize(ev_slot[slot]);  // the slot's previous H2D has left the staging buffers
-        pool.run(T * 4, [&, qa, qb, slot](unsigned t) { part_max[t] = kb::query_lengths_host(q_offsets, qa, qb, h_lens[slot], t, T * 4); });
-        uint64_t mx = 0;
-        for (uint64_t v : part_max) mx = std::max(mx, v);
-        max_len[c] = mx;
-        stride[c] = (uint32_t)std::max<uint64_t>(1, (mx + spw - 1) / spw);
-        if (mx > 65535 || stride[c] > max_stride) {
-            unsupported = true;
-            return 0;
-        }
-        const size_t need = (qb - qa) * stride[c] * sizeof(uint64_t);
-        if (need > cap_words[slot]) {
-            pinned_put(h_words[slot], cap_words[slot]);
-            h_words[slot] = (uint64_t *)pinned_get(need, &cap_words[slot]);
-            if (!h_words[slot]) return fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed");
-        }
-        std::fill(part_ok.begin(), part_ok.end(), 1);
-        const uint32_t sc = stride[c];
-        pool.submit(T * 4, [&, qa, qb, slot, sc](unsigned t) {
-            part_ok[t] = kb::pack_queries_host(q_ranks, q_offsets, qa, qb, ix->bits, ix->sigma, sc, h_words[slot], t, T * 4) ? 1 : 0;
-        });
-        return 0;
-    };
-    auto finish_pack_and_upload = [&](int c) -> int {
-        const uint64_t qa = c0[c], qb = c0[c + 1];
-        pool.wait();
-        if (qb == qa || unsupported) return 0;
-        for (uint8_t ok : part_ok) bad_rank = bad_rank || !ok;
-        const int slot = c % kRing;
-        const uint64_t Qc = qb - qa;
-        KB_TRY(dev_alloc(ix, &d_words[c], Qc * stride[c], false));
-        KB_TRY(dev_alloc(ix, &d_lens[c], Qc, false));
-        cudaEvent_t ev_alloc;  // the allocations are ordered on `st`
-        cudaEventCreateWithFlags(&ev_alloc, cudaEventDisableTiming);
-        cudaEventRecord(ev_alloc, st);
-        cudaStreamWaitEvent(ix->copy_in, ev_alloc, 0);
-        cudaEventDestroy(ev_alloc);
-        cudaMemcpyAsync(d_words[c], h_words[slot], Qc * stride[c] * sizeof(uint64_t), cudaMemcpyHostToDevice, ix->copy_in);
-        cudaMemcpyAsync(d_lens[c], h_lens[slot], Qc * sizeof(uint16_t), cudaMemcpyHostToDevice, ix->copy_in);
-        h2d += Qc * stride[c] * sizeof(uint64_t) + Qc * sizeof(uint16_t);
-        cudaEventRecord(ev_in[c], ix->copy_in);
-        cudaEventRecord(ev_slot[slot], ix->copy_in);
-        return 0;
-    };
-
-    {
-        cudaEvent_t ev0;  // the copy-out stream must not run ahead of work already queued on `st`
-        cudaEventCreateWithFlags(&ev0, cudaEventDisableTiming);
-        cudaEventRecord(ev0, st);
-        cudaStreamWaitEvent(ix->copy_out, ev0, 0);
-        cudaEventDestroy(ev0);
-    }
-    if (int s = start_pack(0)) return cleanup(s);
-    if (int s = finish_pack_and_upload(0)) return cleanup(s);
-    if (kChunks > 1)
-        if (int s = start_pack(1)) return cleanup(s);
-    uint64_t base = 0;
-    for (int c = 0; c < kChunks && !unsupported; ++c) {
-        if (c + 1 < kChunks) {
-            if (int s = finish_pack_and_upload(c + 1)) return cleanup(s);
-            if (c + 2 < kChunks)
-                if (int s = start_pack(c + 2)) return cleanup(s);
-        }
-        if (unsupported || bad_rank) break;
-        const uint64_t qa = c0[c], qb = c0[c + 1], Qc = qb - qa;
-        if (Qc == 0) continue;
-        cudaStreamWaitEvent(st, ev_in[c], 0);
-        PackedQueries pk{d_words[c], d_lens[c], stride[c]};
-        int s = search_device_impl(ix, nullptr, nullptr, Qc, max_len[c], mode, nullptr, 0, kFlavorFull, &chunk_res[c], &pk);
-        if (s != 0) return cleanup(s);
-        kmer_b200_result *cr = chunk_res[c];
-        if (base) add_base_kernel<<<(unsigned)((Qc + 1 + 255) / 256), 256, 0, st>>>(cr->offsets, Qc + 1, base);
-        cudaEventRecord(ev_done[c], st);
-        cudaStreamWaitEvent(ix->copy_out, ev_done[c], 0);
-        cudaMemcpyAsync(res->offsets + qa, cr->offsets, Qc * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->copy_out);
-        cudaMemcpyAsync(res->status + qa, cr->status, Qc, cudaMemcpyDeviceToHost, ix->copy_out);
-        base += cr->n_positions;
-    }
-    if (bad_rank) return cleanup(fail(KMER_B200_ERR_INVALID_RANK, "a query contains a rank >= sigma"));
-    if (unsupported) return cleanup(KMER_B200_ERR_UNSUPPORTED);  // the caller falls back to the unpacked pipeline
-    res->n_positions = base;
-    const size_t pos_bytes = base * sizeof(uint32_t);
-    if (pos_bytes > (8ull << 30)) {
-        res->positions = (uint32_t *)std::malloc(pos_bytes);
-        res->positions_pageable = true;
-        res->cap_positions = pos_bytes;
-    } else {
-        res->positions = (uint32_t *)pinned_get(pos_bytes, &res->cap_positions);
-    }
-    if (!res->positions) return cleanup(fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation for the positions failed"));
-    uint64_t at = 0;
-    for (int c = 0; c < kChunks; ++c) {
-        if (!chunk_res[c] || !chunk_res[c]->n_positions) continue;
-        cudaMemcpyAsync(res->positions + at, chunk_res[c]->positions, chunk_res[c]->n_positions * sizeof(uint32_t),
-                        cudaMemcpyDeviceToHost, ix->copy_out);
-        at += chunk_res[c]->n_positions;
-    }
-    cudaError_t e = cudaStreamSynchronize(ix->copy_out);
-    res->offsets[Q] = base;
-    if (e != cudaSuccess) return cleanup(fail(KMER_B200_ERR_CUDA, std::string("search (D2H): ") + cudaGetErrorString(e)));
-    ix->last_h2d = h2d;
-    ix->last_d2h = Q * 9 + base * sizeof(uint32_t);
-    *out = res;
-    return cleanup(0);
-}
-
-// Large host batches, round 2's final form. Per-query packing on the host cores costs more than the PCIe bytes it saves
-// (search_batch_host_packed: 16 cores pack ~30 GB/s of variable-length queries, the link moves 55 GB/s). What the host
-// cores do fast is a pure streaming pack of the concatenated ranks, query boundaries ignored (kb::pack_stream_host: 128
-// ranks -> 32 bytes in ten AVX2 instructions, bound by what a core streams from DRAM: ~100 GB/s on 16 cores); cutting
-// that stream into per-query words is a ~1 ms kernel on the device (align_stream_kernel). The batch is cut into chunks of
-// queries of two kinds that keep BOTH resources busy:
-//   * stream chunks: 16-bit lengths + streaming pack by the pool, then (bits / 8) of the bytes over PCIe;
-//   * raw chunks (pinned input only, `raw_pct` percent of the chunks): the copy engine moves the caller's 1-byte ranks
-//     as they are -- no host work beyond the lengths.
+// Large host batches, in chunks of queries: the H2D copy of later chunks, the search of chunk c and the D2H copy of
+// earlier chunks' offsets and status run concurrently. Per-query packing on the host cores costs more than the PCIe bytes
+// it saves (16 cores pack ~30 GB/s of variable-length queries, the link moves 55 GB/s). What the host cores do fast is a
+// pure streaming pack of the concatenated ranks, query boundaries ignored (kb::pack_stream_host: 128 ranks -> 32 bytes in
+// ten AVX2 instructions, bound by what a core streams from DRAM: ~100 GB/s on 16 cores); cutting that stream into
+// per-query words is a ~1 ms kernel on the device (align_stream_kernel). The batch is cut into chunks of queries of two
+// kinds that keep BOTH resources busy:
+//   * packed chunks: 16-bit lengths + streaming pack by the pool, then (bits / 8) of the bytes over PCIe;
+//   * raw chunks (`raw_pct` percent of the chunks): the copy engine moves the caller's 1-byte ranks as they are -- no host
+//     work beyond the lengths. A raw chunk with a query of 65 536 symbols or more sends its offsets as they are instead.
 // A producer thread walks the chunks in order and never waits for the device except for a free slot of the pinned ring:
 // raw chunks are queued on one H2D stream, packed chunks on another, so neither kind waits behind the other. The calling
 // thread searches the chunks in order as they arrive (device buffers are allocated up front, so the producer makes no
-// stream-ordered allocation); offsets and status of finished chunks leave on the D2H stream. Results are identical to
-// the plain path's (tests/test_gpu_full_size.py).
-static int search_batch_host_stream(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q,
-                                    uint32_t mode, uint32_t raw_pct, kmer_b200_result **out) {
+// stream-ordered allocation); offsets and status of finished chunks leave on the D2H stream. Position lists stay on the
+// device until the last chunk is done (their total size is only known then) and are copied out in one sweep. Results
+// are identical to the single-copy path's (tests/test_gpu_full_size.py). KMER_B200_ERR_UNSUPPORTED: a packed chunk holds
+// a query longer than 16 words or 65 535 symbols, or no producer thread could be started.
+static int search_batch_host_chunked(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q,
+                                     uint32_t mode, uint32_t raw_pct, kmer_b200_result **out) {
     constexpr int kChunks = 24, kRing = 4;
-    if (ix->bits != 2 && ix->bits != 4) return KMER_B200_ERR_UNSUPPORTED;
     // KMER_B200_HOST_TRACE=1: where the time went (ms), printed to stderr at the end of the call
     const bool trace = std::getenv("KMER_B200_HOST_TRACE") != nullptr;
     auto now = [] { return std::chrono::steady_clock::now(); };
@@ -2365,29 +2067,18 @@ static int search_batch_host_stream(kmer_b200_index *ix, const uint8_t *q_ranks,
     const uint64_t per = (Q + kChunks - 1) / kChunks;
     uint64_t c0[kChunks + 1];
     for (int c = 0; c <= kChunks; ++c) c0[c] = std::min<uint64_t>((uint64_t)c * per, Q);
-    // which chunks travel raw: spread evenly (error diffusion), the first one among them -- the copy engine starts on it at
-    // once while the pool packs chunk 1
-    bool raw[kChunks] = {};
-    {
-        uint32_t acc = raw_pct ? 99 : 0;
-        for (int c = 0; c < kChunks; ++c) {
-            acc += std::min(raw_pct, 100u);
-            if (acc >= 100) {
-                raw[c] = true;
-                acc -= 100;
-            }
-        }
-    }
+    const std::vector<uint8_t> raw = raw_chunk_choice(raw_pct, kChunks);
 
     const uint64_t max_stride = 16;
     uint16_t *h_lens = nullptr;
     size_t cap_lens = 0;
     uint64_t *h_words[kRing] = {};
     size_t cap_words[kRing] = {};
-    void *d_in[kChunks] = {};        // raw chunk: its ranks; stream chunk: its packed stream (+ one word of padding)
-    uint64_t *d_words[kChunks] = {}; // stream chunk: per-query words after the alignment
+    void *d_in[kChunks] = {};        // raw chunk: its ranks; packed chunk: its packed stream (+ one word of padding)
+    uint64_t *d_words[kChunks] = {}; // packed chunk: per-query words after the alignment
     uint16_t *d_lens[kChunks] = {};
-    uint64_t *d_off[kChunks] = {};   // chunk-relative symbol offsets, rebuilt from the lengths on the device
+    uint64_t *d_off[kChunks] = {};   // chunk-relative symbol offsets, rebuilt on the device
+    bool lens16[kChunks] = {};       // the chunk sent 16-bit lengths (else its offsets as they are)
     uint64_t *d_scan = nullptr;
     uint32_t stride[kChunks] = {};
     uint64_t max_len[kChunks] = {}, n_sym_c[kChunks] = {}, n_stream_words[kChunks] = {};
@@ -2463,14 +2154,8 @@ static int search_batch_host_stream(kmer_b200_index *ix, const uint8_t *q_ranks,
         cudaStreamWaitEvent(ix->copy_out, ev0, 0);
         cudaEventDestroy(ev0);
     }
-    res = new (std::nothrow) kmer_b200_result();
-    if (!res) return cleanup(fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation failed"));
-    res->index = ix;
-    res->on_device = false;
-    res->n_queries = Q;
-    res->offsets = (uint64_t *)pinned_get((Q + 1) * sizeof(uint64_t), &res->cap_offsets);
-    res->status = (uint8_t *)pinned_get(Q, &res->cap_status);
-    if (!res->offsets || !res->status) return cleanup(fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed"));
+    res = host_result_new(ix, Q);
+    if (!res) return cleanup(fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed"));
 
     const int device = ix->device;
     auto produce = [&] {
@@ -2485,9 +2170,18 @@ static int search_batch_host_stream(kmer_b200_index *ix, const uint8_t *q_ranks,
             if (Qc) {
                 const uint8_t *src = q_ranks + q_offsets[qa];
                 const uint64_t n_sym = n_sym_c[c];
+                const bool is_raw = raw[c];
+                // raw chunks on their own H2D stream: a 175 MB copy does not hold up the packed chunk behind it, whose
+                // ring slot the packers want back (queueing every raw chunk up front was tried: the raw stream then
+                // starves the packed one and the ring stalls -- 64 ms against 54)
+                cudaStream_t cs = is_raw ? ix->copy_in2 : ix->copy_in;
                 int slot = 0;
                 auto t0 = now();
-                if (!raw[c]) {
+                if (is_raw) {
+                    // the ranks first: the copy engine moves them while the host threads compute this chunk's lengths
+                    if (n_sym) cudaMemcpyAsync(d_in[c], src, n_sym, cudaMemcpyHostToDevice, cs);
+                    h2d += n_sym;
+                } else {
                     slot = used++ % kRing;
                     if (used > kRing) cudaEventSynchronize(ev_slot[slot]);  // the slot's previous H2D has left the staging buffer
                     t_slot += since(t0);
@@ -2495,7 +2189,6 @@ static int search_batch_host_stream(kmer_b200_index *ix, const uint8_t *q_ranks,
                     std::fill(part_ok.begin(), part_ok.end(), 1);
                 }
                 uint64_t *dst = h_words[slot];
-                const bool is_raw = raw[c];
                 pool.run(T * 4, [&, qa, qb, src, n_sym, dst, is_raw](unsigned t) {
                     part_max[t] = kb::query_lengths_host(q_offsets, qa, qb, h_lens + qa, t, T * 4);
                     if (!is_raw) part_ok[t] = kb::pack_stream_host(src, n_sym, bits, sigma, dst, t, T * 4) ? 1 : 0;
@@ -2506,24 +2199,24 @@ static int search_batch_host_stream(kmer_b200_index *ix, const uint8_t *q_ranks,
                 for (uint64_t v : part_max) mx = std::max(mx, v);
                 max_len[c] = mx;
                 stride[c] = (uint32_t)std::max<uint64_t>(1, (mx + spw - 1) / spw);
-                if (mx > 65535 || (!is_raw && stride[c] > max_stride)) unsupported = failed = true;
+                lens16[c] = mx < 65536;
+                if (!is_raw && (!lens16[c] || stride[c] > max_stride)) unsupported = failed = true;
                 if (!is_raw)
                     for (uint8_t ok : part_ok)
                         if (!ok) bad_rank = failed = true;
                 if (!failed) {
-                    // raw chunks on their own H2D stream: a 175 MB copy does not hold up the packed chunk behind it, whose
-                    // ring slot the packers want back (queueing every raw chunk up front was tried: the raw stream then
-                    // starves the packed one and the ring stalls -- 64 ms against 54)
-                    cudaStream_t cs = is_raw ? ix->copy_in2 : ix->copy_in;
-                    if (is_raw) {
-                        if (n_sym) cudaMemcpyAsync(d_in[c], src, n_sym, cudaMemcpyHostToDevice, cs);
-                        h2d += n_sym + Qc * sizeof(uint16_t);
-                    } else {
+                    if (!is_raw) {
                         dst[n_stream_words[c]] = 0;  // the padding word align_stream_kernel may read
                         cudaMemcpyAsync(d_in[c], dst, (n_stream_words[c] + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, cs);
-                        h2d += (n_stream_words[c] + 1) * sizeof(uint64_t) + Qc * sizeof(uint16_t);
+                        h2d += (n_stream_words[c] + 1) * sizeof(uint64_t);
                     }
-                    cudaMemcpyAsync(d_lens[c], h_lens + qa, Qc * sizeof(uint16_t), cudaMemcpyHostToDevice, cs);
+                    if (lens16[c]) {
+                        cudaMemcpyAsync(d_lens[c], h_lens + qa, Qc * sizeof(uint16_t), cudaMemcpyHostToDevice, cs);
+                        h2d += Qc * sizeof(uint16_t);
+                    } else {
+                        cudaMemcpyAsync(d_off[c], q_offsets + qa, (Qc + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, cs);
+                        h2d += (Qc + 1) * sizeof(uint64_t);
+                    }
                     cudaEventRecord(ev_in[c], cs);
                     if (!is_raw) cudaEventRecord(ev_slot[slot], cs);
                 }
@@ -2540,7 +2233,7 @@ static int search_batch_host_stream(kmer_b200_index *ix, const uint8_t *q_ranks,
     };
     try {
         producer = std::thread(produce);
-    } catch (const std::system_error &) {  // no thread to be had: the caller takes one of the single-threaded pipelines
+    } catch (const std::system_error &) {  // no thread to be had: the caller takes the single-copy path
         return cleanup(KMER_B200_ERR_UNSUPPORTED);
     }
 
@@ -2561,9 +2254,13 @@ static int search_batch_host_stream(kmer_b200_index *ix, const uint8_t *q_ranks,
         if (Qc == 0) continue;
         const auto t0 = now();
         cudaStreamWaitEvent(st, ev_in[c], 0);
-        // lengths -> chunk-relative offsets: widen, exclusive scan (the total lands in entry Qc)
-        widen_lens_kernel<<<(unsigned)((Qc + 255) / 256), 256, 0, st>>>(d_lens[c], Qc, d_off[c]);
-        kb::launch_offsets_scan(d_off[c], Qc, d_scan, st);
+        if (lens16[c]) {
+            // lengths -> chunk-relative offsets: widen, exclusive scan (the total lands in entry Qc)
+            widen_lens_kernel<<<(unsigned)((Qc + 255) / 256), 256, 0, st>>>(d_lens[c], Qc, d_off[c]);
+            kb::launch_offsets_scan(d_off[c], Qc, d_scan, st);
+        } else {
+            add_base_kernel<<<(unsigned)((Qc + 1 + 255) / 256), 256, 0, st>>>(d_off[c], Qc + 1, 0 - q_offsets[qa]);
+        }
         int s;
         if (raw[c]) {
             s = search_device_impl(ix, (const uint8_t *)d_in[c], d_off[c], Qc, max_len[c], mode, nullptr, 0, kFlavorFull, &chunk_res[c]);
@@ -2589,17 +2286,8 @@ static int search_batch_host_stream(kmer_b200_index *ix, const uint8_t *q_ranks,
     }
     producer.join();
     if (bad_rank) return cleanup(fail(KMER_B200_ERR_INVALID_RANK, "a query contains a rank >= sigma"));
-    if (unsupported || !ok_so_far) return cleanup(KMER_B200_ERR_UNSUPPORTED);  // the caller falls back to the unpacked pipeline
-    res->n_positions = base;
-    const size_t pos_bytes = base * sizeof(uint32_t);
-    if (pos_bytes > (8ull << 30)) {
-        res->positions = (uint32_t *)std::malloc(pos_bytes);
-        res->positions_pageable = true;
-        res->cap_positions = pos_bytes;
-    } else {
-        res->positions = (uint32_t *)pinned_get(pos_bytes, &res->cap_positions);
-    }
-    if (!res->positions) return cleanup(fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation for the positions failed"));
+    if (unsupported || !ok_so_far) return cleanup(KMER_B200_ERR_UNSUPPORTED);  // the caller reruns the batch with every chunk raw
+    if (!host_result_positions(res, base)) return cleanup(fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation for the positions failed"));
     uint64_t at = 0;
     for (int c = 0; c < kChunks; ++c) {
         if (!chunk_res[c] || !chunk_res[c]->n_positions) continue;
@@ -2660,27 +2348,8 @@ static int search_batch_host_single_copy(kmer_b200_index *ix, const uint8_t *q_r
                                max_mismatches);
     if (s != 0) return s;
     // device result -> pinned host buffers
-    kmer_b200_result *res = new (std::nothrow) kmer_b200_result();
-    if (!res) {
-        kmer_b200_result_free(dres);
-        return fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation failed");
-    }
-    res->index = ix;
-    res->on_device = false;
-    res->n_queries = Q;
-    res->n_positions = dres->n_positions;
-    res->offsets = (uint64_t *)pinned_get((Q + 1) * sizeof(uint64_t), &res->cap_offsets);
-    res->status = (uint8_t *)pinned_get(Q, &res->cap_status);
-    // pinning tens of gigabytes is slow and can starve the host: beyond 8 GiB the positions go to pageable memory
-    const size_t pos_bytes = res->n_positions * sizeof(uint32_t);
-    if (pos_bytes > (8ull << 30)) {
-        res->positions = (uint32_t *)std::malloc(pos_bytes);
-        res->positions_pageable = true;
-        res->cap_positions = pos_bytes;
-    } else {
-        res->positions = (uint32_t *)pinned_get(pos_bytes, &res->cap_positions);
-    }
-    if (!res->offsets || !res->status || !res->positions) {
+    kmer_b200_result *res = host_result_new(ix, Q);
+    if (!res || !host_result_positions(res, dres->n_positions)) {
         kmer_b200_result_free(dres);
         kmer_b200_result_free(res);
         return fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed");
@@ -2714,73 +2383,33 @@ static int search_batch_host(kmer_b200_index *ix, const uint8_t *q_ranks, const 
     if (n_sym && !q_ranks) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "q_ranks is null");
     // batches whose transfer dominates (>= 256 MiB over PCIe) are pipelined in chunks
     if (!lut256 && Q >= (1u << 18) && n_sym + Q * 17 >= (256ull << 20) && !std::getenv("KMER_B200_NO_PIPELINE")) {
-        // Which pipeline. 2- and 4-bit alphabets: search_batch_host_stream -- the host threads pack chunks of the batch as a
-        // stream (a quarter / half of the bytes), and when the input is pinned the copy engine moves the other chunks as
-        // they are at the same time; the share of raw chunks comes from the host's streaming pack rate, measured once per
-        // process on the first large batch (other processes sharing the cores -- one per GPU under torchrun -- lower the
-        // rate and so raise the share). Pageable input cannot be DMA-ed directly (the driver would stage it at a fraction
-        // of the link rate): every chunk is packed straight out of the caller's memory into a pinned ring. 8-bit alphabets
-        // (nothing to gain from packing) and batches the streaming pipeline refuses (a query >= 65 536 symbols) keep round
-        // 2's first two pipelines: per-query packing for pageable input, raw chunks for pinned input.
+        // The share of raw chunks. Pageable input cannot be DMA-ed directly (the driver would stage it at a fraction of the
+        // link rate): every chunk is packed straight out of the caller's memory into a pinned ring. Pinned input of 2- and
+        // 4-bit alphabets: the share comes from the host's streaming pack rate, measured once per process on the first
+        // large batch (other processes sharing the cores -- one per GPU under torchrun -- lower the rate and so raise the
+        // share). Pinned input of 8-bit alphabets: packing saves no link bytes, every chunk travels raw.
         cudaPointerAttributes attr{};
-        bool pageable = cudaPointerGetAttributes(&attr, q_ranks) != cudaSuccess || attr.type == cudaMemoryTypeUnregistered;
+        const bool pageable = cudaPointerGetAttributes(&attr, q_ranks) != cudaSuccess || attr.type == cudaMemoryTypeUnregistered;
         cudaGetLastError();
-        const bool input_pageable = pageable;
-        if (!pageable && ix->bits == 8) {  // (2- and 4-bit alphabets take the streaming pipeline below)
-            static std::atomic<int> pack_wins{-1};  // -1 unknown, 0 no, 1 yes
-            if (pack_wins.load() < 0) {
-                kb::HostPool &pool = kb::HostPool::instance();
-                const unsigned T = pool.threads();
-                const uint64_t Qs = std::min<uint64_t>(Q, 1u << 22);
-                const uint32_t spw = 64 / ix->bits;
-                std::vector<uint16_t> lens(Qs);
-                std::vector<uint64_t> part_max(T * 4, 0);
-                pool.run(T * 4, [&](unsigned t) { part_max[t] = kb::query_lengths_host(q_offsets, 0, Qs, lens.data(), t, T * 4); });
-                uint64_t mx = 1;
-                for (uint64_t v : part_max) mx = std::max(mx, v);
-                const uint64_t stride = (mx + spw - 1) / spw;
-                int wins = 0;
-                if (stride <= 16) {
-                    std::vector<uint64_t> words(Qs * stride);
-                    const auto t0 = std::chrono::steady_clock::now();
-                    pool.run(T * 4, [&](unsigned t) {
-                        kb::pack_queries_host(q_ranks, q_offsets, 0, Qs, ix->bits, ix->sigma, (uint32_t)stride, words.data(), t, T * 4);
-                    });
-                    const double sec = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
-                    const double in_bytes = (double)(q_offsets[Qs] - q_offsets[0]) + 8.0 * Qs;
-                    wins = in_bytes / sec > 75e9 ? 1 : 0;  // must beat the ~55 GB/s link with margin (the pack also shares memory bandwidth with the DMA)
-                }
-                pack_wins.store(wins);
-            }
-            pageable = pack_wins.load() == 1;
+        uint32_t raw_pct = 0;
+        double rate = 0;
+        if (!pageable && ix->bits == 8) {
+            raw_pct = 100;
+        } else if (!pageable) {
+            rate = stream_pack_rate(q_ranks + q_offsets[0], n_sym, ix->bits, ix->sigma);
+            raw_pct = raw_chunk_percent(rate / std::max(1u, ix->host_sharers), ix->bits, n_sym, Q);
         }
-        // KMER_B200_HOST_PACK: 0 = raw chunks only, 1 = per-query packing on the host, 2 = streaming pack only,
-        // 3 = streaming pack + raw chunks (KMER_B200_HOST_RAW_PCT percent of the chunks, default from the calibration)
-        int forced = -1;
-        if (const char *env = std::getenv("KMER_B200_HOST_PACK")) forced = std::atoi(env);
-        const bool can_stream = ix->bits == 2 || ix->bits == 4;
-        if ((forced < 0 && can_stream) || forced == 2 || forced == 3) {
-            uint32_t raw_pct = 0;
-            double rate = 0;
-            if (!input_pageable && forced != 2) {
-                rate = stream_pack_rate(q_ranks + q_offsets[0], n_sym, ix->bits, ix->sigma);
-                raw_pct = raw_chunk_percent(rate / std::max(1u, ix->host_sharers), ix->bits, n_sym, Q);
-                if (const char *env = std::getenv("KMER_B200_HOST_RAW_PCT")) raw_pct = (uint32_t)std::max(0, std::min(100, std::atoi(env)));
-            }
-            const int s = search_batch_host_stream(ix, q_ranks, q_offsets, Q, mode, raw_pct, out);
-            if (s != KMER_B200_ERR_UNSUPPORTED) {
-                ix->last_host_path = 3, ix->last_raw_pct = raw_pct, ix->last_pack_gbs = rate / 1e9;
-                return s;
-            }
+        if (const char *env = std::getenv("KMER_B200_HOST_RAW_PCT")) raw_pct = (uint32_t)std::max(0, std::min(100, std::atoi(env)));
+        int s = search_batch_host_chunked(ix, q_ranks, q_offsets, Q, mode, raw_pct, out);
+        if (s == KMER_B200_ERR_UNSUPPORTED && raw_pct < 100) {  // a packed chunk refused its queries: every chunk raw
+            raw_pct = 100;
+            s = search_batch_host_chunked(ix, q_ranks, q_offsets, Q, mode, raw_pct, out);
         }
-        if (forced >= 0) pageable = forced == 1;
-        if (pageable) {
-            const int s = search_batch_host_packed(ix, q_ranks, q_offsets, Q, mode, out);
-            ix->last_host_path = 2, ix->last_raw_pct = 0, ix->last_pack_gbs = 0;
-            if (s != KMER_B200_ERR_UNSUPPORTED) return s;  // queries longer than 16 packed words: the unpacked pipeline
+        if (s != KMER_B200_ERR_UNSUPPORTED) {
+            ix->last_host_path = 3, ix->last_raw_pct = raw_pct, ix->last_pack_gbs = rate / 1e9;
+            return s;
         }
-        ix->last_host_path = 1, ix->last_raw_pct = 100, ix->last_pack_gbs = 0;
-        return search_batch_host_pipelined(ix, q_ranks, q_offsets, Q, mode, out);
+        // no producer thread to be had: one copy each way
     }
     return search_batch_host_single_copy(ix, q_ranks, q_offsets, Q, mode, lut256, -1, out);
 }
@@ -3832,28 +3461,10 @@ static int search_batch_multi(kmer_b200_index *group, const uint8_t *q_ranks, co
             free_parts();
             return fail(code, msg);
         }
-    kmer_b200_result *res = new (std::nothrow) kmer_b200_result();
-    if (!res) {
-        free_parts();
-        return fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation failed");
-    }
-    res->index = group;
-    res->on_device = false;
-    res->n_queries = Q;
     std::vector<uint64_t> p0(N + 1, 0);
     for (uint32_t i = 0; i < N; ++i) p0[i + 1] = p0[i] + part[i]->n_positions;
-    res->n_positions = p0[N];
-    res->offsets = (uint64_t *)pinned_get((Q + 1) * sizeof(uint64_t), &res->cap_offsets);
-    res->status = (uint8_t *)pinned_get(Q, &res->cap_status);
-    const size_t pos_bytes = p0[N] * sizeof(uint32_t);
-    if (pos_bytes > (8ull << 30)) {
-        res->positions = (uint32_t *)std::malloc(pos_bytes);
-        res->positions_pageable = true;
-        res->cap_positions = pos_bytes;
-    } else {
-        res->positions = (uint32_t *)pinned_get(pos_bytes, &res->cap_positions);
-    }
-    if (!res->offsets || !res->status || !res->positions) {
+    kmer_b200_result *res = host_result_new(group, Q);
+    if (!res || !host_result_positions(res, p0[N])) {
         free_parts();
         kmer_b200_result_free(res);
         return fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation failed");

@@ -109,28 +109,8 @@ inline uint64_t pack8(uint64_t v) {
 #endif
 }
 
+// ---- streaming pack: a contiguous run of ranks -> words, query boundaries ignored ---------------------------------
 #if defined(__AVX2__)
-alignas(32) static const uint8_t kTailMask[64] = {
-    0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF,
-    0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF, 0xFF};  // then 32 zeros
-
-// the first min(left, 32) bytes of a 32-byte load kept, the rest zeroed
-static inline __m256i keep_first(__m256i v, uint32_t left) {
-    const uint32_t keep = left < 32 ? left : 32;
-    return _mm256_and_si256(v, _mm256_loadu_si256(reinterpret_cast<const __m256i *>(kTailMask + 32 - keep)));
-}
-
-// 32 two-bit ranks (one per byte) -> 64 bits, symbol 0 in the top two bits: two multiply-adds merge neighbours
-// (4 a + b, then 16 x + y), a byte shuffle collects the eight finished bytes
-static inline uint64_t pack32x2(__m256i v) {
-    const __m256i x = _mm256_maddubs_epi16(v, _mm256_set1_epi16(0x0104));
-    const __m256i y = _mm256_madd_epi16(x, _mm256_set1_epi32(0x00010010));
-    const __m256i sh = _mm256_setr_epi8(12, 8, 4, 0, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, 12, 8, 4, 0, -1, -1, -1, -1, -1,
-                                        -1, -1, -1, -1, -1, -1, -1);
-    const __m256i z = _mm256_shuffle_epi8(y, sh);
-    return ((uint64_t)(uint32_t)_mm256_extract_epi32(z, 0) << 32) | (uint32_t)_mm256_extract_epi32(z, 4);
-}
-
 // 32 four-bit ranks -> two 64-bit words (16 symbols each)
 static inline void pack32x4(__m256i v, uint64_t &w0, uint64_t &w1) {
     const __m256i x = _mm256_maddubs_epi16(v, _mm256_set1_epi16(0x0110));  // 16 a + b in every 16-bit lane
@@ -140,103 +120,7 @@ static inline void pack32x4(__m256i v, uint64_t &w0, uint64_t &w1) {
     w0 = (uint64_t)_mm256_extract_epi64(z, 0);
     w1 = (uint64_t)_mm256_extract_epi64(z, 2);
 }
-#endif
 
-// `safe_end`: reading at any address below it is inside the caller's buffer (a query's last chunk is fetched with one
-// unconditional wide load and masked, instead of a variable-length copy)
-template <int BITS>
-bool pack_range(const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t q_begin, uint64_t lo, uint64_t hi, uint32_t sigma,
-                uint32_t stride, uint64_t *words, const uint8_t *safe_end) {
-    constexpr uint32_t SPW = 64 / BITS;  // symbols per word
-    constexpr uint32_t CPW = SPW / 8;    // 8-symbol chunks per word
-    const uint64_t guard = (uint64_t)(0x80u - (sigma > 128 ? 128u : sigma)) * 0x0101010101010101ull;
-    uint64_t inval = 0;  // bit 7 of a byte ends up set <=> that rank is >= sigma (sigma <= 128)
-    bool bad = false;
-#if defined(__AVX2__)
-    __m256i vmax = _mm256_setzero_si256();  // largest rank seen (BITS 2 / 4 paths)
-#endif
-    uint64_t off = q_offsets[lo];
-    for (uint64_t i = lo; i < hi; ++i) {
-        const uint64_t next = q_offsets[i + 1];
-        const uint8_t *src = q_ranks + off;
-        const uint32_t m = (uint32_t)(next - off);
-        off = next;
-        uint64_t *dst = words + (i - q_begin) * stride;
-        const uint32_t n_words = (m + SPW - 1) / SPW;
-        uint32_t w = 0;
-#if defined(__AVX2__)
-        if ((BITS == 2 || BITS == 4) && src + (size_t)n_words * SPW + 32 <= safe_end) {
-            if (BITS == 2) {
-                for (; w < n_words; ++w) {
-                    __m256i v = _mm256_loadu_si256(reinterpret_cast<const __m256i *>(src + 32 * w));
-                    v = keep_first(v, m - 32 * w);
-                    vmax = _mm256_max_epu8(vmax, v);
-                    dst[w] = pack32x2(v);
-                }
-            } else {
-                for (uint32_t s = 0; s < m; s += 32) {
-                    __m256i v = _mm256_loadu_si256(reinterpret_cast<const __m256i *>(src + s));
-                    v = keep_first(v, m - s);
-                    vmax = _mm256_max_epu8(vmax, v);
-                    uint64_t a, b;
-                    pack32x4(v, a, b);
-                    dst[w++] = a;
-                    if (w < n_words) dst[w++] = b;
-                }
-            }
-        } else
-#endif
-        if (src + (size_t)n_words * SPW + 8 <= safe_end) {
-            // branch-free per word: always CPW 8-byte loads (those behind the query's end are masked to zero; they stay
-            // inside the batch buffer), one PEXT each
-            for (; w < n_words; ++w) {
-                const uint8_t *p = src + w * SPW;
-                const int32_t left = (int32_t)(m - w * SPW);  // symbols of the query from this word on, >= 1
-                uint64_t acc = 0;
-#pragma GCC unroll 8
-                for (uint32_t c = 0; c < CPW; ++c) {
-                    uint64_t v;
-                    std::memcpy(&v, p + 8 * c, 8);
-                    const int32_t l = left - (int32_t)(8 * c);
-                    const uint64_t keep = l >= 8 ? ~0ull : (l <= 0 ? 0ull : ((1ull << (8 * l)) - 1));
-                    v &= keep;
-                    inval |= (v + guard) | v;
-                    acc |= pack8<BITS>(v) << (64 - 8 * BITS * (c + 1));
-                }
-                dst[w] = acc;
-            }
-        } else {  // the last few queries of the batch: byte by byte
-            for (; w < n_words; ++w) {
-                uint64_t acc = 0;
-                for (uint32_t c = 0; c < CPW; ++c) {
-                    uint64_t v = 0;
-                    for (uint32_t j = 0; j < 8; ++j) {
-                        const uint32_t sidx = w * SPW + 8 * c + j;
-                        if (sidx < m) v |= (uint64_t)src[sidx] << (8 * j);
-                    }
-                    inval |= (v + guard) | v;
-                    acc |= pack8<BITS>(v) << (64 - 8 * BITS * (c + 1));
-                }
-                dst[w] = acc;
-            }
-        }
-        for (; w < stride; ++w) dst[w] = 0;
-        if (sigma > 128)
-            for (uint32_t j = 0; j < m; ++j) bad |= src[j] >= sigma;
-    }
-    if (sigma <= 128) bad = (inval & 0x8080808080808080ull) != 0;
-#if defined(__AVX2__)
-    {
-        alignas(32) uint8_t mx[32];
-        _mm256_store_si256(reinterpret_cast<__m256i *>(mx), vmax);
-        for (int j = 0; j < 32; ++j) bad |= mx[j] >= sigma;
-    }
-#endif
-    return !bad;
-}
-
-// ---- streaming pack: a contiguous run of ranks -> words, query boundaries ignored ---------------------------------
-#if defined(__AVX2__)
 // 128 two-bit ranks -> four words: per 32-byte vector two multiply-adds leave one finished byte (4 symbols, the first on
 // top) in every 32-bit lane; two saturating packs bring the 32 finished bytes of four vectors together, a byte shuffle
 // and a lane permutation put them in word order (byte 7 - l of word t = symbols 4 l .. 4 l + 3 of vector t)
@@ -278,6 +162,15 @@ bool pack_stream_range(const uint8_t *ranks, uint64_t n, uint32_t sigma, uint64_
             vmax = _mm256_max_epu8(vmax, v);
             pack32x4(v, words[w], words[w + 1]);
         }
+    } else {
+        // 8 bits: a word is its 8 ranks with the byte order reversed (symbol 0 on top)
+        const __m256i rev = _mm256_setr_epi8(7, 6, 5, 4, 3, 2, 1, 0, 15, 14, 13, 12, 11, 10, 9, 8, 7, 6, 5, 4, 3, 2, 1, 0, 15, 14, 13,
+                                             12, 11, 10, 9, 8);
+        for (; w + 4 <= full_hi; w += 4) {
+            const __m256i v = _mm256_loadu_si256(reinterpret_cast<const __m256i *>(ranks + w * 8));
+            vmax = _mm256_max_epu8(vmax, v);
+            _mm256_storeu_si256(reinterpret_cast<__m256i *>(words + w), _mm256_shuffle_epi8(v, rev));
+        }
     }
     {
         alignas(32) uint8_t mx[32];
@@ -316,16 +209,6 @@ bool pack_stream_host(const uint8_t *ranks, uint64_t n, uint32_t bits, uint32_t 
     if (bits == 2) return pack_stream_range<2>(ranks, n, sigma, words, w_lo, w_hi);
     if (bits == 4) return pack_stream_range<4>(ranks, n, sigma, words, w_lo, w_hi);
     return pack_stream_range<8>(ranks, n, sigma, words, w_lo, w_hi);
-}
-
-bool pack_queries_host(const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t q_begin, uint64_t q_end, uint32_t bits,
-                       uint32_t sigma, uint32_t stride, uint64_t *words, unsigned part, unsigned n_parts) {
-    const uint64_t n = q_end - q_begin;
-    const uint64_t lo = q_begin + n * part / n_parts, hi = q_begin + n * (part + 1) / n_parts;
-    const uint8_t *safe_end = q_ranks + q_offsets[q_end];  // the batch's last byte + 1 (the buffer may end there)
-    if (bits == 2) return pack_range<2>(q_ranks, q_offsets, q_begin, lo, hi, sigma, stride, words, safe_end);
-    if (bits == 4) return pack_range<4>(q_ranks, q_offsets, q_begin, lo, hi, sigma, stride, words, safe_end);
-    return pack_range<8>(q_ranks, q_offsets, q_begin, lo, hi, sigma, stride, words, safe_end);
 }
 
 }  // namespace kb

@@ -1,5 +1,5 @@
-// Host-side helpers of the C ABI's host-buffer search (capi.cu): a small persistent thread pool and the packing of
-// query batches (1 byte per rank -> the device's b-bit MSB-first words) before they cross PCIe.
+// Host-side helpers of the C ABI's host-buffer search (capi.cu): a small persistent thread pool, the query lengths and the
+// streaming pack of query batches and texts (1 byte per rank -> the device's b-bit MSB-first words) before they cross PCIe.
 #pragma once
 
 #include <cstdint>
@@ -26,15 +26,10 @@ class HostPool {
     Impl *impl_;
 };
 
-// Queries [q_begin, q_end) of a host batch: lens[i - q_begin] = length (must fit 16 bits) and the longest length.
+// Queries [q_begin, q_end) of a host batch: lens[i - q_begin] = length (its low 16 bits: valid when the returned longest
+// length is below 65 536) and the longest length.
 uint64_t query_lengths_host(const uint64_t *q_offsets, uint64_t q_begin, uint64_t q_end, uint16_t *lens, unsigned part,
                             unsigned n_parts);
-// Packs the same queries: word j of query i at words[(i - q_begin) * stride + j], symbol s of a query in bits
-// [64 - bits (s % spw + 1), 64 - bits (s % spw)) of word s / spw (spw = 64 / bits); unused words are zero.
-// Returns false when a rank >= sigma was seen. `part` of `n_parts`: the slice of the queries this call handles.
-bool pack_queries_host(const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t q_begin, uint64_t q_end, uint32_t bits,
-                       uint32_t sigma, uint32_t stride, uint64_t *words, unsigned part, unsigned n_parts);
-
 
 // Streaming pack of a contiguous run of n ranks, query boundaries ignored: symbol s lands in bits
 // [64 - bits (s % spw + 1), 64 - bits (s % spw)) of words[s / spw]; the unused low bits of the last word are zero. The

@@ -1,5 +1,6 @@
-"""Config 5 through the host C ABI (kmer_b200_search_batch, kmer_b200_create) under each host pipeline: which one is
-the fastest on this box, and how the share of raw chunks moves the time. Prints one line per setting.
+"""Config 5 through the host C ABI (kmer_b200_search_batch, kmer_b200_create) under each share of raw chunks
+(KMER_B200_HOST_RAW_PCT), pinned and pageable, and a sigma-27 batch of as many queries: which share is the fastest on
+this box. Prints one line per setting.
 usage: python profiles/tools/host_path_sweep.py [text_symbols] [queries]"""
 import os
 import sys
@@ -35,8 +36,7 @@ torch.cuda.synchronize()
 
 
 def run(label, env, qa, oa, reps=3):
-    for k in ("KMER_B200_HOST_PACK", "KMER_B200_HOST_RAW_PCT"):
-        os.environ.pop(k, None)
+    os.environ.pop("KMER_B200_HOST_RAW_PCT", None)
     os.environ.update(env)
     best, fp = 1e30, None
     for _ in range(reps + 1):
@@ -51,16 +51,33 @@ def run(label, env, qa, oa, reps=3):
 
 
 run("pinned, default", {}, h_q.numpy(), h_off.numpy())
-run("pinned, raw chunks only (round-2 start)", {"KMER_B200_HOST_PACK": "0"}, h_q.numpy(), h_off.numpy())
-run("pinned, streaming pack only", {"KMER_B200_HOST_PACK": "2"}, h_q.numpy(), h_off.numpy())
+run("pinned, raw chunks only (round-2 start)", {"KMER_B200_HOST_RAW_PCT": "100"}, h_q.numpy(), h_off.numpy())
+run("pinned, streaming pack only", {"KMER_B200_HOST_RAW_PCT": "0"}, h_q.numpy(), h_off.numpy())
 for pct in (20, 30, 40, 50, 60):
-    run(f"pinned, streaming pack + {pct} % raw", {"KMER_B200_HOST_PACK": "3", "KMER_B200_HOST_RAW_PCT": str(pct)}, h_q.numpy(), h_off.numpy())
-run("pinned, per-query pack", {"KMER_B200_HOST_PACK": "1"}, h_q.numpy(), h_off.numpy(), reps=1)
+    run(f"pinned, streaming pack + {pct} % raw", {"KMER_B200_HOST_RAW_PCT": str(pct)}, h_q.numpy(), h_off.numpy())
 run("pageable, default (streaming pack)", {}, p_q, p_off)
-run("pageable, per-query pack", {"KMER_B200_HOST_PACK": "1"}, p_q, p_off, reps=1)
-run("pageable, raw chunks (driver-staged copies)", {"KMER_B200_HOST_PACK": "0"}, p_q, p_off, reps=1)
-for k in ("KMER_B200_HOST_PACK", "KMER_B200_HOST_RAW_PCT"):
-    os.environ.pop(k, None)
+run("pageable, raw chunks (driver-staged copies)", {"KMER_B200_HOST_RAW_PCT": "100"}, p_q, p_off, reps=1)
+os.environ.pop("KMER_B200_HOST_RAW_PCT", None)
+ix.close()
+del text
+
+# sigma 27 (8-bit words: packing saves no link bytes): the same query lengths over a 200 Mbp text, k = 5
+n27 = min(n, 200_000_000)
+text = torch.empty(n27, dtype=torch.uint8, device=dev)
+_capi.check(L.kmer_b200_synth_ranks_device(text.data_ptr(), n27, 0, 27, 206, None))
+q = torch.from_numpy(p_q).to(dev)
+_capi.check(L.kmer_b200_synth_ranks_device(q.data_ptr(), n_sym, 0, 27, 1240, None))
+torch.cuda.synchronize()
+h_q.copy_(q.cpu())
+p_q = h_q.numpy().copy()
+del q
+ix = kb.KmerIndex(None, 27, [5], text_device_ptr=text.data_ptr(), n=n27)
+torch.cuda.synchronize()
+run("sigma 27 pinned, default (raw chunks)", {}, h_q.numpy(), h_off.numpy())
+run("sigma 27 pinned, streaming pack only", {"KMER_B200_HOST_RAW_PCT": "0"}, h_q.numpy(), h_off.numpy())
+run("sigma 27 pageable, default (streaming pack)", {}, p_q, p_off)
+run("sigma 27 pageable, raw chunks (driver-staged copies)", {"KMER_B200_HOST_RAW_PCT": "100"}, p_q, p_off, reps=1)
+os.environ.pop("KMER_B200_HOST_RAW_PCT", None)
 ix.close()
 del text
 if os.environ.get("SWEEP_NO_BUILD"):

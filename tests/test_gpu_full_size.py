@@ -123,7 +123,7 @@ def test_pipelined_text_upload_equals_plain(kb, sigma, k):
         del os.environ["KMER_B200_HOST_RAW_PCT"]
 
 
-def test_pipelined_host_batch_equals_plain(kb):
+def test_chunked_host_batch_equals_plain(kb):
     """Host batches >= 256 MiB are searched in pipelined chunks (H2D / search / D2H overlapped); the result must be
     the plain path's, offsets included."""
     import os
@@ -147,7 +147,6 @@ def test_pipelined_host_batch_equals_plain(kb):
         mixed_auto = ix.search_batch(pin_q.numpy(), pin_off.numpy()).as_tuple()
         path_auto = ix.last_search_host_path()
         assert path_auto["pipeline"].startswith("streaming") and path_auto["host_pack_gbs"] > 0, path_auto
-        os.environ["KMER_B200_HOST_PACK"] = "3"
         mixed = {}
         try:
             for pct in (0, 30, 50, 100):
@@ -162,34 +161,28 @@ def test_pipelined_host_batch_equals_plain(kb):
                     ix.search_batch(torch.from_numpy(bad).pin_memory().numpy(), pin_off.numpy())
                 assert e.value.code == -4
                 bad[at] = q[at]
-            os.environ["KMER_B200_HOST_PACK"] = "1"
-            packed_per_query = ix.search_batch(q, off).as_tuple()   # round 2's first host packer: query by query
-            assert ix.last_search_host_path()["pipeline"].startswith("per-query")
-        finally:
-            os.environ.pop("KMER_B200_HOST_PACK", None)
-            os.environ.pop("KMER_B200_HOST_RAW_PCT", None)
-        os.environ["KMER_B200_HOST_PACK"] = "0"
-        try:
+            os.environ["KMER_B200_HOST_RAW_PCT"] = "100"
             piped = ix.search_batch(q, off).as_tuple()       # 1-byte ranks over PCIe, chunks pipelined
             # the offsets crossed the link as 16-bit lengths
             assert ix.last_search_transfer()[0] == q.size + 2 * (off.size - 1)
-            os.environ["KMER_B200_NO_LENS16"] = "1"
-            piped_off = ix.search_batch(q, off).as_tuple()   # ... and as they are
-            assert ix.last_search_transfer()[0] == q.size + 8 * (off.size - 1 + 8)
-            del os.environ["KMER_B200_NO_LENS16"]
-            # a query of 65 536 symbols or more: its chunk sends offsets, the other chunks lengths (CORRECT mode: the
-            # reference's table stops at 10 000 symbols)
+            # a query of 65 536 symbols or more: its chunk (the last one of 24) sends its offsets, the other chunks
+            # lengths (CORRECT mode: the reference's table stops at 10 000 symbols)
             q_long = np.concatenate([q, text[1000:71_000]])
             off_long = np.concatenate([off, [off[-1] + 70_000]]).astype(np.uint64)
             piped_long = ix.search_batch(q_long, off_long, mode=kb.MODE_CORRECT).as_tuple()
+            n_long = off_long.size - 1
+            last = n_long - 23 * -(-n_long // 24)
+            assert ix.last_search_transfer()[0] == q_long.size + 2 * (n_long - last) + 8 * (last + 1)
         finally:
-            os.environ.pop("KMER_B200_HOST_PACK", None)
-            os.environ.pop("KMER_B200_NO_LENS16", None)
-        # the same long query through the default choice: the streaming pipeline refuses the batch part-way (its lengths
-        # travel as 16 bits), the per-query packer refuses it too (> 16 words), the raw-chunk pipeline answers
+            os.environ.pop("KMER_B200_HOST_RAW_PCT", None)
+        # the same long query through the default choice. Pageable: the packed chunk that holds it refuses the batch
+        # (its lengths travel as 16 bits), which is searched again with every chunk raw
         default_long = ix.search_batch(q_long, off_long, mode=kb.MODE_CORRECT).as_tuple()
-        assert ix.last_search_host_path()["pipeline"] == "raw chunks"
+        path_long = ix.last_search_host_path()
+        assert path_long["pipeline"].startswith("streaming") and path_long["raw_chunk_pct"] == 100, path_long
+        # pinned: the same unless the long query's chunk is one of the raw chunks
         pinned_long = ix.search_batch(torch.from_numpy(q_long).pin_memory().numpy(), off_long, mode=kb.MODE_CORRECT).as_tuple()
+        assert ix.last_search_host_path()["pipeline"].startswith("streaming")
         os.environ["KMER_B200_NO_PIPELINE"] = "1"
         try:
             plain = ix.search_batch(q, off).as_tuple()
@@ -203,16 +196,57 @@ def test_pipelined_host_batch_equals_plain(kb):
         assert e.value.code == -4
     assert piped[1].size > 500_000
     assert_results_equal(piped, plain, label="pipelined vs plain")
-    assert_results_equal(piped_off, plain, label="pipelined (offsets as they are) vs plain")
     assert plain_long[0][-1] - plain_long[0][-2] == 1          # the long query occurs once, at position 1000
     assert_results_equal(piped_long, plain_long, label="pipelined with a 70 000-symbol query vs plain")
     assert_results_equal(default_long, plain_long, label="default pipeline choice with a 70 000-symbol query vs plain")
     assert_results_equal(pinned_long, plain_long, label="default pipeline choice, pinned, with a 70 000-symbol query vs plain")
     assert_results_equal(packed, plain, label="stream-packed pipeline (pageable input) vs plain")
-    assert_results_equal(packed_per_query, plain, label="per-query host-packed pipeline vs plain")
     assert_results_equal(mixed_auto, plain, label=f"stream-packed + raw chunks ({path_auto}) vs plain")
     for pct, got in mixed.items():
         assert_results_equal(got, plain, label=f"stream-packed + {pct} % raw chunks vs plain")
+
+
+def test_chunked_host_batch_8bit_equals_plain(kb):
+    """An 8-bit alphabet (sigma 27) through the chunked pipeline: pageable input packed as a stream on the host threads
+    (a byte reversal per word), pinned input sent as 1-byte ranks. Both must give the plain path's result, and a rank
+    >= sigma must be reported from either."""
+    import os
+
+    import torch
+
+    from kmer_index_b200 import synth
+    sigma = 27
+    text = synth.random_text(20_000_000, sigma, TEXT_SEED + 7)
+    q1, off1 = synth.random_queries(3_000_000, 12, 100, sigma, QUERY_SEED + 7)
+    q2, off2 = _planted(text, 3_000_000, 12, 100, QUERY_SEED + 8)
+    q = np.concatenate([q1, q2])
+    off = np.concatenate([off1, off2[1:] + off1[-1]])
+    assert q.size + 17 * (off.size - 1) >= (256 << 20)
+    pin_q = torch.from_numpy(q).pin_memory()
+    with kb.KmerIndex(text, sigma, [5]) as ix:
+        pageable = ix.search_batch(q, off).as_tuple()
+        path = ix.last_search_host_path()
+        assert path["pipeline"].startswith("streaming") and path["raw_chunk_pct"] == 0, path
+        assert ix.last_search_transfer()[0] < q.size + 2 * (off.size - 1) + 4096
+        pinned = ix.search_batch(pin_q.numpy(), off).as_tuple()
+        path = ix.last_search_host_path()
+        assert path["pipeline"].startswith("streaming") and path["raw_chunk_pct"] == 100, path
+        assert ix.last_search_transfer()[0] == q.size + 2 * (off.size - 1)
+        os.environ["KMER_B200_NO_PIPELINE"] = "1"
+        try:
+            plain = ix.search_batch(q, off).as_tuple()
+        finally:
+            del os.environ["KMER_B200_NO_PIPELINE"]
+        for at in (3, q.size // 2, q.size - 1):
+            bad = q.copy()
+            bad[at] = sigma
+            for label, src in (("pageable", bad), ("pinned", torch.from_numpy(bad).pin_memory().numpy())):
+                with pytest.raises(kb.KmerB200Error) as e:
+                    ix.search_batch(src, off)
+                assert e.value.code == -4, (label, at)
+    assert plain[1].size > 500_000
+    assert_results_equal(pageable, plain, label="sigma 27, stream-packed chunks (pageable input) vs plain")
+    assert_results_equal(pinned, plain, label="sigma 27, raw chunks (pinned input) vs plain")
 
 
 def test_config3_full_text_counts_and_subsample(kb, oracle_mod):
