@@ -208,6 +208,47 @@ int kmer_b200_count_approx_batch_device(kmer_b200_index *index, const uint8_t *d
                                         uint64_t n_queries, uint64_t max_query_len, uint32_t max_mismatches,
                                         kmer_b200_result **out);
 
+/* ---- hit strategies of approximate search (the seqan3 search_cfg::hit_* choices). With d(p) = the Hamming distance
+   between T[p, p+m) and the query, H = the hits of kmer_b200_search_approx_batch and d_min = the smallest d(p) over H:
+     KMER_B200_HITS_ALL          H
+     KMER_B200_HITS_ALL_BEST     the p in H with d(p) = d_min
+     KMER_B200_HITS_SINGLE_BEST  the one p in H with the smallest (d(p), p): ties go to the lowest position
+     KMER_B200_HITS_STRATA       the p in H with d(p) <= min(e, d_min + strata); strata = 0 is ALL_BEST, >= e is ALL
+   Positions are ascending per query; an empty H gives no hits under every strategy. A query of m <= e symbols has
+   d_min < m if some window is within m - 1 substitutions, else d_min = m (every window; none when m > n). Statuses as
+   for kmer_b200_search_approx_batch. Every strategy other than ALL runs a best pass first (budget min(e, m - 1) per
+   query); ALL_BEST and STRATA then search the queries that have hits again, each with budget min(e, d_min + strata).
+   The result carries kmer_b200_result_best_distances (u8[Q]: d_min, 0xFF where H is empty or the status is not OK)
+   for every strategy other than ALL, and kmer_b200_result_distances (u8[n_positions]: d(p) of each position, in the
+   same order) when KMER_B200_APPROX_DISTANCES is set (the count-only form ignores it). KMER_B200_ERR_INVALID_ARGUMENT
+   for null options, e > 8, an unknown strategy or unknown flag bits; the handles kmer_b200_search_approx_batch refuses
+   are refused the same way. Host batches are staged in one copy; kmer_b200_last_search_transfer counts the two
+   arrays. */
+typedef enum kmer_b200_approx_hits {
+    KMER_B200_HITS_ALL = 0,
+    KMER_B200_HITS_ALL_BEST = 1,
+    KMER_B200_HITS_SINGLE_BEST = 2,
+    KMER_B200_HITS_STRATA = 3
+} kmer_b200_approx_hits;
+
+enum { KMER_B200_APPROX_DISTANCES = 1 }; /* kmer_b200_approx_options.flags */
+
+typedef struct kmer_b200_approx_options {
+    uint32_t max_mismatches; /* e <= 8 */
+    uint32_t hits;           /* kmer_b200_approx_hits */
+    uint32_t strata;         /* s, KMER_B200_HITS_STRATA only */
+    uint32_t flags;          /* KMER_B200_APPROX_DISTANCES: return d(p) per hit (ignored by the count-only form) */
+} kmer_b200_approx_options;
+
+int kmer_b200_search_approx_batch_ex(kmer_b200_index *index, const uint8_t *q_ranks, const uint64_t *q_offsets,
+                                     uint64_t n_queries, const kmer_b200_approx_options *options, kmer_b200_result **out);
+int kmer_b200_search_approx_batch_device_ex(kmer_b200_index *index, const uint8_t *d_q_ranks, const uint64_t *d_q_offsets,
+                                            uint64_t n_queries, uint64_t max_query_len,
+                                            const kmer_b200_approx_options *options, kmer_b200_result **out);
+int kmer_b200_count_approx_batch_device_ex(kmer_b200_index *index, const uint8_t *d_q_ranks, const uint64_t *d_q_offsets,
+                                           uint64_t n_queries, uint64_t max_query_len,
+                                           const kmer_b200_approx_options *options, kmer_b200_result **out);
+
 uint64_t kmer_b200_result_n_queries(const kmer_b200_result *r);
 uint64_t kmer_b200_result_n_positions(const kmer_b200_result *r);
 int kmer_b200_result_on_device(const kmer_b200_result *r);
@@ -219,6 +260,8 @@ const uint32_t *kmer_b200_result_hit_queries(const kmer_b200_result *r);
 const uint64_t *kmer_b200_result_offsets(const kmer_b200_result *r);   /* [Q+1] */
 const uint32_t *kmer_b200_result_positions(const kmer_b200_result *r); /* [offsets[Q]], NULL if count-only */
 const uint8_t *kmer_b200_result_status(const kmer_b200_result *r);     /* [Q] */
+const uint8_t *kmer_b200_result_distances(const kmer_b200_result *r);      /* [n_positions] or NULL (approximate search) */
+const uint8_t *kmer_b200_result_best_distances(const kmer_b200_result *r); /* [Q] or NULL (approximate search) */
 void kmer_b200_result_free(kmer_b200_result *r);
 
 /* ---- sharded (multi-GPU) search, two phases around one cross-rank exchange.

@@ -246,6 +246,10 @@ namespace kmer
         detail::array_view<std::uint64_t> offsets;   // [n_queries + 1]
         positions_t positions;                       // ascending per query
         detail::array_view<std::uint8_t> status;     // kmer_b200_query_status per query
+        // approximate search with a hit strategy (empty otherwise): the Hamming distance of each position (same order),
+        // when asked for, and d_min per query (0xFF without a hit) for every strategy but approx_hits::all()
+        detail::array_view<std::uint8_t> distances;
+        detail::array_view<std::uint8_t> best_distance;
 
         std::size_t size() const noexcept { return status.size(); }
         bool threw(std::size_t i) const { return status[i] == KMER_B200_QUERY_THROW_INVALID_ARGUMENT; }
@@ -261,6 +265,8 @@ namespace kmer
             const std::uint64_t n_q = kmer_b200_result_n_queries(r), n_p = kmer_b200_result_n_positions(r);
             offsets = {kmer_b200_result_offsets(r), std::size_t(n_q + 1)};
             status = {kmer_b200_result_status(r), std::size_t(n_q)};
+            if (kmer_b200_result_distances(r)) distances = {kmer_b200_result_distances(r), std::size_t(n_p)};
+            if (kmer_b200_result_best_distances(r)) best_distance = {kmer_b200_result_best_distances(r), std::size_t(n_q)};
             if constexpr (std::is_same_v<position_t, std::uint32_t>)
                 positions = {kmer_b200_result_positions(r), std::size_t(n_p)};
             else if (n_p)
@@ -269,6 +275,19 @@ namespace kmer
 
     private:
         std::shared_ptr<kmer_b200_result> _owner;
+    };
+
+    // which hits of an approximate search (search_approx_batch): the seqan3 search_cfg::hit_all / hit_all_best /
+    // hit_single_best / hit_strata{s} choices (kmer_b200_approx_hits)
+    struct approx_hits
+    {
+        std::uint32_t strategy = KMER_B200_HITS_ALL;  // kmer_b200_approx_hits
+        std::uint32_t s = 0;                          // strata(s) only
+
+        static constexpr approx_hits all() noexcept { return {KMER_B200_HITS_ALL, 0}; }
+        static constexpr approx_hits all_best() noexcept { return {KMER_B200_HITS_ALL_BEST, 0}; }
+        static constexpr approx_hits single_best() noexcept { return {KMER_B200_HITS_SINGLE_BEST, 0}; }
+        static constexpr approx_hits strata(std::uint32_t s) noexcept { return {KMER_B200_HITS_STRATA, s}; }
     };
 
     // tag for the shared-positions constructor below
@@ -451,9 +470,48 @@ namespace kmer
         template<std::ranges::range queries_t>
         kmer_batch_result<position_t> search_approx_batch(queries_t const& queries, std::uint32_t max_mismatches) const
         {
-            using query_t = std::remove_cvref_t<std::ranges::range_reference_t<queries_t const>>;
             std::vector<std::uint8_t> ranks;
             std::vector<std::uint64_t> offsets{0};
+            gather_ranks(queries, ranks, offsets);
+            kmer_b200_result* r = nullptr;
+            detail::check(kmer_b200_search_approx_batch(_handle, ranks.data(), offsets.data(), offsets.size() - 1, max_mismatches, &r));
+            return kmer_batch_result<position_t>(r);
+        }
+
+        // Approximate search with a hit strategy (kmer_b200_search_approx_batch_ex): approx_hits::all() (every hit),
+        // all_best() (the hits at the smallest distance d_min), single_best() (the lowest such position) or strata(s)
+        // (distance <= min(max_mismatches, d_min + s)). The result's best_distance holds d_min per query (not for all()),
+        // and `distances` the Hamming distance of every position when asked for.
+        template<std::ranges::range queries_t>
+        kmer_batch_result<position_t> search_approx_batch(queries_t const& queries, std::uint32_t max_mismatches, approx_hits hits,
+                                                          bool distances = false) const
+        {
+            std::vector<std::uint8_t> ranks;
+            std::vector<std::uint64_t> offsets{0};
+            gather_ranks(queries, ranks, offsets);
+            kmer_b200_approx_options opt{max_mismatches, hits.strategy, hits.s, distances ? std::uint32_t(KMER_B200_APPROX_DISTANCES) : 0u};
+            kmer_b200_result* r = nullptr;
+            detail::check(kmer_b200_search_approx_batch_ex(_handle, ranks.data(), offsets.data(), offsets.size() - 1, &opt, &r));
+            return kmer_batch_result<position_t>(r);
+        }
+
+        // one query: its positions within max_mismatches substitutions, ascending; throws for an empty query
+        std::vector<position_t> search_approx(std::vector<alphabet_t> const& query, std::uint32_t max_mismatches) const
+        {
+            std::array<std::vector<alphabet_t> const*, 1> one{&query};
+            auto deref = one | std::views::transform([](auto const* p) -> std::vector<alphabet_t> const& { return *p; });
+            auto batch = search_approx_batch(deref, max_mismatches);
+            if (batch.status[0] != KMER_B200_QUERY_OK)
+                throw std::invalid_argument("approximate search of an empty query is undefined");
+            return std::vector<position_t>(batch.positions.begin(), batch.positions.end());
+        }
+
+    private:
+        // a batch as one rank buffer and its offsets (a copy of the bytes when the queries hold their ranks in place)
+        template<std::ranges::range queries_t>
+        static void gather_ranks(queries_t const& queries, std::vector<std::uint8_t>& ranks, std::vector<std::uint64_t>& offsets)
+        {
+            using query_t = std::remove_cvref_t<std::ranges::range_reference_t<queries_t const>>;
             for (auto const& q : queries)
             {
                 if constexpr (detail::ranks_in_place<query_t>)
@@ -468,21 +526,9 @@ namespace kmer
                 }
                 offsets.push_back(ranks.size());
             }
-            kmer_b200_result* r = nullptr;
-            detail::check(kmer_b200_search_approx_batch(_handle, ranks.data(), offsets.data(), offsets.size() - 1, max_mismatches, &r));
-            return kmer_batch_result<position_t>(r);
         }
 
-        // one query: its positions within max_mismatches substitutions, ascending; throws for an empty query
-        std::vector<position_t> search_approx(std::vector<alphabet_t> const& query, std::uint32_t max_mismatches) const
-        {
-            std::array<std::vector<alphabet_t> const*, 1> one{&query};
-            auto deref = one | std::views::transform([](auto const* p) -> std::vector<alphabet_t> const& { return *p; });
-            auto batch = search_approx_batch(deref, max_mismatches);
-            if (batch.status[0] != KMER_B200_QUERY_OK)
-                throw std::invalid_argument("approximate search of an empty query is undefined");
-            return std::vector<position_t>(batch.positions.begin(), batch.positions.end());
-        }
+    public:
 
         // kmer_index_element::search_k (kmer_index.hpp:182-190): the bucket of the k symbols starting at `it`, for one
         // of the index's ks; empty when the k-mer does not occur (the reference returns a null pointer)

@@ -74,13 +74,30 @@ def gather_probe(table_bytes: int = 16 << 30, n_gathers: int = 1 << 30, stream: 
     return n_gathers / (ms.value * 1e-3)
 
 
-class BatchResult:
-    """CSR result of a batch: offsets[Q+1], positions (ascending per query), status[Q]."""
+APPROX_HITS = {"all": _capi.HITS_ALL, "all_best": _capi.HITS_ALL_BEST, "single_best": _capi.HITS_SINGLE_BEST,
+               "strata": _capi.HITS_STRATA}
 
-    def __init__(self, offsets: np.ndarray, positions: np.ndarray, status: np.ndarray, _owner=None):
+
+def approx_options(max_mismatches: int, hits: str = "all", strata: int = 0, distances: bool = False) -> _capi.ApproxOptions:
+    """kmer_b200_approx_options of a search_approx call (hits: a key of APPROX_HITS)."""
+    if hits not in APPROX_HITS:
+        raise ValueError(f"hits must be one of {sorted(APPROX_HITS)}, not {hits!r}")
+    return _capi.ApproxOptions(int(max_mismatches), APPROX_HITS[hits], int(strata),
+                               _capi.APPROX_DISTANCES if distances else 0)
+
+
+class BatchResult:
+    """CSR result of a batch: offsets[Q+1], positions (ascending per query), status[Q]. Approximate search with a hit
+    strategy also fills `distances` (uint8 per position: its Hamming distance, with distances=True) and `best_distance`
+    (uint8 per query: d_min, 0xFF without a hit; every strategy but "all"); both are None otherwise."""
+
+    def __init__(self, offsets: np.ndarray, positions: np.ndarray, status: np.ndarray, _owner=None,
+                 distances: np.ndarray | None = None, best_distance: np.ndarray | None = None):
         self.offsets = offsets
         self.positions = positions
         self.status = status
+        self.distances = distances
+        self.best_distance = best_distance
         self._owner = _owner   # (lib, C result handle) when the arrays are views of the pinned C result
 
     def free(self):
@@ -88,7 +105,7 @@ class BatchResult:
         if self._owner is not None:
             L, r = self._owner
             self._owner = None
-            self.offsets = self.positions = self.status = None
+            self.offsets = self.positions = self.status = self.distances = self.best_distance = None
             L.kmer_b200_result_free(r)
 
     def __del__(self):
@@ -206,6 +223,16 @@ class DeviceResult:
 
     def status(self):
         return _DevArray(self.status_ptr, self.n_queries, "|u1", self)
+
+    def distances(self):
+        """uint8 view of d(p) per position (approximate search with distances=True), or None."""
+        ptr = self._L.kmer_b200_result_distances(self._r) or 0
+        return _DevArray(ptr, self.n_positions, "|u1", self) if ptr else None
+
+    def best_distances(self):
+        """uint8 view of d_min per query (approximate search with a hit strategy other than "all"), or None."""
+        ptr = self._L.kmer_b200_result_best_distances(self._r) or 0
+        return _DevArray(ptr, self.n_queries, "|u1", self) if ptr else None
 
     def hit_queries(self):
         """int32 view of [n, id_1 .. id_n, ...]: the queries the count pass found hits for (unordered), or None."""
@@ -366,16 +393,25 @@ class KmerIndex:
         L.kmer_b200_result_free(r)
         return BatchResult(offsets, positions, status)
 
-    def search_approx(self, q_ranks, q_offsets, max_mismatches: int, copy: bool = True) -> BatchResult:
+    def search_approx(self, q_ranks, q_offsets, max_mismatches: int, copy: bool = True, *, hits: str = "all",
+                      strata: int = 0, distances: bool = False) -> BatchResult:
         """Approximate search of a host batch (kmer_b200_search_approx_batch): per query, every position p, ascending,
         where the text window T[p, p+m) differs from the query in at most max_mismatches (<= 8) symbols. Substitutions
         only; max_mismatches=0 is exact search in MODE_CORRECT. copy=False: views of the library's pinned buffers (valid
-        until BatchResult.free())."""
+        until BatchResult.free()).
+        hits: "all", "all_best" (the hits at the smallest distance d_min), "single_best" (the lowest such position) or
+        "strata" (distance <= d_min + strata); every choice but "all" sets BatchResult.best_distance. distances=True
+        sets BatchResult.distances (kmer_b200_search_approx_batch_ex)."""
         q = np.ascontiguousarray(np.asarray(q_ranks, dtype=np.uint8))
         off = np.ascontiguousarray(np.asarray(q_offsets, dtype=np.uint64))
         r = C.c_void_p()
-        _capi.check(self._L.kmer_b200_search_approx_batch(self._h, q.ctypes.data, off.ctypes.data, off.size - 1,
-                                                          int(max_mismatches), C.byref(r)))
+        if hits == "all" and not distances:
+            _capi.check(self._L.kmer_b200_search_approx_batch(self._h, q.ctypes.data, off.ctypes.data, off.size - 1,
+                                                              int(max_mismatches), C.byref(r)))
+        else:
+            opt = approx_options(max_mismatches, hits, strata, distances)
+            _capi.check(self._L.kmer_b200_search_approx_batch_ex(self._h, q.ctypes.data, off.ctypes.data, off.size - 1,
+                                                                 C.byref(opt), C.byref(r)))
         return self._host_result(r, off.size - 1, copy)
 
     def _host_result(self, r, Q: int, copy: bool) -> BatchResult:
@@ -386,9 +422,13 @@ class KmerIndex:
                   if Q else np.zeros(0, dtype=np.uint8))
         positions = (np.ctypeslib.as_array(C.cast(L.kmer_b200_result_positions(r), _capi.u32p), shape=(total,))
                      if total else np.zeros(0, dtype=np.uint32))
+        d_ptr, b_ptr = L.kmer_b200_result_distances(r), L.kmer_b200_result_best_distances(r)
+        dist = (np.ctypeslib.as_array(C.cast(d_ptr, _capi.u8p), shape=(total,)) if total else np.zeros(0, np.uint8)) if d_ptr else None
+        best = (np.ctypeslib.as_array(C.cast(b_ptr, _capi.u8p), shape=(Q,)) if Q else np.zeros(0, np.uint8)) if b_ptr else None
         if not copy:
-            return BatchResult(offsets, positions, status, _owner=(L, r))
-        out = BatchResult(offsets.copy(), positions.copy(), status.copy())
+            return BatchResult(offsets, positions, status, _owner=(L, r), distances=dist, best_distance=best)
+        out = BatchResult(offsets.copy(), positions.copy(), status.copy(), distances=None if dist is None else dist.copy(),
+                          best_distance=None if best is None else best.copy())
         L.kmer_b200_result_free(r)
         return out
 
@@ -417,13 +457,23 @@ class KmerIndex:
     def count_batch_device(self, q_ptr: int, off_ptr: int, Q: int, max_len: int, mode: int = MODE_DEFAULT):
         return self._device_call(self._L.kmer_b200_count_batch_device, q_ptr, off_ptr, Q, max_len, mode)
 
-    def search_approx_batch_device(self, q_ptr: int, off_ptr: int, Q: int, max_len: int, max_mismatches: int):
-        """Approximate search (see search_approx) of a device-resident batch; the result stays on the device."""
-        return self._device_call(self._L.kmer_b200_search_approx_batch_device, q_ptr, off_ptr, Q, max_len, max_mismatches)
+    def search_approx_batch_device(self, q_ptr: int, off_ptr: int, Q: int, max_len: int, max_mismatches: int, *,
+                                   hits: str = "all", strata: int = 0, distances: bool = False):
+        """Approximate search (see search_approx, including hits / strata / distances) of a device-resident batch; the
+        result stays on the device."""
+        if hits == "all" and not distances:
+            return self._device_call(self._L.kmer_b200_search_approx_batch_device, q_ptr, off_ptr, Q, max_len, max_mismatches)
+        opt = approx_options(max_mismatches, hits, strata, distances)
+        return self._device_call(self._L.kmer_b200_search_approx_batch_device_ex, q_ptr, off_ptr, Q, max_len, C.byref(opt))
 
-    def count_approx_batch_device(self, q_ptr: int, off_ptr: int, Q: int, max_len: int, max_mismatches: int):
-        """Count-only approximate search of a device-resident batch: offsets and status, no positions."""
-        return self._device_call(self._L.kmer_b200_count_approx_batch_device, q_ptr, off_ptr, Q, max_len, max_mismatches)
+    def count_approx_batch_device(self, q_ptr: int, off_ptr: int, Q: int, max_len: int, max_mismatches: int, *,
+                                  hits: str = "all", strata: int = 0, distances: bool = False):
+        """Count-only approximate search of a device-resident batch: offsets and status (and best_distances() for a hit
+        strategy other than "all"), no positions."""
+        if hits == "all" and not distances:
+            return self._device_call(self._L.kmer_b200_count_approx_batch_device, q_ptr, off_ptr, Q, max_len, max_mismatches)
+        opt = approx_options(max_mismatches, hits, strata, distances)
+        return self._device_call(self._L.kmer_b200_count_approx_batch_device_ex, q_ptr, off_ptr, Q, max_len, C.byref(opt))
 
     def presence_batch_device(self, q_ptr: int, off_ptr: int, Q: int, max_len: int, present_ptr: int,
                               mode: int = MODE_DEFAULT, fmt: int = 0) -> None:

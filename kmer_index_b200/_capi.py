@@ -29,6 +29,18 @@ class Config(C.Structure):
                 ("device_ids", C.POINTER(C.c_int32)), ("n_devices", C.c_uint32)]
 
 
+HITS_ALL = 0
+HITS_ALL_BEST = 1
+HITS_SINGLE_BEST = 2
+HITS_STRATA = 3
+APPROX_DISTANCES = 1
+
+
+class ApproxOptions(C.Structure):
+    """kmer_b200_approx_options"""
+    _fields_ = [("max_mismatches", C.c_uint32), ("hits", C.c_uint32), ("strata", C.c_uint32), ("flags", C.c_uint32)]
+
+
 class ElementInfo(C.Structure):
     _fields_ = [("k", C.c_uint32), ("key_bits", C.c_uint32), ("directory_shift", C.c_uint32),
                 ("sort_passes", C.c_uint32), ("n_kmers", C.c_uint64), ("directory_entries", C.c_uint64),
@@ -94,6 +106,12 @@ SYMBOLS = {
                                                        C.c_uint32, C.POINTER(C.c_void_p)]),
     "kmer_b200_count_approx_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64,
                                                       C.c_uint32, C.POINTER(C.c_void_p)]),
+    "kmer_b200_search_approx_batch_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(ApproxOptions),
+                                                   C.POINTER(C.c_void_p)]),
+    "kmer_b200_search_approx_batch_device_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64,
+                                                          C.POINTER(ApproxOptions), C.POINTER(C.c_void_p)]),
+    "kmer_b200_count_approx_batch_device_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64,
+                                                         C.POINTER(ApproxOptions), C.POINTER(C.c_void_p)]),
     "kmer_b200_result_n_queries": (C.c_uint64, [C.c_void_p]),
     "kmer_b200_result_n_positions": (C.c_uint64, [C.c_void_p]),
     "kmer_b200_result_on_device": (C.c_int, [C.c_void_p]),
@@ -101,6 +119,8 @@ SYMBOLS = {
     "kmer_b200_result_offsets": (C.c_void_p, [C.c_void_p]),
     "kmer_b200_result_positions": (C.c_void_p, [C.c_void_p]),
     "kmer_b200_result_status": (C.c_void_p, [C.c_void_p]),
+    "kmer_b200_result_distances": (C.c_void_p, [C.c_void_p]),
+    "kmer_b200_result_best_distances": (C.c_void_p, [C.c_void_p]),
     "kmer_b200_result_free": (None, [C.c_void_p]),
     "kmer_b200_presence_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64,
                                                   C.c_uint32, C.c_void_p, C.c_uint32]),

@@ -79,12 +79,16 @@ enum KernelId : int {
     K_SEARCH_PRESENCE,
     K_OFFSETS_SCAN,
     K_SEGMENT_SORT,
+    K_APPROX_BEST,
+    K_APPROX_SINGLE,
+    K_APPROX_DISTANCES,
     K_COUNT_
 };
 
 const char *const kKernelNames[K_COUNT_] = {
     "pack_text",       "radix_hist_text", "radix_hist_pairs", "column_scan",     "radix_scatter_text", "radix_scatter_pairs",
-    "directory_fill",  "search_count",    "search_write",     "search_presence", "offsets_scan",       "segment_sort"};
+    "directory_fill",  "search_count",    "search_write",     "search_presence", "offsets_scan",       "segment_sort",
+    "approx_best",     "approx_single",   "approx_distances"};
 
 struct Profiler {
     bool enabled = false;
@@ -240,7 +244,10 @@ struct kmer_b200_result {
     uint32_t *positions = nullptr;
     uint8_t *status = nullptr;
     uint32_t *hit_queries = nullptr;  // device results: [0] = n, [1..n] = ids of the queries the count pass found hits for
+    uint8_t *distances = nullptr;      // approximate search with KMER_B200_APPROX_DISTANCES: d(p) per position, or null
+    uint8_t *best_distance = nullptr;  // approximate search, hit strategies other than "all": d_min per query, or null
     size_t cap_offsets = 0, cap_positions = 0, cap_status = 0;  // host buffers: byte capacities
+    size_t cap_distances = 0, cap_best_distance = 0;
     bool positions_pageable = false;  // very large position lists live in plain malloc memory
 };
 
@@ -1303,7 +1310,15 @@ struct PendingSearch {
     size_t h_scratch_cap = 0;
     bool presence_applied = false;  // deferred mode: the whole-text rule has been applied to the counts
     bool merge_checked = false;     // add_counts: the batch has no segment that the sort pass would have to visit
+    // approximate search with a hit strategy (kmer_b200_approx_options; null = every hit, no distances)
+    const kmer_b200_approx_options *hit_opt = nullptr;
+    uint8_t *d_budget = nullptr;     // [Q]: per-query budget of the re-seeded passes (all best, strata)
+    uint32_t *d_best_pos = nullptr;  // [Q]: the best pass's lowest position with d_min
     void release() {
+        dev_free(ix, d_budget);
+        dev_free(ix, d_best_pos);
+        d_budget = nullptr;
+        d_best_pos = nullptr;
         dev_free(ix, d_flags);
         d_flags = nullptr;
         pinned_put(h_scratch, h_scratch_cap);
@@ -1329,9 +1344,20 @@ struct PackedQueries {
     uint32_t stride;
 };
 
+// the device arrays of a hit strategy (search_begin allocates them)
+kb::ApproxHitArgs approx_hit_args(const PendingSearch *p) {
+    kb::ApproxHitArgs h{};
+    h.budget = p->d_budget;
+    h.best_dist = p->res->best_distance;
+    h.best_pos = p->d_best_pos;
+    h.strata = p->hit_opt && p->hit_opt->hits == KMER_B200_HITS_STRATA ? std::min(p->hit_opt->strata, kb::kMaxMismatches) : 0;
+    return h;
+}
+
 int search_begin(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len,
                  uint32_t mode, const void *d_present_global, uint32_t present_format, uint32_t *d_present4,
-                 PendingSearch *p, const PackedQueries *packed = nullptr, int32_t max_mismatches = -1) {
+                 PendingSearch *p, const PackedQueries *packed = nullptr, int32_t max_mismatches = -1,
+                 const kmer_b200_approx_options *hit_opt = nullptr) {
     using namespace kb;
     const bool approx = max_mismatches >= 0;  // approximate search: the semantics of CORRECT mode, any query length
     if (approx) mode = KMER_B200_MODE_CORRECT;
@@ -1359,6 +1385,11 @@ int search_begin(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off,
         dev_alloc(ix, &p->d_unsorted, Q, false) || dev_alloc(ix, &p->d_block_sums, offsets_scan_blocks(Q) + 1, false) ||
         (d_present4 && dev_alloc(ix, &p->d_defer, Q, false)) || dev_alloc(ix, &p->d_heavy, Q + 1, false) ||
         dev_alloc(ix, &p->d_hits, Q + 1, false) || dev_alloc(ix, &p->d_flags, 4, false))
+        return bail(KMER_B200_ERR_OUT_OF_MEMORY);
+    const bool best_pass = approx && hit_opt && hit_opt->hits != KMER_B200_HITS_ALL;
+    p->hit_opt = approx ? hit_opt : nullptr;
+    if (best_pass && (dev_alloc(ix, &res->best_distance, Q, false) || dev_alloc(ix, &p->d_best_pos, Q, false) ||
+                      (hit_opt->hits != KMER_B200_HITS_SINGLE_BEST && dev_alloc(ix, &p->d_budget, Q, false))))
         return bail(KMER_B200_ERR_OUT_OF_MEMORY);
     p->h_scratch = (uint64_t *)pinned_get(8 * sizeof(uint64_t), &p->h_scratch_cap);
     if (!p->h_scratch) return bail(fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed"));
@@ -1409,13 +1440,29 @@ int search_begin(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off,
     if (a.gather_count) cudaMemsetAsync(ix->d_gathers, 0, sizeof(unsigned long long), st);
 
     cudaMemsetAsync(p->d_flags, 0, 4 * sizeof(uint32_t), st);
-    ix->prof.begin(K_SEARCH_COUNT, 0);
-    if (approx)
+    if (best_pass) {
+        // best pass over every query; all best and strata then count again over the queries it listed, each with its budget
+        const ApproxHitArgs h = approx_hit_args(p);
+        const SearchPass count = a.gather_count ? kPassCountAccount : kPassCount;
+        ix->prof.begin(K_APPROX_BEST, 0);
+        launch_search_approx_hits(a, h, kApproxBest, count, st);
+        ix->prof.end();
+        if (hit_opt->hits != KMER_B200_HITS_SINGLE_BEST) {
+            cudaMemsetAsync(p->d_heavy, 0, sizeof(uint32_t), st);
+            ix->prof.begin(K_SEARCH_COUNT, 0);
+            launch_search_approx_hits(a, h, kApproxListed, count, st);
+            ix->prof.end();
+        }
+    } else if (approx) {
+        ix->prof.begin(K_SEARCH_COUNT, 0);
         launch_search_approx(a, a.gather_count ? kPassCountAccount : kPassCount, st);
-    else
+        ix->prof.end();
+    } else {
+        ix->prof.begin(K_SEARCH_COUNT, 0);
         launch_search(a, d_present4 ? (a.gather_count ? kPassCountDeferredAccount : kPassCountDeferred)
                                     : (a.gather_count ? kPassCountAccount : kPassCount), st);
-    ix->prof.end();
+        ix->prof.end();
+    }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return bail(fail(KMER_B200_ERR_CUDA, std::string("search (count pass): ") + cudaGetErrorString(e)));
     return KMER_B200_OK;
@@ -1490,11 +1537,28 @@ int search_finish(PendingSearch *p, const uint32_t *d_present4_global, SearchFla
     // below already reads through it, so those results come out sorted and skip the segment sort
     uint64_t aux_missing = want_aux;
     if (flavor == kFlavorFull && want_aux && !(ix->cfg.reserved & KMER_B200_FLAG_NO_AUX)) aux_missing = ensure_aux_elements(ix, want_aux);
-    if (flavor == kFlavorFull && total > 0) {
-        if (dev_alloc(ix, &res->positions, total, false)) return bail(KMER_B200_ERR_OUT_OF_MEMORY);
+    const kmer_b200_approx_options *hit_opt = p->hit_opt;
+    const uint32_t hits = hit_opt ? hit_opt->hits : (uint32_t)KMER_B200_HITS_ALL;
+    const bool want_distances = hit_opt && (hit_opt->flags & KMER_B200_APPROX_DISTANCES);
+    // asked-for distances are present even without a hit (an empty array, not NULL)
+    if (flavor == kFlavorFull && want_distances && total == 0 && dev_alloc(ix, &res->distances, 1, false))
+        return bail(KMER_B200_ERR_OUT_OF_MEMORY);
+    if (flavor == kFlavorFull && total > 0 && hits == KMER_B200_HITS_SINGLE_BEST) {
+        // one hit per listed query: the best pass has it already
+        if (dev_alloc(ix, &res->positions, total, false) || (want_distances && dev_alloc(ix, &res->distances, total, false)))
+            return bail(KMER_B200_ERR_OUT_OF_MEMORY);
+        a.positions = res->positions;
+        ix->prof.begin(K_APPROX_SINGLE, 0);
+        launch_approx_single(a, approx_hit_args(p), res->distances, st);
+        ix->prof.end();
+    } else if (flavor == kFlavorFull && total > 0) {
+        if (dev_alloc(ix, &res->positions, total, false) || (want_distances && dev_alloc(ix, &res->distances, total, false)))
+            return bail(KMER_B200_ERR_OUT_OF_MEMORY);
         a.positions = res->positions;
         ix->prof.begin(K_SEARCH_WRITE, 0);
-        if (a.approx)
+        if (a.approx && hits != KMER_B200_HITS_ALL)
+            launch_search_approx_hits(a, approx_hit_args(p), kApproxListed, kPassWrite, st);
+        else if (a.approx)
             launch_search_approx(a, kPassWrite, st);
         else
             launch_search(a, kPassWrite, st);
@@ -1509,6 +1573,16 @@ int search_finish(PendingSearch *p, const uint32_t *d_present4_global, SearchFla
             launch_segment_sort(res->positions, d_tmp, res->offsets, p->d_unsorted, Q, key_bits, st);
             ix->prof.end();
             dev_free(ix, d_tmp);
+        }
+        if (want_distances) {
+            // d(p) in position order, after the sort; its gathered sectors join the count passes' under profile = 2
+            ix->prof.begin(K_APPROX_DISTANCES, 0);
+            launch_approx_distances(a, approx_hit_args(p), res->distances, st);
+            ix->prof.end();
+            if (a.gather_count) {
+                cudaMemcpyAsync(&hs[3], ix->d_gathers, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+                if (cudaStreamSynchronize(st) == cudaSuccess) ix->last_gathers = hs[3];
+            }
         }
     }
     res->hit_queries = p->d_hits;  // stays with the result (the sharded merge works from it)
@@ -1528,9 +1602,11 @@ int search_finish(PendingSearch *p, const uint32_t *d_present4_global, SearchFla
 // queries already on the device; result stays on the device
 int search_device_impl(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len,
                        uint32_t mode, const void *d_present_global, uint32_t present_format, SearchFlavor flavor,
-                       kmer_b200_result **out, const PackedQueries *packed = nullptr, int32_t max_mismatches = -1) {
+                       kmer_b200_result **out, const PackedQueries *packed = nullptr, int32_t max_mismatches = -1,
+                       const kmer_b200_approx_options *hit_opt = nullptr) {
     PendingSearch p;
-    KB_TRY(search_begin(ix, d_q, d_off, Q, max_len, mode, d_present_global, present_format, nullptr, &p, packed, max_mismatches));
+    KB_TRY(search_begin(ix, d_q, d_off, Q, max_len, mode, d_present_global, present_format, nullptr, &p, packed, max_mismatches,
+                        hit_opt));
     return search_finish(&p, nullptr, flavor, out);
 }
 
@@ -1572,6 +1648,18 @@ int approx_check(const kmer_b200_index *ix, uint32_t max_mismatches) {
     for (size_t e = 0; e < ix->ks.size(); ++e)
         if (ix->elems[e].dev.key_lo != 0 || ix->elems[e].dev.key_hi != UINT64_MAX)
             return fail(KMER_B200_ERR_UNSUPPORTED, "approximate search needs the whole key space: adopt the assembled element first");
+    return KMER_B200_OK;
+}
+
+// the options of the _ex entry points: INVALID_ARGUMENT for null options, e > 8, an unknown strategy or unknown flag
+// bits, then the handle checks of approx_check. Every hit without distances takes the plain approximate path (null).
+int approx_options_check(const kmer_b200_index *ix, const kmer_b200_approx_options *opt, const kmer_b200_approx_options **hit_opt) {
+    if (!opt) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "approximate search: null options");
+    if (opt->hits > KMER_B200_HITS_STRATA) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "approximate search: unknown hit strategy");
+    if (opt->flags & ~(uint32_t)KMER_B200_APPROX_DISTANCES)
+        return fail(KMER_B200_ERR_INVALID_ARGUMENT, "approximate search: unknown option flags");
+    KB_TRY(approx_check(ix, opt->max_mismatches));
+    *hit_opt = (opt->hits == KMER_B200_HITS_ALL && !(opt->flags & KMER_B200_APPROX_DISTANCES)) ? nullptr : opt;
     return KMER_B200_OK;
 }
 
@@ -1831,6 +1919,30 @@ int kmer_b200_count_approx_batch_device(kmer_b200_index *ix, const uint8_t *d_q,
     std::lock_guard<std::mutex> lock(ix->mu);
     return search_device_impl(ix, d_q, d_off, Q, max_len, KMER_B200_MODE_CORRECT, nullptr, 0, kFlavorCountOnly, out, nullptr,
                               (int32_t)max_mismatches);
+}
+
+int kmer_b200_search_approx_batch_device_ex(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
+                                            uint64_t max_len, const kmer_b200_approx_options *opt, kmer_b200_result **out) {
+    if (!ix || !out || !d_off) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    *out = nullptr;
+    const kmer_b200_approx_options *hit_opt = nullptr;
+    KB_TRY(approx_options_check(ix, opt, &hit_opt));
+    DeviceGuard guard(ix->device);
+    std::lock_guard<std::mutex> lock(ix->mu);
+    return search_device_impl(ix, d_q, d_off, Q, max_len, KMER_B200_MODE_CORRECT, nullptr, 0, kFlavorFull, out, nullptr,
+                              (int32_t)opt->max_mismatches, hit_opt);
+}
+
+int kmer_b200_count_approx_batch_device_ex(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
+                                           uint64_t max_len, const kmer_b200_approx_options *opt, kmer_b200_result **out) {
+    if (!ix || !out || !d_off) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    *out = nullptr;
+    const kmer_b200_approx_options *hit_opt = nullptr;
+    KB_TRY(approx_options_check(ix, opt, &hit_opt));
+    DeviceGuard guard(ix->device);
+    std::lock_guard<std::mutex> lock(ix->mu);
+    return search_device_impl(ix, d_q, d_off, Q, max_len, KMER_B200_MODE_CORRECT, nullptr, 0, kFlavorCountOnly, out, nullptr,
+                              (int32_t)opt->max_mismatches, hit_opt);
 }
 
 int kmer_b200_search_batch_device_global(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
@@ -2314,7 +2426,8 @@ static int search_batch_host_chunked(kmer_b200_index *ix, const uint8_t *q_ranks
 // Small exact batches, and every approximate batch (max_mismatches >= 0), take this path. The caller holds the
 // handle's lock and device.
 static int search_batch_host_single_copy(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q,
-                                         uint32_t mode, const uint8_t *lut256, int32_t max_mismatches, kmer_b200_result **out) {
+                                         uint32_t mode, const uint8_t *lut256, int32_t max_mismatches, kmer_b200_result **out,
+                                         const kmer_b200_approx_options *hit_opt = nullptr) {
     cudaStream_t st = ix->stream;
     const uint64_t n_sym = q_offsets[Q] - q_offsets[0];
     uint8_t *d_q = nullptr;
@@ -2345,11 +2458,16 @@ static int search_batch_host_single_copy(kmer_b200_index *ix, const uint8_t *q_r
     const uint64_t max_len = ix->h_pinned[2];
     kmer_b200_result *dres = nullptr;
     int s = search_device_impl(ix, d_q - q_offsets[0], d_off, Q, max_len, mode, nullptr, 0, kFlavorFull, &dres, nullptr,
-                               max_mismatches);
+                               max_mismatches, hit_opt);
     if (s != 0) return s;
     // device result -> pinned host buffers
     kmer_b200_result *res = host_result_new(ix, Q);
-    if (!res || !host_result_positions(res, dres->n_positions)) {
+    bool extra_ok = res != nullptr;
+    if (res && dres->distances)
+        extra_ok = (res->distances = (uint8_t *)pinned_get(std::max<uint64_t>(dres->n_positions, 1), &res->cap_distances)) != nullptr;
+    if (extra_ok && dres->best_distance)
+        extra_ok = (res->best_distance = (uint8_t *)pinned_get(std::max<uint64_t>(Q, 1), &res->cap_best_distance)) != nullptr;
+    if (!res || !extra_ok || !host_result_positions(res, dres->n_positions)) {
         kmer_b200_result_free(dres);
         kmer_b200_result_free(res);
         return fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed");
@@ -2358,6 +2476,9 @@ static int search_batch_host_single_copy(kmer_b200_index *ix, const uint8_t *q_r
     if (Q) cudaMemcpyAsync(res->status, dres->status, Q, cudaMemcpyDeviceToHost, st);
     if (res->n_positions)
         cudaMemcpyAsync(res->positions, dres->positions, res->n_positions * sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
+    const uint64_t n_dist = dres->distances ? res->n_positions : 0, n_best = dres->best_distance ? Q : 0;
+    if (n_dist) cudaMemcpyAsync(res->distances, dres->distances, n_dist, cudaMemcpyDeviceToHost, st);
+    if (n_best) cudaMemcpyAsync(res->best_distance, dres->best_distance, n_best, cudaMemcpyDeviceToHost, st);
     cudaError_t e = cudaStreamSynchronize(st);
     kmer_b200_result_free(dres);
     if (e != cudaSuccess) {
@@ -2366,7 +2487,7 @@ static int search_batch_host_single_copy(kmer_b200_index *ix, const uint8_t *q_r
         return fail(KMER_B200_ERR_CUDA, std::string("search (D2H): ") + cudaGetErrorString(e));
     }
     ix->last_h2d = n_sym + (Q + 1) * sizeof(uint64_t);
-    ix->last_d2h = (Q + 1) * sizeof(uint64_t) + Q + res->n_positions * sizeof(uint32_t);
+    ix->last_d2h = (Q + 1) * sizeof(uint64_t) + Q + res->n_positions * sizeof(uint32_t) + n_dist + n_best;
     ix->last_host_path = 0, ix->last_raw_pct = 100, ix->last_pack_gbs = 0;
     *out = res;
     return KMER_B200_OK;
@@ -2428,6 +2549,19 @@ int kmer_b200_search_approx_batch(kmer_b200_index *ix, const uint8_t *q_ranks, c
     DeviceGuard guard(ix->device);
     std::lock_guard<std::mutex> lock(ix->mu);
     return search_batch_host_single_copy(ix, q_ranks, q_offsets, Q, KMER_B200_MODE_CORRECT, nullptr, (int32_t)max_mismatches, out);
+}
+
+int kmer_b200_search_approx_batch_ex(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q,
+                                     const kmer_b200_approx_options *opt, kmer_b200_result **out) {
+    if (!ix || !out || !q_offsets) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    *out = nullptr;
+    const kmer_b200_approx_options *hit_opt = nullptr;
+    KB_TRY(approx_options_check(ix, opt, &hit_opt));
+    if (q_offsets[Q] != q_offsets[0] && !q_ranks) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "q_ranks is null");
+    DeviceGuard guard(ix->device);
+    std::lock_guard<std::mutex> lock(ix->mu);
+    return search_batch_host_single_copy(ix, q_ranks, q_offsets, Q, KMER_B200_MODE_CORRECT, nullptr, (int32_t)opt->max_mismatches,
+                                         out, hit_opt);
 }
 
 int kmer_b200_search_batch_ptrs(kmer_b200_index *ix, const uint8_t *const *q_ptrs, const uint64_t *q_lens, uint64_t Q,
@@ -2503,6 +2637,8 @@ const uint32_t *kmer_b200_result_hit_queries(const kmer_b200_result *r) { return
 const uint64_t *kmer_b200_result_offsets(const kmer_b200_result *r) { return r ? r->offsets : nullptr; }
 const uint32_t *kmer_b200_result_positions(const kmer_b200_result *r) { return r ? r->positions : nullptr; }
 const uint8_t *kmer_b200_result_status(const kmer_b200_result *r) { return r ? r->status : nullptr; }
+const uint8_t *kmer_b200_result_distances(const kmer_b200_result *r) { return r ? r->distances : nullptr; }
+const uint8_t *kmer_b200_result_best_distances(const kmer_b200_result *r) { return r ? r->best_distance : nullptr; }
 
 void kmer_b200_result_free(kmer_b200_result *r) {
     if (!r) return;
@@ -2513,6 +2649,8 @@ void kmer_b200_result_free(kmer_b200_result *r) {
         dev_free(ix, r->positions);
         dev_free(ix, r->status);
         dev_free(ix, r->hit_queries);
+        dev_free(ix, r->distances);
+        dev_free(ix, r->best_distance);
     } else {
         pinned_put(r->offsets, r->cap_offsets);
         if (r->positions_pageable)
@@ -2520,6 +2658,8 @@ void kmer_b200_result_free(kmer_b200_result *r) {
         else
             pinned_put(r->positions, r->cap_positions);
         pinned_put(r->status, r->cap_status);
+        pinned_put(r->distances, r->cap_distances);
+        pinned_put(r->best_distance, r->cap_best_distance);
     }
     delete r;
 }

@@ -109,6 +109,24 @@ void launch_search(const SearchArgs &args, SearchPass pass, cudaStream_t stream)
 // elements hold their positions (whole or in peer parts); queries as 1-byte ranks (q_packed unused)
 constexpr uint32_t kMaxMismatches = 8;
 void launch_search_approx(const SearchArgs &args, SearchPass pass, cudaStream_t stream);
+// hit strategies of approximate search (search_approx.cu). kApproxBest: count passes over every query with budget
+// min(e, m - 1) -> best_dist / best_pos per query, counts = 1 where a hit exists, those queries listed in args.hits,
+// budget[q] = min(e, d_min + strata) when budget != null. kApproxListed: count and write passes over the queries of
+// args.hits with budget[q] each (the count pass leaves the list as it is).
+enum ApproxMode : int { kApproxAll = 0, kApproxListed = 1, kApproxBest = 2 };
+struct ApproxHitArgs {
+    uint8_t *budget;     // device or null, [Q]: per-query budget e_q
+    uint8_t *best_dist;  // device (kApproxBest), [Q]: d_min, 0xFF = no hit
+    uint32_t *best_pos;  // device (kApproxBest), [Q]: the lowest position with d_min
+    uint32_t strata;     // s of the strata strategy (0 = all best)
+};
+void launch_search_approx_hits(const SearchArgs &args, const ApproxHitArgs &h, ApproxMode mode, SearchPass pass,
+                               cudaStream_t stream);
+// after the offsets scan: positions[offsets[q]] = best_pos[q] (+ distances) for each listed query
+void launch_approx_single(const SearchArgs &args, const ApproxHitArgs &h, uint8_t *d_distances, cudaStream_t stream);
+// after the write pass (and segment sort): d_distances[j] = d(positions[j]) over the listed queries' hits; budget
+// h.budget[q], else args.max_mismatches
+void launch_approx_distances(const SearchArgs &args, const ApproxHitArgs &h, uint8_t *d_distances, cudaStream_t stream);
 uint32_t search_q_words(uint32_t group, uint32_t bits, uint64_t max_len);
 // deferred count pass epilogue: zero the counts / set THROW according to the combined presence flags
 void launch_finalize_deferred(uint64_t *d_counts, uint8_t *d_status, const uint8_t *d_defer, const uint32_t *d_present4_global,

@@ -14,6 +14,13 @@
 // One group of G lanes per query, as the general search kernel; two passes (count -> scan -> write); candidate lists
 // longer than kHeavyCandidates go to a warp-per-query launch. Hits of several seeds, or of a slab, are not ascending:
 // such a query is flagged for launch_segment_sort.
+//
+// Hit strategies (kmer_b200_approx_hits) other than "all" start with a best pass (kApproxBest): the count-pass
+// enumeration of every query with budget min(e, m - 1), each lane keeping the smallest (d << 32 | p) of its survivors;
+// it writes d_min and the lowest position with that distance, and lists the queries that have one. Single-best ends
+// there (one hit per listed query, launch_approx_single). All-best and strata run the count and write passes again
+// over the listed queries only (kApproxListed), each with its own budget e_q = min(e, d_min + s): the e_q + 1 seeds
+// enumerate exactly the windows with d <= e_q. launch_approx_distances recomputes d(p) of every written hit.
 #include <algorithm>
 
 #include "launch.h"
@@ -24,11 +31,14 @@ namespace kb {
 constexpr int kApproxThreads = 256;
 
 // PASS: kPassCount, kPassCountAccount (count + gathered sectors) or kPassWrite. HEAVY: the warp-per-query launch over
-// the heavy list.
-template <int PASS_, int G, bool HEAVY>
-__device__ __forceinline__ void approx_query(const SearchArgs &a, const uint64_t q, uint64_t *smem_q) {
+// the heavy list. MODE: kApproxAll (budget a.max_mismatches, every query), kApproxListed (budget h.budget[q], the
+// queries of a.hits; the count pass does not list them again) or kApproxBest (count passes only: the best pass).
+template <int PASS_, int G, bool HEAVY, int MODE = kApproxAll>
+__device__ __forceinline__ void approx_query(const SearchArgs &a, const uint64_t q, uint64_t *smem_q,
+                                             const ApproxHitArgs &h = ApproxHitArgs{}) {
     constexpr bool kAccount = PASS_ == kPassCountAccount;
     constexpr int PASS = kAccount ? (int)kPassCount : PASS_;
+    constexpr bool kBest = MODE == kApproxBest;
     const int lane = threadIdx.x & 31;
     const int gl = threadIdx.x & (G - 1);
     const int group = threadIdx.x / G;
@@ -61,7 +71,7 @@ __device__ __forceinline__ void approx_query(const SearchArgs &a, const uint64_t
     const PackedText T = ix.text;
     const uint64_t off0 = a.q_offsets[q];
     const uint64_t m64 = a.q_offsets[q + 1] - off0;
-    const uint32_t e = a.max_mismatches;
+    uint32_t e = MODE == kApproxListed ? (uint32_t)h.budget[q] : a.max_mismatches;
     uint32_t status = KMER_B200_QUERY_OK;
     if (m64 == 0) status = KMER_B200_QUERY_UNDEFINED;
     else if (m64 > a.max_len) status = KMER_B200_QUERY_TOO_LONG_FOR_SHARD;  // longer than the caller's max_query_len
@@ -70,10 +80,13 @@ __device__ __forceinline__ void approx_query(const SearchArgs &a, const uint64_t
             a.counts[q] = 0;
             a.status[q] = (uint8_t)status;
             a.unsorted[q] = 0;
+            if (kBest) h.best_dist[q] = 0xFF;
         }
         return;
     }
     const uint32_t m = (uint32_t)m64;
+    if (kBest && e >= m) e = m - 1;  // d_min of a query of m <= e symbols: below m if a window is found, else m
+    uint64_t best = ~0ull;           // kApproxBest: this lane's smallest (d << 32 | p)
     uint64_t *qw = smem_q + (size_t)group * a.q_words;
     pack_query_group<G>(a.q_ranks, off0, m, a.q_offsets[a.n_queries], T, (uint32_t)gl, gmask, a.error_flag, qw);
 
@@ -162,7 +175,15 @@ __device__ __forceinline__ void approx_query(const SearchArgs &a, const uint64_t
                         if (kAccount) ++n_gather;
                     }
                     if (ok) {
-                        ok = mismatches_span(T, qw, p, 0, m, e) <= e;
+                        if (kBest) {
+                            // the limit follows this lane's best distance: equal distances are still counted exactly
+                            const uint32_t lim = best == ~0ull ? e : (uint32_t)(best >> 32);
+                            const uint32_t d = mismatches_span(T, qw, p, 0, m, lim);
+                            if (d <= lim) best = min(best, ((uint64_t)d << 32) | p);
+                            ok = false;
+                        } else {
+                            ok = mismatches_span(T, qw, p, 0, m, e) <= e;
+                        }
                         if (kAccount) n_gather += 1 + (m * T.bits >> 8);
                     }
                 }
@@ -179,13 +200,29 @@ __device__ __forceinline__ void approx_query(const SearchArgs &a, const uint64_t
         for (int o = G >> 1; o > 0; o >>= 1) n_gather += __shfl_xor_sync(gmask, n_gather, o, G);
         if (gl == 0) atomicAdd(a.gather_count, (unsigned long long)n_gather);
     }
+    if (kBest) {
+        for (int o = G >> 1; o > 0; o >>= 1) best = min(best, (uint64_t)__shfl_xor_sync(gmask, best, o, G));
+        if (best == ~0ull && m <= a.max_mismatches && (uint64_t)m <= T.n) best = (uint64_t)m << 32;  // every window: d = m
+        if (gl == 0) {
+            const bool found = best != ~0ull;
+            const uint32_t d = (uint32_t)(best >> 32);
+            a.counts[q] = found ? 1 : 0;
+            a.status[q] = KMER_B200_QUERY_OK;
+            a.unsorted[q] = HEAVY ? 2 : 0;
+            h.best_dist[q] = found ? (uint8_t)d : (uint8_t)0xFF;
+            h.best_pos[q] = (uint32_t)best;
+            if (h.budget && found) h.budget[q] = (uint8_t)min(a.max_mismatches, d + h.strata);
+            if (found) a.hits[1 + atomicAdd(a.hits, 1u)] = (uint32_t)q;
+        }
+        return;
+    }
     if (PASS == kPassCount && gl == 0) {
         a.counts[q] = n_hits;
         a.status[q] = KMER_B200_QUERY_OK;
         const bool flag = unsorted && n_hits > 1;
         a.unsorted[q] = (flag ? 1 : 0) | (HEAVY ? 2 : 0);
         if (flag) atomicAdd(a.error_flag + 1, 1u);  // number of segments the sort pass has to visit
-        if (a.hits != nullptr && n_hits > 0) {
+        if (MODE == kApproxAll && a.hits != nullptr && n_hits > 0) {
             // the write pass only visits the queries listed here
             const uint32_t act = __activemask();
             const int leader = __ffs(act) - 1;
@@ -200,67 +237,192 @@ __device__ __forceinline__ void approx_query(const SearchArgs &a, const uint64_t
 #undef GSHFL
 }
 
-// count pass: one group per query; write pass: the queries the count pass listed as having hits
-template <int PASS, int G>
-__global__ void __launch_bounds__(kApproxThreads) search_approx_kernel(const SearchArgs a) {
+// count pass: one group per query; write pass (and every pass of kApproxListed): the queries the count pass listed as
+// having hits
+template <int PASS, int G, int MODE>
+__device__ __forceinline__ void approx_grid(const SearchArgs &a, const ApproxHitArgs &h, uint64_t *smem_q) {
     constexpr int kGroups = kApproxThreads / G;
-    extern __shared__ uint64_t smem_q[];
-    if (PASS == kPassWrite && a.hits != nullptr) {
+    if ((PASS == kPassWrite || MODE == kApproxListed) && a.hits != nullptr) {
         const uint32_t n_listed = a.hits[0];
         for (uint64_t i = (uint64_t)blockIdx.x * kGroups + threadIdx.x / G; i < n_listed; i += (uint64_t)gridDim.x * kGroups) {
-            approx_query<PASS, G, false>(a, (uint64_t)a.hits[1 + i], smem_q);
+            approx_query<PASS, G, false, MODE>(a, (uint64_t)a.hits[1 + i], smem_q, h);
             __syncwarp();
         }
     } else {
         const uint64_t q = (uint64_t)blockIdx.x * kGroups + threadIdx.x / G;
-        if (q < a.n_queries) approx_query<PASS, G, false>(a, q, smem_q);
-    }
-}
-
-// second launch of a pass: one warp per query of the heavy list (a.heavy[0] = length, a.heavy[1..] = query ids)
-template <int PASS>
-__global__ void __launch_bounds__(kApproxThreads) search_approx_heavy_kernel(const SearchArgs a) {
-    constexpr int kGroups = kApproxThreads / 32;
-    extern __shared__ uint64_t smem_q[];
-    const uint32_t n_heavy = a.heavy[0];
-    for (uint32_t i = blockIdx.x * kGroups + threadIdx.x / 32; i < n_heavy; i += gridDim.x * kGroups) {
-        approx_query<PASS, 32, true>(a, (uint64_t)a.heavy[1 + i], smem_q);
-        __syncwarp();
+        if (q < a.n_queries) approx_query<PASS, G, false, MODE>(a, q, smem_q, h);
     }
 }
 
 template <int PASS, int G>
-static void launch_approx_pg(const SearchArgs &args, cudaStream_t stream) {
+__global__ void __launch_bounds__(kApproxThreads) search_approx_kernel(const SearchArgs a) {
+    extern __shared__ uint64_t smem_q[];
+    approx_grid<PASS, G, kApproxAll>(a, ApproxHitArgs{}, smem_q);
+}
+
+template <int PASS, int G, int MODE>
+__global__ void __launch_bounds__(kApproxThreads) search_approx_hits_kernel(const SearchArgs a, const ApproxHitArgs h) {
+    extern __shared__ uint64_t smem_q[];
+    approx_grid<PASS, G, MODE>(a, h, smem_q);
+}
+
+// second launch of a pass: one warp per query of the heavy list (a.heavy[0] = length, a.heavy[1..] = query ids)
+template <int PASS, int MODE>
+__device__ __forceinline__ void approx_heavy(const SearchArgs &a, const ApproxHitArgs &h, uint64_t *smem_q) {
+    constexpr int kGroups = kApproxThreads / 32;
+    const uint32_t n_heavy = a.heavy[0];
+    for (uint32_t i = blockIdx.x * kGroups + threadIdx.x / 32; i < n_heavy; i += gridDim.x * kGroups) {
+        approx_query<PASS, 32, true, MODE>(a, (uint64_t)a.heavy[1 + i], smem_q, h);
+        __syncwarp();
+    }
+}
+
+template <int PASS>
+__global__ void __launch_bounds__(kApproxThreads) search_approx_heavy_kernel(const SearchArgs a) {
+    extern __shared__ uint64_t smem_q[];
+    approx_heavy<PASS, kApproxAll>(a, ApproxHitArgs{}, smem_q);
+}
+
+template <int PASS, int MODE>
+__global__ void __launch_bounds__(kApproxThreads) search_approx_heavy_hits_kernel(const SearchArgs a, const ApproxHitArgs h) {
+    extern __shared__ uint64_t smem_q[];
+    approx_heavy<PASS, MODE>(a, h, smem_q);
+}
+
+template <int PASS, int G, int MODE>
+static void launch_approx_pg(const SearchArgs &args, const ApproxHitArgs &h, cudaStream_t stream) {
     constexpr int kGroups = kApproxThreads / G;
     const size_t smem = (size_t)kGroups * args.q_words * sizeof(uint64_t);
     uint64_t blocks = (args.n_queries + kGroups - 1) / kGroups;
-    if (PASS == kPassWrite && args.hits != nullptr) blocks = std::min<uint64_t>(blocks, (uint64_t)device_sm_count() * 16);
-    cudaFuncSetAttribute(search_approx_kernel<PASS, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    search_approx_kernel<PASS, G><<<(unsigned)blocks, kApproxThreads, smem, stream>>>(args);
+    if ((PASS == kPassWrite || MODE == kApproxListed) && args.hits != nullptr)
+        blocks = std::min<uint64_t>(blocks, (uint64_t)device_sm_count() * 16);
+    if (MODE == kApproxAll) {
+        cudaFuncSetAttribute(search_approx_kernel<PASS, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        search_approx_kernel<PASS, G><<<(unsigned)blocks, kApproxThreads, smem, stream>>>(args);
+    } else {
+        cudaFuncSetAttribute(search_approx_hits_kernel<PASS, G, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        search_approx_hits_kernel<PASS, G, MODE><<<(unsigned)blocks, kApproxThreads, smem, stream>>>(args, h);
+    }
     if (G < 32 && args.heavy != nullptr) {
         // queries with long candidate lists, if any (the list length lives on the device: fixed grid, no host sync)
-        SearchArgs h = args;
-        h.q_words = search_q_words(32, args.bits, args.max_len);
-        const size_t hsmem = (size_t)(kApproxThreads / 32) * h.q_words * sizeof(uint64_t);
-        cudaFuncSetAttribute(search_approx_heavy_kernel<PASS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hsmem);
-        search_approx_heavy_kernel<PASS><<<device_sm_count() * 2, kApproxThreads, hsmem, stream>>>(h);
+        SearchArgs ha = args;
+        ha.q_words = search_q_words(32, args.bits, args.max_len);
+        const size_t hsmem = (size_t)(kApproxThreads / 32) * ha.q_words * sizeof(uint64_t);
+        if (MODE == kApproxAll) {
+            cudaFuncSetAttribute(search_approx_heavy_kernel<PASS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hsmem);
+            search_approx_heavy_kernel<PASS><<<device_sm_count() * 2, kApproxThreads, hsmem, stream>>>(ha);
+        } else {
+            cudaFuncSetAttribute(search_approx_heavy_hits_kernel<PASS, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hsmem);
+            search_approx_heavy_hits_kernel<PASS, MODE><<<device_sm_count() * 2, kApproxThreads, hsmem, stream>>>(ha, h);
+        }
+    }
+}
+
+template <int G, int MODE>
+static void launch_approx_g(const SearchArgs &args, const ApproxHitArgs &h, SearchPass pass, cudaStream_t stream) {
+    if (pass == kPassCount) launch_approx_pg<kPassCount, G, MODE>(args, h, stream);
+    if (pass == kPassCountAccount) launch_approx_pg<kPassCountAccount, G, MODE>(args, h, stream);
+    if constexpr (MODE != kApproxBest)
+        if (pass == kPassWrite) launch_approx_pg<kPassWrite, G, MODE>(args, h, stream);
+}
+
+template <int MODE>
+static void launch_approx_m(const SearchArgs &args, const ApproxHitArgs &h, SearchPass pass, cudaStream_t stream) {
+    if (args.n_queries == 0) return;
+    if (args.group == 1) launch_approx_g<1, MODE>(args, h, pass, stream);
+    else if (args.group == 2) launch_approx_g<2, MODE>(args, h, pass, stream);
+    else if (args.group == 4) launch_approx_g<4, MODE>(args, h, pass, stream);
+    else if (args.group == 8) launch_approx_g<8, MODE>(args, h, pass, stream);
+    else launch_approx_g<32, MODE>(args, h, pass, stream);
+}
+
+void launch_search_approx(const SearchArgs &args, SearchPass pass, cudaStream_t stream) {
+    launch_approx_m<kApproxAll>(args, ApproxHitArgs{}, pass, stream);
+}
+
+void launch_search_approx_hits(const SearchArgs &args, const ApproxHitArgs &h, ApproxMode mode, SearchPass pass,
+                               cudaStream_t stream) {
+    if (mode == kApproxBest) launch_approx_m<kApproxBest>(args, h, pass, stream);
+    else if (mode == kApproxListed) launch_approx_m<kApproxListed>(args, h, pass, stream);
+    else launch_approx_m<kApproxAll>(args, h, pass, stream);
+}
+
+// single best: the one hit of each listed query at its offset (the scan of counts = found)
+__global__ void __launch_bounds__(256) approx_single_kernel(const uint32_t *__restrict__ hits, const uint64_t *__restrict__ offsets,
+                                                            const uint32_t *__restrict__ best_pos, const uint8_t *__restrict__ best_dist,
+                                                            uint32_t *__restrict__ positions, uint8_t *__restrict__ distances) {
+    const uint32_t n = hits[0];
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const uint32_t q = hits[1 + i];
+        const uint64_t o = offsets[q];
+        positions[o] = best_pos[q];
+        if (distances) distances[o] = best_dist[q];
+    }
+}
+
+void launch_approx_single(const SearchArgs &args, const ApproxHitArgs &h, uint8_t *d_distances, cudaStream_t stream) {
+    if (args.n_queries == 0) return;
+    const uint64_t blocks = std::min<uint64_t>((args.n_queries + 255) / 256, (uint64_t)device_sm_count() * 8);
+    approx_single_kernel<<<(unsigned)blocks, 256, 0, stream>>>(args.hits, args.counts, h.best_pos, h.best_dist, args.positions,
+                                                               d_distances);
+}
+
+// d(p) of every written hit of the listed queries, in position order: one group per query packs it again and counts the
+// mismatches of each of its windows (limit e_q: every written hit is within it, so the count is exact)
+template <int G, bool ACCOUNT>
+__global__ void __launch_bounds__(kApproxThreads) approx_distances_kernel(const SearchArgs a, const ApproxHitArgs h,
+                                                                          uint8_t *__restrict__ distances) {
+    constexpr int kGroups = kApproxThreads / G;
+    extern __shared__ uint64_t smem_q[];
+    const int lane = threadIdx.x & 31;
+    const int gl = threadIdx.x & (G - 1);
+    const uint32_t gfull = G == 32 ? 0xFFFFFFFFu : ((1u << G) - 1);
+    const uint32_t gmask = gfull << (uint32_t)(lane - gl);
+    uint64_t *qw = smem_q + (size_t)(threadIdx.x / G) * a.q_words;
+    const PackedText T = a.index->text;
+    const uint32_t n_listed = a.hits[0];
+    for (uint64_t i = (uint64_t)blockIdx.x * kGroups + threadIdx.x / G; i < n_listed; i += (uint64_t)gridDim.x * kGroups) {
+        const uint64_t q = a.hits[1 + i];
+        const uint64_t o0 = a.counts[q], o1 = a.counts[q + 1];
+        if (o0 == o1) continue;
+        const uint64_t off0 = a.q_offsets[q];
+        const uint32_t m = (uint32_t)(a.q_offsets[q + 1] - off0);
+        const uint32_t e = h.budget ? (uint32_t)h.budget[q] : a.max_mismatches;
+        pack_query_group<G>(a.q_ranks, off0, m, a.q_offsets[a.n_queries], T, (uint32_t)gl, gmask, a.error_flag, qw);
+        uint32_t n_gather = 0;
+        for (uint64_t j = o0 + gl; j < o1; j += G) {
+            distances[j] = (uint8_t)mismatches_span(T, qw, a.positions[j], 0, m, e);
+            if (ACCOUNT) n_gather += 1 + (m * T.bits >> 8);
+        }
+        if (ACCOUNT) {
+            for (int o = G >> 1; o > 0; o >>= 1) n_gather += __shfl_xor_sync(gmask, n_gather, o, G);
+            if (gl == 0) atomicAdd(a.gather_count, (unsigned long long)n_gather);
+        }
+        __syncwarp();
     }
 }
 
 template <int G>
-static void launch_approx_g(const SearchArgs &args, SearchPass pass, cudaStream_t stream) {
-    if (pass == kPassCount) launch_approx_pg<kPassCount, G>(args, stream);
-    if (pass == kPassCountAccount) launch_approx_pg<kPassCountAccount, G>(args, stream);
-    if (pass == kPassWrite) launch_approx_pg<kPassWrite, G>(args, stream);
+static void launch_distances_g(const SearchArgs &args, const ApproxHitArgs &h, uint8_t *d_distances, cudaStream_t stream) {
+    constexpr int kGroups = kApproxThreads / G;
+    const size_t smem = (size_t)kGroups * args.q_words * sizeof(uint64_t);
+    const uint64_t blocks = std::min<uint64_t>((args.n_queries + kGroups - 1) / kGroups, (uint64_t)device_sm_count() * 16);
+    if (args.gather_count) {
+        cudaFuncSetAttribute(approx_distances_kernel<G, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        approx_distances_kernel<G, true><<<(unsigned)blocks, kApproxThreads, smem, stream>>>(args, h, d_distances);
+    } else {
+        cudaFuncSetAttribute(approx_distances_kernel<G, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        approx_distances_kernel<G, false><<<(unsigned)blocks, kApproxThreads, smem, stream>>>(args, h, d_distances);
+    }
 }
 
-void launch_search_approx(const SearchArgs &args, SearchPass pass, cudaStream_t stream) {
+void launch_approx_distances(const SearchArgs &args, const ApproxHitArgs &h, uint8_t *d_distances, cudaStream_t stream) {
     if (args.n_queries == 0) return;
-    if (args.group == 1) launch_approx_g<1>(args, pass, stream);
-    else if (args.group == 2) launch_approx_g<2>(args, pass, stream);
-    else if (args.group == 4) launch_approx_g<4>(args, pass, stream);
-    else if (args.group == 8) launch_approx_g<8>(args, pass, stream);
-    else launch_approx_g<32>(args, pass, stream);
+    if (args.group == 1) launch_distances_g<1>(args, h, d_distances, stream);
+    else if (args.group == 2) launch_distances_g<2>(args, h, d_distances, stream);
+    else if (args.group == 4) launch_distances_g<4>(args, h, d_distances, stream);
+    else if (args.group == 8) launch_distances_g<8>(args, h, d_distances, stream);
+    else launch_distances_g<32>(args, h, d_distances, stream);
 }
 
 }  // namespace kb
