@@ -148,6 +148,33 @@ int kmer_b200_records_locate(const kmer_b200_records *r, const uint32_t *positio
                              uint32_t *record_out, uint32_t *offset_out);
 void kmer_b200_records_free(kmer_b200_records *r);
 
+/* ---- sequence collections: an index plus a record table starts[0..R] (starts[0] = 0, non-decreasing, starts[R] = n;
+   empty records allowed). On a collection index a window [p, p+m) exists only inside one record (no record start s with
+   p < s < p + m), so every search returns what searching each record on its own would, positions offset by the
+   record's start (seqan3: a search over a collection, reference id = record). An index without records is unchanged.
+   - Approximate search (every entry point, strategy and distances) honours the boundaries.
+   - Exact search (_search_batch, _ptrs, _text, _batch_device, _count_batch_device) runs in CORRECT mode, as approximate
+     search with max_mismatches = 0; mode UINT32_MAX means CORRECT, KMER_B200_MODE_REFERENCE_EXACT is refused with
+     KMER_B200_ERR_INVALID_ARGUMENT (the reference has no collections).
+   - Host batches take the single-copy staging (kmer_b200_last_search_host_path reports 0): the chunked pipeline does not
+     serve collections.
+   - The cross-shard and routed entry points (presence_batch_device, search_batch_device_global, search_sharded_*,
+     route_*, search_routed_device, unroute_device) return KMER_B200_ERR_UNSUPPORTED.
+   - kmer_b200_save writes file version 4 (version 3 plus the table); kmer_b200_load rebuilds it.
+   The device holds the table and a bitmap of the record starts (n / 8 bytes), counted by kmer_b200_device_bytes. */
+/* Attach the table once: KMER_B200_ERR_INVALID_ARGUMENT for null pointers, n_records = 0 or >= 2^32, starts[0] != 0, a
+   decreasing entry, starts[R] != n or records already attached; KMER_B200_ERR_UNSUPPORTED on the handles approximate
+   search refuses. kmer_b200_records_starts / _count of a parsed file fit as they are. */
+int kmer_b200_attach_records(kmer_b200_index *index, const uint64_t *starts, uint64_t n_records);
+/* The host copy of the table ([*n_records + 1]), or NULL (and *n_records = 0) for an index without records. */
+const uint64_t *kmer_b200_index_records(const kmer_b200_index *index, uint64_t *n_records);
+/* positions -> record (the last r with starts[r] <= p) and offset p - starts[r]; a position >= n gives UINT32_MAX and 0.
+   kmer_b200_locate takes host arrays, kmer_b200_locate_device device arrays (a kernel on the index's stream).
+   KMER_B200_ERR_INVALID_ARGUMENT on an index without records. */
+int kmer_b200_locate(kmer_b200_index *index, const uint32_t *positions, uint64_t n, uint32_t *record_out, uint32_t *offset_out);
+int kmer_b200_locate_device(kmer_b200_index *index, const uint32_t *d_positions, uint64_t n, uint32_t *d_record_out,
+                            uint32_t *d_offset_out);
+
 void kmer_b200_destroy(kmer_b200_index *index);
 
 /* ---- serialization: construct once, load later (the thesis assumes it, thesis/content/02_implementation.tex:44-46,
@@ -165,7 +192,8 @@ int kmer_b200_load(const char *path, const kmer_b200_config *cfg, kmer_b200_inde
    Batches of 256 MiB or more are cut into chunks that are uploaded, searched and downloaded concurrently; for 2- and
    4-bit alphabets the library's host threads pack part of the chunks before they cross PCIe (all of them when the
    buffers are pageable), the copy engine moves the rest as they are (DESIGN.md section 7, "Host path"). The buffers may
-   be pinned or pageable; they are only read, and only during the call. */
+   be pinned or pageable; they are only read, and only during the call. A collection index (kmer_b200_attach_records)
+   answers in CORRECT mode, with hits inside one record only. */
 int kmer_b200_search_batch(kmer_b200_index *index, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t n_queries,
                            uint32_t mode, kmer_b200_result **out);
 

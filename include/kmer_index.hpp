@@ -26,6 +26,7 @@
 //     std::vector<std::vector<dna4>> take 0.47 s, 63 ms of it inside the library (profiles/r02/header_bench.txt).
 //   * an index can span several GPUs: kmer_index(text, devices) builds it from key-range parts on all of them and
 //     search_batch() stripes the batch over them (kmer_b200_config.device_ids).
+//   * kmer_index(texts, kmer::collection) indexes a collection of texts: no hit spans two of them, locate() gives (text, offset).
 //   * the alphabet requirement is `a.to_rank()` plus kmer::alphabet_size<A>; seqan3 alphabets satisfy it when
 //     seqan3 is available, kmer::dna4 / dna5 / dna15 / aa27 below are rank-only stand-ins.
 #pragma once
@@ -292,6 +293,16 @@ namespace kmer
 
     // tag for the shared-positions constructor below
     inline constexpr struct shared_positions_t {} shared_positions{};
+    // tag for the collection constructor below
+    inline constexpr struct collection_t {} collection{};
+
+    // where a hit of a collection index lies: the text (record) and the offset inside it (kmer_index::locate)
+    struct record_hit
+    {
+        std::uint32_t record = 0;
+        std::uint32_t offset = 0;
+        friend constexpr bool operator==(record_hit a, record_hit b) noexcept { return a.record == b.record && a.offset == b.offset; }
+    };
 
     // kmer_index.hpp:350-566
     template<alphabet alphabet_t, typename position_t, std::size_t... ks>
@@ -334,6 +345,32 @@ namespace kmer
         {
             std::vector<std::int32_t> ids(devices.begin(), devices.end());
             build(text, mode, ids.empty() ? -1 : ids[0], ids.data(), std::uint32_t(ids.size()));
+        }
+
+        // kmer_index(texts, kmer::collection): one index over a collection of texts (a genome's chromosomes, a set of
+        // transcripts), searched in CORRECT mode. No hit spans two texts: search_batch / search_approx_batch return what
+        // searching each text on its own would, positions offset by the text's start in the concatenation; locate()
+        // maps them to (text, offset) -- seqan3's (reference id, position) (kmer_b200_attach_records)
+        template<std::ranges::range texts_t>
+        kmer_index(texts_t const& texts, collection_t, int device = -1)
+        {
+            std::vector<std::uint8_t> ranks;
+            std::vector<std::uint64_t> starts{0};
+            gather_ranks(texts, ranks, starts);
+            build(ranks, KMER_B200_MODE_CORRECT, device, nullptr, 0);
+            detail::check(kmer_b200_attach_records(_handle, starts.data(), starts.size() - 1));
+        }
+
+        // (text, offset) of every position of a search result on a collection index, in the result's order; throws on an
+        // index without texts
+        std::vector<record_hit> locate(kmer_batch_result<position_t> const& result) const
+        {
+            const std::size_t n = result.positions.size();
+            std::vector<std::uint32_t> rec(n), off(n);
+            detail::check(kmer_b200_locate(_handle, result.positions.data(), n, rec.data(), off.data()));
+            std::vector<record_hit> out(n);
+            for (std::size_t i = 0; i < n; ++i) out[i] = record_hit{rec[i], off[i]};
+            return out;
         }
 
     private:

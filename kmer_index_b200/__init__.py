@@ -151,9 +151,16 @@ class Records:
         end = self._data.find(b"\n", o)
         return self._data[o + 1:end if end >= 0 else len(self._data)].rstrip(b"\r").decode(errors="replace")
 
-    def index(self, ks: Sequence[int], **kw) -> "KmerIndex":
-        return KmerIndex(None, self.sigma, ks, text_device_ptr=int(self._L.kmer_b200_records_ranks_device(self._h)),
-                         n=self.n_symbols, **kw)
+    def index(self, ks: Sequence[int], collection: bool = False, **kw) -> "KmerIndex":
+        """KmerIndex over the concatenated records. collection=True: a collection index (KmerIndex.attach_records with
+        these starts, built in MODE_CORRECT): no hit spans two records, KmerIndex.locate gives (record, offset)."""
+        if collection:
+            kw["mode"] = MODE_CORRECT
+        ix = KmerIndex(None, self.sigma, ks, text_device_ptr=int(self._L.kmer_b200_records_ranks_device(self._h)),
+                       n=self.n_symbols, **kw)
+        if collection:
+            ix.attach_records(self.starts)
+        return ix
 
     def locate(self, positions, query_len: int = 0):
         """(record, offset) of each position; record == 0xFFFFFFFF where a match of query_len symbols would run over the
@@ -326,6 +333,47 @@ class KmerIndex:
         self.sigma = None
         self.n = int(self.element_info(0).n_kmers) + self.ks[0] - 1
         return self
+
+    # -- sequence collections
+    def attach_records(self, starts) -> None:
+        """Make this a collection index (kmer_b200_attach_records): starts[0..R] with starts[0] = 0, non-decreasing,
+        starts[R] = n. Every search then reports only windows inside one record; exact search runs in MODE_CORRECT."""
+        s = np.ascontiguousarray(np.asarray(starts, dtype=np.uint64))
+        if s.size < 2:
+            raise ValueError("starts needs at least two entries (one record)")
+        _capi.check(self._L.kmer_b200_attach_records(self._h, s.ctypes.data_as(_capi.u64p), s.size - 1))
+
+    @property
+    def records(self) -> np.ndarray | None:
+        """The record table starts[0..R] of a collection index (uint64), or None."""
+        n = C.c_uint64(0)
+        p = self._L.kmer_b200_index_records(self._h, C.byref(n))
+        return np.ctypeslib.as_array(p, shape=(n.value + 1,)).copy() if p else None
+
+    def locate(self, positions):
+        """(record, offset) of each hit position of a collection index: record = the last r with starts[r] <= p, offset =
+        p - starts[r] (0xFFFFFFFF, 0 for p >= n). A numpy array (or list) is located on the host and gives uint32 numpy
+        arrays; a torch tensor or device view (int32 / uint32) is located by a kernel and gives int32 tensors on its
+        device."""
+        if hasattr(positions, "__cuda_array_interface__") or type(positions).__module__.startswith("torch"):
+            import torch
+            t = torch.as_tensor(positions, device="cuda") if not isinstance(positions, torch.Tensor) else positions
+            if t.dtype not in (torch.int32, torch.uint32) or not t.is_cuda:
+                raise TypeError("device positions must be an int32 / uint32 CUDA tensor or view")
+            t = t.contiguous()
+            rec = torch.empty(t.numel(), dtype=torch.int32, device=t.device)
+            off = torch.empty(t.numel(), dtype=torch.int32, device=t.device)
+            torch.cuda.current_stream(t.device).synchronize()
+            _capi.check(self._L.kmer_b200_locate_device(self._h, C.c_void_p(t.data_ptr()), t.numel(), C.c_void_p(rec.data_ptr()),
+                                                        C.c_void_p(off.data_ptr())))
+            torch.cuda.synchronize(t.device)   # the kernel ran on the index's stream
+            return rec, off
+        p = np.ascontiguousarray(np.asarray(positions, dtype=np.uint32))
+        rec = np.zeros(p.size, dtype=np.uint32)
+        off = np.zeros(p.size, dtype=np.uint32)
+        _capi.check(self._L.kmer_b200_locate(self._h, p.ctypes.data_as(_capi.u32p), p.size, rec.ctypes.data_as(_capi.u32p),
+                                             off.ctypes.data_as(_capi.u32p)))
+        return rec, off
 
     # -- lifetime
     def close(self):

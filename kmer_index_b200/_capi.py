@@ -89,6 +89,10 @@ SYMBOLS = {
     "kmer_b200_records_ranks_device": (C.c_void_p, [C.c_void_p]),
     "kmer_b200_records_locate": (C.c_int, [C.c_void_p, u32p, C.c_uint64, C.c_uint64, u32p, u32p]),
     "kmer_b200_records_free": (None, [C.c_void_p]),
+    "kmer_b200_attach_records": (C.c_int, [C.c_void_p, u64p, C.c_uint64]),
+    "kmer_b200_index_records": (u64p, [C.c_void_p, u64p]),
+    "kmer_b200_locate": (C.c_int, [C.c_void_p, u32p, C.c_uint64, u32p, u32p]),
+    "kmer_b200_locate_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
     "kmer_b200_destroy": (None, [C.c_void_p]),
     "kmer_b200_save": (C.c_int, [C.c_void_p, C.c_char_p]),
     "kmer_b200_load": (C.c_int, [C.c_char_p, C.POINTER(Config), C.POINTER(C.c_void_p)]),

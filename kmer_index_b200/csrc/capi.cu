@@ -231,6 +231,11 @@ struct kmer_b200_index {
     size_t h_pinned_cap = 0;
     // a multi-device handle (cfg.n_devices > 1) owns one whole index per device and nothing else
     std::vector<kmer_b200_index *> replicas;
+    // collection index (kmer_b200_attach_records): the record table starts[0..R] (host and device) and the boundary
+    // bitmap of DeviceIndex::boundary; empty / null otherwise
+    std::vector<uint64_t> starts;
+    uint64_t *d_starts = nullptr;
+    uint64_t *d_boundary = nullptr;
 };
 
 static inline kmer_b200_index *primary(kmer_b200_index *ix) { return (ix && !ix->replicas.empty()) ? ix->replicas[0] : ix; }
@@ -908,6 +913,56 @@ int finalize_index(kmer_b200_index *ix) {
     return KMER_B200_OK;
 }
 
+// a record table starts[0..R] of this index's text: 0 < R < 2^32, starts[0] = 0, non-decreasing, starts[R] = n
+int records_check(const kmer_b200_index *ix, const uint64_t *starts, uint64_t n_records) {
+    if (n_records == 0 || n_records >= (1ull << 32)) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "n_records must be in [1, 2^32)");
+    if (starts[0] != 0 || starts[n_records] != ix->n) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "starts[0] must be 0 and starts[R] = n");
+    for (uint64_t r = 0; r < n_records; ++r)
+        if (starts[r + 1] < starts[r]) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "record starts must not decrease");
+    return KMER_B200_OK;
+}
+
+// Make ix a collection index (the table passed records_check): the device copy of the table, the boundary bitmap
+// (one scatter of the record starts) and the per-m window tables of DeviceIndex.
+int attach_records_impl(kmer_b200_index *ix, const uint64_t *starts, uint64_t n_records) {
+    const uint64_t words = ix->n / 64 + 1;
+    uint64_t *d_starts = nullptr, *d_bits = nullptr;
+    const uint64_t bytes_before = ix->device_bytes;
+    if (dev_alloc(ix, &d_starts, n_records + 1, true) || dev_alloc(ix, &d_bits, words, true)) {
+        dev_free(ix, d_starts);
+        ix->device_bytes = bytes_before;
+        return KMER_B200_ERR_OUT_OF_MEMORY;
+    }
+    cudaMemcpyAsync(d_starts, starts, (n_records + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, ix->stream);
+    cudaMemsetAsync(d_bits, 0, words * sizeof(uint64_t), ix->stream);
+    kb::launch_record_boundaries(d_starts, n_records, ix->n, d_bits, ix->stream);
+    kb::DeviceIndex &D = ix->host_index;
+    D.boundary = d_bits;
+    for (uint32_t m = 0; m < 9; ++m) D.n_win[m] = 0, D.first_win[m] = UINT64_MAX;
+    for (uint64_t r = 0; r < n_records; ++r) {
+        const uint64_t len = starts[r + 1] - starts[r];
+        for (uint32_t m = 1; m < 9 && m <= len; ++m) {
+            D.n_win[m] += len - m + 1;
+            D.first_win[m] = std::min(D.first_win[m], starts[r]);
+        }
+    }
+    cudaMemcpyAsync(ix->d_index, &D, sizeof(D), cudaMemcpyHostToDevice, ix->stream);
+    cudaError_t e = cudaStreamSynchronize(ix->stream);
+    if (e == cudaSuccess) e = cudaGetLastError();
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        D.boundary = nullptr;
+        dev_free(ix, d_starts);
+        dev_free(ix, d_bits);
+        ix->device_bytes = bytes_before;
+        return fail(KMER_B200_ERR_CUDA, std::string("attach_records: ") + cudaGetErrorString(e));
+    }
+    ix->starts.assign(starts, starts + n_records + 1);
+    ix->d_starts = d_starts;
+    ix->d_boundary = d_bits;
+    return KMER_B200_OK;
+}
+
 // characters -> ranks through a 256-entry table, in place (SURVEY.md 8f.3: real inputs are characters)
 __global__ void __launch_bounds__(256) translate_kernel(uint8_t *__restrict__ data, uint64_t n, const uint8_t *__restrict__ lut) {
     __shared__ uint8_t s_lut[256];
@@ -1166,6 +1221,7 @@ struct FileElement {
 };
 constexpr uint32_t kFileVersion = 3;  // 2: an element's sorted hashes are optional (FileElement::has_keys bit 0)
                                       // 3: has_keys bit 1 = a view of the largest k's arrays (shared positions): no arrays follow
+constexpr uint32_t kFileVersionRecords = 4;  // a collection index: version 3, then R and starts[0..R] (u64) after the elements
 constexpr size_t kIoChunk = 64u << 20;
 
 // Double-buffered: h_buf holds two halves of kIoChunk bytes; the copy of chunk c + 1 runs while chunk c is written to
@@ -1359,6 +1415,17 @@ int search_begin(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off,
                  PendingSearch *p, const PackedQueries *packed = nullptr, int32_t max_mismatches = -1,
                  const kmer_b200_approx_options *hit_opt = nullptr) {
     using namespace kb;
+    const bool collection = !ix->starts.empty();
+    if (collection && max_mismatches < 0) {
+        // exact search on a collection: CORRECT mode, answered by approximate search with e = 0 (the same result on a
+        // plain index), whose kernels honour the record boundaries
+        if (mode == KMER_B200_MODE_REFERENCE_EXACT)
+            return fail(KMER_B200_ERR_INVALID_ARGUMENT, "a collection index searches in CORRECT mode only: the reference has no collections");
+        if (mode != UINT32_MAX && mode != KMER_B200_MODE_CORRECT) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "unknown mode");
+        if (d_present4 || d_present_global || packed)
+            return fail(KMER_B200_ERR_UNSUPPORTED, "a collection index is unsharded: no cross-shard search");
+        max_mismatches = 0;
+    }
     const bool approx = max_mismatches >= 0;  // approximate search: the semantics of CORRECT mode, any query length
     if (approx) mode = KMER_B200_MODE_CORRECT;
     if (mode == UINT32_MAX) mode = ix->cfg.mode;
@@ -1431,7 +1498,7 @@ int search_begin(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off,
         for (int r = 0; r <= kb::kMaxPosParts; ++r) a.parts0.first[r] = E0.part_first[r];
         for (int r = 0; r < kb::kMaxPosParts; ++r) a.parts0.ptr[r] = E0.pos_part[r];
     }
-    a.approx = approx ? 1 : 0;
+    a.approx = approx ? (collection ? 2 : 1) : 0;
     a.max_mismatches = approx ? (uint32_t)max_mismatches : 0;
     a.lean_ok = !approx && a.single_k && ix->sigma == 4 && ix->elems[0].dev.shift == 0 && ix->elems[0].key_bytes == 4 && !d_present4 &&
                 !d_present_global && ix->cfg.profile < 2 && !std::getenv("KMER_B200_NO_LEAN");
@@ -1685,6 +1752,9 @@ static int search_batch_multi(kmer_b200_index *group, const uint8_t *q_ranks, co
 #define KB_NOT_ON_GROUP(ix)                                                                                         \
     if ((ix) && !(ix)->replicas.empty())                                                                            \
         return fail(KMER_B200_ERR_UNSUPPORTED, "device-pointer entry points are not available on a multi-device handle")
+#define KB_NOT_ON_COLLECTION(ix)                                                                                    \
+    if ((ix) && !(ix)->starts.empty())                                                                              \
+        return fail(KMER_B200_ERR_UNSUPPORTED, "cross-shard and routed searches are not available on a collection index")
 
 int kmer_b200_create(const uint8_t *ranks, uint64_t n, uint32_t sigma, const uint32_t *ks, uint32_t n_ks,
                      const kmer_b200_config *cfg, kmer_b200_index **out) {
@@ -1713,7 +1783,7 @@ int kmer_b200_save(kmer_b200_index *ix, const char *path) {
     int s = h_buf ? 0 : fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed");
     FileHeader h{};
     std::memcpy(h.magic, "KMERB200", 8);
-    h.version = kFileVersion;
+    h.version = ix->starts.empty() ? kFileVersion : kFileVersionRecords;
     h.sigma = ix->sigma;
     h.bits = ix->bits;
     h.n_ks = (uint32_t)ix->ks.size();
@@ -1737,6 +1807,11 @@ int kmer_b200_save(kmer_b200_index *ix, const char *path) {
         if (s == 0) s = write_device_array(ix, f, he.d_pos, he.dev.n_kmers * 4, h_buf);
         if (s == 0) s = write_device_array(ix, f, he.d_dir, he.dev.dir_entries * 4, h_buf);
     }
+    if (s == 0 && !ix->starts.empty()) {
+        const uint64_t n_records = ix->starts.size() - 1;
+        if (fwrite(&n_records, sizeof(n_records), 1, f) != 1 || fwrite(ix->starts.data(), sizeof(uint64_t), n_records + 1, f) != n_records + 1)
+            s = fail(KMER_B200_ERR_INVALID_ARGUMENT, "short write");
+    }
     pinned_put(h_buf, cap);
     if (std::fclose(f) != 0 && s == 0) s = fail(KMER_B200_ERR_INVALID_ARGUMENT, "close failed");
     return s;
@@ -1748,7 +1823,7 @@ int kmer_b200_load(const char *path, const kmer_b200_config *cfg_in, kmer_b200_i
     FILE *f = std::fopen(path, "rb");
     if (!f) return fail(KMER_B200_ERR_INVALID_ARGUMENT, std::string("cannot open ") + path);
     FileHeader h{};
-    if (fread(&h, sizeof(h), 1, f) != 1 || std::memcmp(h.magic, "KMERB200", 8) != 0 || (h.version != kFileVersion && h.version != 2) ||
+    if (fread(&h, sizeof(h), 1, f) != 1 || std::memcmp(h.magic, "KMERB200", 8) != 0 || h.version < 2 || h.version > kFileVersionRecords ||
         h.n_ks == 0 || h.n_ks > (uint32_t)kb::kMaxElements) {
         std::fclose(f);
         return fail(KMER_B200_ERR_INVALID_ARGUMENT, "not a kmer_b200 index file (or an unknown version)");
@@ -1834,7 +1909,20 @@ int kmer_b200_load(const char *path, const kmer_b200_config *cfg_in, kmer_b200_i
         } else {
             ix->cfg.reserved &= ~(uint32_t)KMER_B200_FLAG_SHARED_POSITIONS;  // what the file holds decides
         }
-        return r ? r : finalize_index(ix);
+        std::vector<uint64_t> rec;  // version 4: the record table of a collection index
+        if (r == 0 && h.version >= kFileVersionRecords) {
+            uint64_t n_records = 0;
+            if (fread(&n_records, sizeof(n_records), 1, f) != 1 || n_records == 0 || n_records >= (1ull << 32))
+                return fail(KMER_B200_ERR_INVALID_ARGUMENT, "corrupt record table in index file");
+            rec.resize(n_records + 1);
+            if (fread(rec.data(), sizeof(uint64_t), n_records + 1, f) != n_records + 1)
+                return fail(KMER_B200_ERR_INVALID_ARGUMENT, "truncated index file");
+            if ((r = records_check(ix, rec.data(), n_records)) != 0) return r;
+        }
+        if (r == 0) r = finalize_index(ix);
+        if (r == 0 && !rec.empty()) r = approx_check(ix, 0);
+        if (r == 0 && !rec.empty()) r = attach_records_impl(ix, rec.data(), rec.size() - 1);
+        return r;
     };
     if (s == 0) s = load();
     std::fclose(f);
@@ -1864,6 +1952,8 @@ void kmer_b200_destroy(kmer_b200_index *ix) {
         dev_free(ix, (uint8_t *)he.d_keys);
     }
     dev_free(ix, ix->d_text);
+    dev_free(ix, ix->d_starts);
+    dev_free(ix, ix->d_boundary);
     dev_free(ix, ix->d_sum_off);
     dev_free(ix, ix->d_sum_elem);
     dev_free(ix, ix->d_use_multi);
@@ -1949,6 +2039,7 @@ int kmer_b200_search_batch_device_global(kmer_b200_index *ix, const uint8_t *d_q
                                          uint64_t max_len, uint32_t mode, const void *d_present_global,
                                          uint32_t present_format, kmer_b200_result **out) {
     KB_NOT_ON_GROUP(ix);
+    KB_NOT_ON_COLLECTION(ix);
     if (!ix || !out || !d_off || !d_present_global || present_format > 1)
         return fail(KMER_B200_ERR_INVALID_ARGUMENT, "bad argument");
     *out = nullptr;
@@ -1964,6 +2055,7 @@ struct kmer_b200_pending {
 int kmer_b200_search_sharded_begin(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
                                    uint64_t max_len, uint32_t mode, uint32_t *d_present4, kmer_b200_pending **out) {
     KB_NOT_ON_GROUP(ix);
+    KB_NOT_ON_COLLECTION(ix);
     if (!ix || !out || !d_off || !d_present4) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
     *out = nullptr;
     DeviceGuard guard(ix->device);
@@ -2045,6 +2137,7 @@ int kmer_b200_search_sharded_add_counts(kmer_b200_pending *h, const uint32_t *d_
 int kmer_b200_presence_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
                                     uint64_t max_len, uint32_t mode, void *d_present, uint32_t present_format) {
     KB_NOT_ON_GROUP(ix);
+    KB_NOT_ON_COLLECTION(ix);
     using namespace kb;
     if (!ix || !d_off || !d_present || present_format > 1) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "bad argument");
     if (ix->cfg.reserved & KMER_B200_FLAG_SHARED_POSITIONS)
@@ -2503,7 +2596,7 @@ static int search_batch_host(kmer_b200_index *ix, const uint8_t *q_ranks, const 
     const uint64_t n_sym = q_offsets[Q] - q_offsets[0];
     if (n_sym && !q_ranks) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "q_ranks is null");
     // batches whose transfer dominates (>= 256 MiB over PCIe) are pipelined in chunks
-    if (!lut256 && Q >= (1u << 18) && n_sym + Q * 17 >= (256ull << 20) && !std::getenv("KMER_B200_NO_PIPELINE")) {
+    if (!lut256 && ix->starts.empty() && Q >= (1u << 18) && n_sym + Q * 17 >= (256ull << 20) && !std::getenv("KMER_B200_NO_PIPELINE")) {
         // The share of raw chunks. Pageable input cannot be DMA-ed directly (the driver would stage it at a fraction of the
         // link rate): every chunk is packed straight out of the caller's memory into a pinned ring. Pinned input of 2- and
         // 4-bit alphabets: the share comes from the host's streaming pack rate, measured once per process on the first
@@ -3113,10 +3206,9 @@ const uint64_t *kmer_b200_records_starts(const kmer_b200_records *r) { return r 
 const uint64_t *kmer_b200_records_header_offsets(const kmer_b200_records *r) { return r ? r->header_offsets.data() : nullptr; }
 const uint8_t *kmer_b200_records_ranks_device(const kmer_b200_records *r) { return r ? r->d_ranks : nullptr; }
 
-int kmer_b200_records_locate(const kmer_b200_records *r, const uint32_t *positions, uint64_t n, uint64_t query_len,
-                             uint32_t *record_out, uint32_t *offset_out) {
-    if (!r || (n && (!positions || !record_out || !offset_out))) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
-    const std::vector<uint64_t> &s = r->starts;
+// positions -> (record, offset) by a binary search in the record table s[0..R]; see kmer_b200_records_locate
+static void locate_host(const std::vector<uint64_t> &s, const uint32_t *positions, uint64_t n, uint64_t query_len,
+                        uint32_t *record_out, uint32_t *offset_out) {
     for (uint64_t i = 0; i < n; ++i) {
         const uint64_t p = positions[i];
         const size_t rec = (size_t)(std::upper_bound(s.begin(), s.end(), p) - s.begin()) - 1;
@@ -3128,6 +3220,48 @@ int kmer_b200_records_locate(const kmer_b200_records *r, const uint32_t *positio
         record_out[i] = (query_len && p + query_len > s[rec + 1]) ? UINT32_MAX : (uint32_t)rec;
         offset_out[i] = (uint32_t)(p - s[rec]);
     }
+}
+
+int kmer_b200_records_locate(const kmer_b200_records *r, const uint32_t *positions, uint64_t n, uint64_t query_len,
+                             uint32_t *record_out, uint32_t *offset_out) {
+    if (!r || (n && (!positions || !record_out || !offset_out))) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    locate_host(r->starts, positions, n, query_len, record_out, offset_out);
+    return KMER_B200_OK;
+}
+
+// ---- collection index ----------------------------------------------------------------------------------------------
+int kmer_b200_attach_records(kmer_b200_index *ix, const uint64_t *starts, uint64_t n_records) {
+    if (!ix || !starts) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    if (n_records == 0 || n_records >= (1ull << 32)) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "n_records must be in [1, 2^32)");
+    KB_TRY(approx_check(ix, 0));  // the handles approximate search refuses hold no collection either
+    if (!ix->starts.empty()) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "records are attached already");
+    KB_TRY(records_check(ix, starts, n_records));
+    DeviceGuard guard(ix->device);
+    std::lock_guard<std::mutex> lock(ix->mu);
+    return attach_records_impl(ix, starts, n_records);
+}
+
+const uint64_t *kmer_b200_index_records(const kmer_b200_index *ix, uint64_t *n_records) {
+    const bool has = ix && !ix->starts.empty();
+    if (n_records) *n_records = has ? ix->starts.size() - 1 : 0;
+    return has ? ix->starts.data() : nullptr;
+}
+
+int kmer_b200_locate(kmer_b200_index *ix, const uint32_t *positions, uint64_t n, uint32_t *record_out, uint32_t *offset_out) {
+    if (!ix || (n && (!positions || !record_out || !offset_out))) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    if (ix->starts.empty()) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "the index has no records: kmer_b200_attach_records");
+    locate_host(ix->starts, positions, n, 0, record_out, offset_out);
+    return KMER_B200_OK;
+}
+
+int kmer_b200_locate_device(kmer_b200_index *ix, const uint32_t *d_positions, uint64_t n, uint32_t *d_record_out,
+                            uint32_t *d_offset_out) {
+    if (!ix || (n && (!d_positions || !d_record_out || !d_offset_out))) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    if (ix->starts.empty()) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "the index has no records: kmer_b200_attach_records");
+    DeviceGuard guard(ix->device);
+    std::lock_guard<std::mutex> lock(ix->mu);
+    kb::launch_locate(ix->d_starts, ix->starts.size() - 1, d_positions, n, d_record_out, d_offset_out, ix->stream);
+    KB_CUDA(cudaGetLastError());
     return KMER_B200_OK;
 }
 
@@ -3145,6 +3279,7 @@ void kmer_b200_records_free(kmer_b200_records *r) {
 static int routable(const kmer_b200_index *ix) {
     if (!ix) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null index");
     if (!ix->replicas.empty()) return fail(KMER_B200_ERR_UNSUPPORTED, "not available on a multi-device handle");
+    KB_NOT_ON_COLLECTION(ix);
     if (ix->ks.size() != 1 || ix->elems[0].key_bytes != 4 || ix->elems[0].dev.shift != 0)
         return fail(KMER_B200_ERR_UNSUPPORTED, "query routing needs a single-k index with 32-bit hashes and a dense directory");
     return 0;

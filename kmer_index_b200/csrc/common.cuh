@@ -278,6 +278,28 @@ struct DeviceIndex {
     // key-range multi-GPU search: per element, a bitmap over the WHOLE key space (bit h = hash h occurs in the text),
     // or null. With it a part answers "does this part of the query occur anywhere" for hashes other parts own.
     const uint64_t *presence[kMaxElements];
+    // Collection index (kmer_b200_attach_records), else null / zero: bit s of `boundary` is set for every record start
+    // 0 < s < n, so a window [p, p+m) lies inside one record exactly when no bit of [p+1, p+m) is set. Per query length
+    // m = 1..8 (the "every window" answer of m <= e): n_win[m] = in-record windows, first_win[m] = the lowest one.
+    const uint64_t *boundary;
+    uint64_t n_win[9];
+    uint64_t first_win[9];
 };
+
+// no record of a collection index starts inside (p, p+m): ceil(m / 64) + 1 words at most, read like the text
+__device__ __forceinline__ bool window_in_record(const uint64_t *boundary, uint64_t p, uint32_t m) {
+    if (m <= 1) return true;
+    const uint64_t a = p + 1, b = p + m - 1;  // the bits [a, b]
+    uint64_t w = a >> 6;
+    const uint64_t w_last = b >> 6;
+    uint64_t x = gather64(boundary + w) & (~0ull << (a & 63));
+    while (w < w_last) {
+        if (x) return false;
+        x = gather64(boundary + ++w);
+    }
+    const uint32_t hb = (uint32_t)(b & 63);
+    if (hb != 63) x &= (2ull << hb) - 1;
+    return x == 0;
+}
 
 }  // namespace kb

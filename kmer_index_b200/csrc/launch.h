@@ -97,7 +97,8 @@ struct SearchArgs {
     unsigned long long *gather_count;  // device or null: accumulates the 32-byte sectors the batch must gather
     uint32_t *error_flag;            // device u32[4]: [0] bit 0 = query rank >= sigma; [1] = #segments to sort;
                                      // [2..3] = u64 mask of sub-k query lengths that found no auxiliary element
-    uint32_t approx;                 // 1: approximate search (search_approx.cu): every window within max_mismatches substitutions
+    uint32_t approx;                 // 1: approximate search (search_approx.cu): every window within max_mismatches substitutions;
+                                     // 2: the same on a collection index (windows inside one record only)
     uint32_t max_mismatches;         // e <= kMaxMismatches
 };
 
@@ -128,6 +129,11 @@ void launch_approx_single(const SearchArgs &args, const ApproxHitArgs &h, uint8_
 // h.budget[q], else args.max_mismatches
 void launch_approx_distances(const SearchArgs &args, const ApproxHitArgs &h, uint8_t *d_distances, cudaStream_t stream);
 uint32_t search_q_words(uint32_t group, uint32_t bits, uint64_t max_len);
+// collection index (search_approx.cu; SearchArgs::approx = 2 selects the record-boundary check of the approximate
+// kernels): bit s of d_bits (zeroed, n / 64 + 1 words) = a record starts at s, 0 < s < n; and (record, offset) per position
+void launch_record_boundaries(const uint64_t *d_starts, uint64_t n_records, uint64_t n, uint64_t *d_bits, cudaStream_t stream);
+void launch_locate(const uint64_t *d_starts, uint64_t n_records, const uint32_t *d_positions, uint64_t n_pos, uint32_t *d_record,
+                   uint32_t *d_offset, cudaStream_t stream);
 // deferred count pass epilogue: zero the counts / set THROW according to the combined presence flags
 void launch_finalize_deferred(uint64_t *d_counts, uint8_t *d_status, const uint8_t *d_defer, const uint32_t *d_present4_global,
                               uint64_t n_queries, cudaStream_t stream);

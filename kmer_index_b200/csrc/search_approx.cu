@@ -21,6 +21,11 @@
 // there (one hit per listed query, launch_approx_single). All-best and strata run the count and write passes again
 // over the listed queries only (kApproxListed), each with its own budget e_q = min(e, d_min + s): the e_q + 1 seeds
 // enumerate exactly the windows with d <= e_q. launch_approx_distances recomputes d(p) of every written hit.
+//
+// Collection index (COLL, args.approx == 2): a window counts only when it lies inside one record (window_in_record on
+// the boundary bitmap), checked where a verified window becomes a hit or a lane's best, so every pass and strategy sees
+// in-record windows only. The check depends on p alone, so the first-error-free-seed dedup stays exact. The kernels of
+// a plain index are instantiated without it.
 #include <algorithm>
 
 #include "launch.h"
@@ -33,7 +38,7 @@ constexpr int kApproxThreads = 256;
 // PASS: kPassCount, kPassCountAccount (count + gathered sectors) or kPassWrite. HEAVY: the warp-per-query launch over
 // the heavy list. MODE: kApproxAll (budget a.max_mismatches, every query), kApproxListed (budget h.budget[q], the
 // queries of a.hits; the count pass does not list them again) or kApproxBest (count passes only: the best pass).
-template <int PASS_, int G, bool HEAVY, int MODE = kApproxAll>
+template <int PASS_, int G, bool HEAVY, int MODE = kApproxAll, bool COLL = false>
 __device__ __forceinline__ void approx_query(const SearchArgs &a, const uint64_t q, uint64_t *smem_q,
                                              const ApproxHitArgs &h = ApproxHitArgs{}) {
     constexpr bool kAccount = PASS_ == kPassCountAccount;
@@ -94,12 +99,23 @@ __device__ __forceinline__ void approx_query(const SearchArgs &a, const uint64_t
     uint64_t n_hits = 0;
     bool unsorted = false;
     if (m <= e || (uint64_t)m > T.n) {
-        // every window is within e substitutions of a query of at most e symbols (or no window fits)
-        const uint64_t n_win = (uint64_t)m > T.n ? 0 : T.n - m + 1;
+        // every window is within e substitutions of a query of at most e symbols (or no window fits); on a collection
+        // the in-record ones: counted from the table, written by scanning every window start
+        const uint64_t n_win = (uint64_t)m > T.n ? 0 : (COLL ? ix.n_win[m] : T.n - m + 1);
         HAND_OFF_IF_HEAVY(n_win)
         n_hits = n_win;
-        if (PASS == kPassWrite)
+        if (PASS == kPassWrite && !COLL)
             for (uint64_t p = gl; p < n_win; p += G) a.positions[out_base + p] = (uint32_t)p;
+        if (PASS == kPassWrite && COLL) {
+            uint64_t k = 0;
+            for (uint64_t p0 = 0; p0 + m <= T.n && k < n_win; p0 += G) {
+                const uint64_t p = p0 + gl;
+                const bool ok = p + m <= T.n && window_in_record(ix.boundary, p, m);
+                const uint32_t b = GBALLOT(ok);
+                if (ok) a.positions[out_base + k + __popc(b & lt_mask)] = (uint32_t)p;
+                k += __popc(b);
+            }
+        }
     } else {
         const uint32_t L = m / (e + 1);
         // the seed element: the largest k <= L, else the smallest k (> L), enumerated as prefix slabs
@@ -179,10 +195,19 @@ __device__ __forceinline__ void approx_query(const SearchArgs &a, const uint64_t
                             // the limit follows this lane's best distance: equal distances are still counted exactly
                             const uint32_t lim = best == ~0ull ? e : (uint32_t)(best >> 32);
                             const uint32_t d = mismatches_span(T, qw, p, 0, m, lim);
-                            if (d <= lim) best = min(best, ((uint64_t)d << 32) | p);
+                            bool in = d <= lim;
+                            if (COLL && in) {
+                                in = window_in_record(ix.boundary, p, m);
+                                if (kAccount) ++n_gather;
+                            }
+                            if (in) best = min(best, ((uint64_t)d << 32) | p);
                             ok = false;
                         } else {
                             ok = mismatches_span(T, qw, p, 0, m, e) <= e;
+                            if (COLL && ok) {
+                                ok = window_in_record(ix.boundary, p, m);
+                                if (kAccount) ++n_gather;
+                            }
                         }
                         if (kAccount) n_gather += 1 + (m * T.bits >> 8);
                     }
@@ -202,7 +227,11 @@ __device__ __forceinline__ void approx_query(const SearchArgs &a, const uint64_t
     }
     if (kBest) {
         for (int o = G >> 1; o > 0; o >>= 1) best = min(best, (uint64_t)__shfl_xor_sync(gmask, best, o, G));
-        if (best == ~0ull && m <= a.max_mismatches && (uint64_t)m <= T.n) best = (uint64_t)m << 32;  // every window: d = m
+        if (best == ~0ull && m <= a.max_mismatches && (uint64_t)m <= T.n) {
+            // every window: d = m, lowest at 0 (on a collection: at the first in-record window, if any)
+            if (!COLL) best = (uint64_t)m << 32;
+            else if (ix.n_win[m] != 0) best = ((uint64_t)m << 32) | ix.first_win[m];
+        }
         if (gl == 0) {
             const bool found = best != ~0ull;
             const uint32_t d = (uint32_t)(best >> 32);
@@ -239,18 +268,18 @@ __device__ __forceinline__ void approx_query(const SearchArgs &a, const uint64_t
 
 // count pass: one group per query; write pass (and every pass of kApproxListed): the queries the count pass listed as
 // having hits
-template <int PASS, int G, int MODE>
+template <int PASS, int G, int MODE, bool COLL = false>
 __device__ __forceinline__ void approx_grid(const SearchArgs &a, const ApproxHitArgs &h, uint64_t *smem_q) {
     constexpr int kGroups = kApproxThreads / G;
     if ((PASS == kPassWrite || MODE == kApproxListed) && a.hits != nullptr) {
         const uint32_t n_listed = a.hits[0];
         for (uint64_t i = (uint64_t)blockIdx.x * kGroups + threadIdx.x / G; i < n_listed; i += (uint64_t)gridDim.x * kGroups) {
-            approx_query<PASS, G, false, MODE>(a, (uint64_t)a.hits[1 + i], smem_q, h);
+            approx_query<PASS, G, false, MODE, COLL>(a, (uint64_t)a.hits[1 + i], smem_q, h);
             __syncwarp();
         }
     } else {
         const uint64_t q = (uint64_t)blockIdx.x * kGroups + threadIdx.x / G;
-        if (q < a.n_queries) approx_query<PASS, G, false, MODE>(a, q, smem_q, h);
+        if (q < a.n_queries) approx_query<PASS, G, false, MODE, COLL>(a, q, smem_q, h);
     }
 }
 
@@ -267,12 +296,12 @@ __global__ void __launch_bounds__(kApproxThreads) search_approx_hits_kernel(cons
 }
 
 // second launch of a pass: one warp per query of the heavy list (a.heavy[0] = length, a.heavy[1..] = query ids)
-template <int PASS, int MODE>
+template <int PASS, int MODE, bool COLL = false>
 __device__ __forceinline__ void approx_heavy(const SearchArgs &a, const ApproxHitArgs &h, uint64_t *smem_q) {
     constexpr int kGroups = kApproxThreads / 32;
     const uint32_t n_heavy = a.heavy[0];
     for (uint32_t i = blockIdx.x * kGroups + threadIdx.x / 32; i < n_heavy; i += gridDim.x * kGroups) {
-        approx_query<PASS, 32, true, MODE>(a, (uint64_t)a.heavy[1 + i], smem_q, h);
+        approx_query<PASS, 32, true, MODE, COLL>(a, (uint64_t)a.heavy[1 + i], smem_q, h);
         __syncwarp();
     }
 }
@@ -289,6 +318,19 @@ __global__ void __launch_bounds__(kApproxThreads) search_approx_heavy_hits_kerne
     approx_heavy<PASS, MODE>(a, h, smem_q);
 }
 
+// every pass and mode of a collection index (approx == 2)
+template <int PASS, int G, int MODE>
+__global__ void __launch_bounds__(kApproxThreads) search_approx_coll_kernel(const SearchArgs a, const ApproxHitArgs h) {
+    extern __shared__ uint64_t smem_q[];
+    approx_grid<PASS, G, MODE, true>(a, h, smem_q);
+}
+
+template <int PASS, int MODE>
+__global__ void __launch_bounds__(kApproxThreads) search_approx_heavy_coll_kernel(const SearchArgs a, const ApproxHitArgs h) {
+    extern __shared__ uint64_t smem_q[];
+    approx_heavy<PASS, MODE, true>(a, h, smem_q);
+}
+
 template <int PASS, int G, int MODE>
 static void launch_approx_pg(const SearchArgs &args, const ApproxHitArgs &h, cudaStream_t stream) {
     constexpr int kGroups = kApproxThreads / G;
@@ -296,7 +338,11 @@ static void launch_approx_pg(const SearchArgs &args, const ApproxHitArgs &h, cud
     uint64_t blocks = (args.n_queries + kGroups - 1) / kGroups;
     if ((PASS == kPassWrite || MODE == kApproxListed) && args.hits != nullptr)
         blocks = std::min<uint64_t>(blocks, (uint64_t)device_sm_count() * 16);
-    if (MODE == kApproxAll) {
+    const bool coll = args.approx == 2;
+    if (coll) {
+        cudaFuncSetAttribute(search_approx_coll_kernel<PASS, G, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        search_approx_coll_kernel<PASS, G, MODE><<<(unsigned)blocks, kApproxThreads, smem, stream>>>(args, h);
+    } else if (MODE == kApproxAll) {
         cudaFuncSetAttribute(search_approx_kernel<PASS, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         search_approx_kernel<PASS, G><<<(unsigned)blocks, kApproxThreads, smem, stream>>>(args);
     } else {
@@ -308,7 +354,10 @@ static void launch_approx_pg(const SearchArgs &args, const ApproxHitArgs &h, cud
         SearchArgs ha = args;
         ha.q_words = search_q_words(32, args.bits, args.max_len);
         const size_t hsmem = (size_t)(kApproxThreads / 32) * ha.q_words * sizeof(uint64_t);
-        if (MODE == kApproxAll) {
+        if (coll) {
+            cudaFuncSetAttribute(search_approx_heavy_coll_kernel<PASS, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hsmem);
+            search_approx_heavy_coll_kernel<PASS, MODE><<<device_sm_count() * 2, kApproxThreads, hsmem, stream>>>(ha, h);
+        } else if (MODE == kApproxAll) {
             cudaFuncSetAttribute(search_approx_heavy_kernel<PASS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hsmem);
             search_approx_heavy_kernel<PASS><<<device_sm_count() * 2, kApproxThreads, hsmem, stream>>>(ha);
         } else {
@@ -423,6 +472,53 @@ void launch_approx_distances(const SearchArgs &args, const ApproxHitArgs &h, uin
     else if (args.group == 4) launch_distances_g<4>(args, h, d_distances, stream);
     else if (args.group == 8) launch_distances_g<8>(args, h, d_distances, stream);
     else launch_distances_g<32>(args, h, d_distances, stream);
+}
+
+// ---- collection index: the record boundary bitmap (built once per attach or load) and locating hits
+
+__global__ void __launch_bounds__(256) record_boundaries_kernel(const uint64_t *__restrict__ starts, uint64_t n_records, uint64_t n,
+                                                                unsigned long long *__restrict__ bits) {
+    for (uint64_t r = 1 + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n_records; r += (uint64_t)gridDim.x * blockDim.x) {
+        const uint64_t s = starts[r];
+        if (s > 0 && s < n) atomicOr(bits + (s >> 6), 1ull << (s & 63));
+    }
+}
+
+void launch_record_boundaries(const uint64_t *d_starts, uint64_t n_records, uint64_t n, uint64_t *d_bits, cudaStream_t stream) {
+    if (n_records < 2) return;
+    const uint64_t blocks = std::min<uint64_t>((n_records + 255) / 256, (uint64_t)device_sm_count() * 8);
+    record_boundaries_kernel<<<(unsigned)blocks, 256, 0, stream>>>(d_starts, n_records, n, (unsigned long long *)d_bits);
+}
+
+// record = the last r with starts[r] <= p (empty records share their start with the next one), offset = p - starts[r];
+// a position at or past the end of the text gives (UINT32_MAX, 0)
+__global__ void __launch_bounds__(256) locate_kernel(const uint64_t *__restrict__ starts, uint64_t n_records,
+                                                     const uint32_t *__restrict__ positions, uint64_t n_pos,
+                                                     uint32_t *__restrict__ record_out, uint32_t *__restrict__ offset_out) {
+    const uint64_t n = __ldg(starts + n_records);
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_pos; i += (uint64_t)gridDim.x * blockDim.x) {
+        const uint64_t p = positions[i];
+        if (p >= n) {
+            record_out[i] = 0xFFFFFFFFu;
+            offset_out[i] = 0;
+            continue;
+        }
+        uint64_t lo = 0, hi = n_records;  // starts[lo] <= p < starts[hi]
+        while (hi - lo > 1) {
+            const uint64_t mid = (lo + hi) >> 1;
+            if (__ldg(starts + mid) <= p) lo = mid;
+            else hi = mid;
+        }
+        record_out[i] = (uint32_t)lo;
+        offset_out[i] = (uint32_t)(p - __ldg(starts + lo));
+    }
+}
+
+void launch_locate(const uint64_t *d_starts, uint64_t n_records, const uint32_t *d_positions, uint64_t n_pos, uint32_t *d_record,
+                   uint32_t *d_offset, cudaStream_t stream) {
+    if (n_pos == 0) return;
+    const uint64_t blocks = std::min<uint64_t>((n_pos + 255) / 256, (uint64_t)device_sm_count() * 16);
+    locate_kernel<<<(unsigned)blocks, 256, 0, stream>>>(d_starts, n_records, d_positions, n_pos, d_record, d_offset);
 }
 
 }  // namespace kb
