@@ -277,6 +277,29 @@ int kmer_b200_count_approx_batch_device_ex(kmer_b200_index *index, const uint8_t
                                            uint64_t n_queries, uint64_t max_query_len,
                                            const kmer_b200_approx_options *options, kmer_b200_result **out);
 
+/* ---- k-mer seeding (the reference's kmer_index_element::search_k, kmer_index.hpp:182-190, for every k-mer of every
+   query in one call): for each query q of length m and each offset j in [0, m - k], every text position p with
+   T[p, p+k) = q[j, j+k). k must be one of the index's ks (auxiliary elements do not count), else
+   KMER_B200_ERR_INVALID_ARGUMENT. On a collection index only windows inside one record count. A query shorter than k has
+   no k-mers and no hits; every status is KMER_B200_QUERY_OK; a rank >= sigma fails the call with
+   KMER_B200_ERR_INVALID_RANK. A query's hits are ordered by (j, p) ascending, and kmer_b200_result_seed_offsets gives
+   the j of each one. kmer_b200_result_kmer_counts holds one u32 per k-mer of the batch (sum over q of max(0, m_q - k + 1)
+   entries, query order then j order): the k-mer's occurrence count (in-record occurrences on a collection index).
+   max_occ > 0 is a repeat cap: a k-mer with more than max_occ occurrences contributes no hits, and its count entry reads
+   max_occ + 1. max_occ = 0: no cap. Query length is not bounded by a shared-memory staging (each query is walked in
+   tiles); j is reported in 32 bits, so max_query_len < 2^32. Refused (KMER_B200_ERR_UNSUPPORTED) on the handles
+   approximate search refuses. The host form stages the batch in one copy (counted by kmer_b200_last_search_transfer);
+   the device forms take max_query_len >= the longest query; the count-only form returns offsets, status and the k-mer
+   counts but no positions. */
+int kmer_b200_seed_batch(kmer_b200_index *index, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t n_queries,
+                         uint32_t k, uint32_t max_occ, kmer_b200_result **out);
+int kmer_b200_seed_batch_device(kmer_b200_index *index, const uint8_t *d_q_ranks, const uint64_t *d_q_offsets,
+                                uint64_t n_queries, uint64_t max_query_len, uint32_t k, uint32_t max_occ,
+                                kmer_b200_result **out);
+int kmer_b200_count_seeds_batch_device(kmer_b200_index *index, const uint8_t *d_q_ranks, const uint64_t *d_q_offsets,
+                                       uint64_t n_queries, uint64_t max_query_len, uint32_t k, uint32_t max_occ,
+                                       kmer_b200_result **out);
+
 uint64_t kmer_b200_result_n_queries(const kmer_b200_result *r);
 uint64_t kmer_b200_result_n_positions(const kmer_b200_result *r);
 int kmer_b200_result_on_device(const kmer_b200_result *r);
@@ -290,6 +313,9 @@ const uint32_t *kmer_b200_result_positions(const kmer_b200_result *r); /* [offse
 const uint8_t *kmer_b200_result_status(const kmer_b200_result *r);     /* [Q] */
 const uint8_t *kmer_b200_result_distances(const kmer_b200_result *r);      /* [n_positions] or NULL (approximate search) */
 const uint8_t *kmer_b200_result_best_distances(const kmer_b200_result *r); /* [Q] or NULL (approximate search) */
+const uint32_t *kmer_b200_result_seed_offsets(const kmer_b200_result *r);  /* [n_positions] or NULL (seeding, not count-only) */
+const uint32_t *kmer_b200_result_kmer_counts(const kmer_b200_result *r);   /* [n_kmers] or NULL (seeding) */
+uint64_t kmer_b200_result_n_kmers(const kmer_b200_result *r);              /* k-mers of a seeding batch, else 0 */
 void kmer_b200_result_free(kmer_b200_result *r);
 
 /* ---- sharded (multi-GPU) search, two phases around one cross-rank exchange.

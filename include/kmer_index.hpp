@@ -251,6 +251,10 @@ namespace kmer
         // when asked for, and d_min per query (0xFF without a hit) for every strategy but approx_hits::all()
         detail::array_view<std::uint8_t> distances;
         detail::array_view<std::uint8_t> best_distance;
+        // seeding (seed_batch; empty otherwise): the query offset j of each position, and the occurrence count of every
+        // k-mer of the batch (query order, then j order; max_occ + 1 for a k-mer above the cap)
+        detail::array_view<std::uint32_t> seed_offsets;
+        detail::array_view<std::uint32_t> kmer_counts;
 
         std::size_t size() const noexcept { return status.size(); }
         bool threw(std::size_t i) const { return status[i] == KMER_B200_QUERY_THROW_INVALID_ARGUMENT; }
@@ -268,6 +272,9 @@ namespace kmer
             status = {kmer_b200_result_status(r), std::size_t(n_q)};
             if (kmer_b200_result_distances(r)) distances = {kmer_b200_result_distances(r), std::size_t(n_p)};
             if (kmer_b200_result_best_distances(r)) best_distance = {kmer_b200_result_best_distances(r), std::size_t(n_q)};
+            if (kmer_b200_result_seed_offsets(r)) seed_offsets = {kmer_b200_result_seed_offsets(r), std::size_t(n_p)};
+            if (kmer_b200_result_kmer_counts(r))
+                kmer_counts = {kmer_b200_result_kmer_counts(r), std::size_t(kmer_b200_result_n_kmers(r))};
             if constexpr (std::is_same_v<position_t, std::uint32_t>)
                 positions = {kmer_b200_result_positions(r), std::size_t(n_p)};
             else if (n_p)
@@ -529,6 +536,22 @@ namespace kmer
             kmer_b200_approx_options opt{max_mismatches, hits.strategy, hits.s, distances ? std::uint32_t(KMER_B200_APPROX_DISTANCES) : 0u};
             kmer_b200_result* r = nullptr;
             detail::check(kmer_b200_search_approx_batch_ex(_handle, ranks.data(), offsets.data(), offsets.size() - 1, &opt, &r));
+            return kmer_batch_result<position_t>(r);
+        }
+
+        // k-mer seeding (kmer_b200_seed_batch; search_k<k> for every offset of every query in one call): per query, for
+        // every offset j in [0, m - k], every position p of the k-mer q[j, j+k), ordered by (j, p), with j in
+        // seed_offsets and each k-mer's occurrence count in kmer_counts. max_occ > 0: k-mers occurring more often give no
+        // positions and count max_occ + 1. On a collection index only windows inside one record count.
+        template<std::size_t k, std::ranges::range queries_t>
+        kmer_batch_result<position_t> seed_batch(queries_t const& queries, std::uint32_t max_occ = 0) const
+        {
+            static_assert(((k == ks) || ...), "seed_batch<k>: k is not one of this index's ks");
+            std::vector<std::uint8_t> ranks;
+            std::vector<std::uint64_t> offsets{0};
+            gather_ranks(queries, ranks, offsets);
+            kmer_b200_result* r = nullptr;
+            detail::check(kmer_b200_seed_batch(_handle, ranks.data(), offsets.data(), offsets.size() - 1, std::uint32_t(k), max_occ, &r));
             return kmer_batch_result<position_t>(r);
         }
 

@@ -89,15 +89,20 @@ def approx_options(max_mismatches: int, hits: str = "all", strata: int = 0, dist
 class BatchResult:
     """CSR result of a batch: offsets[Q+1], positions (ascending per query), status[Q]. Approximate search with a hit
     strategy also fills `distances` (uint8 per position: its Hamming distance, with distances=True) and `best_distance`
-    (uint8 per query: d_min, 0xFF without a hit; every strategy but "all"); both are None otherwise."""
+    (uint8 per query: d_min, 0xFF without a hit; every strategy but "all"); both are None otherwise. Seeding (KmerIndex.seeds) fills
+    `seed_offsets` (uint32 per position: the query offset j of its k-mer) and `kmer_counts` (uint32 per k-mer of the batch);
+    both are None for other searches."""
 
     def __init__(self, offsets: np.ndarray, positions: np.ndarray, status: np.ndarray, _owner=None,
-                 distances: np.ndarray | None = None, best_distance: np.ndarray | None = None):
+                 distances: np.ndarray | None = None, best_distance: np.ndarray | None = None,
+                 seed_offsets: np.ndarray | None = None, kmer_counts: np.ndarray | None = None):
         self.offsets = offsets
         self.positions = positions
         self.status = status
         self.distances = distances
         self.best_distance = best_distance
+        self.seed_offsets = seed_offsets
+        self.kmer_counts = kmer_counts
         self._owner = _owner   # (lib, C result handle) when the arrays are views of the pinned C result
 
     def free(self):
@@ -106,6 +111,7 @@ class BatchResult:
             L, r = self._owner
             self._owner = None
             self.offsets = self.positions = self.status = self.distances = self.best_distance = None
+            self.seed_offsets = self.kmer_counts = None
             L.kmer_b200_result_free(r)
 
     def __del__(self):
@@ -240,6 +246,16 @@ class DeviceResult:
         """uint8 view of d_min per query (approximate search with a hit strategy other than "all"), or None."""
         ptr = self._L.kmer_b200_result_best_distances(self._r) or 0
         return _DevArray(ptr, self.n_queries, "|u1", self) if ptr else None
+
+    def seed_offsets(self):
+        """int32 view of the query offset j of each position (seeding, not count-only), or None."""
+        ptr = self._L.kmer_b200_result_seed_offsets(self._r) or 0
+        return _DevArray(ptr, self.n_positions, "<i4", self) if ptr else None
+
+    def kmer_counts(self):
+        """int32 view of the occurrence count of each k-mer of the batch (seeding), or None."""
+        ptr = self._L.kmer_b200_result_kmer_counts(self._r) or 0
+        return _DevArray(ptr, int(self._L.kmer_b200_result_n_kmers(self._r)), "<i4", self) if ptr else None
 
     def hit_queries(self):
         """int32 view of [n, id_1 .. id_n, ...]: the queries the count pass found hits for (unordered), or None."""
@@ -462,6 +478,35 @@ class KmerIndex:
                                                                  C.byref(opt), C.byref(r)))
         return self._host_result(r, off.size - 1, copy)
 
+    def _seed_k(self, k: int | None) -> int:
+        if k is None:
+            if len(self.ks) != 1:
+                raise ValueError("seeding an index with several ks needs k")
+            return self.ks[0]
+        return int(k)
+
+    def seeds(self, q_ranks, q_offsets, k: int | None = None, max_occ: int = 0, copy: bool = True) -> BatchResult:
+        """k-mer seeding of a host batch (kmer_b200_seed_batch): per query, for every offset j in [0, m - k], every text
+        position p with T[p, p+k) = q[j, j+k), ordered by (j, p); BatchResult.seed_offsets holds each hit's j and
+        BatchResult.kmer_counts each k-mer's occurrence count (query order, then j order). k defaults to the index's only
+        k. max_occ > 0: k-mers with more than max_occ occurrences give no hits and report max_occ + 1. On a collection
+        index only windows inside one record count."""
+        q = np.ascontiguousarray(np.asarray(q_ranks, dtype=np.uint8))
+        off = np.ascontiguousarray(np.asarray(q_offsets, dtype=np.uint64))
+        r = C.c_void_p()
+        _capi.check(self._L.kmer_b200_seed_batch(self._h, q.ctypes.data, off.ctypes.data, off.size - 1, self._seed_k(k),
+                                                 int(max_occ), C.byref(r)))
+        return self._host_result(r, off.size - 1, copy)
+
+    def seeds_batch_device(self, q_ptr: int, off_ptr: int, Q: int, max_len: int, k: int | None = None, max_occ: int = 0):
+        """Seeding (see seeds) of a device-resident batch; the result stays on the device."""
+        return self._device_call(self._L.kmer_b200_seed_batch_device, q_ptr, off_ptr, Q, max_len, self._seed_k(k), int(max_occ))
+
+    def count_seeds_batch_device(self, q_ptr: int, off_ptr: int, Q: int, max_len: int, k: int | None = None, max_occ: int = 0):
+        """Count-only seeding of a device-resident batch: offsets, status and kmer_counts(), no positions."""
+        return self._device_call(self._L.kmer_b200_count_seeds_batch_device, q_ptr, off_ptr, Q, max_len, self._seed_k(k),
+                                 int(max_occ))
+
     def _host_result(self, r, Q: int, copy: bool) -> BatchResult:
         L = self._L
         total = L.kmer_b200_result_n_positions(r)
@@ -473,10 +518,15 @@ class KmerIndex:
         d_ptr, b_ptr = L.kmer_b200_result_distances(r), L.kmer_b200_result_best_distances(r)
         dist = (np.ctypeslib.as_array(C.cast(d_ptr, _capi.u8p), shape=(total,)) if total else np.zeros(0, np.uint8)) if d_ptr else None
         best = (np.ctypeslib.as_array(C.cast(b_ptr, _capi.u8p), shape=(Q,)) if Q else np.zeros(0, np.uint8)) if b_ptr else None
+        s_ptr, c_ptr, n_kmers = L.kmer_b200_result_seed_offsets(r), L.kmer_b200_result_kmer_counts(r), L.kmer_b200_result_n_kmers(r)
+        seed = (np.ctypeslib.as_array(C.cast(s_ptr, _capi.u32p), shape=(total,)) if total else np.zeros(0, np.uint32)) if s_ptr else None
+        kc = (np.ctypeslib.as_array(C.cast(c_ptr, _capi.u32p), shape=(n_kmers,)) if n_kmers else np.zeros(0, np.uint32)) if c_ptr else None
         if not copy:
-            return BatchResult(offsets, positions, status, _owner=(L, r), distances=dist, best_distance=best)
+            return BatchResult(offsets, positions, status, _owner=(L, r), distances=dist, best_distance=best, seed_offsets=seed,
+                               kmer_counts=kc)
         out = BatchResult(offsets.copy(), positions.copy(), status.copy(), distances=None if dist is None else dist.copy(),
-                          best_distance=None if best is None else best.copy())
+                          best_distance=None if best is None else best.copy(), seed_offsets=None if seed is None else seed.copy(),
+                          kmer_counts=None if kc is None else kc.copy())
         L.kmer_b200_result_free(r)
         return out
 

@@ -116,6 +116,12 @@ SYMBOLS = {
                                                           C.POINTER(ApproxOptions), C.POINTER(C.c_void_p)]),
     "kmer_b200_count_approx_batch_device_ex": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64,
                                                          C.POINTER(ApproxOptions), C.POINTER(C.c_void_p)]),
+    "kmer_b200_seed_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32,
+                                       C.POINTER(C.c_void_p)]),
+    "kmer_b200_seed_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32,
+                                              C.c_uint32, C.POINTER(C.c_void_p)]),
+    "kmer_b200_count_seeds_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32,
+                                                     C.c_uint32, C.POINTER(C.c_void_p)]),
     "kmer_b200_result_n_queries": (C.c_uint64, [C.c_void_p]),
     "kmer_b200_result_n_positions": (C.c_uint64, [C.c_void_p]),
     "kmer_b200_result_on_device": (C.c_int, [C.c_void_p]),
@@ -125,6 +131,9 @@ SYMBOLS = {
     "kmer_b200_result_status": (C.c_void_p, [C.c_void_p]),
     "kmer_b200_result_distances": (C.c_void_p, [C.c_void_p]),
     "kmer_b200_result_best_distances": (C.c_void_p, [C.c_void_p]),
+    "kmer_b200_result_seed_offsets": (C.c_void_p, [C.c_void_p]),
+    "kmer_b200_result_kmer_counts": (C.c_void_p, [C.c_void_p]),
+    "kmer_b200_result_n_kmers": (C.c_uint64, [C.c_void_p]),
     "kmer_b200_result_free": (None, [C.c_void_p]),
     "kmer_b200_presence_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64,
                                                   C.c_uint32, C.c_void_p, C.c_uint32]),

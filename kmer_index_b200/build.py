@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.environ.get("KMER_B200_LIB_OUT") or os.path.join(HERE, "libkmer_b200.so")   # KMER_B200_LIB_OUT: tuning builds
-SOURCES = ["capi.cu", "build_kernels.cu", "onesweep.cu", "search_kernels.cu", "search_lean.cu", "search_approx.cu", "route_kernels.cu", "fastx_kernels.cu", "synth.cu", "host_pack.cpp"]
+SOURCES = ["capi.cu", "build_kernels.cu", "onesweep.cu", "search_kernels.cu", "search_lean.cu", "search_approx.cu", "search_seeds.cu", "route_kernels.cu", "fastx_kernels.cu", "synth.cu", "host_pack.cpp"]
 HEADERS = ["common.cuh", "radix.cuh", "launch.h", "host_pack.h", "query_pack.cuh", os.path.join("..", "..", "include", "kmer_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC,-O3,-Wall", "-Xptxas", "-v"]

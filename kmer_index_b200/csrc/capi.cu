@@ -82,13 +82,15 @@ enum KernelId : int {
     K_APPROX_BEST,
     K_APPROX_SINGLE,
     K_APPROX_DISTANCES,
+    K_SEED_COUNT,
+    K_SEED_WRITE,
     K_COUNT_
 };
 
 const char *const kKernelNames[K_COUNT_] = {
     "pack_text",       "radix_hist_text", "radix_hist_pairs", "column_scan",     "radix_scatter_text", "radix_scatter_pairs",
     "directory_fill",  "search_count",    "search_write",     "search_presence", "offsets_scan",       "segment_sort",
-    "approx_best",     "approx_single",   "approx_distances"};
+    "approx_best",     "approx_single",   "approx_distances", "seed_count",      "seed_write"};
 
 struct Profiler {
     bool enabled = false;
@@ -251,8 +253,11 @@ struct kmer_b200_result {
     uint32_t *hit_queries = nullptr;  // device results: [0] = n, [1..n] = ids of the queries the count pass found hits for
     uint8_t *distances = nullptr;      // approximate search with KMER_B200_APPROX_DISTANCES: d(p) per position, or null
     uint8_t *best_distance = nullptr;  // approximate search, hit strategies other than "all": d_min per query, or null
+    uint32_t *seed_offsets = nullptr;  // seeding: the query offset j of each position, or null
+    uint32_t *kmer_counts = nullptr;   // seeding: the occurrence count of each k-mer of the batch, or null
+    uint64_t n_kmers = 0;
     size_t cap_offsets = 0, cap_positions = 0, cap_status = 0;  // host buffers: byte capacities
-    size_t cap_distances = 0, cap_best_distance = 0;
+    size_t cap_distances = 0, cap_best_distance = 0, cap_seed_offsets = 0, cap_kmer_counts = 0;
     bool positions_pageable = false;  // very large position lists live in plain malloc memory
 };
 
@@ -1703,19 +1708,25 @@ __global__ void max_len_kernel(const uint64_t *__restrict__ off, uint64_t Q, uns
     if ((threadIdx.x & 31) == 0 && m) atomicMax(out, m);
 }
 
-// Approximate search needs the whole text and every position of every element on this device: refused (with the reason)
+// Approximate search, collections and seeding need the whole text and every position of every element on this device
+// (whole or in peer parts), each bucket in ascending position order: refused (with the reason, `what` = the feature)
 // for the handles where one of them lives elsewhere.
-int approx_check(const kmer_b200_index *ix, uint32_t max_mismatches) {
-    if (max_mismatches > kb::kMaxMismatches) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "approximate search: max_mismatches above 8");
-    if (!ix->replicas.empty()) return fail(KMER_B200_ERR_UNSUPPORTED, "approximate search is not available on a multi-device handle");
+int whole_index_check(const kmer_b200_index *ix, const char *what) {
+    const std::string w(what);
+    if (!ix->replicas.empty()) return fail(KMER_B200_ERR_UNSUPPORTED, w + " is not available on a multi-device handle");
     if (ix->sharded || !ix->reaches_end || ix->cfg.halo != 0)
-        return fail(KMER_B200_ERR_UNSUPPORTED, "approximate search is not available on a position-range shard");
+        return fail(KMER_B200_ERR_UNSUPPORTED, w + " is not available on a position-range shard");
     if (ix->cfg.reserved & KMER_B200_FLAG_SHARED_POSITIONS)
-        return fail(KMER_B200_ERR_UNSUPPORTED, "approximate search is not available on a shared-positions index");
+        return fail(KMER_B200_ERR_UNSUPPORTED, w + " is not available on a shared-positions index");
     for (size_t e = 0; e < ix->ks.size(); ++e)
         if (ix->elems[e].dev.key_lo != 0 || ix->elems[e].dev.key_hi != UINT64_MAX)
-            return fail(KMER_B200_ERR_UNSUPPORTED, "approximate search needs the whole key space: adopt the assembled element first");
+            return fail(KMER_B200_ERR_UNSUPPORTED, w + " needs the whole key space: adopt the assembled element first");
     return KMER_B200_OK;
+}
+
+int approx_check(const kmer_b200_index *ix, uint32_t max_mismatches) {
+    if (max_mismatches > kb::kMaxMismatches) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "approximate search: max_mismatches above 8");
+    return whole_index_check(ix, "approximate search");
 }
 
 // the options of the _ex entry points: INVALID_ARGUMENT for null options, e > 8, an unknown strategy or unknown flag
@@ -1729,6 +1740,167 @@ int approx_options_check(const kmer_b200_index *ix, const kmer_b200_approx_optio
     *hit_opt = (opt->hits == KMER_B200_HITS_ALL && !(opt->flags & KMER_B200_APPROX_DISTANCES)) ? nullptr : opt;
     return KMER_B200_OK;
 }
+
+// The checks of the seeding entry points: the element of k (not an auxiliary one), or INVALID_ARGUMENT; the handle checks
+// of whole_index_check.
+int seed_check(const kmer_b200_index *ix, uint32_t k, uint32_t *elem) {
+    KB_TRY(whole_index_check(ix, "seeding"));
+    for (size_t e = 0; e < ix->ks.size(); ++e)
+        if (ix->ks[e] == k) {
+            *elem = (uint32_t)e;
+            return KMER_B200_OK;
+        }
+    return fail(KMER_B200_ERR_INVALID_ARGUMENT, "seeding: k is not one of the index's ks");
+}
+
+// Seeding of a batch already on the device (kmer_b200_seed_batch_device): k-mers per query -> scan -> count pass -> scan
+// -> [write pass + heavy launch]. Two synchronisations: the number of k-mers (sizes kmer_counts), then the number of hits
+// (sizes the positions). The caller holds the handle's lock and device.
+int seed_device_impl(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len, uint32_t elem,
+                     uint32_t max_occ, SearchFlavor flavor, kmer_b200_result **out) {
+    using namespace kb;
+    if (Q >= 0xFFFFFFFFull) return fail(KMER_B200_ERR_UNSUPPORTED, "more than 2^32 - 2 queries in one batch: split the batch");
+    if (max_len >= (1ull << 32)) return fail(KMER_B200_ERR_UNSUPPORTED, "seeding: a query offset j is reported in 32 bits");
+    cudaStream_t st = ix->stream;
+    kmer_b200_result *res = new (std::nothrow) kmer_b200_result();
+    if (!res) return fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation failed");
+    res->index = ix;
+    res->on_device = true;
+    res->n_queries = Q;
+    uint64_t *d_kbase = nullptr, *d_block_sums = nullptr;
+    uint32_t *d_flags = nullptr, *d_lo = nullptr;
+    unsigned long long *d_n_heavy = nullptr;
+    HeavySeed *d_heavy = nullptr;
+    size_t hs_cap = 0;
+    uint64_t *hs = nullptr;
+    auto release = [&] {
+        dev_free(ix, d_kbase);
+        dev_free(ix, d_block_sums);
+        dev_free(ix, d_flags);
+        dev_free(ix, d_lo);
+        dev_free(ix, d_n_heavy);
+        dev_free(ix, d_heavy);
+        pinned_put(hs, hs_cap);
+    };
+    auto bail = [&](int code) {
+        release();
+        kmer_b200_result_free(res);
+        return code;
+    };
+    auto sync = [&](const char *what) -> int {
+        cudaError_t e = cudaStreamSynchronize(st);
+        if (e == cudaSuccess) e = cudaGetLastError();
+        if (e == cudaSuccess) return KMER_B200_OK;
+        cudaGetLastError();
+        return fail(KMER_B200_ERR_CUDA, std::string(what) + cudaGetErrorString(e));
+    };
+    hs = (uint64_t *)pinned_get(8 * sizeof(uint64_t), &hs_cap);
+    if (!hs) return bail(fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed"));
+    if (dev_alloc(ix, &res->offsets, Q + 1, false) || dev_alloc(ix, &res->status, Q, false) || dev_alloc(ix, &d_kbase, Q + 1, false) ||
+        dev_alloc(ix, &d_block_sums, offsets_scan_blocks(Q) + 1, false) || dev_alloc(ix, &d_flags, 1, false) ||
+        dev_alloc(ix, &d_n_heavy, 1, false))
+        return bail(KMER_B200_ERR_OUT_OF_MEMORY);
+    // each query's first k-mer in the batch's k-mer order
+    launch_seed_kmers_per_query(d_off, Q, ix->ks[elem], d_kbase, st);
+    launch_offsets_scan(d_kbase, Q, d_block_sums, st);
+    cudaMemcpyAsync(&hs[0], d_kbase + Q, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+    if (int s = sync("seeding (k-mers per query): ")) return bail(s);
+    res->n_kmers = Q ? hs[0] : 0;
+    if (dev_alloc(ix, &res->kmer_counts, res->n_kmers, false) ||
+        (flavor == kFlavorFull && dev_alloc(ix, &d_lo, res->n_kmers, false)))
+        return bail(KMER_B200_ERR_OUT_OF_MEMORY);
+
+    SeedArgs a{};
+    a.index = ix->d_index;
+    a.q_ranks = d_q;
+    a.q_offsets = d_off;
+    a.n_queries = Q;
+    a.elem = elem;
+    a.k = ix->ks[elem];
+    a.max_occ = max_occ;
+    a.coll = ix->starts.empty() ? 0 : 1;
+    a.kmer_base = d_kbase;
+    a.kmer_counts = res->kmer_counts;
+    a.bucket_lo = d_lo;
+    a.counts = res->offsets;
+    a.status = res->status;
+    a.n_heavy = d_n_heavy;
+    a.error_flag = d_flags;
+    a.gather_count = ix->cfg.profile >= 2 ? ix->d_gathers : nullptr;  // profile = 2: also count gathered sectors
+    cudaMemsetAsync(d_flags, 0, sizeof(uint32_t), st);
+    cudaMemsetAsync(d_n_heavy, 0, sizeof(unsigned long long), st);
+    if (a.gather_count) cudaMemsetAsync(ix->d_gathers, 0, sizeof(unsigned long long), st);
+    ix->prof.begin(K_SEED_COUNT, 0);
+    launch_seed_count(a, st);
+    ix->prof.end();
+    ix->prof.begin(K_OFFSETS_SCAN, 3.0 * 8 * Q, 3);
+    launch_offsets_scan(res->offsets, Q, d_block_sums, st);
+    ix->prof.end();
+    cudaMemcpyAsync(&hs[0], res->offsets + Q, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+    cudaMemcpyAsync(&hs[1], d_n_heavy, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+    cudaMemcpyAsync(&hs[2], d_flags, sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
+    if (a.gather_count) cudaMemcpyAsync(&hs[3], ix->d_gathers, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+    if (int s = sync("seeding (count pass): ")) return bail(s);
+    if (a.gather_count) ix->last_gathers = hs[3];
+    if (hs[2] & 1u) return bail(fail(KMER_B200_ERR_INVALID_RANK, "a query contains a rank >= sigma"));
+    const uint64_t total = Q ? hs[0] : 0, n_heavy = hs[1];
+    res->n_positions = total;
+    if (flavor == kFlavorFull && total > 0) {
+        if (dev_alloc(ix, &res->positions, total, false) || dev_alloc(ix, &res->seed_offsets, total, false) ||
+            (n_heavy && dev_alloc(ix, &d_heavy, n_heavy, false)))
+            return bail(KMER_B200_ERR_OUT_OF_MEMORY);
+        a.positions = res->positions;
+        a.seed_offsets = res->seed_offsets;
+        a.heavy = d_heavy;
+        cudaMemsetAsync(d_n_heavy, 0, sizeof(unsigned long long), st);
+        ix->prof.begin(K_SEED_WRITE, 0);
+        launch_seed_write(a, st);
+        ix->prof.end();
+        if (a.gather_count) cudaMemcpyAsync(&hs[3], ix->d_gathers, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+        if (int s = sync("seeding (write pass): ")) return bail(s);
+        if (a.gather_count) ix->last_gathers = hs[3];
+    } else if (flavor == kFlavorFull && dev_alloc(ix, &res->seed_offsets, 1, false)) {
+        return bail(KMER_B200_ERR_OUT_OF_MEMORY);  // a full result without hits: empty arrays, not NULL
+    }
+    release();
+    *out = res;
+    return KMER_B200_OK;
+}
+
+// Query lengths of a host batch: the batch and its offsets staged on the device, and the longest query. The staging is
+// released with the object.
+struct StagedBatch {
+    kmer_b200_index *ix;
+    uint8_t *d_q = nullptr;
+    uint64_t *d_off = nullptr;
+    unsigned long long *d_max = nullptr;
+    uint64_t max_len = 0;
+    explicit StagedBatch(kmer_b200_index *x) : ix(x) {}
+    ~StagedBatch() {
+        dev_free(ix, d_q);
+        dev_free(ix, d_off);
+        dev_free(ix, d_max);
+    }
+    // one copy each of the ranks (translated with lut256 when given) and the offsets; d_q is indexed by the caller's
+    // offsets (it points q_offsets[0] symbols before the copy)
+    int stage(const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q, const uint8_t *lut256) {
+        cudaStream_t st = ix->stream;
+        const uint64_t n_sym = q_offsets[Q] - q_offsets[0];
+        KB_TRY(dev_alloc(ix, &d_q, n_sym, false));
+        KB_TRY(dev_alloc(ix, &d_off, Q + 1, false));
+        KB_TRY(dev_alloc(ix, &d_max, 1, false));
+        KB_CUDA(cudaMemcpyAsync(d_off, q_offsets, (Q + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+        if (n_sym) KB_CUDA(cudaMemcpyAsync(d_q, q_ranks + q_offsets[0], n_sym, cudaMemcpyHostToDevice, st));
+        if (lut256) KB_TRY(translate_on_device(ix, d_q, n_sym, lut256));
+        KB_CUDA(cudaMemsetAsync(d_max, 0, sizeof(unsigned long long), st));
+        if (Q) max_len_kernel<<<(unsigned)std::min<uint64_t>((Q + 255) / 256, (uint64_t)kb::device_sm_count() * 8), 256, 0, st>>>(d_off, Q, d_max);
+        KB_CUDA(cudaMemcpyAsync(&ix->h_pinned[2], d_max, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+        KB_CUDA(cudaStreamSynchronize(st));
+        max_len = ix->h_pinned[2];
+        return KMER_B200_OK;
+    }
+    const uint8_t *ranks(const uint64_t *q_offsets) const { return d_q - q_offsets[0]; }
+};
 
 }  // namespace
 
@@ -1920,7 +2092,7 @@ int kmer_b200_load(const char *path, const kmer_b200_config *cfg_in, kmer_b200_i
             if ((r = records_check(ix, rec.data(), n_records)) != 0) return r;
         }
         if (r == 0) r = finalize_index(ix);
-        if (r == 0 && !rec.empty()) r = approx_check(ix, 0);
+        if (r == 0 && !rec.empty()) r = whole_index_check(ix, "a collection index");
         if (r == 0 && !rec.empty()) r = attach_records_impl(ix, rec.data(), rec.size() - 1);
         return r;
     };
@@ -2523,34 +2695,10 @@ static int search_batch_host_single_copy(kmer_b200_index *ix, const uint8_t *q_r
                                          const kmer_b200_approx_options *hit_opt = nullptr) {
     cudaStream_t st = ix->stream;
     const uint64_t n_sym = q_offsets[Q] - q_offsets[0];
-    uint8_t *d_q = nullptr;
-    uint64_t *d_off = nullptr;
-    unsigned long long *d_max = nullptr;
-    struct Staging {  // the device copies of the batch are released on every exit path
-        kmer_b200_index *ix;
-        uint8_t *&q;
-        uint64_t *&off;
-        unsigned long long *&mx;
-        ~Staging() {
-            dev_free(ix, q);
-            dev_free(ix, off);
-            dev_free(ix, mx);
-        }
-    } staging{ix, d_q, d_off, d_max};
-    KB_TRY(dev_alloc(ix, &d_q, n_sym, false));
-    KB_TRY(dev_alloc(ix, &d_off, Q + 1, false));
-    KB_TRY(dev_alloc(ix, &d_max, 1, false));
-    // offsets are rebased on the device side by passing q_ranks - q_offsets[0]
-    KB_CUDA(cudaMemcpyAsync(d_off, q_offsets, (Q + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    if (n_sym) KB_CUDA(cudaMemcpyAsync(d_q, q_ranks + q_offsets[0], n_sym, cudaMemcpyHostToDevice, st));
-    if (lut256) KB_TRY(translate_on_device(ix, d_q, n_sym, lut256));
-    KB_CUDA(cudaMemsetAsync(d_max, 0, sizeof(unsigned long long), st));
-    if (Q) max_len_kernel<<<(unsigned)std::min<uint64_t>((Q + 255) / 256, (uint64_t)kb::device_sm_count() * 8), 256, 0, st>>>(d_off, Q, d_max);
-    KB_CUDA(cudaMemcpyAsync(&ix->h_pinned[2], d_max, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    KB_CUDA(cudaStreamSynchronize(st));
-    const uint64_t max_len = ix->h_pinned[2];
+    StagedBatch staged(ix);
+    KB_TRY(staged.stage(q_ranks, q_offsets, Q, lut256));
     kmer_b200_result *dres = nullptr;
-    int s = search_device_impl(ix, d_q - q_offsets[0], d_off, Q, max_len, mode, nullptr, 0, kFlavorFull, &dres, nullptr,
+    int s = search_device_impl(ix, staged.ranks(q_offsets), staged.d_off, Q, staged.max_len, mode, nullptr, 0, kFlavorFull, &dres, nullptr,
                                max_mismatches, hit_opt);
     if (s != 0) return s;
     // device result -> pinned host buffers
@@ -2657,6 +2805,75 @@ int kmer_b200_search_approx_batch_ex(kmer_b200_index *ix, const uint8_t *q_ranks
                                          out, hit_opt);
 }
 
+int kmer_b200_seed_batch(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q, uint32_t k,
+                         uint32_t max_occ, kmer_b200_result **out) {
+    if (!ix || !out || !q_offsets) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    *out = nullptr;
+    uint32_t elem = 0;
+    KB_TRY(seed_check(ix, k, &elem));
+    if (q_offsets[Q] != q_offsets[0] && !q_ranks) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "q_ranks is null");
+    DeviceGuard guard(ix->device);
+    std::lock_guard<std::mutex> lock(ix->mu);
+    cudaStream_t st = ix->stream;
+    StagedBatch staged(ix);
+    KB_TRY(staged.stage(q_ranks, q_offsets, Q, nullptr));
+    kmer_b200_result *dres = nullptr;
+    KB_TRY(seed_device_impl(ix, staged.ranks(q_offsets), staged.d_off, Q, staged.max_len, elem, max_occ, kFlavorFull, &dres));
+    // device result -> pinned host buffers
+    kmer_b200_result *res = host_result_new(ix, Q);
+    bool ok = res != nullptr;
+    if (ok) {
+        res->n_kmers = dres->n_kmers;
+        ok = (res->kmer_counts = (uint32_t *)pinned_get(std::max<uint64_t>(dres->n_kmers, 1) * sizeof(uint32_t), &res->cap_kmer_counts)) &&
+             (res->seed_offsets = (uint32_t *)pinned_get(std::max<uint64_t>(dres->n_positions, 1) * sizeof(uint32_t), &res->cap_seed_offsets)) &&
+             host_result_positions(res, dres->n_positions);
+    }
+    if (!ok) {
+        kmer_b200_result_free(dres);
+        kmer_b200_result_free(res);
+        return fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed");
+    }
+    const uint64_t n_pos = res->n_positions, n_kmers = res->n_kmers;
+    cudaMemcpyAsync(res->offsets, dres->offsets, (Q + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+    if (Q) cudaMemcpyAsync(res->status, dres->status, Q, cudaMemcpyDeviceToHost, st);
+    if (n_pos) cudaMemcpyAsync(res->positions, dres->positions, n_pos * sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
+    if (n_pos) cudaMemcpyAsync(res->seed_offsets, dres->seed_offsets, n_pos * sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
+    if (n_kmers) cudaMemcpyAsync(res->kmer_counts, dres->kmer_counts, n_kmers * sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
+    cudaError_t e = cudaStreamSynchronize(st);
+    kmer_b200_result_free(dres);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        kmer_b200_result_free(res);
+        return fail(KMER_B200_ERR_CUDA, std::string("seeding (D2H): ") + cudaGetErrorString(e));
+    }
+    ix->last_h2d = (q_offsets[Q] - q_offsets[0]) + (Q + 1) * sizeof(uint64_t);
+    ix->last_d2h = (Q + 1) * sizeof(uint64_t) + Q + 2 * n_pos * sizeof(uint32_t) + n_kmers * sizeof(uint32_t);
+    ix->last_host_path = 0, ix->last_raw_pct = 100, ix->last_pack_gbs = 0;
+    *out = res;
+    return KMER_B200_OK;
+}
+
+static int seed_device_entry(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len, uint32_t k,
+                             uint32_t max_occ, SearchFlavor flavor, kmer_b200_result **out) {
+    if (!ix || !out || !d_off) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    *out = nullptr;
+    uint32_t elem = 0;
+    KB_TRY(seed_check(ix, k, &elem));
+    DeviceGuard guard(ix->device);
+    std::lock_guard<std::mutex> lock(ix->mu);
+    return seed_device_impl(ix, d_q, d_off, Q, max_len, elem, max_occ, flavor, out);
+}
+
+int kmer_b200_seed_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len,
+                                uint32_t k, uint32_t max_occ, kmer_b200_result **out) {
+    return seed_device_entry(ix, d_q, d_off, Q, max_len, k, max_occ, kFlavorFull, out);
+}
+
+int kmer_b200_count_seeds_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len,
+                                       uint32_t k, uint32_t max_occ, kmer_b200_result **out) {
+    return seed_device_entry(ix, d_q, d_off, Q, max_len, k, max_occ, kFlavorCountOnly, out);
+}
+
 int kmer_b200_search_batch_ptrs(kmer_b200_index *ix, const uint8_t *const *q_ptrs, const uint64_t *q_lens, uint64_t Q,
                                 uint32_t mode, kmer_b200_result **out) {
     if (!ix || !out || (Q && (!q_ptrs || !q_lens))) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
@@ -2732,6 +2949,9 @@ const uint32_t *kmer_b200_result_positions(const kmer_b200_result *r) { return r
 const uint8_t *kmer_b200_result_status(const kmer_b200_result *r) { return r ? r->status : nullptr; }
 const uint8_t *kmer_b200_result_distances(const kmer_b200_result *r) { return r ? r->distances : nullptr; }
 const uint8_t *kmer_b200_result_best_distances(const kmer_b200_result *r) { return r ? r->best_distance : nullptr; }
+const uint32_t *kmer_b200_result_seed_offsets(const kmer_b200_result *r) { return r ? r->seed_offsets : nullptr; }
+const uint32_t *kmer_b200_result_kmer_counts(const kmer_b200_result *r) { return r ? r->kmer_counts : nullptr; }
+uint64_t kmer_b200_result_n_kmers(const kmer_b200_result *r) { return r ? r->n_kmers : 0; }
 
 void kmer_b200_result_free(kmer_b200_result *r) {
     if (!r) return;
@@ -2744,6 +2964,8 @@ void kmer_b200_result_free(kmer_b200_result *r) {
         dev_free(ix, r->hit_queries);
         dev_free(ix, r->distances);
         dev_free(ix, r->best_distance);
+        dev_free(ix, r->seed_offsets);
+        dev_free(ix, r->kmer_counts);
     } else {
         pinned_put(r->offsets, r->cap_offsets);
         if (r->positions_pageable)
@@ -2753,6 +2975,8 @@ void kmer_b200_result_free(kmer_b200_result *r) {
         pinned_put(r->status, r->cap_status);
         pinned_put(r->distances, r->cap_distances);
         pinned_put(r->best_distance, r->cap_best_distance);
+        pinned_put(r->seed_offsets, r->cap_seed_offsets);
+        pinned_put(r->kmer_counts, r->cap_kmer_counts);
     }
     delete r;
 }
@@ -3233,7 +3457,7 @@ int kmer_b200_records_locate(const kmer_b200_records *r, const uint32_t *positio
 int kmer_b200_attach_records(kmer_b200_index *ix, const uint64_t *starts, uint64_t n_records) {
     if (!ix || !starts) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
     if (n_records == 0 || n_records >= (1ull << 32)) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "n_records must be in [1, 2^32)");
-    KB_TRY(approx_check(ix, 0));  // the handles approximate search refuses hold no collection either
+    KB_TRY(whole_index_check(ix, "a collection index"));
     if (!ix->starts.empty()) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "records are attached already");
     KB_TRY(records_check(ix, starts, n_records));
     DeviceGuard guard(ix->device);

@@ -134,6 +134,40 @@ uint32_t search_q_words(uint32_t group, uint32_t bits, uint64_t max_len);
 void launch_record_boundaries(const uint64_t *d_starts, uint64_t n_records, uint64_t n, uint64_t *d_bits, cudaStream_t stream);
 void launch_locate(const uint64_t *d_starts, uint64_t n_records, const uint32_t *d_positions, uint64_t n_pos, uint32_t *d_record,
                    uint32_t *d_offset, cudaStream_t stream);
+// ---- k-mer seeding (search_seeds.cu): every k-mer of every query looked up in one element, one warp per query
+struct HeavySeed {  // a bucket the write pass hands to the warp-per-bucket launch
+    uint64_t out;   // its first output slot
+    uint64_t cnt;   // hits to write
+    uint32_t lo;    // its first CSR entry
+    uint32_t j;     // the k-mer's query offset
+};
+struct SeedArgs {
+    const DeviceIndex *index;        // device pointer
+    const uint8_t *q_ranks;          // device
+    const uint64_t *q_offsets;       // device, [Q + 1]
+    uint64_t n_queries;
+    uint32_t elem;                   // the element of k (not an auxiliary one)
+    uint32_t k;
+    uint32_t max_occ;                // 0 = no cap
+    uint32_t coll;                   // collection index: in-record windows only
+    const uint64_t *kmer_base;       // device, [Q + 1]: index of each query's first k-mer in the batch's k-mer order
+    uint32_t *kmer_counts;           // device, [n_kmers]
+    uint32_t *bucket_lo;             // device, [n_kmers], or null (count only): each k-mer's first CSR entry
+    uint64_t *counts;                // device, [Q + 1]: hits per query (count pass), then offsets
+    uint8_t *status;                 // device, [Q]
+    uint32_t *positions;             // device (write pass)
+    uint32_t *seed_offsets;          // device (write pass): the j of each position
+    HeavySeed *heavy;                // device (write pass) or null: room for every bucket above kHeavyCandidates hits
+    unsigned long long *n_heavy;     // device: such buckets (count pass), then the heavy list's length (zeroed before the write pass)
+    uint32_t *error_flag;            // device u32: bit 0 = query rank >= sigma
+    unsigned long long *gather_count;  // device or null: accumulates the 32-byte sectors gathered
+};
+// n_kmers[q] = max(0, m_q - k + 1), to be turned into SeedArgs::kmer_base by launch_offsets_scan
+void launch_seed_kmers_per_query(const uint64_t *d_q_offsets, uint64_t n_queries, uint32_t k, uint64_t *d_n_kmers, cudaStream_t stream);
+void launch_seed_count(const SeedArgs &a, cudaStream_t stream);
+// after the offsets scan of the count pass's counts: the write pass and, when a.heavy != null, the heavy launch
+void launch_seed_write(const SeedArgs &a, cudaStream_t stream);
+
 // deferred count pass epilogue: zero the counts / set THROW according to the combined presence flags
 void launch_finalize_deferred(uint64_t *d_counts, uint8_t *d_status, const uint8_t *d_defer, const uint32_t *d_present4_global,
                               uint64_t n_queries, cudaStream_t stream);
