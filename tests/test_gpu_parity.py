@@ -1,5 +1,7 @@
 """GPU parity: the CUDA path (through the C ABI) against the golden fixtures generated from the compiled
 reference, against the C restatement oracle on larger seeded inputs, and against ground truth (CORRECT mode)."""
+import contextlib
+
 import numpy as np
 import pytest
 
@@ -159,18 +161,35 @@ def test_edge_cases(kb):
         assert ix.search(np.array([0, 1, 2], np.uint8)).tolist() == [0, 4]
 
 
+def _sharded_shape(sigma, ks, n, m_lo, m_hi, world, group, i):
+    label = f"{sigma}-ks{i}-{n}-{m_lo}-{m_hi}-{world}" + (f"-G{group}" if group else "")
+    return pytest.param(sigma, ks, n, m_lo, m_hi, world, group, id=label)
+
+
 @pytest.mark.parametrize("fmt", [0, 1, "fused"])
-@pytest.mark.parametrize("sigma,ks,n,m_lo,m_hi,world", [(4, [16], 400_000, 16, 64, 2), (4, [12], 300_000, 13, 64, 3),
-                                                       (4, [5, 7, 9, 11, 13], 200_000, 4, 40, 2), (15, [8], 200_000, 3, 20, 4),
-                                                       (27, [12], 200_000, 8, 40, 2)])
-def test_sharded_search_emulated_on_one_gpu(kb, oracle_mod, sigma, ks, n, m_lo, m_hi, world, fmt):
+@pytest.mark.parametrize("sigma,ks,n,m_lo,m_hi,world,group", [
+    _sharded_shape(*shape, i) for i, shape in enumerate([
+        (4, [16], 400_000, 16, 64, 2, 0), (4, [12], 300_000, 13, 64, 3, 0), (4, [5, 7, 9, 11, 13], 200_000, 4, 40, 2, 0),
+        (15, [8], 200_000, 3, 20, 4, 0), (27, [12], 200_000, 8, 40, 2, 0)])] + [
+    # the presence and deferred passes with G lanes per query forced (KMER_B200_GROUP)
+    _sharded_shape(sigma, ks, n, m_lo, m_hi, world, group, i)
+    for i, (sigma, ks, n, m_lo, m_hi, world) in ((2, (4, [5, 7, 9, 11, 13], 200_000, 4, 40, 2)), (3, (15, [8], 200_000, 3, 20, 4)))
+    for group in (2, 4, 8)])
+def test_sharded_search_emulated_on_one_gpu(kb, oracle_mod, monkeypatch, sigma, ks, n, m_lo, m_hi, world, group, fmt):
     """The sharded path (position-range shards with halo, presence OR, global-presence search, rank-order merge)
     run as `world` indices on one GPU must equal the unsharded reference-exact result."""
     import torch
 
     from kmer_index_b200 import sharded, synth
+    from test_gpu_variants import kernel_summary, kernels_launched, lanes, template_args
     dev = torch.device("cuda", 0)
+    stack = contextlib.ExitStack()
+    if group:
+        monkeypatch.setenv("KMER_B200_GROUP", str(group))
+        names = stack.enter_context(kernels_launched())
     text = synth.random_text(n, sigma, 91)
+    if group:
+        text[30_000:31_500] = 1     # ~1500 consecutive hits for the constant queries, answered by the G-lane launch
     q, off = synth.stress_queries(text, 5000, m_lo, m_hi, sigma, 92)
     Q = off.size - 1
     d_q = torch.from_numpy(q).to(dev)
@@ -215,10 +234,16 @@ def test_sharded_search_emulated_on_one_gpu(kb, oracle_mod, sigma, ks, n, m_lo, 
     finally:
         for ix in idx:
             ix.close()
+        stack.close()
     with oracle_mod.Oracle(text, sigma, ks) as o:
         want = o.search(q, off)
-    assert_results_equal(got, want, label=f"sharded x{world} {ks}")
+    assert_results_equal(got, want, label=f"sharded x{world} {ks} G={group}")
     assert want[1].size > 0
+    if group:
+        # the presence pass (fmt 0, 1) or the deferred count pass (fused) ran with G lanes, and so did every other pass
+        first_pass = "4" if fmt == "fused" else "2"
+        assert lanes(names, "search_kernel") == {group}, kernel_summary(names)
+        assert any(a[0] == first_pass for a in template_args(names, "search_kernel")), kernel_summary(names)
 
 
 @pytest.mark.parametrize("sigma,ks,n,m_lo,m_hi,world", [(4, [16], 400_000, 16, 64, 2), (4, [5, 7, 9, 11, 13], 200_000, 4, 40, 3),
