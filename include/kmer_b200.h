@@ -221,7 +221,8 @@ int kmer_b200_count_batch_device(kmer_b200_index *index, const uint8_t *d_q_rank
    result of KMER_B200_MODE_CORRECT search. Not available (KMER_B200_ERR_UNSUPPORTED) on a multi-device handle, a
    position-range shard, a shared-positions index or a key-range part that has not been adopted. Query length is
    bounded by the shared-memory staging as for exact search. Same host buffers and result layout as
-   kmer_b200_search_batch; the whole batch is staged on the device in one copy. */
+   kmer_b200_search_batch; the whole batch is staged on the device in one copy. This and the two device forms below
+   are the _ex forms (hit strategies, below) with options {max_mismatches, KMER_B200_HITS_ALL, 0, 0}. */
 int kmer_b200_search_approx_batch(kmer_b200_index *index, const uint8_t *q_ranks, const uint64_t *q_offsets,
                                   uint64_t n_queries, uint32_t max_mismatches, kmer_b200_result **out);
 

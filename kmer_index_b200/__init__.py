@@ -418,64 +418,39 @@ class KmerIndex:
     def search_batch(self, q_ranks, q_offsets, mode: int = MODE_DEFAULT, copy: bool = True) -> BatchResult:
         """Batch of queries in host memory -> host CSR result (kmer_index::search + to_vector per query).
         copy=False returns views of the library's pinned result buffers (valid until BatchResult.free())."""
-        L = self._L
         q = np.ascontiguousarray(np.asarray(q_ranks, dtype=np.uint8))
         off = np.ascontiguousarray(np.asarray(q_offsets, dtype=np.uint64))
-        Q = off.size - 1
         r = C.c_void_p()
-        _capi.check(L.kmer_b200_search_batch(self._h, q.ctypes.data, off.ctypes.data, Q, mode, C.byref(r)))
-        total = L.kmer_b200_result_n_positions(r)
-        offsets = np.ctypeslib.as_array(C.cast(L.kmer_b200_result_offsets(r), _capi.u64p), shape=(Q + 1,))
-        status = (np.ctypeslib.as_array(C.cast(L.kmer_b200_result_status(r), _capi.u8p), shape=(Q,))
-                  if Q else np.zeros(0, dtype=np.uint8))
-        positions = (np.ctypeslib.as_array(C.cast(L.kmer_b200_result_positions(r), _capi.u32p), shape=(total,))
-                     if total else np.zeros(0, dtype=np.uint32))
-        if not copy:
-            return BatchResult(offsets, positions, status, _owner=(L, r))
-        out = BatchResult(offsets.copy(), positions.copy(), status.copy())
-        L.kmer_b200_result_free(r)
-        return out
+        _capi.check(self._L.kmer_b200_search_batch(self._h, q.ctypes.data, off.ctypes.data, off.size - 1, mode, C.byref(r)))
+        return self._host_result(r, off.size - 1, copy)
 
     def search_batch_text(self, queries, lut: np.ndarray | None = None, mode: int = MODE_DEFAULT) -> BatchResult:
         """Batch of character queries (list of str/bytes); translated to ranks on the device."""
-        L = self._L
         lut = np.ascontiguousarray(np.asarray(lut if lut is not None else self._lut, dtype=np.uint8))
         raw = [x.encode() if isinstance(x, str) else bytes(x) for x in queries]
         off = np.zeros(len(raw) + 1, dtype=np.uint64)
         np.cumsum([len(x) for x in raw], out=off[1:])
         q = np.frombuffer(b"".join(raw), dtype=np.uint8)
         r = C.c_void_p()
-        _capi.check(L.kmer_b200_search_batch_text(self._h, q.ctypes.data_as(C.c_char_p), off.ctypes.data, len(raw),
-                                                  lut.ctypes.data_as(_capi.u8p), mode, C.byref(r)))
-        Q = len(raw)
-        total = L.kmer_b200_result_n_positions(r)
-        offsets = np.ctypeslib.as_array(C.cast(L.kmer_b200_result_offsets(r), _capi.u64p), shape=(Q + 1,)).copy()
-        status = (np.ctypeslib.as_array(C.cast(L.kmer_b200_result_status(r), _capi.u8p), shape=(Q,)).copy()
-                  if Q else np.zeros(0, dtype=np.uint8))
-        positions = (np.ctypeslib.as_array(C.cast(L.kmer_b200_result_positions(r), _capi.u32p), shape=(total,)).copy()
-                     if total else np.zeros(0, dtype=np.uint32))
-        L.kmer_b200_result_free(r)
-        return BatchResult(offsets, positions, status)
+        _capi.check(self._L.kmer_b200_search_batch_text(self._h, q.ctypes.data_as(C.c_char_p), off.ctypes.data, len(raw),
+                                                        lut.ctypes.data_as(_capi.u8p), mode, C.byref(r)))
+        return self._host_result(r, len(raw), True)
 
     def search_approx(self, q_ranks, q_offsets, max_mismatches: int, copy: bool = True, *, hits: str = "all",
                       strata: int = 0, distances: bool = False) -> BatchResult:
-        """Approximate search of a host batch (kmer_b200_search_approx_batch): per query, every position p, ascending,
+        """Approximate search of a host batch (kmer_b200_search_approx_batch_ex): per query, every position p, ascending,
         where the text window T[p, p+m) differs from the query in at most max_mismatches (<= 8) symbols. Substitutions
         only; max_mismatches=0 is exact search in MODE_CORRECT. copy=False: views of the library's pinned buffers (valid
         until BatchResult.free()).
         hits: "all", "all_best" (the hits at the smallest distance d_min), "single_best" (the lowest such position) or
         "strata" (distance <= d_min + strata); every choice but "all" sets BatchResult.best_distance. distances=True
-        sets BatchResult.distances (kmer_b200_search_approx_batch_ex)."""
+        sets BatchResult.distances."""
         q = np.ascontiguousarray(np.asarray(q_ranks, dtype=np.uint8))
         off = np.ascontiguousarray(np.asarray(q_offsets, dtype=np.uint64))
         r = C.c_void_p()
-        if hits == "all" and not distances:
-            _capi.check(self._L.kmer_b200_search_approx_batch(self._h, q.ctypes.data, off.ctypes.data, off.size - 1,
-                                                              int(max_mismatches), C.byref(r)))
-        else:
-            opt = approx_options(max_mismatches, hits, strata, distances)
-            _capi.check(self._L.kmer_b200_search_approx_batch_ex(self._h, q.ctypes.data, off.ctypes.data, off.size - 1,
-                                                                 C.byref(opt), C.byref(r)))
+        opt = approx_options(max_mismatches, hits, strata, distances)
+        _capi.check(self._L.kmer_b200_search_approx_batch_ex(self._h, q.ctypes.data, off.ctypes.data, off.size - 1, C.byref(opt),
+                                                             C.byref(r)))
         return self._host_result(r, off.size - 1, copy)
 
     def _seed_k(self, k: int | None) -> int:
@@ -559,8 +534,6 @@ class KmerIndex:
                                    hits: str = "all", strata: int = 0, distances: bool = False):
         """Approximate search (see search_approx, including hits / strata / distances) of a device-resident batch; the
         result stays on the device."""
-        if hits == "all" and not distances:
-            return self._device_call(self._L.kmer_b200_search_approx_batch_device, q_ptr, off_ptr, Q, max_len, max_mismatches)
         opt = approx_options(max_mismatches, hits, strata, distances)
         return self._device_call(self._L.kmer_b200_search_approx_batch_device_ex, q_ptr, off_ptr, Q, max_len, C.byref(opt))
 
@@ -568,8 +541,6 @@ class KmerIndex:
                                   hits: str = "all", strata: int = 0, distances: bool = False):
         """Count-only approximate search of a device-resident batch: offsets and status (and best_distances() for a hit
         strategy other than "all"), no positions."""
-        if hits == "all" and not distances:
-            return self._device_call(self._L.kmer_b200_count_approx_batch_device, q_ptr, off_ptr, Q, max_len, max_mismatches)
         opt = approx_options(max_mismatches, hits, strata, distances)
         return self._device_call(self._L.kmer_b200_count_approx_batch_device_ex, q_ptr, off_ptr, Q, max_len, C.byref(opt))
 

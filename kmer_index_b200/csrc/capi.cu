@@ -263,6 +263,22 @@ struct kmer_b200_result {
 
 namespace {
 
+// Every array a result can hold: f(array member, capacity member of its host buffer, element count). The one list that
+// kmer_b200_result_free and result_to_host walk; hit_queries lives on the device only (no capacity).
+template <typename F>
+void for_each_result_array(const kmer_b200_result &r, F &&f) {
+    using R = kmer_b200_result;
+    const uint64_t Q = r.n_queries, P = r.n_positions;
+    f(&R::offsets, &R::cap_offsets, Q + 1);
+    f(&R::status, &R::cap_status, Q);
+    f(&R::positions, &R::cap_positions, P);
+    f(&R::distances, &R::cap_distances, P);
+    f(&R::best_distance, &R::cap_best_distance, Q);
+    f(&R::seed_offsets, &R::cap_seed_offsets, P);
+    f(&R::kmer_counts, &R::cap_kmer_counts, r.n_kmers);
+    f(&R::hit_queries, (size_t R::*)nullptr, Q + 1);
+}
+
 struct DeviceGuard {
     int prev = -1;
     explicit DeviceGuard(int dev) {
@@ -1405,6 +1421,24 @@ struct PackedQueries {
     uint32_t stride;
 };
 
+// A device result of Q queries with its offsets and status allocated, or null (the error is recorded); the caller places
+// the rest and releases it with kmer_b200_result_free.
+kmer_b200_result *device_result_new(kmer_b200_index *ix, uint64_t Q) {
+    kmer_b200_result *res = new (std::nothrow) kmer_b200_result();
+    if (!res) {
+        fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation failed");
+        return nullptr;
+    }
+    res->index = ix;
+    res->on_device = true;
+    res->n_queries = Q;
+    if (dev_alloc(ix, &res->offsets, Q + 1, false) || dev_alloc(ix, &res->status, Q, false)) {
+        kmer_b200_result_free(res);
+        return nullptr;
+    }
+    return res;
+}
+
 // the device arrays of a hit strategy (search_begin allocates them)
 kb::ApproxHitArgs approx_hit_args(const PendingSearch *p) {
     kb::ApproxHitArgs h{};
@@ -1440,11 +1474,8 @@ int search_begin(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off,
     if ((ix->cfg.reserved & KMER_B200_FLAG_SHARED_POSITIONS) && (d_present4 || d_present_global))
         return fail(KMER_B200_ERR_UNSUPPORTED, "a shared-positions index is unsharded: no cross-shard presence exchange");
     cudaStream_t st = ix->stream;
-    kmer_b200_result *res = new (std::nothrow) kmer_b200_result();
-    if (!res) return fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation failed");
-    res->index = ix;
-    res->on_device = true;
-    res->n_queries = Q;
+    kmer_b200_result *res = device_result_new(ix, Q);
+    if (!res) return KMER_B200_ERR_OUT_OF_MEMORY;
     p->ix = ix;
     p->res = res;
     auto bail = [&](int code) {
@@ -1453,8 +1484,7 @@ int search_begin(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off,
         p->res = nullptr;
         return code;
     };
-    if (dev_alloc(ix, &res->offsets, Q + 1, false) || dev_alloc(ix, &res->status, Q, false) ||
-        dev_alloc(ix, &p->d_unsorted, Q, false) || dev_alloc(ix, &p->d_block_sums, offsets_scan_blocks(Q) + 1, false) ||
+    if (dev_alloc(ix, &p->d_unsorted, Q, false) || dev_alloc(ix, &p->d_block_sums, offsets_scan_blocks(Q) + 1, false) ||
         (d_present4 && dev_alloc(ix, &p->d_defer, Q, false)) || dev_alloc(ix, &p->d_heavy, Q + 1, false) ||
         dev_alloc(ix, &p->d_hits, Q + 1, false) || dev_alloc(ix, &p->d_flags, 4, false))
         return bail(KMER_B200_ERR_OUT_OF_MEMORY);
@@ -1724,19 +1754,16 @@ int whole_index_check(const kmer_b200_index *ix, const char *what) {
     return KMER_B200_OK;
 }
 
-int approx_check(const kmer_b200_index *ix, uint32_t max_mismatches) {
-    if (max_mismatches > kb::kMaxMismatches) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "approximate search: max_mismatches above 8");
-    return whole_index_check(ix, "approximate search");
-}
-
-// the options of the _ex entry points: INVALID_ARGUMENT for null options, e > 8, an unknown strategy or unknown flag
-// bits, then the handle checks of approx_check. Every hit without distances takes the plain approximate path (null).
+// The options of approximate search: INVALID_ARGUMENT for null options, an unknown strategy, unknown flag bits or e > 8,
+// then the handle checks of whole_index_check. Every hit without distances takes the plain approximate path (null).
 int approx_options_check(const kmer_b200_index *ix, const kmer_b200_approx_options *opt, const kmer_b200_approx_options **hit_opt) {
     if (!opt) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "approximate search: null options");
     if (opt->hits > KMER_B200_HITS_STRATA) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "approximate search: unknown hit strategy");
     if (opt->flags & ~(uint32_t)KMER_B200_APPROX_DISTANCES)
         return fail(KMER_B200_ERR_INVALID_ARGUMENT, "approximate search: unknown option flags");
-    KB_TRY(approx_check(ix, opt->max_mismatches));
+    if (opt->max_mismatches > kb::kMaxMismatches)
+        return fail(KMER_B200_ERR_INVALID_ARGUMENT, "approximate search: max_mismatches above 8");
+    KB_TRY(whole_index_check(ix, "approximate search"));
     *hit_opt = (opt->hits == KMER_B200_HITS_ALL && !(opt->flags & KMER_B200_APPROX_DISTANCES)) ? nullptr : opt;
     return KMER_B200_OK;
 }
@@ -1762,11 +1789,8 @@ int seed_device_impl(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_
     if (Q >= 0xFFFFFFFFull) return fail(KMER_B200_ERR_UNSUPPORTED, "more than 2^32 - 2 queries in one batch: split the batch");
     if (max_len >= (1ull << 32)) return fail(KMER_B200_ERR_UNSUPPORTED, "seeding: a query offset j is reported in 32 bits");
     cudaStream_t st = ix->stream;
-    kmer_b200_result *res = new (std::nothrow) kmer_b200_result();
-    if (!res) return fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation failed");
-    res->index = ix;
-    res->on_device = true;
-    res->n_queries = Q;
+    kmer_b200_result *res = device_result_new(ix, Q);
+    if (!res) return KMER_B200_ERR_OUT_OF_MEMORY;
     uint64_t *d_kbase = nullptr, *d_block_sums = nullptr;
     uint32_t *d_flags = nullptr, *d_lo = nullptr;
     unsigned long long *d_n_heavy = nullptr;
@@ -1796,9 +1820,8 @@ int seed_device_impl(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_
     };
     hs = (uint64_t *)pinned_get(8 * sizeof(uint64_t), &hs_cap);
     if (!hs) return bail(fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed"));
-    if (dev_alloc(ix, &res->offsets, Q + 1, false) || dev_alloc(ix, &res->status, Q, false) || dev_alloc(ix, &d_kbase, Q + 1, false) ||
-        dev_alloc(ix, &d_block_sums, offsets_scan_blocks(Q) + 1, false) || dev_alloc(ix, &d_flags, 1, false) ||
-        dev_alloc(ix, &d_n_heavy, 1, false))
+    if (dev_alloc(ix, &d_kbase, Q + 1, false) || dev_alloc(ix, &d_block_sums, offsets_scan_blocks(Q) + 1, false) ||
+        dev_alloc(ix, &d_flags, 1, false) || dev_alloc(ix, &d_n_heavy, 1, false))
         return bail(KMER_B200_ERR_OUT_OF_MEMORY);
     // each query's first k-mer in the batch's k-mer order
     launch_seed_kmers_per_query(d_off, Q, ix->ks[elem], d_kbase, st);
@@ -1901,6 +1924,66 @@ struct StagedBatch {
     }
     const uint8_t *ranks(const uint64_t *q_offsets) const { return d_q - q_offsets[0]; }
 };
+
+// What a batch entry point asks for. Every device entry point and every single-copy host batch is one of these four kinds.
+struct BatchRequest {
+    enum Kind { kExact, kExactGlobal, kApprox, kSeeds } kind = kExact;
+    SearchFlavor flavor = kFlavorFull;
+    uint32_t mode = UINT32_MAX;     // exact: a kmer_b200_mode, or UINT32_MAX for the index default
+    const void *present = nullptr;  // exact global: the whole-text presence flags and their format
+    uint32_t present_format = 0;
+    const kmer_b200_approx_options *opt = nullptr;      // approximate: the caller's options
+    const kmer_b200_approx_options *hit_opt = nullptr;  // approximate: the effective options (request_check)
+    uint32_t k = 0, elem = 0, max_occ = 0;              // seeding: k, its element (request_check) and the repeat cap
+    static BatchRequest exact(uint32_t mode, SearchFlavor f) {
+        BatchRequest r;
+        r.mode = mode, r.flavor = f;
+        return r;
+    }
+    static BatchRequest exact_global(uint32_t mode, const void *present, uint32_t format) {
+        BatchRequest r;
+        r.kind = kExactGlobal, r.mode = mode, r.present = present, r.present_format = format;
+        return r;
+    }
+    static BatchRequest approx(const kmer_b200_approx_options *opt, SearchFlavor f) {
+        BatchRequest r;
+        r.kind = kApprox, r.opt = opt, r.flavor = f;
+        return r;
+    }
+    static BatchRequest seeds(uint32_t k, uint32_t max_occ, SearchFlavor f) {
+        BatchRequest r;
+        r.kind = kSeeds, r.k = k, r.max_occ = max_occ, r.flavor = f;
+        return r;
+    }
+};
+
+// The checks of a request before the device is touched (the batch's offsets, on the host or the device, must not be
+// null); fills in the effective hit options of approximate search and the element of seeding.
+int request_check(const kmer_b200_index *ix, const uint64_t *offsets, BatchRequest *req, kmer_b200_result **out) {
+    if (!ix || !out || !offsets) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    *out = nullptr;
+    switch (req->kind) {
+    case BatchRequest::kExactGlobal:
+        if (!req->present || req->present_format > 1) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "bad argument");
+        return KMER_B200_OK;
+    case BatchRequest::kApprox: return approx_options_check(ix, req->opt, &req->hit_opt);
+    case BatchRequest::kSeeds: return seed_check(ix, req->k, &req->elem);
+    default: return KMER_B200_OK;
+    }
+}
+
+// A checked request over queries on the device; the result stays on the device. The caller holds the handle's lock and
+// device.
+int request_run(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len, const BatchRequest &req,
+                kmer_b200_result **out) {
+    switch (req.kind) {
+    case BatchRequest::kApprox:
+        return search_device_impl(ix, d_q, d_off, Q, max_len, KMER_B200_MODE_CORRECT, nullptr, 0, req.flavor, out, nullptr,
+                                  (int32_t)req.opt->max_mismatches, req.hit_opt);
+    case BatchRequest::kSeeds: return seed_device_impl(ix, d_q, d_off, Q, max_len, req.elem, req.max_occ, req.flavor, out);
+    default: return search_device_impl(ix, d_q, d_off, Q, max_len, req.mode, req.present, req.present_format, req.flavor, out);
+    }
+}
 
 }  // namespace
 
@@ -2141,83 +2224,65 @@ void kmer_b200_destroy(kmer_b200_index *ix) {
     delete ix;
 }
 
-int kmer_b200_search_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
-                                  uint64_t max_len, uint32_t mode, kmer_b200_result **out) {
-    KB_NOT_ON_GROUP(ix);
-    if (!ix || !out || (!d_off)) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
-    *out = nullptr;
+// The device entry points: the request's checks, then the device and the handle's lock, once for all of them. The exact
+// forms refuse multi-device handles first, the global-presence form collection indexes too; approximate search and
+// seeding refuse those handles in their own checks.
+static int device_entry(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len, BatchRequest req,
+                        kmer_b200_result **out) {
+    if (req.kind == BatchRequest::kExact || req.kind == BatchRequest::kExactGlobal) { KB_NOT_ON_GROUP(ix); }
+    if (req.kind == BatchRequest::kExactGlobal) { KB_NOT_ON_COLLECTION(ix); }
+    KB_TRY(request_check(ix, d_off, &req, out));
     DeviceGuard guard(ix->device);
     std::lock_guard<std::mutex> lock(ix->mu);
-    return search_device_impl(ix, d_q, d_off, Q, max_len, mode, nullptr, 0, kFlavorFull, out);
+    return request_run(ix, d_q, d_off, Q, max_len, req, out);
+}
+
+int kmer_b200_search_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
+                                  uint64_t max_len, uint32_t mode, kmer_b200_result **out) {
+    return device_entry(ix, d_q, d_off, Q, max_len, BatchRequest::exact(mode, kFlavorFull), out);
 }
 
 int kmer_b200_count_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
                                  uint64_t max_len, uint32_t mode, kmer_b200_result **out) {
-    KB_NOT_ON_GROUP(ix);
-    if (!ix || !out || (!d_off)) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
-    *out = nullptr;
-    DeviceGuard guard(ix->device);
-    std::lock_guard<std::mutex> lock(ix->mu);
-    return search_device_impl(ix, d_q, d_off, Q, max_len, mode, nullptr, 0, kFlavorCountOnly, out);
+    return device_entry(ix, d_q, d_off, Q, max_len, BatchRequest::exact(mode, kFlavorCountOnly), out);
 }
 
 int kmer_b200_search_approx_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
                                          uint64_t max_len, uint32_t max_mismatches, kmer_b200_result **out) {
-    if (!ix || !out || !d_off) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
-    *out = nullptr;
-    KB_TRY(approx_check(ix, max_mismatches));
-    DeviceGuard guard(ix->device);
-    std::lock_guard<std::mutex> lock(ix->mu);
-    return search_device_impl(ix, d_q, d_off, Q, max_len, KMER_B200_MODE_CORRECT, nullptr, 0, kFlavorFull, out, nullptr,
-                              (int32_t)max_mismatches);
+    const kmer_b200_approx_options opt{max_mismatches, KMER_B200_HITS_ALL, 0, 0};
+    return device_entry(ix, d_q, d_off, Q, max_len, BatchRequest::approx(&opt, kFlavorFull), out);
 }
 
 int kmer_b200_count_approx_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
                                         uint64_t max_len, uint32_t max_mismatches, kmer_b200_result **out) {
-    if (!ix || !out || !d_off) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
-    *out = nullptr;
-    KB_TRY(approx_check(ix, max_mismatches));
-    DeviceGuard guard(ix->device);
-    std::lock_guard<std::mutex> lock(ix->mu);
-    return search_device_impl(ix, d_q, d_off, Q, max_len, KMER_B200_MODE_CORRECT, nullptr, 0, kFlavorCountOnly, out, nullptr,
-                              (int32_t)max_mismatches);
+    const kmer_b200_approx_options opt{max_mismatches, KMER_B200_HITS_ALL, 0, 0};
+    return device_entry(ix, d_q, d_off, Q, max_len, BatchRequest::approx(&opt, kFlavorCountOnly), out);
 }
 
 int kmer_b200_search_approx_batch_device_ex(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
                                             uint64_t max_len, const kmer_b200_approx_options *opt, kmer_b200_result **out) {
-    if (!ix || !out || !d_off) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
-    *out = nullptr;
-    const kmer_b200_approx_options *hit_opt = nullptr;
-    KB_TRY(approx_options_check(ix, opt, &hit_opt));
-    DeviceGuard guard(ix->device);
-    std::lock_guard<std::mutex> lock(ix->mu);
-    return search_device_impl(ix, d_q, d_off, Q, max_len, KMER_B200_MODE_CORRECT, nullptr, 0, kFlavorFull, out, nullptr,
-                              (int32_t)opt->max_mismatches, hit_opt);
+    return device_entry(ix, d_q, d_off, Q, max_len, BatchRequest::approx(opt, kFlavorFull), out);
 }
 
 int kmer_b200_count_approx_batch_device_ex(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
                                            uint64_t max_len, const kmer_b200_approx_options *opt, kmer_b200_result **out) {
-    if (!ix || !out || !d_off) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
-    *out = nullptr;
-    const kmer_b200_approx_options *hit_opt = nullptr;
-    KB_TRY(approx_options_check(ix, opt, &hit_opt));
-    DeviceGuard guard(ix->device);
-    std::lock_guard<std::mutex> lock(ix->mu);
-    return search_device_impl(ix, d_q, d_off, Q, max_len, KMER_B200_MODE_CORRECT, nullptr, 0, kFlavorCountOnly, out, nullptr,
-                              (int32_t)opt->max_mismatches, hit_opt);
+    return device_entry(ix, d_q, d_off, Q, max_len, BatchRequest::approx(opt, kFlavorCountOnly), out);
 }
 
 int kmer_b200_search_batch_device_global(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q,
                                          uint64_t max_len, uint32_t mode, const void *d_present_global,
                                          uint32_t present_format, kmer_b200_result **out) {
-    KB_NOT_ON_GROUP(ix);
-    KB_NOT_ON_COLLECTION(ix);
-    if (!ix || !out || !d_off || !d_present_global || present_format > 1)
-        return fail(KMER_B200_ERR_INVALID_ARGUMENT, "bad argument");
-    *out = nullptr;
-    DeviceGuard guard(ix->device);
-    std::lock_guard<std::mutex> lock(ix->mu);
-    return search_device_impl(ix, d_q, d_off, Q, max_len, mode, d_present_global, present_format, kFlavorFull, out);
+    return device_entry(ix, d_q, d_off, Q, max_len, BatchRequest::exact_global(mode, d_present_global, present_format), out);
+}
+
+int kmer_b200_seed_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len,
+                                uint32_t k, uint32_t max_occ, kmer_b200_result **out) {
+    return device_entry(ix, d_q, d_off, Q, max_len, BatchRequest::seeds(k, max_occ, kFlavorFull), out);
+}
+
+int kmer_b200_count_seeds_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len,
+                                       uint32_t k, uint32_t max_occ, kmer_b200_result **out) {
+    return device_entry(ix, d_q, d_off, Q, max_len, BatchRequest::seeds(k, max_occ, kFlavorCountOnly), out);
 }
 
 struct kmer_b200_pending {
@@ -2687,50 +2752,52 @@ static int search_batch_host_chunked(kmer_b200_index *ix, const uint8_t *q_ranks
     return code;
 }
 
-// One copy each way: the batch is staged on the device whole, searched, and the result copied back into pinned host buffers.
-// Small exact batches, and every approximate batch (max_mismatches >= 0), take this path. The caller holds the
-// handle's lock and device.
-static int search_batch_host_single_copy(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q,
-                                         uint32_t mode, const uint8_t *lut256, int32_t max_mismatches, kmer_b200_result **out,
-                                         const kmer_b200_approx_options *hit_opt = nullptr) {
-    cudaStream_t st = ix->stream;
+// The device result dres copied into a new host result: a pinned buffer for each array dres holds (the positions as
+// host_result_positions places them), copied on the index's stream with one synchronisation. *d2h = the bytes copied.
+static int result_to_host(kmer_b200_index *ix, const kmer_b200_result *dres, kmer_b200_result **out, uint64_t *d2h) {
+    kmer_b200_result *res = host_result_new(ix, dres->n_queries);
+    bool ok = res && host_result_positions(res, dres->n_positions);
+    if (ok) res->n_kmers = dres->n_kmers;
+    uint64_t bytes = 0;
+    for_each_result_array(*dres, [&](auto array, auto cap, uint64_t n) {
+        using T = std::remove_reference_t<decltype(*(dres->*array))>;
+        if (!ok || !cap || !(dres->*array)) return;
+        if (!(res->*array)) ok = (res->*array = (T *)pinned_get(n * sizeof(T), &(res->*cap))) != nullptr;
+        if (ok && n) cudaMemcpyAsync(res->*array, dres->*array, n * sizeof(T), cudaMemcpyDeviceToHost, ix->stream), bytes += n * sizeof(T);
+    });
+    // also when an allocation failed: the copies already queued finish before their buffers go back to the cache
+    const cudaError_t e = cudaStreamSynchronize(ix->stream);
+    if (!ok || e != cudaSuccess) {
+        cudaGetLastError();
+        kmer_b200_result_free(res);
+        return ok ? fail(KMER_B200_ERR_CUDA, std::string("result (D2H): ") + cudaGetErrorString(e))
+                  : fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed");
+    }
+    *d2h = bytes;
+    *out = res;
+    return KMER_B200_OK;
+}
+
+// One copy each way: the batch is staged on the device whole, the request runs there, and the result comes back into
+// pinned host buffers. Small exact batches, collections, approximate search and seeding take this path.
+static int host_batch(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q, const uint8_t *lut256,
+                      BatchRequest req, kmer_b200_result **out) {
+    KB_TRY(request_check(ix, q_offsets, &req, out));
     const uint64_t n_sym = q_offsets[Q] - q_offsets[0];
+    if (n_sym && !q_ranks) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "q_ranks is null");
+    DeviceGuard guard(ix->device);
+    std::lock_guard<std::mutex> lock(ix->mu);
     StagedBatch staged(ix);
     KB_TRY(staged.stage(q_ranks, q_offsets, Q, lut256));
     kmer_b200_result *dres = nullptr;
-    int s = search_device_impl(ix, staged.ranks(q_offsets), staged.d_off, Q, staged.max_len, mode, nullptr, 0, kFlavorFull, &dres, nullptr,
-                               max_mismatches, hit_opt);
-    if (s != 0) return s;
-    // device result -> pinned host buffers
-    kmer_b200_result *res = host_result_new(ix, Q);
-    bool extra_ok = res != nullptr;
-    if (res && dres->distances)
-        extra_ok = (res->distances = (uint8_t *)pinned_get(std::max<uint64_t>(dres->n_positions, 1), &res->cap_distances)) != nullptr;
-    if (extra_ok && dres->best_distance)
-        extra_ok = (res->best_distance = (uint8_t *)pinned_get(std::max<uint64_t>(Q, 1), &res->cap_best_distance)) != nullptr;
-    if (!res || !extra_ok || !host_result_positions(res, dres->n_positions)) {
-        kmer_b200_result_free(dres);
-        kmer_b200_result_free(res);
-        return fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed");
-    }
-    cudaMemcpyAsync(res->offsets, dres->offsets, (Q + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
-    if (Q) cudaMemcpyAsync(res->status, dres->status, Q, cudaMemcpyDeviceToHost, st);
-    if (res->n_positions)
-        cudaMemcpyAsync(res->positions, dres->positions, res->n_positions * sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
-    const uint64_t n_dist = dres->distances ? res->n_positions : 0, n_best = dres->best_distance ? Q : 0;
-    if (n_dist) cudaMemcpyAsync(res->distances, dres->distances, n_dist, cudaMemcpyDeviceToHost, st);
-    if (n_best) cudaMemcpyAsync(res->best_distance, dres->best_distance, n_best, cudaMemcpyDeviceToHost, st);
-    cudaError_t e = cudaStreamSynchronize(st);
+    KB_TRY(request_run(ix, staged.ranks(q_offsets), staged.d_off, Q, staged.max_len, req, &dres));
+    uint64_t d2h = 0;
+    const int s = result_to_host(ix, dres, out, &d2h);
     kmer_b200_result_free(dres);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        kmer_b200_result_free(res);
-        return fail(KMER_B200_ERR_CUDA, std::string("search (D2H): ") + cudaGetErrorString(e));
-    }
+    if (s != 0) return s;
     ix->last_h2d = n_sym + (Q + 1) * sizeof(uint64_t);
-    ix->last_d2h = (Q + 1) * sizeof(uint64_t) + Q + res->n_positions * sizeof(uint32_t) + n_dist + n_best;
+    ix->last_d2h = d2h;
     ix->last_host_path = 0, ix->last_raw_pct = 100, ix->last_pack_gbs = 0;
-    *out = res;
     return KMER_B200_OK;
 }
 
@@ -2739,12 +2806,12 @@ static int search_batch_host(kmer_b200_index *ix, const uint8_t *q_ranks, const 
     if (!ix || !out || !q_offsets) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
     *out = nullptr;
     if (!ix->replicas.empty()) return search_batch_multi(ix, q_ranks, q_offsets, Q, mode, lut256, out);
-    DeviceGuard guard(ix->device);
-    std::lock_guard<std::mutex> lock(ix->mu);
     const uint64_t n_sym = q_offsets[Q] - q_offsets[0];
     if (n_sym && !q_ranks) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "q_ranks is null");
     // batches whose transfer dominates (>= 256 MiB over PCIe) are pipelined in chunks
     if (!lut256 && ix->starts.empty() && Q >= (1u << 18) && n_sym + Q * 17 >= (256ull << 20) && !std::getenv("KMER_B200_NO_PIPELINE")) {
+        DeviceGuard guard(ix->device);
+        std::lock_guard<std::mutex> lock(ix->mu);
         // The share of raw chunks. Pageable input cannot be DMA-ed directly (the driver would stage it at a fraction of the
         // link rate): every chunk is packed straight out of the caller's memory into a pinned ring. Pinned input of 2- and
         // 4-bit alphabets: the share comes from the host's streaming pack rate, measured once per process on the first
@@ -2773,7 +2840,7 @@ static int search_batch_host(kmer_b200_index *ix, const uint8_t *q_ranks, const 
         }
         // no producer thread to be had: one copy each way
     }
-    return search_batch_host_single_copy(ix, q_ranks, q_offsets, Q, mode, lut256, -1, out);
+    return host_batch(ix, q_ranks, q_offsets, Q, lut256, BatchRequest::exact(mode, kFlavorFull), out);
 }
 
 int kmer_b200_search_batch(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q,
@@ -2783,95 +2850,18 @@ int kmer_b200_search_batch(kmer_b200_index *ix, const uint8_t *q_ranks, const ui
 
 int kmer_b200_search_approx_batch(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q,
                                   uint32_t max_mismatches, kmer_b200_result **out) {
-    if (!ix || !out || !q_offsets) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
-    *out = nullptr;
-    KB_TRY(approx_check(ix, max_mismatches));
-    if (q_offsets[Q] != q_offsets[0] && !q_ranks) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "q_ranks is null");
-    DeviceGuard guard(ix->device);
-    std::lock_guard<std::mutex> lock(ix->mu);
-    return search_batch_host_single_copy(ix, q_ranks, q_offsets, Q, KMER_B200_MODE_CORRECT, nullptr, (int32_t)max_mismatches, out);
+    const kmer_b200_approx_options opt{max_mismatches, KMER_B200_HITS_ALL, 0, 0};
+    return host_batch(ix, q_ranks, q_offsets, Q, nullptr, BatchRequest::approx(&opt, kFlavorFull), out);
 }
 
 int kmer_b200_search_approx_batch_ex(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q,
                                      const kmer_b200_approx_options *opt, kmer_b200_result **out) {
-    if (!ix || !out || !q_offsets) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
-    *out = nullptr;
-    const kmer_b200_approx_options *hit_opt = nullptr;
-    KB_TRY(approx_options_check(ix, opt, &hit_opt));
-    if (q_offsets[Q] != q_offsets[0] && !q_ranks) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "q_ranks is null");
-    DeviceGuard guard(ix->device);
-    std::lock_guard<std::mutex> lock(ix->mu);
-    return search_batch_host_single_copy(ix, q_ranks, q_offsets, Q, KMER_B200_MODE_CORRECT, nullptr, (int32_t)opt->max_mismatches,
-                                         out, hit_opt);
+    return host_batch(ix, q_ranks, q_offsets, Q, nullptr, BatchRequest::approx(opt, kFlavorFull), out);
 }
 
 int kmer_b200_seed_batch(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q, uint32_t k,
                          uint32_t max_occ, kmer_b200_result **out) {
-    if (!ix || !out || !q_offsets) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
-    *out = nullptr;
-    uint32_t elem = 0;
-    KB_TRY(seed_check(ix, k, &elem));
-    if (q_offsets[Q] != q_offsets[0] && !q_ranks) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "q_ranks is null");
-    DeviceGuard guard(ix->device);
-    std::lock_guard<std::mutex> lock(ix->mu);
-    cudaStream_t st = ix->stream;
-    StagedBatch staged(ix);
-    KB_TRY(staged.stage(q_ranks, q_offsets, Q, nullptr));
-    kmer_b200_result *dres = nullptr;
-    KB_TRY(seed_device_impl(ix, staged.ranks(q_offsets), staged.d_off, Q, staged.max_len, elem, max_occ, kFlavorFull, &dres));
-    // device result -> pinned host buffers
-    kmer_b200_result *res = host_result_new(ix, Q);
-    bool ok = res != nullptr;
-    if (ok) {
-        res->n_kmers = dres->n_kmers;
-        ok = (res->kmer_counts = (uint32_t *)pinned_get(std::max<uint64_t>(dres->n_kmers, 1) * sizeof(uint32_t), &res->cap_kmer_counts)) &&
-             (res->seed_offsets = (uint32_t *)pinned_get(std::max<uint64_t>(dres->n_positions, 1) * sizeof(uint32_t), &res->cap_seed_offsets)) &&
-             host_result_positions(res, dres->n_positions);
-    }
-    if (!ok) {
-        kmer_b200_result_free(dres);
-        kmer_b200_result_free(res);
-        return fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed");
-    }
-    const uint64_t n_pos = res->n_positions, n_kmers = res->n_kmers;
-    cudaMemcpyAsync(res->offsets, dres->offsets, (Q + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
-    if (Q) cudaMemcpyAsync(res->status, dres->status, Q, cudaMemcpyDeviceToHost, st);
-    if (n_pos) cudaMemcpyAsync(res->positions, dres->positions, n_pos * sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
-    if (n_pos) cudaMemcpyAsync(res->seed_offsets, dres->seed_offsets, n_pos * sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
-    if (n_kmers) cudaMemcpyAsync(res->kmer_counts, dres->kmer_counts, n_kmers * sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
-    cudaError_t e = cudaStreamSynchronize(st);
-    kmer_b200_result_free(dres);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        kmer_b200_result_free(res);
-        return fail(KMER_B200_ERR_CUDA, std::string("seeding (D2H): ") + cudaGetErrorString(e));
-    }
-    ix->last_h2d = (q_offsets[Q] - q_offsets[0]) + (Q + 1) * sizeof(uint64_t);
-    ix->last_d2h = (Q + 1) * sizeof(uint64_t) + Q + 2 * n_pos * sizeof(uint32_t) + n_kmers * sizeof(uint32_t);
-    ix->last_host_path = 0, ix->last_raw_pct = 100, ix->last_pack_gbs = 0;
-    *out = res;
-    return KMER_B200_OK;
-}
-
-static int seed_device_entry(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len, uint32_t k,
-                             uint32_t max_occ, SearchFlavor flavor, kmer_b200_result **out) {
-    if (!ix || !out || !d_off) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
-    *out = nullptr;
-    uint32_t elem = 0;
-    KB_TRY(seed_check(ix, k, &elem));
-    DeviceGuard guard(ix->device);
-    std::lock_guard<std::mutex> lock(ix->mu);
-    return seed_device_impl(ix, d_q, d_off, Q, max_len, elem, max_occ, flavor, out);
-}
-
-int kmer_b200_seed_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len,
-                                uint32_t k, uint32_t max_occ, kmer_b200_result **out) {
-    return seed_device_entry(ix, d_q, d_off, Q, max_len, k, max_occ, kFlavorFull, out);
-}
-
-int kmer_b200_count_seeds_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len,
-                                       uint32_t k, uint32_t max_occ, kmer_b200_result **out) {
-    return seed_device_entry(ix, d_q, d_off, Q, max_len, k, max_occ, kFlavorCountOnly, out);
+    return host_batch(ix, q_ranks, q_offsets, Q, nullptr, BatchRequest::seeds(k, max_occ, kFlavorFull), out);
 }
 
 int kmer_b200_search_batch_ptrs(kmer_b200_index *ix, const uint8_t *const *q_ptrs, const uint64_t *q_lens, uint64_t Q,
@@ -2958,25 +2948,15 @@ void kmer_b200_result_free(kmer_b200_result *r) {
     kmer_b200_index *ix = r->index;
     if (r->on_device) {
         DeviceGuard guard(ix->device);
-        dev_free(ix, r->offsets);
-        dev_free(ix, r->positions);
-        dev_free(ix, r->status);
-        dev_free(ix, r->hit_queries);
-        dev_free(ix, r->distances);
-        dev_free(ix, r->best_distance);
-        dev_free(ix, r->seed_offsets);
-        dev_free(ix, r->kmer_counts);
+        for_each_result_array(*r, [&](auto array, auto, uint64_t) { dev_free(ix, r->*array); });
     } else {
-        pinned_put(r->offsets, r->cap_offsets);
-        if (r->positions_pageable)
+        if (r->positions_pageable) {
             std::free(r->positions);
-        else
-            pinned_put(r->positions, r->cap_positions);
-        pinned_put(r->status, r->cap_status);
-        pinned_put(r->distances, r->cap_distances);
-        pinned_put(r->best_distance, r->cap_best_distance);
-        pinned_put(r->seed_offsets, r->cap_seed_offsets);
-        pinned_put(r->kmer_counts, r->cap_kmer_counts);
+            r->positions = nullptr;
+        }
+        for_each_result_array(*r, [&](auto array, auto cap, uint64_t) {
+            if (cap) pinned_put(r->*array, r->*cap);
+        });
     }
     delete r;
 }
@@ -3634,20 +3614,15 @@ int kmer_b200_unroute_device(kmer_b200_index *ix, uint8_t *d_send_blocks, uint8_
         sent.p[b + 1] = sent.p[b] + sent_counts[b];
         seg.p[b + 1] = seg.p[b] + recv_splits[b];
     }
-    kmer_b200_result *res = new (std::nothrow) kmer_b200_result();
-    if (!res) return fail(KMER_B200_ERR_OUT_OF_MEMORY, "host allocation failed");
-    res->index = ix;
-    res->on_device = true;
-    res->n_queries = Q;
+    kmer_b200_result *res = device_result_new(ix, Q);
+    if (!res) return KMER_B200_ERR_OUT_OF_MEMORY;
     uint64_t *d_block_sums = nullptr;
     auto bail = [&](int code) {
         dev_free(ix, d_block_sums);
         kmer_b200_result_free(res);
         return code;
     };
-    if (dev_alloc(ix, &res->offsets, Q + 1, false) || dev_alloc(ix, &res->status, Q, false) ||
-        dev_alloc(ix, &d_block_sums, kb::offsets_scan_blocks(Q) + 1, false))
-        return bail(KMER_B200_ERR_OUT_OF_MEMORY);
+    if (dev_alloc(ix, &d_block_sums, kb::offsets_scan_blocks(Q) + 1, false)) return bail(KMER_B200_ERR_OUT_OF_MEMORY);
     cudaMemsetAsync(res->offsets, 0, (Q + 1) * sizeof(uint64_t), st);
     if (Q) cudaMemcpyAsync(res->status, d_status, Q, cudaMemcpyDeviceToDevice, st);
     kb::launch_unroute_counts(d_send_blocks, plan->block_bytes, plan->stride, d_ret_blocks, plan->return_block_bytes, plan->capacity, N, sent,
