@@ -132,7 +132,8 @@ int kmer_b200_search_batch_text(kmer_b200_index *index, const char *q_chars, con
    '+' and quality lines too) are dropped, sequence characters are translated through lut256 (a character outside the
    alphabet fails with KMER_B200_ERR_INVALID_RANK), all records are concatenated into one rank text that stays in device
    memory -- feed it to kmer_b200_create_from_device -- and a record table maps positions back. format: 0 = by the
-   first byte ('>' / ';' FASTA, '@' FASTQ), 1 = FASTA, 2 = FASTQ (four lines per record). */
+   first byte ('>' / ';' FASTA, '@' FASTQ), 1 = FASTA, 2 = FASTQ (four lines per record; blank lines at the end of the
+   file are no records). */
 typedef struct kmer_b200_records kmer_b200_records;
 int kmer_b200_parse_sequences(const char *data, uint64_t n_bytes, const uint8_t *lut256, uint32_t sigma, uint32_t format,
                               const kmer_b200_config *cfg, kmer_b200_records **out);

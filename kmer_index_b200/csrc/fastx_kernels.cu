@@ -108,7 +108,7 @@ struct FxClass {
 };
 
 // classification of the thread's kFxPer bytes. format 1 = FASTA (header lines start with '>' or ';'), 2 = FASTQ (records of
-// four lines: @name, sequence, +, qualities)
+// four lines: @name, sequence, +, qualities; an empty line where a header would be starts no record)
 __device__ __forceinline__ FxClass fastx_classify(const uint8_t *__restrict__ data, uint64_t n, uint32_t format, uint64_t nl_before_tile,
                                                   int64_t last_nl_before_tile, int64_t *warp_buf64, uint32_t *warp_buf32, uint8_t (&ch)[kFxPer]) {
     const uint64_t i0 = (uint64_t)blockIdx.x * kFxTile + (uint64_t)threadIdx.x * kFxPer;
@@ -134,7 +134,9 @@ __device__ __forceinline__ FxClass fastx_classify(const uint8_t *__restrict__ da
             const uint8_t first = (uint64_t)line_start == i ? ch[j] : data[line_start];  // first byte of this byte's line
             bool header, seq_line;
             if (format == 2) {
-                header = (line_no & 3) == 0;
+                // an empty line in header position is no record (a file that ends in a blank line); a blank line
+                // between records moves the next '@' line to a sequence line, where '@' is refused
+                header = (line_no & 3) == 0 && first != '\n' && first != '\r';
                 seq_line = (line_no & 3) == 1;
             } else {
                 header = first == '>' || first == ';';
