@@ -302,6 +302,31 @@ int kmer_b200_count_seeds_batch_device(kmer_b200_index *index, const uint8_t *d_
                                        uint64_t n_queries, uint64_t max_query_len, uint32_t k, uint32_t max_occ,
                                        kmer_b200_result **out);
 
+/* ---- k-mer spectrum: what the index holds as a whole, read off the bucket sizes of the element of k (one of the index's
+   ks, views of a shared-positions index included; auxiliary elements do not count, any other k is
+   KMER_B200_ERR_INVALID_ARGUMENT). The counted windows are p in [0, n - k]; on a collection index only those inside one
+   record. count(h) is the number of counted windows with hash h: the uncapped count seeding reports for that k-mer.
+   Refused (KMER_B200_ERR_UNSUPPORTED) on multi-device handles, position-range shards and key-range parts that have not
+   been adopted. Runs on the index's stream and returns when the results are on the host. */
+typedef struct kmer_b200_spectrum_info {
+    uint64_t total;      /* counted windows */
+    uint64_t distinct;   /* #{h : count(h) >= 1} */
+    uint64_t max_count;  /* the largest count(h), 0 when nothing is counted */
+    uint64_t key_space;  /* sigma^k, saturated at UINT64_MAX */
+} kmer_b200_spectrum_info;
+/* hist[c] = #{h : count(h) = c} for 1 <= c < n_bins - 1, hist[n_bins - 1] = #{h : count(h) >= n_bins - 1},
+   hist[0] = sigma^k - distinct (saturated). n_bins >= 2; hist may be NULL (info only), info may be NULL. */
+int kmer_b200_spectrum(kmer_b200_index *index, uint32_t k, uint64_t *hist, uint64_t n_bins, kmer_b200_spectrum_info *info);
+/* Every h with count(h) >= min_count (>= 1), ordered by count descending, then hash ascending: *n_out = how many exist
+   (N), and the first min(N, cap) go to hashes / counts (host arrays; NULL allowed when cap = 0). Jellyfish-style "top
+   100" is min_count = 1, cap = 100. */
+int kmer_b200_frequent_kmers(kmer_b200_index *index, uint32_t k, uint64_t min_count, uint64_t *hashes, uint64_t *counts,
+                             uint64_t cap, uint64_t *n_out);
+/* The repeat cutoff that ignores the most frequent fraction of the distinct k-mers: the smallest c >= 1 with
+   #{h : count(h) > c} <= floor(fraction * distinct), 0 when distinct = 0. fraction in [0, 1). Exact at any count;
+   seeding with max_occ = cutoff drops exactly the k-mers above it. */
+int kmer_b200_occurrence_cutoff(kmer_b200_index *index, uint32_t k, double fraction, uint64_t *cutoff);
+
 uint64_t kmer_b200_result_n_queries(const kmer_b200_result *r);
 uint64_t kmer_b200_result_n_positions(const kmer_b200_result *r);
 int kmer_b200_result_on_device(const kmer_b200_result *r);

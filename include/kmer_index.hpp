@@ -555,6 +555,49 @@ namespace kmer
             return kmer_batch_result<position_t>(r);
         }
 
+        // k-mer spectrum of element k (kmer_b200_spectrum): hist[c] = distinct k-mers occurring c times for
+        // 1 <= c < bins - 1, hist[bins - 1] = those occurring bins - 1 times or more, hist[0] = sigma^k - distinct. On a
+        // collection index only windows inside one record count.
+        struct kmer_spectrum
+        {
+            std::vector<std::uint64_t> hist;
+            kmer_b200_spectrum_info info{};
+        };
+        template<std::size_t k>
+        kmer_spectrum spectrum(std::uint64_t bins = 10001) const
+        {
+            static_assert(((k == ks) || ...), "spectrum<k>: k is not one of this index's ks");
+            kmer_spectrum s;
+            s.hist.resize(bins);
+            detail::check(kmer_b200_spectrum(_handle, std::uint32_t(k), s.hist.data(), bins, &s.info));
+            return s;
+        }
+
+        // the k-mers occurring at least min_count times as (hash, count), count descending then hash ascending, the
+        // first cap of them (kmer_b200_frequent_kmers)
+        template<std::size_t k>
+        std::vector<std::pair<std::uint64_t, std::uint64_t>> frequent_kmers(std::uint64_t min_count, std::uint64_t cap) const
+        {
+            static_assert(((k == ks) || ...), "frequent_kmers<k>: k is not one of this index's ks");
+            std::vector<std::uint64_t> hashes(cap), counts(cap);
+            std::uint64_t n = 0;
+            detail::check(kmer_b200_frequent_kmers(_handle, std::uint32_t(k), min_count, hashes.data(), counts.data(), cap, &n));
+            std::vector<std::pair<std::uint64_t, std::uint64_t>> out(std::min(n, cap));
+            for (std::size_t i = 0; i < out.size(); ++i) out[i] = {hashes[i], counts[i]};
+            return out;
+        }
+
+        // the repeat cap that ignores the most frequent `fraction` of the distinct k-mers (kmer_b200_occurrence_cutoff);
+        // seed_batch<k>(queries, cutoff) drops exactly the k-mers above it
+        template<std::size_t k>
+        std::uint64_t occurrence_cutoff(double fraction) const
+        {
+            static_assert(((k == ks) || ...), "occurrence_cutoff<k>: k is not one of this index's ks");
+            std::uint64_t c = 0;
+            detail::check(kmer_b200_occurrence_cutoff(_handle, std::uint32_t(k), fraction, &c));
+            return c;
+        }
+
         // one query: its positions within max_mismatches substitutions, ascending; throws for an empty query
         std::vector<position_t> search_approx(std::vector<alphabet_t> const& query, std::uint32_t max_mismatches) const
         {

@@ -16,7 +16,7 @@ from . import _capi
 from ._capi import (MODE_CORRECT, MODE_DEFAULT, MODE_REFERENCE_EXACT, QUERY_OK, QUERY_THROW_INVALID_ARGUMENT,
                     QUERY_TOO_LONG_FOR_SHARD, QUERY_UNDEFINED, KmerB200Error)
 
-__all__ = ["KmerIndex", "make_kmer_index", "BatchResult", "Records", "parse_sequences", "fast_pow", "kmer_hash", "choose_best_k", "scheme_for_ks",
+__all__ = ["KmerIndex", "make_kmer_index", "BatchResult", "Records", "parse_sequences", "fast_pow", "kmer_hash", "kmer_from_hash", "Spectrum", "choose_best_k", "scheme_for_ks",
            "char_lut", "ALPHABET_CHARS",
            "MODE_REFERENCE_EXACT", "MODE_CORRECT", "KmerB200Error", "ALPHABETS"]
 
@@ -46,6 +46,34 @@ def kmer_hash(ranks, sigma: int) -> int:
     """The k-mer hash of `ranks` (kmer_index.hpp:56-73)."""
     r = np.ascontiguousarray(np.asarray(ranks, dtype=np.uint8))
     return int(_capi.lib().kmer_b200_hash(r.ctypes.data_as(_capi.u8p), r.size, sigma))
+
+
+def kmer_from_hash(h: int, k: int, sigma: int) -> np.ndarray:
+    """The k ranks whose kmer_hash is h (first symbol most significant): the inverse of kmer_hash, for printing the
+    k-mers of KmerIndex.frequent_kmers."""
+    h, k, sigma = int(h), int(k), int(sigma)
+    if k < 1 or not 0 <= h < sigma ** k:
+        raise ValueError(f"hash {h} is not the hash of a {k}-mer over {sigma} symbols")
+    out = np.zeros(k, dtype=np.uint8)
+    for i in range(k - 1, -1, -1):
+        h, out[i] = divmod(h, sigma)
+    return out
+
+
+class Spectrum:
+    """The k-mer spectrum of one element (KmerIndex.spectrum): hist[c] = distinct k-mers occurring c times for
+    1 <= c < len(hist) - 1, hist[-1] = those occurring len(hist) - 1 times or more, hist[0] = sigma^k - distinct; total
+    = counted windows, distinct = k-mers occurring at least once, max_count = the largest count (0 when none)."""
+
+    def __init__(self, hist: np.ndarray, info):
+        self.hist = hist
+        self.total = int(info.total)
+        self.distinct = int(info.distinct)
+        self.max_count = int(info.max_count)
+        self.key_space = int(info.key_space)
+
+    def __repr__(self):
+        return f"Spectrum(total={self.total}, distinct={self.distinct}, max_count={self.max_count}, bins={self.hist.size})"
 
 
 def choose_best_k(query_lengths: Iterable[int], n_k: int = 4) -> list[int]:
@@ -459,6 +487,39 @@ class KmerIndex:
                 raise ValueError("seeding an index with several ks needs k")
             return self.ks[0]
         return int(k)
+
+    # -- k-mer spectrum
+    def spectrum(self, k: int | None = None, bins: int = 10001) -> Spectrum:
+        """Occurrence histogram of the k-mers of element k (kmer_b200_spectrum); k defaults to the index's only k. On a
+        collection index only windows inside one record count (the counts seeding reports)."""
+        hist = np.zeros(int(bins), dtype=np.uint64)
+        info = _capi.SpectrumInfo()
+        _capi.check(self._L.kmer_b200_spectrum(self._h, self._seed_k(k), hist.ctypes.data_as(_capi.u64p), hist.size,
+                                               C.byref(info)))
+        return Spectrum(hist, info)
+
+    def frequent_kmers(self, k: int | None = None, min_count: int = 2, limit: int | None = None):
+        """(hashes, counts) as uint64 arrays: every k-mer occurring at least min_count times, by count descending then hash
+        ascending, the first `limit` of them (None: all). kmer_from_hash turns a hash back into ranks."""
+        k = self._seed_k(k)
+        n = C.c_uint64(0)
+        if limit is None:
+            _capi.check(self._L.kmer_b200_frequent_kmers(self._h, k, int(min_count), None, None, 0, C.byref(n)))
+            limit = n.value
+        hashes = np.zeros(int(limit), dtype=np.uint64)
+        counts = np.zeros(int(limit), dtype=np.uint64)
+        _capi.check(self._L.kmer_b200_frequent_kmers(self._h, k, int(min_count), hashes.ctypes.data_as(_capi.u64p),
+                                                     counts.ctypes.data_as(_capi.u64p), hashes.size, C.byref(n)))
+        m = min(n.value, hashes.size)
+        return hashes[:m], counts[:m]
+
+    def occurrence_cutoff(self, fraction: float, k: int | None = None) -> int:
+        """The repeat cap that ignores the most frequent `fraction` of the distinct k-mers (kmer_b200_occurrence_cutoff):
+        the smallest c >= 1 with #{count > c} <= floor(fraction * distinct), 0 for an empty spectrum. seeds(...,
+        max_occ=cutoff) then drops exactly the k-mers above it."""
+        c = C.c_uint64(0)
+        _capi.check(self._L.kmer_b200_occurrence_cutoff(self._h, self._seed_k(k), float(fraction), C.byref(c)))
+        return int(c.value)
 
     def seeds(self, q_ranks, q_offsets, k: int | None = None, max_occ: int = 0, copy: bool = True) -> BatchResult:
         """k-mer seeding of a host batch (kmer_b200_seed_batch): per query, for every offset j in [0, m - k], every text

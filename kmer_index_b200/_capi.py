@@ -62,6 +62,10 @@ class PlanRow(C.Structure):
                 ("expected_candidates", C.c_double), ("expected_sectors", C.c_double)]
 
 
+class SpectrumInfo(C.Structure):
+    _fields_ = [("total", C.c_uint64), ("distinct", C.c_uint64), ("max_count", C.c_uint64), ("key_space", C.c_uint64)]
+
+
 class KernelStat(C.Structure):
     _fields_ = [("name", C.c_char_p), ("launches", C.c_uint64), ("device_ms", C.c_double),
                 ("algorithmic_bytes", C.c_double)]
@@ -122,6 +126,9 @@ SYMBOLS = {
                                               C.c_uint32, C.POINTER(C.c_void_p)]),
     "kmer_b200_count_seeds_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32,
                                                      C.c_uint32, C.POINTER(C.c_void_p)]),
+    "kmer_b200_spectrum": (C.c_int, [C.c_void_p, C.c_uint32, u64p, C.c_uint64, C.POINTER(SpectrumInfo)]),
+    "kmer_b200_frequent_kmers": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint64, u64p, u64p, C.c_uint64, u64p]),
+    "kmer_b200_occurrence_cutoff": (C.c_int, [C.c_void_p, C.c_uint32, C.c_double, u64p]),
     "kmer_b200_result_n_queries": (C.c_uint64, [C.c_void_p]),
     "kmer_b200_result_n_positions": (C.c_uint64, [C.c_void_p]),
     "kmer_b200_result_on_device": (C.c_int, [C.c_void_p]),

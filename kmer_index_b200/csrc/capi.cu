@@ -1740,13 +1740,14 @@ __global__ void max_len_kernel(const uint64_t *__restrict__ off, uint64_t Q, uns
 
 // Approximate search, collections and seeding need the whole text and every position of every element on this device
 // (whole or in peer parts), each bucket in ascending position order: refused (with the reason, `what` = the feature)
-// for the handles where one of them lives elsewhere.
-int whole_index_check(const kmer_b200_index *ix, const char *what) {
+// for the handles where one of them lives elsewhere. views_ok: the feature also reads the views of a shared-positions
+// index (the k-mer spectrum needs bucket sizes only, not their order).
+int whole_index_check(const kmer_b200_index *ix, const char *what, bool views_ok = false) {
     const std::string w(what);
     if (!ix->replicas.empty()) return fail(KMER_B200_ERR_UNSUPPORTED, w + " is not available on a multi-device handle");
     if (ix->sharded || !ix->reaches_end || ix->cfg.halo != 0)
         return fail(KMER_B200_ERR_UNSUPPORTED, w + " is not available on a position-range shard");
-    if (ix->cfg.reserved & KMER_B200_FLAG_SHARED_POSITIONS)
+    if (!views_ok && (ix->cfg.reserved & KMER_B200_FLAG_SHARED_POSITIONS))
         return fail(KMER_B200_ERR_UNSUPPORTED, w + " is not available on a shared-positions index");
     for (size_t e = 0; e < ix->ks.size(); ++e)
         if (ix->elems[e].dev.key_lo != 0 || ix->elems[e].dev.key_hi != UINT64_MAX)
@@ -3467,6 +3468,288 @@ int kmer_b200_locate_device(kmer_b200_index *ix, const uint32_t *d_positions, ui
     kb::launch_locate(ix->d_starts, ix->starts.size() - 1, d_positions, n, d_record_out, d_offset_out, ix->stream);
     KB_CUDA(cudaGetLastError());
     return KMER_B200_OK;
+}
+
+// ---- k-mer spectrum (spectrum.cu). The caller of each helper holds the handle's lock and device.
+
+// bins of the histogram behind kmer_b200_frequent_kmers and kmer_b200_occurrence_cutoff: counts up to 65 534 are read off
+// it, larger ones (at most n / 65 535 hashes) are selected and sorted
+constexpr uint64_t kSpectrumSelectBins = 1ull << 16;
+constexpr uint64_t kSpectrumMaxBins = 1ull << 24;
+
+// the element of k (not an auxiliary one; views included), after the handle checks of whole_index_check
+static int spectrum_check(const kmer_b200_index *ix, uint32_t k, uint32_t *elem) {
+    KB_TRY(whole_index_check(ix, "the k-mer spectrum", true));
+    for (size_t e = 0; e < ix->ks.size(); ++e)
+        if (ix->ks[e] == k) {
+            *elem = (uint32_t)e;
+            return KMER_B200_OK;
+        }
+    return fail(KMER_B200_ERR_INVALID_ARGUMENT, "k-mer spectrum: k is not one of the index's ks");
+}
+
+// windows p < s < p + k charged to record start r (no start in (p, s)); the rule of spectrum_corrections_kernel
+static uint64_t junction_windows(const std::vector<uint64_t> &starts, uint64_t r, uint64_t n, uint32_t k) {
+    const uint64_t s = starts[r], prev = starts[r - 1];
+    if (s == 0 || s <= prev) return 0;
+    const uint64_t lo = std::max<uint64_t>(s + 1 >= k ? s + 1 - k : 0, prev), hi = std::min<uint64_t>(s - 1, n - k);
+    return hi >= lo ? hi - lo + 1 : 0;
+}
+
+// One spectrum of one element: the raw sweep of its directory, then the corrections (record junctions of a collection,
+// tail starts of a view). Kept for the selections of kmer_b200_frequent_kmers and kmer_b200_occurrence_cutoff.
+struct Spectrum {
+    kmer_b200_index *ix = nullptr;
+    kb::SpectrumArgs a{};
+    std::vector<uint64_t> hist;
+    uint64_t total = 0, distinct = 0, max_count = 0, key_space = 0;
+    ~Spectrum() {
+        if (!ix) return;
+        dev_free(ix, a.hist);
+        dev_free(ix, a.stats);
+        dev_free(ix, a.tab_keys);
+        dev_free(ix, a.tab_delta);
+    }
+};
+
+// the hashes with corrected count >= thr, in hash order: *n_sel of them, the largest count *max_sel. d_hashes == null:
+// count pass only; else *d_hashes / *d_counts are allocated here and freed by the caller.
+static int spectrum_select(Spectrum &sp, uint64_t thr, uint64_t *n_sel, uint64_t *max_sel, uint64_t **d_hashes = nullptr,
+                           uint32_t **d_counts = nullptr) {
+    kmer_b200_index *ix = sp.ix;
+    cudaStream_t st = ix->stream;
+    const uint64_t tiles = kb::spectrum_tiles(sp.a.n_items);
+    kb::SpectrumSelect sel{thr, nullptr, nullptr, nullptr};
+    uint64_t *block_sums = nullptr;
+    auto done = [&](int r) {
+        dev_free(ix, sel.tile);
+        dev_free(ix, block_sums);
+        return r;
+    };
+    if (dev_alloc(ix, &sel.tile, tiles + 1, false) || dev_alloc(ix, &block_sums, kb::offsets_scan_blocks(tiles) + 1, false))
+        return done(KMER_B200_ERR_OUT_OF_MEMORY);
+    cudaMemsetAsync(sp.a.stats + 3, 0, sizeof(uint64_t), st);
+    kb::launch_spectrum_select(sp.a, sel, false, st);
+    kb::launch_offsets_scan(sel.tile, tiles, block_sums, st);
+    cudaMemcpyAsync(&ix->h_pinned[6], sel.tile + tiles, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+    cudaMemcpyAsync(&ix->h_pinned[7], sp.a.stats + 3, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+    cudaError_t e = cudaStreamSynchronize(st);
+    if (e == cudaSuccess) e = cudaGetLastError();
+    if (e != cudaSuccess) return done(fail(KMER_B200_ERR_CUDA, std::string("k-mer spectrum: ") + cudaGetErrorString(e)));
+    *n_sel = ix->h_pinned[6];
+    *max_sel = ix->h_pinned[7];
+    if (d_hashes) {
+        if (dev_alloc(ix, d_hashes, *n_sel, false) || dev_alloc(ix, d_counts, *n_sel, false)) return done(KMER_B200_ERR_OUT_OF_MEMORY);
+        sel.hashes = *d_hashes;
+        sel.counts = *d_counts;
+        kb::launch_spectrum_select(sp.a, sel, true, st);
+    }
+    return done(KMER_B200_OK);
+}
+
+static int spectrum_compute(kmer_b200_index *ix, uint32_t elem, uint64_t n_bins, Spectrum &sp) {
+    using namespace kb;
+    cudaStream_t st = ix->stream;
+    const Element &E = ix->elems[elem].dev;
+    sp.ix = ix;
+    sp.a.E = E;
+    sp.key_space = 1;
+    for (uint32_t i = 0; i < E.k; ++i)
+        if (__builtin_mul_overflow(sp.key_space, (uint64_t)ix->sigma, &sp.key_space)) {
+            sp.key_space = UINT64_MAX;
+            break;
+        }
+    sp.a.source = E.width != 1 ? kSpectrumSlabs : (E.shift == 0 ? kSpectrumDense : kSpectrumRuns);
+    sp.a.n_items = sp.a.source == kSpectrumRuns ? E.n_kmers : sp.key_space;
+    sp.a.n_bins = (uint32_t)n_bins;
+    KB_TRY(dev_alloc(ix, &sp.a.hist, n_bins, false));
+    KB_TRY(dev_alloc(ix, &sp.a.stats, 4, false));
+    KB_CUDA(cudaMemsetAsync(sp.a.hist, 0, n_bins * sizeof(uint64_t), st));
+    KB_CUDA(cudaMemsetAsync(sp.a.stats, 0, 4 * sizeof(uint64_t), st));
+    launch_spectrum_sweep(sp.a, st);
+    // corrections: every window across a record start (a collection; charged to the first start above it) and the
+    // k_phys - k tail starts of a view (a collection is never a shared-positions index)
+    const uint64_t R = ix->starts.empty() ? 0 : ix->starts.size() - 1;
+    const uint32_t n_tail = E.k_phys - E.k;
+    uint64_t n_corr = n_tail;
+    for (uint64_t r = 1; r < R; ++r) n_corr += junction_windows(ix->starts, r, ix->n, E.k);
+    if (n_corr) {
+        uint64_t cap = 64;
+        while (cap < 2 * n_corr) cap <<= 1;
+        if (cap > (1ull << 32)) return fail(KMER_B200_ERR_UNSUPPORTED, "k-mer spectrum: more than 2^31 windows cross a record start");
+        KB_TRY(dev_alloc(ix, &sp.a.tab_keys, cap, false));
+        KB_TRY(dev_alloc(ix, &sp.a.tab_delta, cap, false));
+        KB_CUDA(cudaMemsetAsync(sp.a.tab_keys, 0xFF, cap * sizeof(uint64_t), st));
+        KB_CUDA(cudaMemsetAsync(sp.a.tab_delta, 0, cap * sizeof(int), st));
+        sp.a.tab_mask = (uint32_t)(cap - 1);
+        sp.a.tail = n_tail ? 1 : 0;
+        launch_spectrum_corrections(sp.a, ix->host_index.text, ix->d_starts, R, n_tail, st);
+    }
+    sp.hist.assign(n_bins, 0);
+    uint64_t stats[4] = {};
+    KB_CUDA(cudaMemcpyAsync(sp.hist.data(), sp.a.hist, n_bins * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    KB_CUDA(cudaMemcpyAsync(stats, sp.a.stats, sizeof(stats), cudaMemcpyDeviceToHost, st));
+    KB_CUDA(cudaStreamSynchronize(st));
+    KB_CUDA(cudaGetLastError());
+    sp.distinct = stats[0];
+    sp.total = E.n_kmers + stats[2];  // the raw sweep counts the owner's n - k_phys + 1 windows; stats[2] = signed deltas
+    sp.hist[0] = sp.key_space == UINT64_MAX ? UINT64_MAX : sp.key_space - sp.distinct;
+    sp.max_count = stats[1];
+    if (n_corr) {  // a corrected bucket may have held the maximum: read it off the histogram, or select the overflow bin
+        sp.max_count = 0;
+        for (uint64_t c = n_bins - 2; c >= 1 && !sp.max_count; --c)
+            if (sp.hist[c]) sp.max_count = c;
+        if (sp.hist[n_bins - 1]) {
+            uint64_t n_sel = 0;
+            KB_TRY(spectrum_select(sp, n_bins - 1, &n_sel, &sp.max_count));
+        }
+    }
+    return KMER_B200_OK;
+}
+
+// stable LSD sort of (u32 key, u32 value) pairs by the low key_bits bits of the key (the build's tiled pair passes);
+// *vals ends up pointing at the sorted values (the other buffers are freed)
+static int sort_pairs_u32(kmer_b200_index *ix, uint32_t *keys, uint32_t **vals, uint64_t n, uint32_t key_bits) {
+    using namespace kb;
+    cudaStream_t st = ix->stream;
+    const uint32_t passes = (key_bits + kRadixBitsMax - 1) / kRadixBitsMax;
+    const uint32_t bits_per_pass = (key_bits + passes - 1) / passes;
+    const uint32_t mask = (1u << bits_per_pass) - 1;
+    const uint32_t n_tiles = (uint32_t)((n + sort_tile_size() - 1) / sort_tile_size());
+    const uint32_t n_chunks = (n_tiles + scan_chunk_tiles() - 1) / scan_chunk_tiles();
+    uint32_t *k2 = nullptr, *v2 = nullptr, *tile_hist = nullptr, *chunk_sums = nullptr;
+    int r = KMER_B200_OK;
+    if (dev_alloc(ix, &k2, n, false) || dev_alloc(ix, &v2, n, false) || dev_alloc(ix, &tile_hist, (uint64_t)n_tiles * kRadix, false) ||
+        dev_alloc(ix, &chunk_sums, (uint64_t)std::max(n_chunks, 1u) * kRadix, false)) {
+        r = KMER_B200_ERR_OUT_OF_MEMORY;
+    } else {
+        uint32_t *kb_[2] = {keys, k2}, *vb[2] = {*vals, v2};
+        int cur = 0;
+        for (uint32_t p = 0; p < passes; ++p) {
+            launch_hist_pairs(kb_[cur], 4, n, p * bits_per_pass, mask, tile_hist, st);
+            launch_column_scan(tile_hist, n_tiles, chunk_sums, st);
+            launch_scatter_pairs(kb_[cur], vb[cur], 4, n, p * bits_per_pass, mask, tile_hist, kb_[cur ^ 1], vb[cur ^ 1], st);
+            cur ^= 1;
+        }
+        *vals = vb[cur];
+        v2 = vb[cur ^ 1];
+    }
+    dev_free(ix, k2);
+    dev_free(ix, v2);
+    dev_free(ix, tile_hist);
+    dev_free(ix, chunk_sums);
+    return r;
+}
+
+// the selection of hashes with count >= thr, sorted by count descending then hash ascending; entries [first, first + n)
+// to the host arrays (hashes may be null)
+static int spectrum_sorted(Spectrum &sp, uint64_t thr, uint64_t first, uint64_t n, uint64_t *hashes, uint64_t *counts, uint64_t *n_sel) {
+    kmer_b200_index *ix = sp.ix;
+    cudaStream_t st = ix->stream;
+    uint64_t max_sel = 0, *d_h = nullptr, *d_out = nullptr;
+    uint32_t *d_c = nullptr, *d_keys = nullptr, *d_order = nullptr;
+    auto done = [&](int r) {
+        dev_free(ix, d_h);
+        dev_free(ix, d_c);
+        dev_free(ix, d_keys);
+        dev_free(ix, d_order);
+        dev_free(ix, d_out);
+        return r;
+    };
+    int r = spectrum_select(sp, thr, n_sel, &max_sel, &d_h, &d_c);
+    if (r) return done(r);
+    if (*n_sel >= (1ull << 32)) return done(fail(KMER_B200_ERR_UNSUPPORTED, "k-mer spectrum: 2^32 or more k-mers selected"));
+    n = std::min(n, *n_sel > first ? *n_sel - first : 0);
+    if (n == 0) return done(KMER_B200_OK);
+    if (max_sel > thr) {  // hash order already; one stable sort by count
+        if (dev_alloc(ix, &d_keys, *n_sel, false) || dev_alloc(ix, &d_order, *n_sel, false)) return done(KMER_B200_ERR_OUT_OF_MEMORY);
+        kb::launch_spectrum_sort_keys(d_c, *n_sel, (uint32_t)max_sel, d_keys, d_order, st);
+        if ((r = sort_pairs_u32(ix, d_keys, &d_order, *n_sel, bit_length(max_sel - thr)))) return done(r);
+    }
+    if (dev_alloc(ix, &d_out, 2 * n, false)) return done(KMER_B200_ERR_OUT_OF_MEMORY);
+    if (d_order)
+        kb::launch_spectrum_gather(d_h, d_c, d_order + first, n, d_out, d_out + n, st);
+    else
+        kb::launch_spectrum_gather(d_h + first, d_c + first, nullptr, n, d_out, d_out + n, st);
+    if (hashes) cudaMemcpyAsync(hashes, d_out, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+    cudaMemcpyAsync(counts, d_out + n, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+    cudaError_t e = cudaStreamSynchronize(st);
+    if (e == cudaSuccess) e = cudaGetLastError();
+    if (e != cudaSuccess) return done(fail(KMER_B200_ERR_CUDA, std::string("k-mer spectrum: ") + cudaGetErrorString(e)));
+    return done(KMER_B200_OK);
+}
+
+int kmer_b200_spectrum(kmer_b200_index *ix, uint32_t k, uint64_t *hist, uint64_t n_bins, kmer_b200_spectrum_info *info) {
+    if (!ix) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    if (n_bins < 2 || n_bins > kSpectrumMaxBins) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "k-mer spectrum: n_bins must be in [2, 2^24]");
+    uint32_t elem = 0;
+    KB_TRY(spectrum_check(ix, k, &elem));
+    DeviceGuard guard(ix->device);
+    std::lock_guard<std::mutex> lock(ix->mu);
+    Spectrum sp;
+    KB_TRY(spectrum_compute(ix, elem, n_bins, sp));
+    if (hist) std::memcpy(hist, sp.hist.data(), n_bins * sizeof(uint64_t));
+    if (info) *info = kmer_b200_spectrum_info{sp.total, sp.distinct, sp.max_count, sp.key_space};
+    return KMER_B200_OK;
+}
+
+int kmer_b200_frequent_kmers(kmer_b200_index *ix, uint32_t k, uint64_t min_count, uint64_t *hashes, uint64_t *counts, uint64_t cap,
+                             uint64_t *n_out) {
+    if (!ix || !n_out || (cap && (!hashes || !counts))) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    if (min_count == 0) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "frequent k-mers: min_count must be >= 1");
+    uint32_t elem = 0;
+    KB_TRY(spectrum_check(ix, k, &elem));
+    DeviceGuard guard(ix->device);
+    std::lock_guard<std::mutex> lock(ix->mu);
+    Spectrum sp;
+    const uint64_t last = kSpectrumSelectBins - 1;
+    KB_TRY(spectrum_compute(ix, elem, kSpectrumSelectBins, sp));
+    // threshold c*: the largest count whose tail #{count >= c*} holds the min(N, cap) entries wanted (the histogram is
+    // exact below its last bin); above it N itself comes from the selection
+    uint64_t thr = min_count, N = 0;
+    if (min_count <= last) {
+        for (uint64_t c = min_count; c <= last; ++c) N += sp.hist[c];
+        const uint64_t want = std::min(N, cap);
+        *n_out = N;
+        if (want == 0) return KMER_B200_OK;
+        uint64_t cum = 0;
+        for (uint64_t c = last; c >= min_count; --c)
+            if ((cum += sp.hist[c]) >= want) {
+                thr = c;
+                break;
+            }
+    }
+    uint64_t n_sel = 0;
+    KB_TRY(spectrum_sorted(sp, thr, 0, cap, hashes, counts, &n_sel));
+    *n_out = min_count <= last ? N : n_sel;
+    return KMER_B200_OK;
+}
+
+int kmer_b200_occurrence_cutoff(kmer_b200_index *ix, uint32_t k, double fraction, uint64_t *cutoff) {
+    if (!ix || !cutoff) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
+    if (!(fraction >= 0.0 && fraction < 1.0)) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "occurrence cutoff: fraction must be in [0, 1)");
+    uint32_t elem = 0;
+    KB_TRY(spectrum_check(ix, k, &elem));
+    DeviceGuard guard(ix->device);
+    std::lock_guard<std::mutex> lock(ix->mu);
+    Spectrum sp;
+    const uint64_t last = kSpectrumSelectBins - 1;
+    KB_TRY(spectrum_compute(ix, elem, kSpectrumSelectBins, sp));
+    *cutoff = 0;
+    if (sp.distinct == 0) return KMER_B200_OK;
+    // #{count > c} <= F holds exactly from the (F + 1)-th largest count on: the cutoff is that count
+    const uint64_t F = (uint64_t)std::floor(fraction * (double)sp.distinct);
+    uint64_t cum = 0;
+    for (uint64_t c = last; c >= 1; --c) {
+        if ((cum += sp.hist[c]) < F + 1) continue;
+        if (c < last) {
+            *cutoff = c;
+            return KMER_B200_OK;
+        }
+        uint64_t n_sel = 0;
+        return spectrum_sorted(sp, last, F, 1, nullptr, cutoff, &n_sel);
+    }
+    return fail(KMER_B200_ERR_CUDA, "occurrence cutoff: the histogram does not add up to the distinct k-mers");
 }
 
 void kmer_b200_records_free(kmer_b200_records *r) {

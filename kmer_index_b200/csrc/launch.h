@@ -231,6 +231,45 @@ uint64_t sizes_tiles(uint64_t n);
 void launch_sizes_tile_sums(const uint8_t *d_sizes, uint64_t n, uint64_t *d_tile_sums, cudaStream_t stream);
 void launch_sizes_to_dir(const uint8_t *d_sizes, uint64_t n, const uint64_t *d_tile_off, uint32_t *d_dir, cudaStream_t stream);
 
+// ---- k-mer spectrum (spectrum.cu): the occurrence histogram of one element from its directory
+enum SpectrumSource : uint32_t {
+    kSpectrumDense = 0,  // shift 0: count(h) = dir[h + 1] - dir[h], n_items = sigma^k
+    kSpectrumRuns = 1,   // shift > 0: runs of equal sorted hashes, n_items = n_kmers
+    kSpectrumSlabs = 2   // a view (width != 1): the owner's slab of h, n_items = sigma^k of the view's k
+};
+struct SpectrumArgs {
+    Element E;
+    uint32_t source;                 // SpectrumSource
+    uint64_t n_items;
+    uint32_t n_bins;                 // B >= 2: bin min(count, B - 1)
+    unsigned long long *hist;        // device, zeroed u64[B]
+    unsigned long long *stats;       // device, zeroed u64[4]: distinct, max raw count, sum of the deltas, max selected count
+    // corrections, or null: open-addressing table of (hash, delta), tab_mask + 1 slots (keys ~0 = empty, deltas zeroed)
+    unsigned long long *tab_keys;
+    int *tab_delta;
+    uint32_t tab_mask;
+    uint32_t tail;                   // the table holds positive deltas (tail starts of a view)
+};
+struct SpectrumSelect {
+    uint64_t thr;                    // select the hashes with corrected count >= thr (>= 1)
+    uint64_t *tile;                  // device, [spectrum_tiles + 1]: counts, then (launch_offsets_scan) offsets
+    uint64_t *hashes;                // device (write pass)
+    uint32_t *counts;                // device (write pass)
+};
+uint64_t spectrum_tiles(uint64_t n_items);
+// hist, stats[0], stats[1] of the raw counts
+void launch_spectrum_sweep(const SpectrumArgs &s, cudaStream_t stream);
+// fill the table (windows across the record starts d_starts[0..R], delta -1; the n_tail tail starts, delta +1), then move
+// every affected hash to its corrected bin (stats[0], stats[2] follow)
+void launch_spectrum_corrections(const SpectrumArgs &s, const PackedText &text, const uint64_t *d_starts, uint64_t n_records,
+                                 uint32_t n_tail, cudaStream_t stream);
+void launch_spectrum_select(const SpectrumArgs &s, const SpectrumSelect &sel, bool write, cudaStream_t stream);
+void launch_spectrum_sort_keys(const uint32_t *d_counts, uint64_t n, uint32_t max_count, uint32_t *d_keys, uint32_t *d_vals,
+                               cudaStream_t stream);
+// out[i] = selection entry order[i] (order null: i), counts widened to u64
+void launch_spectrum_gather(const uint64_t *d_hashes, const uint32_t *d_counts, const uint32_t *d_order, uint64_t n, uint64_t *d_out_hashes,
+                            uint64_t *d_out_counts, cudaStream_t stream);
+
 // ---- random-gather calibration (the denominator of the search roofline)
 void launch_gather_probe(const uint64_t *d_table, uint64_t n_words, uint64_t n_gathers, uint64_t *d_sink, cudaStream_t stream);
 
