@@ -302,6 +302,29 @@ int kmer_b200_count_seeds_batch_device(kmer_b200_index *index, const uint8_t *d_
                                        uint64_t n_queries, uint64_t max_query_len, uint32_t k, uint32_t max_occ,
                                        kmer_b200_result **out);
 
+/* ---- record votes: which records of a collection index each read comes from (the question behind k-mer classifiers,
+   strain or transcript assignment and contamination screening). For read q of length m and each j in [0, m - k], occ(j)
+   is the number of in-record occurrences of q[j, j+k) (exactly seeding's uncapped k-mer count). k-mer j is counted when
+   occ(j) >= 1 and, with max_occ > 0, occ(j) <= max_occ. recs(j) is the set of records its occurrences lie in (the record
+   of position p is the last r with starts[r] <= p, the rule of kmer_b200_locate, so empty records get no votes), and
+   votes(q, r) = #{counted j : r in recs(j)}: a k-mer occurring five times in one record gives it one vote, the same
+   k-mer at two offsets of the read gives two. Per read, every (record, votes) with votes >= min_votes, ordered by votes
+   descending, then record ascending: kmer_b200_result_positions holds the RECORD IDS of this result, and
+   kmer_b200_result_votes their votes ([n_positions]); kmer_b200_result_kmer_hits gives each read's number of counted
+   k-mers ([n_queries]). Exact for any number of records a read hits (reads beyond a shared-memory table take a
+   global-memory path); running out of device memory is KMER_B200_ERR_OUT_OF_MEMORY, never a truncated list.
+   Every status is KMER_B200_QUERY_OK; a read shorter than k has no entries and 0 k-mer hits; a rank >= sigma anywhere
+   fails the call with KMER_B200_ERR_INVALID_RANK. KMER_B200_ERR_INVALID_ARGUMENT: an index without records, k not one
+   of the index's ks (auxiliary elements do not count), min_votes = 0, null pointers. KMER_B200_ERR_UNSUPPORTED on the
+   handles seeding refuses (multi-device handles, position-range shards, key-range parts not yet adopted). The host form
+   stages the batch in one copy; the device form takes max_query_len >= the longest read (reads are walked in tiles, so
+   their length is not otherwise bounded). Reverse complements are not considered: pass one as a read of its own. */
+int kmer_b200_record_votes(kmer_b200_index *index, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t n_queries,
+                           uint32_t k, uint32_t max_occ, uint32_t min_votes, kmer_b200_result **out);
+int kmer_b200_record_votes_device(kmer_b200_index *index, const uint8_t *d_q_ranks, const uint64_t *d_q_offsets,
+                                  uint64_t n_queries, uint64_t max_query_len, uint32_t k, uint32_t max_occ, uint32_t min_votes,
+                                  kmer_b200_result **out);
+
 /* ---- k-mer spectrum: what the index holds as a whole, read off the bucket sizes of the element of k (one of the index's
    ks, views of a shared-positions index included; auxiliary elements do not count, any other k is
    KMER_B200_ERR_INVALID_ARGUMENT). The counted windows are p in [0, n - k]; on a collection index only those inside one
@@ -343,6 +366,8 @@ const uint8_t *kmer_b200_result_best_distances(const kmer_b200_result *r); /* [Q
 const uint32_t *kmer_b200_result_seed_offsets(const kmer_b200_result *r);  /* [n_positions] or NULL (seeding, not count-only) */
 const uint32_t *kmer_b200_result_kmer_counts(const kmer_b200_result *r);   /* [n_kmers] or NULL (seeding) */
 uint64_t kmer_b200_result_n_kmers(const kmer_b200_result *r);              /* k-mers of a seeding batch, else 0 */
+const uint32_t *kmer_b200_result_votes(const kmer_b200_result *r);         /* [n_positions] or NULL (record votes) */
+const uint32_t *kmer_b200_result_kmer_hits(const kmer_b200_result *r);     /* [n_queries] or NULL (record votes) */
 void kmer_b200_result_free(kmer_b200_result *r);
 
 /* ---- sharded (multi-GPU) search, two phases around one cross-rank exchange.

@@ -285,6 +285,41 @@ namespace kmer
         std::shared_ptr<kmer_b200_result> _owner;
     };
 
+    // result of record_votes<k>(): per read, every (record, votes) with votes >= min_votes, by votes descending then record
+    // ascending (CSR over the batch), and each read's counted k-mers. Views of the library's result buffers, which this
+    // object keeps alive; copies of the object share them.
+    struct record_votes_result
+    {
+        detail::array_view<std::uint64_t> offsets;    // [n_reads + 1]
+        detail::array_view<std::uint32_t> records;    // record ids
+        detail::array_view<std::uint32_t> votes;      // their votes
+        detail::array_view<std::uint32_t> kmer_hits;  // [n_reads]
+        detail::array_view<std::uint8_t> status;      // [n_reads], all KMER_B200_QUERY_OK
+
+        std::size_t size() const noexcept { return status.size(); }
+        // the (record, votes) pairs of read i
+        std::vector<std::pair<std::uint32_t, std::uint32_t>> operator[](std::size_t i) const
+        {
+            std::vector<std::pair<std::uint32_t, std::uint32_t>> out;
+            for (std::uint64_t e = offsets[i]; e < offsets[i + 1]; ++e) out.emplace_back(records[e], votes[e]);
+            return out;
+        }
+
+        record_votes_result() = default;
+        explicit record_votes_result(kmer_b200_result* r) : _owner(r, kmer_b200_result_free)
+        {
+            const std::uint64_t n_q = kmer_b200_result_n_queries(r), n_p = kmer_b200_result_n_positions(r);
+            offsets = {kmer_b200_result_offsets(r), std::size_t(n_q + 1)};
+            records = {kmer_b200_result_positions(r), std::size_t(n_p)};
+            votes = {kmer_b200_result_votes(r), std::size_t(n_p)};
+            kmer_hits = {kmer_b200_result_kmer_hits(r), std::size_t(n_q)};
+            status = {kmer_b200_result_status(r), std::size_t(n_q)};
+        }
+
+    private:
+        std::shared_ptr<kmer_b200_result> _owner;
+    };
+
     // which hits of an approximate search (search_approx_batch): the seqan3 search_cfg::hit_all / hit_all_best /
     // hit_single_best / hit_strata{s} choices (kmer_b200_approx_hits)
     struct approx_hits
@@ -553,6 +588,22 @@ namespace kmer
             kmer_b200_result* r = nullptr;
             detail::check(kmer_b200_seed_batch(_handle, ranks.data(), offsets.data(), offsets.size() - 1, std::uint32_t(k), max_occ, &r));
             return kmer_batch_result<position_t>(r);
+        }
+
+        // record votes on a collection index (kmer_b200_record_votes; attach_records first): per read, every record r that
+        // at least min_votes of its counted k-mers occur in (1 <= in-record occurrences, <= max_occ when max_occ > 0; a
+        // k-mer gives each record it occurs in one vote), by votes descending then record ascending
+        template<std::size_t k, std::ranges::range queries_t>
+        record_votes_result record_votes(queries_t const& queries, std::uint32_t max_occ = 0, std::uint32_t min_votes = 1) const
+        {
+            static_assert(((k == ks) || ...), "record_votes<k>: k is not one of this index's ks");
+            std::vector<std::uint8_t> ranks;
+            std::vector<std::uint64_t> offsets{0};
+            gather_ranks(queries, ranks, offsets);
+            kmer_b200_result* r = nullptr;
+            detail::check(kmer_b200_record_votes(_handle, ranks.data(), offsets.data(), offsets.size() - 1, std::uint32_t(k), max_occ,
+                                                 min_votes, &r));
+            return record_votes_result(r);
         }
 
         // k-mer spectrum of element k (kmer_b200_spectrum): hist[c] = distinct k-mers occurring c times for

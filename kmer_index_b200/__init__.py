@@ -119,11 +119,14 @@ class BatchResult:
     strategy also fills `distances` (uint8 per position: its Hamming distance, with distances=True) and `best_distance`
     (uint8 per query: d_min, 0xFF without a hit; every strategy but "all"); both are None otherwise. Seeding (KmerIndex.seeds) fills
     `seed_offsets` (uint32 per position: the query offset j of its k-mer) and `kmer_counts` (uint32 per k-mer of the batch);
-    both are None for other searches."""
+    both are None for other searches. Record votes (KmerIndex.record_votes) hold record ids where the others hold
+    positions (`records` names them), `votes` (uint32 per entry) and `kmer_hits` (uint32 per read: its counted k-mers);
+    `records`, `votes` and `kmer_hits` are None for other results."""
 
     def __init__(self, offsets: np.ndarray, positions: np.ndarray, status: np.ndarray, _owner=None,
                  distances: np.ndarray | None = None, best_distance: np.ndarray | None = None,
-                 seed_offsets: np.ndarray | None = None, kmer_counts: np.ndarray | None = None):
+                 seed_offsets: np.ndarray | None = None, kmer_counts: np.ndarray | None = None,
+                 votes: np.ndarray | None = None, kmer_hits: np.ndarray | None = None):
         self.offsets = offsets
         self.positions = positions
         self.status = status
@@ -131,6 +134,8 @@ class BatchResult:
         self.best_distance = best_distance
         self.seed_offsets = seed_offsets
         self.kmer_counts = kmer_counts
+        self.votes = votes
+        self.kmer_hits = kmer_hits
         self._owner = _owner   # (lib, C result handle) when the arrays are views of the pinned C result
 
     def free(self):
@@ -139,7 +144,7 @@ class BatchResult:
             L, r = self._owner
             self._owner = None
             self.offsets = self.positions = self.status = self.distances = self.best_distance = None
-            self.seed_offsets = self.kmer_counts = None
+            self.seed_offsets = self.kmer_counts = self.votes = self.kmer_hits = None
             L.kmer_b200_result_free(r)
 
     def __del__(self):
@@ -159,6 +164,28 @@ class BatchResult:
 
     def as_tuple(self):
         return self.offsets, self.positions, self.status
+
+    @property
+    def records(self) -> np.ndarray | None:
+        """Record votes: the record id of each entry (the positions array), else None."""
+        return self.positions if self.votes is not None else None
+
+    def best(self):
+        """Record votes: per read, (record or -1, its votes, the runner-up's votes) as int64 arrays. The runner-up's votes
+        are 0 when there is none; a tie shows as equal votes (the record is then the lower id)."""
+        if self.votes is None:
+            raise ValueError("best() needs a record-vote result")
+        Q = self.status.size
+        lens = np.diff(self.offsets.astype(np.int64))
+        first = self.offsets[:-1].astype(np.int64)
+        has1, has2 = lens >= 1, lens >= 2
+        rec = np.full(Q, -1, np.int64)
+        v1 = np.zeros(Q, np.int64)
+        v2 = np.zeros(Q, np.int64)
+        rec[has1] = self.positions[first[has1]]
+        v1[has1] = self.votes[first[has1]]
+        v2[has2] = self.votes[first[has2] + 1]
+        return rec, v1, v2
 
 
 class Records:
@@ -284,6 +311,16 @@ class DeviceResult:
         """int32 view of the occurrence count of each k-mer of the batch (seeding), or None."""
         ptr = self._L.kmer_b200_result_kmer_counts(self._r) or 0
         return _DevArray(ptr, int(self._L.kmer_b200_result_n_kmers(self._r)), "<i4", self) if ptr else None
+
+    def votes(self):
+        """int32 view of the votes of each entry (record votes; positions() then holds record ids), or None."""
+        ptr = self._L.kmer_b200_result_votes(self._r) or 0
+        return _DevArray(ptr, self.n_positions, "<i4", self) if ptr else None
+
+    def kmer_hits(self):
+        """int32 view of the counted k-mers of each read (record votes), or None."""
+        ptr = self._L.kmer_b200_result_kmer_hits(self._r) or 0
+        return _DevArray(ptr, self.n_queries, "<i4", self) if ptr else None
 
     def hit_queries(self):
         """int32 view of [n, id_1 .. id_n, ...]: the queries the count pass found hits for (unordered), or None."""
@@ -543,6 +580,26 @@ class KmerIndex:
         return self._device_call(self._L.kmer_b200_count_seeds_batch_device, q_ptr, off_ptr, Q, max_len, self._seed_k(k),
                                  int(max_occ))
 
+    def record_votes(self, q_ranks, q_offsets, k: int | None = None, max_occ: int = 0, min_votes: int = 1,
+                     copy: bool = True) -> BatchResult:
+        """Which records of a collection index each read comes from (kmer_b200_record_votes): per read, every record r
+        with votes(q, r) >= min_votes, by votes descending then record ascending, where votes(q, r) is the number of the
+        read's counted k-mers (1 <= in-record occurrences, <= max_occ when max_occ > 0) that occur in r. BatchResult.records
+        holds the record ids, .votes their votes, .kmer_hits each read's counted k-mers; best() gives the top record."""
+        q = np.ascontiguousarray(np.asarray(q_ranks, dtype=np.uint8))
+        off = np.ascontiguousarray(np.asarray(q_offsets, dtype=np.uint64))
+        r = C.c_void_p()
+        _capi.check(self._L.kmer_b200_record_votes(self._h, q.ctypes.data, off.ctypes.data, off.size - 1, self._seed_k(k),
+                                                   int(max_occ), int(min_votes), C.byref(r)))
+        return self._host_result(r, off.size - 1, copy)
+
+    def record_votes_batch_device(self, q_ptr: int, off_ptr: int, Q: int, max_len: int, k: int | None = None, max_occ: int = 0,
+                                  min_votes: int = 1):
+        """Record votes (see record_votes) of a device-resident batch; the result stays on the device: positions() holds
+        the record ids, votes() and kmer_hits() the rest."""
+        return self._device_call(self._L.kmer_b200_record_votes_device, q_ptr, off_ptr, Q, max_len, self._seed_k(k), int(max_occ),
+                                 int(min_votes))
+
     def _host_result(self, r, Q: int, copy: bool) -> BatchResult:
         L = self._L
         total = L.kmer_b200_result_n_positions(r)
@@ -557,12 +614,16 @@ class KmerIndex:
         s_ptr, c_ptr, n_kmers = L.kmer_b200_result_seed_offsets(r), L.kmer_b200_result_kmer_counts(r), L.kmer_b200_result_n_kmers(r)
         seed = (np.ctypeslib.as_array(C.cast(s_ptr, _capi.u32p), shape=(total,)) if total else np.zeros(0, np.uint32)) if s_ptr else None
         kc = (np.ctypeslib.as_array(C.cast(c_ptr, _capi.u32p), shape=(n_kmers,)) if n_kmers else np.zeros(0, np.uint32)) if c_ptr else None
+        v_ptr, h_ptr = L.kmer_b200_result_votes(r), L.kmer_b200_result_kmer_hits(r)
+        votes = (np.ctypeslib.as_array(C.cast(v_ptr, _capi.u32p), shape=(total,)) if total else np.zeros(0, np.uint32)) if v_ptr else None
+        hits = (np.ctypeslib.as_array(C.cast(h_ptr, _capi.u32p), shape=(Q,)) if Q else np.zeros(0, np.uint32)) if h_ptr else None
         if not copy:
             return BatchResult(offsets, positions, status, _owner=(L, r), distances=dist, best_distance=best, seed_offsets=seed,
-                               kmer_counts=kc)
+                               kmer_counts=kc, votes=votes, kmer_hits=hits)
         out = BatchResult(offsets.copy(), positions.copy(), status.copy(), distances=None if dist is None else dist.copy(),
                           best_distance=None if best is None else best.copy(), seed_offsets=None if seed is None else seed.copy(),
-                          kmer_counts=None if kc is None else kc.copy())
+                          kmer_counts=None if kc is None else kc.copy(), votes=None if votes is None else votes.copy(),
+                          kmer_hits=None if hits is None else hits.copy())
         L.kmer_b200_result_free(r)
         return out
 

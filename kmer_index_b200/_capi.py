@@ -126,6 +126,10 @@ SYMBOLS = {
                                               C.c_uint32, C.POINTER(C.c_void_p)]),
     "kmer_b200_count_seeds_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32,
                                                      C.c_uint32, C.POINTER(C.c_void_p)]),
+    "kmer_b200_record_votes": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32,
+                                         C.POINTER(C.c_void_p)]),
+    "kmer_b200_record_votes_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32,
+                                                C.c_uint32, C.c_uint32, C.POINTER(C.c_void_p)]),
     "kmer_b200_spectrum": (C.c_int, [C.c_void_p, C.c_uint32, u64p, C.c_uint64, C.POINTER(SpectrumInfo)]),
     "kmer_b200_frequent_kmers": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint64, u64p, u64p, C.c_uint64, u64p]),
     "kmer_b200_occurrence_cutoff": (C.c_int, [C.c_void_p, C.c_uint32, C.c_double, u64p]),
@@ -141,6 +145,8 @@ SYMBOLS = {
     "kmer_b200_result_seed_offsets": (C.c_void_p, [C.c_void_p]),
     "kmer_b200_result_kmer_counts": (C.c_void_p, [C.c_void_p]),
     "kmer_b200_result_n_kmers": (C.c_uint64, [C.c_void_p]),
+    "kmer_b200_result_votes": (C.c_void_p, [C.c_void_p]),
+    "kmer_b200_result_kmer_hits": (C.c_void_p, [C.c_void_p]),
     "kmer_b200_result_free": (None, [C.c_void_p]),
     "kmer_b200_presence_batch_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64,
                                                   C.c_uint32, C.c_void_p, C.c_uint32]),

@@ -84,13 +84,17 @@ enum KernelId : int {
     K_APPROX_DISTANCES,
     K_SEED_COUNT,
     K_SEED_WRITE,
+    K_VOTES_COUNT,
+    K_VOTES_WRITE,
+    K_VOTES_OVERFLOW,
     K_COUNT_
 };
 
 const char *const kKernelNames[K_COUNT_] = {
     "pack_text",       "radix_hist_text", "radix_hist_pairs", "column_scan",     "radix_scatter_text", "radix_scatter_pairs",
     "directory_fill",  "search_count",    "search_write",     "search_presence", "offsets_scan",       "segment_sort",
-    "approx_best",     "approx_single",   "approx_distances", "seed_count",      "seed_write"};
+    "approx_best",     "approx_single",   "approx_distances", "seed_count",      "seed_write",         "votes_count",
+    "votes_write",     "votes_overflow"};
 
 struct Profiler {
     bool enabled = false;
@@ -255,9 +259,12 @@ struct kmer_b200_result {
     uint8_t *best_distance = nullptr;  // approximate search, hit strategies other than "all": d_min per query, or null
     uint32_t *seed_offsets = nullptr;  // seeding: the query offset j of each position, or null
     uint32_t *kmer_counts = nullptr;   // seeding: the occurrence count of each k-mer of the batch, or null
+    uint32_t *votes = nullptr;         // record votes (positions hold the records): the votes of each entry, or null
+    uint32_t *kmer_hits = nullptr;     // record votes: the counted k-mers of each query, or null
     uint64_t n_kmers = 0;
     size_t cap_offsets = 0, cap_positions = 0, cap_status = 0;  // host buffers: byte capacities
     size_t cap_distances = 0, cap_best_distance = 0, cap_seed_offsets = 0, cap_kmer_counts = 0;
+    size_t cap_votes = 0, cap_kmer_hits = 0;
     bool positions_pageable = false;  // very large position lists live in plain malloc memory
 };
 
@@ -276,6 +283,8 @@ void for_each_result_array(const kmer_b200_result &r, F &&f) {
     f(&R::best_distance, &R::cap_best_distance, Q);
     f(&R::seed_offsets, &R::cap_seed_offsets, P);
     f(&R::kmer_counts, &R::cap_kmer_counts, r.n_kmers);
+    f(&R::votes, &R::cap_votes, P);
+    f(&R::kmer_hits, &R::cap_kmer_hits, Q);
     f(&R::hit_queries, (size_t R::*)nullptr, Q + 1);
 }
 
@@ -1891,6 +1900,183 @@ int seed_device_impl(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_
     return KMER_B200_OK;
 }
 
+// stable LSD sort of (u32 key, u32 value) pairs by the low key_bits bits of the key (the build's tiled pair passes);
+// *vals ends up pointing at the sorted values (the other buffers are freed)
+int sort_pairs_u32(kmer_b200_index *ix, uint32_t *keys, uint32_t **vals, uint64_t n, uint32_t key_bits) {
+    using namespace kb;
+    cudaStream_t st = ix->stream;
+    const uint32_t passes = (key_bits + kRadixBitsMax - 1) / kRadixBitsMax;
+    const uint32_t bits_per_pass = (key_bits + passes - 1) / passes;
+    const uint32_t mask = (1u << bits_per_pass) - 1;
+    const uint32_t n_tiles = (uint32_t)((n + sort_tile_size() - 1) / sort_tile_size());
+    const uint32_t n_chunks = (n_tiles + scan_chunk_tiles() - 1) / scan_chunk_tiles();
+    uint32_t *k2 = nullptr, *v2 = nullptr, *tile_hist = nullptr, *chunk_sums = nullptr;
+    int r = KMER_B200_OK;
+    if (dev_alloc(ix, &k2, n, false) || dev_alloc(ix, &v2, n, false) || dev_alloc(ix, &tile_hist, (uint64_t)n_tiles * kRadix, false) ||
+        dev_alloc(ix, &chunk_sums, (uint64_t)std::max(n_chunks, 1u) * kRadix, false)) {
+        r = KMER_B200_ERR_OUT_OF_MEMORY;
+    } else {
+        uint32_t *kb_[2] = {keys, k2}, *vb[2] = {*vals, v2};
+        int cur = 0;
+        for (uint32_t p = 0; p < passes; ++p) {
+            launch_hist_pairs(kb_[cur], 4, n, p * bits_per_pass, mask, tile_hist, st);
+            launch_column_scan(tile_hist, n_tiles, chunk_sums, st);
+            launch_scatter_pairs(kb_[cur], vb[cur], 4, n, p * bits_per_pass, mask, tile_hist, kb_[cur ^ 1], vb[cur ^ 1], st);
+            cur ^= 1;
+        }
+        *vals = vb[cur];
+        v2 = vb[cur ^ 1];
+    }
+    dev_free(ix, k2);
+    dev_free(ix, v2);
+    dev_free(ix, tile_hist);
+    dev_free(ix, chunk_sums);
+    return r;
+}
+
+// The checks of the record-vote entry points: those of seeding, then a record table and min_votes >= 1.
+int votes_check(const kmer_b200_index *ix, uint32_t k, uint32_t min_votes, uint32_t *elem) {
+    KB_TRY(seed_check(ix, k, elem));
+    if (ix->starts.empty()) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "record votes: the index has no records (attach_records)");
+    if (min_votes == 0) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "record votes: min_votes must be >= 1");
+    return KMER_B200_OK;
+}
+
+// Record votes of a batch already on the device (kmer_b200_record_votes_device): k-mers per query -> scan -> count pass ->
+// [overflow path: scan of the flagged reads' events -> spill, segment sort, runs] -> scan -> write pass -> [the flagged
+// reads' entries: two stable pair sorts and a scatter]. The caller holds the handle's lock and device.
+int votes_device_impl(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len, uint32_t elem,
+                      uint32_t max_occ, uint32_t min_votes, kmer_b200_result **out) {
+    using namespace kb;
+    (void)max_len;  // every read is walked in tiles: no length limit
+    if (Q >= 0xFFFFFFFFull) return fail(KMER_B200_ERR_UNSUPPORTED, "more than 2^32 - 2 queries in one batch: split the batch");
+    cudaStream_t st = ix->stream;
+    kmer_b200_result *res = device_result_new(ix, Q);
+    if (!res) return KMER_B200_ERR_OUT_OF_MEMORY;
+    uint64_t *d_kbase = nullptr, *d_block_sums = nullptr, *d_pairs = nullptr, *d_flagged = nullptr;
+    uint32_t *d_flags = nullptr, *d_counts = nullptr, *d_lo = nullptr, *d_spill = nullptr, *d_run_rec = nullptr, *d_run_votes = nullptr;
+    uint32_t *d_keys = nullptr, *d_vals = nullptr, *d_c_rec = nullptr, *d_c_votes = nullptr, *d_c_read = nullptr;
+    uint8_t *d_ovf = nullptr;
+    unsigned long long *d_n_ovf = nullptr;
+    size_t hs_cap = 0;
+    uint64_t *hs = nullptr;
+    auto release = [&] {
+        for (uint64_t *p : {d_kbase, d_block_sums, d_pairs, d_flagged}) dev_free(ix, p);
+        for (uint32_t *p : {d_flags, d_counts, d_lo, d_spill, d_run_rec, d_run_votes, d_keys, d_vals, d_c_rec, d_c_votes, d_c_read})
+            dev_free(ix, p);
+        dev_free(ix, d_ovf);
+        dev_free(ix, d_n_ovf);
+        pinned_put(hs, hs_cap);
+    };
+    auto bail = [&](int code) {
+        release();
+        kmer_b200_result_free(res);
+        return code;
+    };
+    auto sync = [&](const char *what) -> int {
+        cudaError_t e = cudaStreamSynchronize(st);
+        if (e == cudaSuccess) e = cudaGetLastError();
+        if (e == cudaSuccess) return KMER_B200_OK;
+        cudaGetLastError();
+        return fail(KMER_B200_ERR_CUDA, std::string(what) + cudaGetErrorString(e));
+    };
+    hs = (uint64_t *)pinned_get(8 * sizeof(uint64_t), &hs_cap);
+    if (!hs) return bail(fail(KMER_B200_ERR_OUT_OF_MEMORY, "pinned host allocation failed"));
+    if (dev_alloc(ix, &d_kbase, Q + 1, false) || dev_alloc(ix, &d_block_sums, offsets_scan_blocks(Q) + 1, false) ||
+        dev_alloc(ix, &d_flags, 1, false) || dev_alloc(ix, &d_n_ovf, 1, false) || dev_alloc(ix, &d_pairs, Q + 1, false) ||
+        dev_alloc(ix, &d_ovf, Q, false) || dev_alloc(ix, &res->kmer_hits, Q, false))
+        return bail(KMER_B200_ERR_OUT_OF_MEMORY);
+    launch_seed_kmers_per_query(d_off, Q, ix->ks[elem], d_kbase, st);
+    launch_offsets_scan(d_kbase, Q, d_block_sums, st);
+    cudaMemcpyAsync(&hs[0], d_kbase + Q, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+    if (int s = sync("record votes (k-mers per query): ")) return bail(s);
+    const uint64_t n_kmers = Q ? hs[0] : 0;
+    if (dev_alloc(ix, &d_counts, n_kmers, false) || dev_alloc(ix, &d_lo, n_kmers, false)) return bail(KMER_B200_ERR_OUT_OF_MEMORY);
+
+    VoteArgs a{};
+    a.index = ix->d_index;
+    a.q_ranks = d_q;
+    a.q_offsets = d_off;
+    a.n_queries = Q;
+    a.elem = elem;
+    a.k = ix->ks[elem];
+    a.max_occ = max_occ;
+    a.min_votes = min_votes;
+    a.starts = ix->d_starts;
+    a.n_records = ix->starts.size() - 1;
+    a.record_bits = std::max<uint32_t>(1, bit_length(a.n_records - 1));
+    a.kmer_base = d_kbase;
+    a.kmer_counts = d_counts;
+    a.bucket_lo = d_lo;
+    a.counts = res->offsets;
+    a.status = res->status;
+    a.kmer_hits = res->kmer_hits;
+    a.n_pairs = d_pairs;
+    a.ovf = d_ovf;
+    a.n_ovf = d_n_ovf;
+    a.spill_off = d_pairs;
+    a.error_flag = d_flags;
+    cudaMemsetAsync(d_flags, 0, sizeof(uint32_t), st);
+    cudaMemsetAsync(d_n_ovf, 0, sizeof(unsigned long long), st);
+    ix->prof.begin(K_VOTES_COUNT, 0);
+    launch_votes_count(a, st);
+    ix->prof.end();
+    cudaMemcpyAsync(&hs[1], d_n_ovf, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+    cudaMemcpyAsync(&hs[2], d_flags, sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
+    if (int s = sync("record votes (count pass): ")) return bail(s);
+    if (hs[2] & 1u) return bail(fail(KMER_B200_ERR_INVALID_RANK, "a query contains a rank >= sigma"));
+    const uint64_t n_ovf = hs[1];
+    uint64_t n_flagged = 0;  // survivors of the flagged reads
+    if (n_ovf) {
+        // overflow path: every flagged read's (k-mer, record) events in a segment of their own
+        launch_offsets_scan(d_pairs, Q, d_block_sums, st);
+        cudaMemcpyAsync(&hs[3], d_pairs + Q, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+        if (int s = sync("record votes (overflow sizes): ")) return bail(s);
+        const uint64_t n_events = hs[3];
+        if (dev_alloc(ix, &d_spill, n_events, false) || dev_alloc(ix, &d_run_rec, n_events, false) ||
+            dev_alloc(ix, &d_run_votes, n_events, false) || dev_alloc(ix, &d_flagged, Q + 1, false))
+            return bail(KMER_B200_ERR_OUT_OF_MEMORY);
+        a.spill = d_spill;
+        cudaMemsetAsync(d_flagged, 0, (Q + 1) * sizeof(uint64_t), st);
+        ix->prof.begin(K_VOTES_OVERFLOW, 0, 3);
+        launch_votes_spill(a, d_run_rec, d_run_votes, d_flagged, st);
+        ix->prof.end();
+        launch_offsets_scan(d_flagged, Q, d_block_sums, st);
+        cudaMemcpyAsync(&hs[4], d_flagged + Q, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+    }
+    ix->prof.begin(K_OFFSETS_SCAN, 3.0 * 8 * Q, 3);
+    launch_offsets_scan(res->offsets, Q, d_block_sums, st);
+    ix->prof.end();
+    cudaMemcpyAsync(&hs[0], res->offsets + Q, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+    if (int s = sync("record votes (offsets): ")) return bail(s);
+    const uint64_t total = Q ? hs[0] : 0;
+    if (n_ovf) n_flagged = hs[4];
+    if (n_flagged >= (1ull << 32)) return bail(fail(KMER_B200_ERR_UNSUPPORTED, "record votes: 2^32 or more entries of overflowed reads"));
+    res->n_positions = total;
+    if (dev_alloc(ix, &res->positions, total, false) || dev_alloc(ix, &res->votes, total, false))
+        return bail(KMER_B200_ERR_OUT_OF_MEMORY);
+    a.records = res->positions;
+    a.votes = res->votes;
+    ix->prof.begin(K_VOTES_WRITE, 0);
+    launch_votes_write(a, st);
+    ix->prof.end();
+    if (n_flagged) {
+        if (dev_alloc(ix, &d_keys, n_flagged, false) || dev_alloc(ix, &d_vals, n_flagged, false) || dev_alloc(ix, &d_c_rec, n_flagged, false) ||
+            dev_alloc(ix, &d_c_votes, n_flagged, false) || dev_alloc(ix, &d_c_read, n_flagged, false))
+            return bail(KMER_B200_ERR_OUT_OF_MEMORY);
+        launch_votes_place(a, d_run_rec, d_run_votes, d_flagged, d_keys, d_vals, d_c_rec, d_c_votes, d_c_read, st);
+        // stable: by votes descending, then by read; each read's entries stay in record order between equal votes
+        if (int r = sort_pairs_u32(ix, d_keys, &d_vals, n_flagged, 32)) return bail(r);
+        launch_votes_owner(d_vals, d_c_read, n_flagged, d_keys, st);
+        if (int r = sort_pairs_u32(ix, d_keys, &d_vals, n_flagged, std::max<uint32_t>(1, bit_length(Q - 1)))) return bail(r);
+        launch_votes_scatter(a, d_vals, d_c_rec, d_c_votes, d_c_read, d_flagged, n_flagged, st);
+    }
+    if (int s = sync("record votes (write pass): ")) return bail(s);
+    release();
+    *out = res;
+    return KMER_B200_OK;
+}
+
 // Query lengths of a host batch: the batch and its offsets staged on the device, and the longest query. The staging is
 // released with the object.
 struct StagedBatch {
@@ -1926,16 +2112,17 @@ struct StagedBatch {
     const uint8_t *ranks(const uint64_t *q_offsets) const { return d_q - q_offsets[0]; }
 };
 
-// What a batch entry point asks for. Every device entry point and every single-copy host batch is one of these four kinds.
+// What a batch entry point asks for. Every device entry point and every single-copy host batch is one of these five kinds.
 struct BatchRequest {
-    enum Kind { kExact, kExactGlobal, kApprox, kSeeds } kind = kExact;
+    enum Kind { kExact, kExactGlobal, kApprox, kSeeds, kVotes } kind = kExact;
     SearchFlavor flavor = kFlavorFull;
     uint32_t mode = UINT32_MAX;     // exact: a kmer_b200_mode, or UINT32_MAX for the index default
     const void *present = nullptr;  // exact global: the whole-text presence flags and their format
     uint32_t present_format = 0;
     const kmer_b200_approx_options *opt = nullptr;      // approximate: the caller's options
     const kmer_b200_approx_options *hit_opt = nullptr;  // approximate: the effective options (request_check)
-    uint32_t k = 0, elem = 0, max_occ = 0;              // seeding: k, its element (request_check) and the repeat cap
+    uint32_t k = 0, elem = 0, max_occ = 0;              // seeding, votes: k, its element (request_check) and the repeat cap
+    uint32_t min_votes = 0;                             // votes: the fewest votes an entry needs
     static BatchRequest exact(uint32_t mode, SearchFlavor f) {
         BatchRequest r;
         r.mode = mode, r.flavor = f;
@@ -1956,6 +2143,11 @@ struct BatchRequest {
         r.kind = kSeeds, r.k = k, r.max_occ = max_occ, r.flavor = f;
         return r;
     }
+    static BatchRequest votes(uint32_t k, uint32_t max_occ, uint32_t min_votes) {
+        BatchRequest r;
+        r.kind = kVotes, r.k = k, r.max_occ = max_occ, r.min_votes = min_votes;
+        return r;
+    }
 };
 
 // The checks of a request before the device is touched (the batch's offsets, on the host or the device, must not be
@@ -1969,6 +2161,7 @@ int request_check(const kmer_b200_index *ix, const uint64_t *offsets, BatchReque
         return KMER_B200_OK;
     case BatchRequest::kApprox: return approx_options_check(ix, req->opt, &req->hit_opt);
     case BatchRequest::kSeeds: return seed_check(ix, req->k, &req->elem);
+    case BatchRequest::kVotes: return votes_check(ix, req->k, req->min_votes, &req->elem);
     default: return KMER_B200_OK;
     }
 }
@@ -1982,6 +2175,7 @@ int request_run(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, 
         return search_device_impl(ix, d_q, d_off, Q, max_len, KMER_B200_MODE_CORRECT, nullptr, 0, req.flavor, out, nullptr,
                                   (int32_t)req.opt->max_mismatches, req.hit_opt);
     case BatchRequest::kSeeds: return seed_device_impl(ix, d_q, d_off, Q, max_len, req.elem, req.max_occ, req.flavor, out);
+    case BatchRequest::kVotes: return votes_device_impl(ix, d_q, d_off, Q, max_len, req.elem, req.max_occ, req.min_votes, out);
     default: return search_device_impl(ix, d_q, d_off, Q, max_len, req.mode, req.present, req.present_format, req.flavor, out);
     }
 }
@@ -2227,7 +2421,7 @@ void kmer_b200_destroy(kmer_b200_index *ix) {
 
 // The device entry points: the request's checks, then the device and the handle's lock, once for all of them. The exact
 // forms refuse multi-device handles first, the global-presence form collection indexes too; approximate search and
-// seeding refuse those handles in their own checks.
+// seeding (record votes too) refuse those handles in their own checks.
 static int device_entry(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len, BatchRequest req,
                         kmer_b200_result **out) {
     if (req.kind == BatchRequest::kExact || req.kind == BatchRequest::kExactGlobal) { KB_NOT_ON_GROUP(ix); }
@@ -2284,6 +2478,11 @@ int kmer_b200_seed_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const u
 int kmer_b200_count_seeds_batch_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len,
                                        uint32_t k, uint32_t max_occ, kmer_b200_result **out) {
     return device_entry(ix, d_q, d_off, Q, max_len, BatchRequest::seeds(k, max_occ, kFlavorCountOnly), out);
+}
+
+int kmer_b200_record_votes_device(kmer_b200_index *ix, const uint8_t *d_q, const uint64_t *d_off, uint64_t Q, uint64_t max_len,
+                                  uint32_t k, uint32_t max_occ, uint32_t min_votes, kmer_b200_result **out) {
+    return device_entry(ix, d_q, d_off, Q, max_len, BatchRequest::votes(k, max_occ, min_votes), out);
 }
 
 struct kmer_b200_pending {
@@ -2865,6 +3064,11 @@ int kmer_b200_seed_batch(kmer_b200_index *ix, const uint8_t *q_ranks, const uint
     return host_batch(ix, q_ranks, q_offsets, Q, nullptr, BatchRequest::seeds(k, max_occ, kFlavorFull), out);
 }
 
+int kmer_b200_record_votes(kmer_b200_index *ix, const uint8_t *q_ranks, const uint64_t *q_offsets, uint64_t Q, uint32_t k,
+                           uint32_t max_occ, uint32_t min_votes, kmer_b200_result **out) {
+    return host_batch(ix, q_ranks, q_offsets, Q, nullptr, BatchRequest::votes(k, max_occ, min_votes), out);
+}
+
 int kmer_b200_search_batch_ptrs(kmer_b200_index *ix, const uint8_t *const *q_ptrs, const uint64_t *q_lens, uint64_t Q,
                                 uint32_t mode, kmer_b200_result **out) {
     if (!ix || !out || (Q && (!q_ptrs || !q_lens))) return fail(KMER_B200_ERR_INVALID_ARGUMENT, "null argument");
@@ -2943,6 +3147,8 @@ const uint8_t *kmer_b200_result_best_distances(const kmer_b200_result *r) { retu
 const uint32_t *kmer_b200_result_seed_offsets(const kmer_b200_result *r) { return r ? r->seed_offsets : nullptr; }
 const uint32_t *kmer_b200_result_kmer_counts(const kmer_b200_result *r) { return r ? r->kmer_counts : nullptr; }
 uint64_t kmer_b200_result_n_kmers(const kmer_b200_result *r) { return r ? r->n_kmers : 0; }
+const uint32_t *kmer_b200_result_votes(const kmer_b200_result *r) { return r ? r->votes : nullptr; }
+const uint32_t *kmer_b200_result_kmer_hits(const kmer_b200_result *r) { return r ? r->kmer_hits : nullptr; }
 
 void kmer_b200_result_free(kmer_b200_result *r) {
     if (!r) return;
@@ -3605,40 +3811,6 @@ static int spectrum_compute(kmer_b200_index *ix, uint32_t elem, uint64_t n_bins,
         }
     }
     return KMER_B200_OK;
-}
-
-// stable LSD sort of (u32 key, u32 value) pairs by the low key_bits bits of the key (the build's tiled pair passes);
-// *vals ends up pointing at the sorted values (the other buffers are freed)
-static int sort_pairs_u32(kmer_b200_index *ix, uint32_t *keys, uint32_t **vals, uint64_t n, uint32_t key_bits) {
-    using namespace kb;
-    cudaStream_t st = ix->stream;
-    const uint32_t passes = (key_bits + kRadixBitsMax - 1) / kRadixBitsMax;
-    const uint32_t bits_per_pass = (key_bits + passes - 1) / passes;
-    const uint32_t mask = (1u << bits_per_pass) - 1;
-    const uint32_t n_tiles = (uint32_t)((n + sort_tile_size() - 1) / sort_tile_size());
-    const uint32_t n_chunks = (n_tiles + scan_chunk_tiles() - 1) / scan_chunk_tiles();
-    uint32_t *k2 = nullptr, *v2 = nullptr, *tile_hist = nullptr, *chunk_sums = nullptr;
-    int r = KMER_B200_OK;
-    if (dev_alloc(ix, &k2, n, false) || dev_alloc(ix, &v2, n, false) || dev_alloc(ix, &tile_hist, (uint64_t)n_tiles * kRadix, false) ||
-        dev_alloc(ix, &chunk_sums, (uint64_t)std::max(n_chunks, 1u) * kRadix, false)) {
-        r = KMER_B200_ERR_OUT_OF_MEMORY;
-    } else {
-        uint32_t *kb_[2] = {keys, k2}, *vb[2] = {*vals, v2};
-        int cur = 0;
-        for (uint32_t p = 0; p < passes; ++p) {
-            launch_hist_pairs(kb_[cur], 4, n, p * bits_per_pass, mask, tile_hist, st);
-            launch_column_scan(tile_hist, n_tiles, chunk_sums, st);
-            launch_scatter_pairs(kb_[cur], vb[cur], 4, n, p * bits_per_pass, mask, tile_hist, kb_[cur ^ 1], vb[cur ^ 1], st);
-            cur ^= 1;
-        }
-        *vals = vb[cur];
-        v2 = vb[cur ^ 1];
-    }
-    dev_free(ix, k2);
-    dev_free(ix, v2);
-    dev_free(ix, tile_hist);
-    dev_free(ix, chunk_sums);
-    return r;
 }
 
 // the selection of hashes with count >= thr, sorted by count descending then hash ascending; entries [first, first + n)

@@ -168,6 +168,53 @@ void launch_seed_count(const SeedArgs &a, cudaStream_t stream);
 // after the offsets scan of the count pass's counts: the write pass and, when a.heavy != null, the heavy launch
 void launch_seed_write(const SeedArgs &a, cudaStream_t stream);
 
+// ---- record votes (record_votes.cu): per read of a collection index, the records its k-mers occur in, by shared k-mers
+constexpr uint32_t kVoteCapacity = 384;  // distinct records a read's shared-memory table holds; more take the overflow path
+struct VoteArgs {
+    const DeviceIndex *index;        // device pointer
+    const uint8_t *q_ranks;          // device
+    const uint64_t *q_offsets;       // device, [Q + 1]
+    uint64_t n_queries;
+    uint32_t elem;                   // the element of k (not an auxiliary one)
+    uint32_t k;
+    uint32_t max_occ;                // 0 = no cap
+    uint32_t min_votes;              // >= 1
+    const uint64_t *starts;          // device, the record table starts[0..n_records]
+    uint64_t n_records;
+    uint32_t record_bits;            // bits of the largest record id (the overflow path's segment sort)
+    const uint64_t *kmer_base;       // device, [Q + 1]: index of each read's first k-mer in the batch's k-mer order
+    uint32_t *kmer_counts;           // device, [n_kmers]: in-record occurrences, saturated at max_occ + 1 under a cap
+    uint32_t *bucket_lo;             // device, [n_kmers]: each k-mer's first CSR entry
+    uint64_t *counts;                // device, [Q + 1]: entries per read (count pass, overflow path), then offsets
+    uint8_t *status;                 // device, [Q]
+    uint32_t *kmer_hits;             // device, [Q]: counted k-mers per read
+    uint64_t *n_pairs;               // device, [Q + 1]: new (k-mer, record) events of each flagged read (0 otherwise), then
+                                     // the offsets of their segments in `spill`
+    uint8_t *ovf;                    // device, [Q]: 1 = the read's records overflowed its table
+    unsigned long long *n_ovf;       // device: flagged reads
+    uint32_t *spill;                 // device (overflow path): the flagged reads' records, one segment each
+    const uint64_t *spill_off;       // = n_pairs after its offsets scan
+    uint32_t *records;               // device (write passes): record of each entry
+    uint32_t *votes;                 // device (write passes): its votes
+    uint32_t *error_flag;            // device u32: bit 0 = query rank >= sigma
+};
+// count pass: counts, kmer_hits, kmer_counts / bucket_lo, and the flagged reads with their n_pairs
+void launch_votes_count(const VoteArgs &a, cudaStream_t stream);
+// after the offsets scan of n_pairs: each flagged read's records to its segment of a.spill, sorted (run_records is the
+// sort's scratch), run-length counted and filtered by min_votes into run_records / run_votes (record order) at the front
+// of the segment; counts[q] = flagged[q] = the survivors
+void launch_votes_spill(const VoteArgs &a, uint32_t *run_records, uint32_t *run_votes, uint64_t *flagged, cudaStream_t stream);
+// after the offsets scan of counts: the unflagged reads' entries in (votes desc, record asc) order
+void launch_votes_write(const VoteArgs &a, cudaStream_t stream);
+// the flagged reads' survivors as one list (flagged_off: the offsets scan of flagged): keys = ~votes, vals = list index,
+// and each entry's record, votes and read; after a stable pair sort by keys, launch_votes_owner sets keys = the read of each
+// value, and after a second stable sort launch_votes_scatter writes every entry at its read's offsets
+void launch_votes_place(const VoteArgs &a, const uint32_t *run_records, const uint32_t *run_votes, const uint64_t *flagged_off,
+                        uint32_t *keys, uint32_t *vals, uint32_t *c_rec, uint32_t *c_votes, uint32_t *c_read, cudaStream_t stream);
+void launch_votes_owner(const uint32_t *vals, const uint32_t *c_read, uint64_t n, uint32_t *keys, cudaStream_t stream);
+void launch_votes_scatter(const VoteArgs &a, const uint32_t *vals, const uint32_t *c_rec, const uint32_t *c_votes, const uint32_t *c_read,
+                          const uint64_t *flagged_off, uint64_t n, cudaStream_t stream);
+
 // deferred count pass epilogue: zero the counts / set THROW according to the combined presence flags
 void launch_finalize_deferred(uint64_t *d_counts, uint8_t *d_status, const uint8_t *d_defer, const uint32_t *d_present4_global,
                               uint64_t n_queries, cudaStream_t stream);
